@@ -17,6 +17,7 @@ A "step" = one batch of 70 queries ranked against the whole database.
 
 Launch: python bench.py [--gpus N --steps K --warmup W]; for N > 1 under torchrun
 (python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...).
+--dump-outputs DIR writes the result of the last timed step (DIR/scores.npy, DIR/indices.npy).
 """
 import argparse
 import json
@@ -43,7 +44,22 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the head / CLAHE / C5 side measurements")
     ap.add_argument("--full-dba", action="store_true", help="N=1: run the full 1M-row DBA instead of a 16,384-row slice")
     ap.add_argument("--cpu-rows", type=int, default=200000, help="database row sample for the cpu_baseline leg of our arm")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the (scores, indices) of the last timed step to DIR/*.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
+
+
+def dump_outputs(path, scores, idx):
+    """The result a caller of the timed step receives: top-k scores (float32) and database row indices (float64, exact
+    for every row index), both (queries, k), best first.  The inputs are seeded, so two builds can be compared file by file."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "scores.npy"), scores.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, "indices.npy"), idx.cpu().numpy().astype(np.float64))
 
 
 def measured_peaks():
@@ -294,6 +310,19 @@ def independent_topk(torch, mdir_b200, index, q, k_ext):
     return idx + index.idx_base, v64
 
 
+def synthetic_inputs(torch, dev, lo, hi, rank):
+    """The seeded inputs of our arm: database shard rows [lo, hi) of the 1,001,001 (unit fp32 rows, built on `dev`)
+    and the N_BATCHES query batches (N_BATCHES, N_Q, DIM) on the host."""
+    g = torch.Generator(device=dev).manual_seed(1234 + rank)
+    db32 = torch.empty((hi - lo, DIM), dtype=torch.float32, device=dev)
+    for r0 in range(0, hi - lo, 65536):
+        blk = torch.randn((min(65536, hi - lo - r0), DIM), device=dev, generator=g)
+        db32[r0:r0 + blk.shape[0]] = blk / blk.norm(dim=1, keepdim=True)
+    gq = torch.Generator(device="cpu").manual_seed(99)
+    q = torch.randn((N_BATCHES, N_Q, DIM), generator=gq)
+    return db32, q / q.norm(dim=2, keepdim=True)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -317,17 +346,9 @@ def run_ours(args):
     _lib.check(_lib.lib().mdir_device_check(), "device check")
     lib = _lib.lib()
 
-    # ---- synthetic database shard (rows [lo, hi) of the 1,001,001), built on the device -------
     lo, hi = ShardedIndex.shard_bounds(N_DB, world, rank)
-    g = torch.Generator(device=dev).manual_seed(1234 + rank)
-    db32 = torch.empty((hi - lo, DIM), dtype=torch.float32, device=dev)
-    for r0 in range(0, hi - lo, 65536):
-        blk = torch.randn((min(65536, hi - lo - r0), DIM), device=dev, generator=g)
-        db32[r0:r0 + blk.shape[0]] = blk / blk.norm(dim=1, keepdim=True)
-    # N_BATCHES distinct query batches (pinned host memory; every timed loop rotates through them)
-    gq = torch.Generator(device="cpu").manual_seed(99)
-    q_host = torch.randn((N_BATCHES, N_Q, DIM), generator=gq)
-    q_host = (q_host / q_host.norm(dim=2, keepdim=True)).pin_memory()
+    db32, q_host = synthetic_inputs(torch, dev, lo, hi, rank)
+    q_host = q_host.pin_memory()                                      # every timed loop rotates through these batches
     q_bank = q_host.to(dev)
     torch.cuda.synchronize()
     # cold path of the index build (packing only; the fp32 rows are already resident)
@@ -416,6 +437,8 @@ def run_ours(args):
     sampler.active = False
     launches = launches_per_step * args.steps
     ms_total = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *graphs[(args.steps - 1) % N_BATCHES].out)
     # dominant-kernel duration: the graph carries an event pair around the scan; read it after individual replays
     # of the same graph (a per-step read needs a sync, so not inside the loop above)
     scan_samples = []

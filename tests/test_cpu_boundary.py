@@ -122,7 +122,7 @@ def test_product_never_imports_oracle():
                 assert not re.search(r"^\s*(from|import)\s+oracle", src, flags=re.M), f
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not ref_import.available(), reason="needs the mdir reference checkout (MDIR_REF_ROOT, oracle/_ref or baseline/_ref)")
 def test_install_patches_registries():
     ref_import.import_reference()
     import mdir_b200

@@ -30,7 +30,7 @@ def _run(*args, env=None):
 @pytest.fixture(scope="module")
 def arms(tmp_path_factory):
     if not ref_import.available():
-        pytest.skip("reference checkout not staged (run baseline/stage_ref.py in the build container)")
+        pytest.skip("needs the mdir reference checkout (MDIR_REF_ROOT, oracle/_ref or baseline/_ref)")
     root = str(tmp_path_factory.mktemp("integ"))
     _run("fixture", root)
     out = {}

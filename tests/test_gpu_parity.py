@@ -963,15 +963,16 @@ def test_whitenlearn_matches_reference(m, golden):
     np.testing.assert_allclose(np.abs(out), np.abs(oracle.whitenapply(X32[:, :20].astype(np.float64), mm, P, 32)), rtol=0, atol=1e-5)
 
 
-def test_bench_line_contract():
+def test_bench_line_contract(tmp_path):
     """python bench.py (short run): one JSON line on stdout with the metric, roofline, cpu_baseline, e2e, clocks and
-    gpu_launches objects the measurement contract asks for."""
+    gpu_launches objects the measurement contract asks for; --dump-outputs writes the last timed step's top-100."""
     import json
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "20", "--warmup", "3", "--no-extras", "--cpu-rows", "4000"],
-                         capture_output=True, text=True, timeout=600, cwd=root)
+    dump = str(tmp_path / "dump")
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "20", "--warmup", "3", "--no-extras", "--cpu-rows", "4000",
+                          "--dump-outputs", dump], capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stderr[-800:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1
@@ -990,3 +991,25 @@ def test_bench_line_contract():
     assert pc["checked_queries"] == 8 * 70 and pc["mismatches"] == 0 and pc["certificate_failures"] == 0
     assert d["gpu_launches"] == 20 * 3                         # pack, fused scan, finalize+re-score per step
     assert "sm_mhz" in d["clocks"] or "error" in d["clocks"]
+    sc, ix = np.load(os.path.join(dump, "scores.npy")), np.load(os.path.join(dump, "indices.npy"))
+    assert sorted(os.listdir(dump)) == ["indices.npy", "scores.npy"]
+    assert sc.shape == ix.shape == (70, 100) and sc.dtype == np.float32 and ix.dtype == np.float64
+    assert np.all(np.isfinite(sc)) and np.all(np.diff(sc, axis=1) <= 0)            # best first
+    assert np.all(ix == np.round(ix)) and ix.min() >= 0 and ix.max() < 1001001
+    assert all(len(np.unique(row)) == 100 for row in ix)
+    # the dump is the LAST timed step: query batch (20 - 1) % N_BATCHES of the seeded inputs, ranked independently here
+    # (dense fp32 scores -> 148 candidates -> fp64 re-scoring), swaps accepted only inside 2e-6 gaps as in the bench
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    db32, q_host = bench.synthetic_inputs(torch, torch.device("cuda", 0), 0, bench.N_DB, 0)
+    q = q_host[(20 - 1) % bench.N_BATCHES].to(db32.device)
+    cand = torch.topk(q @ db32.T, 148, dim=1).indices
+    v64 = (db32[cand].double() * q.double()[:, None, :]).sum(-1)
+    r_i, r_v = cand.cpu().numpy(), v64.cpu().numpy()
+    del db32, cand, v64
+    order = np.lexsort((r_i, -r_v), axis=1)[:, :116]
+    r_i, r_v = np.take_along_axis(r_i, order, 1), np.take_along_axis(r_v, order, 1)
+    bad, _ = bench.same_topk(ix.astype(np.int64), sc.astype(np.float64), r_i, r_v, 2e-6)
+    assert bad == 0
