@@ -198,6 +198,16 @@ int mdir_sim_scan_fused_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q
                              uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
                              void* ws, void* stream);
 
+/* mdir_sim_scan_fused_bf16 with int8 operands (tcgen05 kind::i8, s32 accumulate): the first pass of the
+ * certified fp32 search reads n_db * D + 4 n_db bytes instead of 2 n_db * D.  db8 (n_db, D) int8 rows and
+ * row_scale[n_db] from mdir_pack_stats_i8; q8 / q_scale from mdir_pack_q_i8 (two int8 planes per query).
+ * Filter score = row_scale[r] * (s_hi * <x8_r, hi> + s_lo * <x8_r, lo>) in fp32; keys, segments and
+ * counters exactly as mdir_sim_scan_fused_bf16.  D % 128 == 0, n_q <= 128.                  */
+int mdir_sim_scan_fused_i8(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8,
+                           const float* q_scale, int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base,
+                           uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                           void* ws, void* stream);
+
 /* The same scan with fp32 operands consumed as TF32 (tcgen05 kind::tf32, fp32 accumulate):
  * db (n_db, D) and q (n_q, D) row-major fp32, D % 4 == 0.  Used directly it is the TF32
  * similarity variant; fed the (n, 3D) matrices written by mdir_split_tf32x3 (role 0 for the
@@ -255,12 +265,36 @@ int mdir_topk_finalize_rescore(const uint64_t* cand, int64_t cand_row, const uin
                                const float* db_stats,
                                float* out_scores, int32_t* out_idx, uint64_t* out_keys,
                                uint64_t* tau, int32_t* overflow, void* stream);
+/* mdir_topk_finalize_rescore for filter scores of another encoding (mdir_sim_scan_fused_i8): q_eps[q]
+ * (mdir_pack_q_i8) is that encoding's bound for query q, used instead of the bf16 one; db_stats must
+ * still be given.  The extension area grows with the shard (0.2 % of n_db rows, 256 .. 2,048 keys).  */
+int mdir_topk_finalize_rescore_eps(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg,
+                                   int cap0, int cap_l, int n_q, int shortlist, int k_out,
+                                   const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D,
+                                   const float* db_stats, const float* q_eps,
+                                   float* out_scores, int32_t* out_idx, uint64_t* out_keys,
+                                   uint64_t* tau, int32_t* overflow, void* stream);
 #define MDIR_STATUS_OVERFLOW    1
 #define MDIR_STATUS_UNCERTIFIED 2
 
 /* stats[2] (device) = {max_r ||bf16(x_r) - x_r||_2^2, max_r ||x_r||_2^2} over the n rows of a shard:
  * the database half of the certificate's error bound.  db16 = mdir_pack_bf16(db32).            */
 int mdir_pack_stats(const float* db32, const uint16_t* db16, int64_t n, int D, float* stats, void* stream);
+
+/* mdir_pack_stats plus, in the same pass, the int8 plane of the shard: db8 (n, D) with a symmetric
+ * per-row scale row_scale[r] = max_i |x_ri| / 127 (x8 = rint(x / s_r), round half even), and
+ * stats[4] = {the two above, max_r ||x_r - s_r x8_r||^2, max_r ||x_r - s_r x8_r||^2 / ||x_r||^2}.
+ * D % 128 == 0; db32 and db8 16-byte aligned.                                               */
+int mdir_pack_stats_i8(const float* db32, const uint16_t* db16, int64_t n, int D, float* stats,
+                       int8_t* db8, float* row_scale, void* stream);
+
+/* The query operand of mdir_sim_scan_fused_i8 and its certificate bound, one launch: q8 (2 n_pad, D),
+ * n_pad = n_q rounded up to 16, rows [0, n_pad) = hi = rint(q / s_hi), rows [n_pad, 2 n_pad) =
+ * lo = rint((q - s_hi hi) / s_lo) (padding rows zero), s_hi = max|q| / 127, s_lo = max|q - s_hi hi| / 127,
+ * q_scale (n_q, 2) = {s_hi, s_lo}; q_eps[n_q] = the bound on |int8-path score - fp32 score| over every
+ * row of the shard described by stats (mdir_pack_stats_i8).  n_q <= 128, D % 128 == 0.        */
+int mdir_pack_q_i8(const float* q32, int n_q, int D, const float* stats, int8_t* q8, float* q_scale,
+                   float* q_eps, void* stream);
 
 /* Exact fp32 re-scoring of a shortlist: out[q, j] = <db32[idx[q,j]-idx_base], q32[q]>
  * (idx < 0 or outside this shard -> -inf); then callers re-finalize.             */

@@ -42,6 +42,7 @@ PROTOTYPES = {
     "mdir_sim_scan_wide_bf16": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp]),
     "mdir_sim_scan_fused_workspace_bytes": (_sz, [_i]),
     "mdir_sim_scan_fused_bf16": (_i, [_vp, _i64, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp]),
+    "mdir_sim_scan_fused_i8": (_i, [_vp, _vp, _i64, _vp, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp]),
     "mdir_sim_scan_tf32": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp]),
     "mdir_split_tf32x3": (_i, [_vp, _i64, _i, _i, _vp, _vp]),
     "mdir_make_key": (_u64, [_f, _u32]),
@@ -49,7 +50,10 @@ PROTOTYPES = {
     "mdir_select_kth": (_i, [_vp, _i64, _i64, _i, _i, _i, _u32, _vp, _vp, _i64, _vp, _i, _i, _i, _vp]),
     "mdir_topk_finalize": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_topk_finalize_rescore": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mdir_topk_finalize_rescore_eps": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_pack_stats": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
+    "mdir_pack_stats_i8": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
+    "mdir_pack_q_i8": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "mdir_rescore_f32": (_i, [_vp, _i64, _u32, _vp, _i, _i, _vp, _i, _vp, _vp]),
     "mdir_qe_accumulate": (_i, [_vp, _i64, _u32, _i, _vp, _vp, _i, _i, _f, _vp, _vp]),
     "mdir_add_l2n": (_i, [_vp, _vp, _i, _i, _vp, _vp]),

@@ -73,9 +73,20 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-template <bool TF32>
+// operand kinds of sim_scan_kernel: bf16 x bf16 and tf32 x tf32 (fp32 accumulators), s8 x s8 (s32 accumulators)
+constexpr int kKindBf16 = 0, kKindTf32 = 1, kKindI8 = 2;
+
+template <int KIND>
 __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if (TF32) {
+    if (KIND == kKindI8) {
+        asm volatile(
+            "{\n"
+            ".reg .pred p;\n"
+            "setp.ne.b32 p, %4, 0;\n"
+            "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n"
+            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+            : "memory");
+    } else if (KIND == kKindTf32) {
         asm volatile(
             "{\n"
             ".reg .pred p;\n"
@@ -139,11 +150,16 @@ struct ScanParams {
     // FUSED mode only (threshold + filter in one launch): every CTA's first tile is a sample tile; the best two keys
     // of each 32-row group go to grp_top (n_q, grid, 8, 2); CTA q selects the kth smallest of query q's grid*16
     // values as the threshold, published through tau_rw; sync = {arrivals 1, arrivals 2, unused, exits}
-    int acc_bufs, acc_stride;     // TMEM: acc_bufs accumulator tiles of 2 x acc_stride columns (3 x 2 x 80 when N <= 80, else 2 x 2 x 128)
+    int acc_bufs, acc_stride;     // TMEM: acc_bufs accumulator tiles of 2 x acc_stride columns (3 x 2 x 80 when N <= 80, else 2 x 2 x 128);
+                                  // int8: acc_bufs accumulators of ONE 128-row half each (see sim_scan_kernel)
     int kth;
     uint32_t* grp_top;
     uint32_t* sync;
     uint64_t* tau_rw;
+    // int8 only: score(row r, query q) = s_r * (s_hi[q] * acc_hi + s_lo[q] * acc_lo), the query as two int8 planes
+    // (rows [0, n_pad) = hi, [n_pad, 2 n_pad) = lo of the B operand)
+    const float* row_scale;      // s_r, n_db entries
+    const float* q_scale;        // {s_hi, s_lo} per query
 };
 
 constexpr int MDIR_SCAN_FUSED = 3;      // internal mode behind mdir_sim_scan_fused_bf16
@@ -248,9 +264,37 @@ __device__ __forceinline__ int tile_of_work(const ScanParams& p, int j) {
     return p.n_sample * p.sample_stride + (j - in_groups);
 }
 
-template <bool TF32>
+// 16 scores (columns c0 .. c0 + 15 of this warp's TMEM lanes) of one accumulator.  int8: the hi plane's s32 sums sit in
+// columns [0, n_pad), the lo plane's in [n_pad, 2 n_pad); s_r is this lane's row scale and qsc the per-query scales.
+template <int KIND>
+__device__ __forceinline__ void acc_scores16(uint32_t taddr, int c0, int n_pad, float s_r, const float* qsc, float (&s)[16]) {
+    uint32_t v[16];
+    tmem_ld16(taddr + (uint32_t)c0, v);
+    if (KIND == kKindI8) {
+        uint32_t lo[16];
+        tmem_ld16(taddr + (uint32_t)(n_pad + c0), lo);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+            const float2 sc = *reinterpret_cast<const float2*>(qsc + 2 * (c0 + i));
+            s[i] = __fmul_rn(__fmaf_rn((float)(int)v[i], sc.x, __fmul_rn((float)(int)lo[i], sc.y)), s_r);
+        }
+    } else {
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 16; ++i) s[i] = __uint_as_float(v[i]);
+    }
+}
+
+// KIND = kKindI8 (FUSED mode only): the accumulators rotate per 128-row HALF rather than per tile.  Two planes of up
+// to 80 queries make N = 160 columns per half, so two whole tiles (640 columns) no longer fit TMEM's 512; three
+// half-accumulators (480) do.  Half index i = 2 * item + h lives in buffer i % acc_bufs: the MMAs of the next tile wait
+// only for the epilogue of this tile's first half, and the second half's epilogue overlaps them.
+template <int KIND>
 __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_constant__ CUtensorMap tmap_db,
                                                                 const __grid_constant__ CUtensorMap tmap_q, const ScanParams p) {
+    constexpr bool TF32 = KIND == kKindTf32;
+    constexpr bool I8 = KIND == kKindI8;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t full_bar[kMaxStages];
     __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
@@ -260,10 +304,11 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
     __shared__ uint64_t tau_s0[kMaxN];
     __shared__ float tau_f0[kMaxN];
     __shared__ uint32_t cand_n0[kMaxN];    // candidates this CTA has appended per query (CTA-private list: no global atomics)
+    __shared__ __align__(8) float qsc[I8 ? 2 * 128 : 2];    // int8: {s_hi, s_lo} per query
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t b_bytes = (uint32_t)p.n_pad * 128u;
+    const uint32_t b_bytes = (uint32_t)p.n_pad * 128u * (I8 ? 2u : 1u);
     const uint32_t stage_bytes = (uint32_t)kABytes + b_bytes;
     // per-query filter state: the static arrays for one block of queries; behind the operand ring for a wide launch
     // (n_qblocks blocks of n_pad queries: thresholds and counters of all n_q_total queries stay resident)
@@ -298,6 +343,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
     }
     if (p.mode == MDIR_SCAN_FUSED) {
         for (int c = threadIdx.x; c < kMaxN; c += kThreads) cand_n[c] = 0u;
+        if (I8)
+            for (int c = threadIdx.x; c < 2 * p.n_pad; c += kThreads) qsc[c] = c < 2 * p.n_q ? p.q_scale[c] : 0.f;
     } else if (p.mode == MDIR_SCAN_FILTER) {
         for (int c = threadIdx.x; c < n_state; c += kThreads) {
             uint64_t t = c < p.n_q_total ? p.tau[c] : 0ull;
@@ -324,7 +371,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                     const uint32_t fb = smem_u32(&full_bar[stage]);
                     const uint32_t a_dst = smem_base + (uint32_t)stage * stage_bytes;
                     mbar_expect_tx(fb, stage_bytes);
-                    constexpr int kElemsPerBlock = TF32 ? 32 : 64;
+                    constexpr int kElemsPerBlock = TF32 ? 32 : (I8 ? 128 : 64);
                     tma_load_2d(a_dst, &tmap_db, fb, kb * kElemsPerBlock, row0, p.db_hint);
                     tma_load_2d(a_dst + kABytes, &tmap_q, fb, kb * kElemsPerBlock, w.qb * p.n_pad, kEvictLast);
                     if (++stage == p.num_stages) { stage = 0; phase ^= 1u; }
@@ -334,17 +381,31 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
     } else if (warp == 1) {
         // ------------------------------------------------------------ MMA issuer
         if (lane == 0) {
-            // instruction descriptor: D=f32 [4,6)=1, A/B format [7,10)/[10,13) = 1 (bf16) or 2 (tf32), K-major A/B,
-            // N>>3 [17,23), M>>4 [24,29)
+            // instruction descriptor: D format [4,6) = 1 (f32) or 2 (s32), A/B format [7,10)/[10,13) = 1 (bf16 / signed
+            // int8) or 2 (tf32), K-major A/B, N>>3 [17,23), M>>4 [24,29); int8: N = both query planes
             constexpr uint32_t fmt = TF32 ? 2u : 1u;
-            const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(p.n_pad >> 3) << 17) | ((128u >> 4) << 24);
+            constexpr uint32_t dfmt = I8 ? 2u : 1u;
+            const uint32_t n_mma = (uint32_t)p.n_pad * (I8 ? 2u : 1u);
+            const uint32_t idesc = (dfmt << 4) | (fmt << 7) | (fmt << 10) | ((n_mma >> 3) << 17) | ((128u >> 4) << 24);
             int stage = 0;
             uint32_t phase = 0;
             WorkItem w;
             for (int it = 0; next_item(p, it, w); ++it) {
                 const int b = it % p.acc_bufs;
                 const uint32_t acc_phase = (uint32_t)(it / p.acc_bufs) & 1u;
-                mbar_wait(smem_u32(&tmem_empty_bar[b]), acc_phase ^ 1u);
+                uint32_t d_half[2];
+                if (I8) {
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        const int i = 2 * it + h, hb = i % p.acc_bufs;
+                        mbar_wait(smem_u32(&tmem_empty_bar[hb]), ((uint32_t)(i / p.acc_bufs) & 1u) ^ 1u);
+                        d_half[h] = tmem_base + (uint32_t)hb * (uint32_t)p.acc_stride;
+                    }
+                } else {
+                    mbar_wait(smem_u32(&tmem_empty_bar[b]), acc_phase ^ 1u);
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) d_half[h] = tmem_base + (uint32_t)(b * 2 + h) * (uint32_t)p.acc_stride;
+                }
                 tc_fence_after();
                 const int nkb = w.nkb;
                 for (int kb = 0; kb < nkb; ++kb) {
@@ -354,18 +415,22 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                     const uint32_t b_base = a_base + kABytes;
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
-                        const uint32_t d_tmem = tmem_base + (uint32_t)(b * 2 + h) * (uint32_t)p.acc_stride;
 #pragma unroll
                         for (int k = 0; k < kKSteps; ++k) {
                             const uint64_t ad = umma_desc_sw128(a_base + (uint32_t)h * (128u * 128u) + (uint32_t)k * 32u);
                             const uint64_t bd = umma_desc_sw128(b_base + (uint32_t)k * 32u);
-                            umma_ss<TF32>(d_tmem, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+                            umma_ss<KIND>(d_half[h], ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
                         }
                     }
                     umma_commit(smem_u32(&empty_bar[stage]));     // frees the smem slot when these MMAs retire
                     if (++stage == p.num_stages) { stage = 0; phase ^= 1u; }
                 }
-                umma_commit(smem_u32(&tmem_full_bar[b]));         // accumulators of this tile are complete
+                if (I8) {                                          // accumulators of this tile are complete
+                    umma_commit(smem_u32(&tmem_full_bar[(2 * it) % p.acc_bufs]));
+                    umma_commit(smem_u32(&tmem_full_bar[(2 * it + 1) % p.acc_bufs]));
+                } else {
+                    umma_commit(smem_u32(&tmem_full_bar[b]));
+                }
             }
         }
     } else {
@@ -382,8 +447,27 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
             const int tile = w.tile;
             float* dense_out = p.dense_out + (int64_t)w.ks * p.split_stride + (int64_t)w.qb * p.n_pad * p.dense_ld;
             const int nq_here = p.n_qblocks > 1 ? min(p.n_pad, p.n_q_total - w.qb * p.n_pad) : p.n_q;     // queries of this item's block
-            mbar_wait(smem_u32(&tmem_full_bar[b]), acc_phase);
-            tc_fence_after();
+            // int8: this lane's row scales of both halves, loaded before the accumulator waits so that their latency hides
+            // under the MMAs instead of stalling the epilogue (and with it the release of the TMEM buffer)
+            float s_rh[2] = {0.f, 0.f};
+            if (I8) {
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int64_t row = (int64_t)tile * kBlockM + h * 128 + quarter * 32 + lane;
+                    if (row < p.n_db) s_rh[h] = __ldg(p.row_scale + row);
+                }
+            }
+            // TMEM column of half h of this item's accumulators, and (int8) the barrier slot / phase of that half
+            auto acc_col = [&](int h) -> uint32_t {
+                return I8 ? (uint32_t)((2 * it + h) % p.acc_bufs) * (uint32_t)p.acc_stride : (uint32_t)(b * 2 + h) * (uint32_t)p.acc_stride;
+            };
+            if (!I8 || (p.mode == MDIR_SCAN_FUSED && it == 0)) {
+                for (int h = 0; h < (I8 ? 2 : 1); ++h) {
+                    const int i = I8 ? 2 * it + h : it;
+                    mbar_wait(smem_u32(&tmem_full_bar[i % p.acc_bufs]), (uint32_t)(i / p.acc_bufs) & 1u);
+                }
+                tc_fence_after();
+            }
             if (p.mode == MDIR_SCAN_FUSED && it == 0) {
                 // ---- pass A over the sample tile: best two keys of each 32-row group (this warp x half), per query
                 const int et = (int)threadIdx.x - 64;
@@ -391,16 +475,16 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                 for (int h = 0; h < 2; ++h) {
                     const int64_t row = (int64_t)tile * kBlockM + h * 128 + quarter * 32 + lane;
                     const bool row_ok = row < p.n_db;
-                    const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(b * 2 + h) * (uint32_t)p.acc_stride;
+                    const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc_col(h);
+                    const float s_r = h ? s_rh[1] : s_rh[0];
 #pragma unroll 1
                     for (int c0 = 0; c0 < p.n_pad; c0 += 16) {
-                        uint32_t v[16];
-                        tmem_ld16(taddr + (uint32_t)c0, v);
-                        tmem_ld_wait();
+                        float v[16];
+                        acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qsc, v);
                         uint32_t m1 = 0xffffffffu, m2 = 0xffffffffu;
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
-                            const uint32_t key = row_ok ? desc_key(__uint_as_float(v[i])) : 0xffffffffu;
+                            const uint32_t key = row_ok ? desc_key(v[i]) : 0xffffffffu;
                             const uint32_t a = __reduce_min_sync(0xffffffffu, key);
                             const unsigned who = __ballot_sync(0xffffffffu, key == a);
                             const uint32_t key2 = (lane == __ffs(who) - 1) ? 0xffffffffu : key;
@@ -494,14 +578,19 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                 const int r_in_tile = h * 128 + quarter * 32 + lane;
                 const int64_t row = (int64_t)tile * kBlockM + r_in_tile;
                 const bool row_ok = row < p.n_db;
-                const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(b * 2 + h) * (uint32_t)p.acc_stride;
+                if (I8) {
+                    const int i = 2 * it + h;
+                    mbar_wait(smem_u32(&tmem_full_bar[i % p.acc_bufs]), (uint32_t)(i / p.acc_bufs) & 1u);
+                    tc_fence_after();
+                }
+                const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc_col(h);
+                const float s_r = h ? s_rh[1] : s_rh[0];
                 const int64_t out_row = (p.mode == MDIR_SCAN_SAMPLE ? (int64_t)w.j * kBlockM : (int64_t)tile * kBlockM) + r_in_tile;
                 const uint32_t gidx = p.idx_base + (uint32_t)row;
 #pragma unroll 1
                 for (int c0 = 0; c0 < p.n_pad; c0 += 16) {
-                    uint32_t v[16];
-                    tmem_ld16(taddr + (uint32_t)c0, v);
-                    tmem_ld_wait();
+                    float v[16];
+                    acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qsc, v);
                     if (emode != MDIR_SCAN_FILTER) {
                         // rows past the end of the database only exist in the compact SAMPLE buffer: mark them -inf
                         if (p.chain > 1) {
@@ -510,27 +599,27 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                             float* sum = chain_sum + ((int64_t)(h * p.n_pad + c0) * 128 + quarter * 32 + lane);
                             if (w.chunk == 0) {
 #pragma unroll
-                                for (int i = 0; i < 16; ++i) sum[i * 128] = __uint_as_float(v[i]);
+                                for (int i = 0; i < 16; ++i) sum[i * 128] = v[i];
                             } else if (!w.last) {
 #pragma unroll
-                                for (int i = 0; i < 16; ++i) sum[i * 128] = __fadd_rn(sum[i * 128], __uint_as_float(v[i]));
+                                for (int i = 0; i < 16; ++i) sum[i * 128] = __fadd_rn(sum[i * 128], v[i]);
                             } else if (row_ok) {
 #pragma unroll
                                 for (int i = 0; i < 16; ++i)
                                     if (c0 + i < p.n_q)
-                                        dense_out[(int64_t)(c0 + i) * p.dense_ld + out_row] = __fadd_rn(sum[i * 128], __uint_as_float(v[i]));
+                                        dense_out[(int64_t)(c0 + i) * p.dense_ld + out_row] = __fadd_rn(sum[i * 128], v[i]);
                             }
                         } else if (row_ok || p.mode == MDIR_SCAN_SAMPLE) {
 #pragma unroll
                             for (int i = 0; i < 16; ++i)
                                 if (c0 + i < nq_here)
-                                    dense_out[(int64_t)(c0 + i) * p.dense_ld + out_row] = row_ok ? __uint_as_float(v[i]) : -INFINITY;
+                                    dense_out[(int64_t)(c0 + i) * p.dense_ld + out_row] = row_ok ? v[i] : -INFINITY;
                         }
                     } else if (row_ok) {
                         const int qo = w.qb * p.n_pad + c0;               // first query of these 16 columns
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
-                            const float s = __uint_as_float(v[i]);
+                            const float s = v[i];
                             if (s >= tau_f[qo + i] && c0 + i < nq_here) {
                                 const uint64_t key = make_key(s, gidx);
                                 if (key <= tau_s[qo + i]) {
@@ -542,10 +631,17 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                         }
                     }
                 }
+                if (I8) {                                  // this half's accumulator is free for the MMAs of a later tile
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(smem_u32(&tmem_empty_bar[(2 * it + h) % p.acc_bufs]));
+                }
             }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(smem_u32(&tmem_empty_bar[b]));
+            if (!I8) {
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(smem_u32(&tmem_empty_bar[b]));
+            }
         }
         if (emode == MDIR_SCAN_FILTER) {
             asm volatile("bar.sync 1, 128;" ::: "memory");       // the four epilogue warps only
@@ -595,17 +691,20 @@ static EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-static int make_tmap(CUtensorMap* map, bool tf32, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
+static int make_tmap(CUtensorMap* map, int kind, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
     EncodeTiledFn fn = get_encode_fn();
     if (!fn) {
         set_error("cuTensorMapEncodeTiled entry point unavailable");
         return MDIR_E_DRIVER;
     }
     cuuint64_t gdim[2] = {cols, rows};
-    cuuint64_t gstride[1] = {cols * (tf32 ? 4u : 2u)};
-    cuuint32_t box[2] = {(cuuint32_t)(tf32 ? 32 : 64), box_rows};
+    const uint32_t esz = kind == kKindTf32 ? 4u : (kind == kKindI8 ? 1u : 2u);
+    cuuint64_t gstride[1] = {cols * esz};
+    cuuint32_t box[2] = {(cuuint32_t)(kBlockKBytes / esz), box_rows};      // one 128-byte swizzle row per operand row
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(map, tf32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), gdim, gstride, box, estr,
+    const CUtensorMapDataType dt = kind == kKindTf32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                   : (kind == kKindI8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
+    CUresult r = fn(map, dt, 2, const_cast<void*>(ptr), gdim, gstride, box, estr,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
@@ -619,16 +718,23 @@ static int make_tmap(CUtensorMap* map, bool tf32, const void* ptr, uint64_t rows
 
 using namespace mdir;
 
-static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, int n_q, int D, int mode, int sample_stride, int n_sample,
+// kind: kKindBf16 / kKindTf32 (bool false / true at the older call sites) or kKindI8 (FUSED mode only; q = the two
+// int8 planes of mdir_pack_q_i8, row_scale / q_scale = s_r and {s_hi, s_lo})
+static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, int n_q, int D, int mode, int sample_stride, int n_sample,
                        float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base, uint64_t* cand,
                        uint32_t* seg_counts, int cap_s, int cap_l, void* stream, int k_split = 1, int64_t split_stride = 0,
-                       int kth = 0, uint32_t* fused_ws = nullptr, uint64_t* tau_rw = nullptr, int n_q_total = 0) {
-    const int esz = tf32 ? 4 : 2;
+                       int kth = 0, uint32_t* fused_ws = nullptr, uint64_t* tau_rw = nullptr, int n_q_total = 0,
+                       const float* row_scale = nullptr, const float* q_scale = nullptr) {
+    const bool tf32 = kind == kKindTf32, i8 = kind == kKindI8;
+    const int esz = tf32 ? 4 : (i8 ? 1 : 2);
     MDIR_CHECK_ARG(db && q && n_db >= 1 && n_q >= 1 && n_q <= kMaxN && D >= 16 / esz && (D % (16 / esz)) == 0);
     MDIR_CHECK_ARG((((uintptr_t)db | (uintptr_t)q) & 15) == 0);
     MDIR_CHECK_ARG(mode >= 0 && mode <= MDIR_SCAN_FUSED);
     MDIR_CHECK_ARG(n_db + (int64_t)idx_base <= ((int64_t)1 << 32));
+    MDIR_CHECK_ARG(!i8 || (mode == MDIR_SCAN_FUSED && row_scale && q_scale));
     ScanParams p;
+    p.row_scale = row_scale;
+    p.q_scale = q_scale;
     p.n_db = n_db;
     p.n_q = n_q;
     p.n_pad = (n_q + 15) & ~15;
@@ -661,6 +767,11 @@ static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, i
     // then not overlapped with the next tile's MMAs: ~10 % of a D = 2048 tile)
     p.acc_bufs = p.n_pad <= 80 ? 3 : (p.n_pad <= 128 ? 2 : 1);
     p.acc_stride = p.n_pad <= 80 ? 80 : (p.n_pad <= 128 ? 128 : 256);
+    if (i8) {
+        // half-accumulators of both query planes: 3 x 160 columns up to 80 queries, else 2 x (2 n_pad) (= one tile)
+        p.acc_stride = 2 * p.n_pad;
+        p.acc_bufs = p.n_pad <= 80 ? 3 : 2;
+    }
     p.kth = 0;
     p.grp_top = nullptr;
     p.sync = nullptr;
@@ -679,10 +790,10 @@ static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, i
                 // the running sums (256 x n_pad fp32) share the CTA's shared memory with the operand ring: wider query
                 // blocks go as two launches
                 const int n0 = ((n_q / 2) + 15) & ~15;
-                int rc = launch_scan(tf32, db, n_db, q, n0, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+                int rc = launch_scan(kind, db, n_db, q, n0, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
                                      cap_s, cap_l, stream);
                 if (rc) return rc;
-                return launch_scan(tf32, db, n_db, static_cast<const uint8_t*>(q) + (size_t)n0 * D * esz, n_q - n0, D, mode, sample_stride, n_sample,
+                return launch_scan(kind, db, n_db, static_cast<const uint8_t*>(q) + (size_t)n0 * D * esz, n_q - n0, D, mode, sample_stride, n_sample,
                                    dense_out + (int64_t)n0 * dense_ld, dense_ld, tau, idx_base, cand, seg_counts, cap_s, cap_l, stream);
             }
             p.kb_per_chain = kChainKBlocks;
@@ -728,7 +839,7 @@ static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, i
     p.db_hint = ((int64_t)n_db * D * esz > (int64_t)96 * 1024 * 1024) ? kEvictFirst : kEvictNormal;
     if (p.n_work <= 0 && mode != MDIR_SCAN_FUSED) return 0;
 
-    const int stage_bytes = kABytes + p.n_pad * 128;
+    const int stage_bytes = kABytes + p.n_pad * 128 * (i8 ? 2 : 1);
     int chain_bytes = p.chain > 1 ? kBlockM * p.n_pad * 4 : 0;            // running sums of the chained tf32 DENSE scan
     if (p.n_qblocks > 1 && mode == MDIR_SCAN_FILTER) chain_bytes = p.n_qblocks * p.n_pad * 16;      // wide FILTER: per-query thresholds + counters
     int stages = (232448 - 1024 - 8192 - chain_bytes) / stage_bytes;      // 8 KB left for the static shared arrays
@@ -738,15 +849,17 @@ static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, i
     const size_t smem = (size_t)stages * stage_bytes + 1024 + chain_bytes;
 
     CUtensorMap tmap_db, tmap_q;
-    int rc = make_tmap(&tmap_db, tf32, db, (uint64_t)n_db, (uint64_t)D, kBlockM);
+    int rc = make_tmap(&tmap_db, kind, db, (uint64_t)n_db, (uint64_t)D, kBlockM);
     if (rc) return rc;
-    rc = make_tmap(&tmap_q, tf32, q, (uint64_t)p.n_q_total, (uint64_t)D, (uint32_t)p.n_pad);
+    const int q_rows = i8 ? 2 * p.n_pad : p.n_q_total;         // int8: hi plane rows [0, n_pad), lo plane rows [n_pad, 2 n_pad)
+    rc = make_tmap(&tmap_q, kind, q, (uint64_t)q_rows, (uint64_t)D, (uint32_t)(i8 ? 2 * p.n_pad : p.n_pad));
     if (rc) return rc;
 
     static PerDeviceOnce once;
     if (once.first() != 0) {
-        MDIR_CUDA(cudaFuncSetAttribute(sim_scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 8192));
-        MDIR_CUDA(cudaFuncSetAttribute(sim_scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 8192));
+        MDIR_CUDA(cudaFuncSetAttribute(sim_scan_kernel<kKindBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 8192));
+        MDIR_CUDA(cudaFuncSetAttribute(sim_scan_kernel<kKindTf32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 8192));
+        MDIR_CUDA(cudaFuncSetAttribute(sim_scan_kernel<kKindI8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 8192));
     }
     const int n_ctas_wanted = p.chain > 1 ? p.n_tiles : p.n_work;
     int grid = mode == MDIR_SCAN_FUSED ? p.n_sample : balanced_grid(n_ctas_wanted, kNumSMs);
@@ -770,12 +883,13 @@ static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, i
         attr[0].val.cooperative = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        MDIR_CUDA(cudaLaunchKernelEx(&cfg, sim_scan_kernel<false>, tmap_db, tmap_q, p));
+        if (i8) MDIR_CUDA(cudaLaunchKernelEx(&cfg, sim_scan_kernel<kKindI8>, tmap_db, tmap_q, p));
+        else MDIR_CUDA(cudaLaunchKernelEx(&cfg, sim_scan_kernel<kKindBf16>, tmap_db, tmap_q, p));
         MDIR_LAUNCH_CHECK();
         return 0;
     }
-    if (tf32) sim_scan_kernel<true><<<grid, kThreads, smem, (cudaStream_t)stream>>>(tmap_db, tmap_q, p);
-    else sim_scan_kernel<false><<<grid, kThreads, smem, (cudaStream_t)stream>>>(tmap_db, tmap_q, p);
+    if (tf32) sim_scan_kernel<kKindTf32><<<grid, kThreads, smem, (cudaStream_t)stream>>>(tmap_db, tmap_q, p);
+    else sim_scan_kernel<kKindBf16><<<grid, kThreads, smem, (cudaStream_t)stream>>>(tmap_db, tmap_q, p);
     MDIR_LAUNCH_CHECK();
     return 0;
 }
@@ -783,7 +897,7 @@ static int launch_scan(bool tf32, const void* db, int64_t n_db, const void* q, i
 extern "C" int mdir_sim_scan_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
                                   int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
                                   uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* stream) {
-    return launch_scan(false, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+    return launch_scan(kKindBf16, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
                        cap_s, cap_l, stream);
 }
 
@@ -793,7 +907,7 @@ extern "C" int mdir_sim_scan_dense_bf16(const uint16_t* db, int64_t n_db, const 
     // 128 queries per work item: 256 (all of TMEM for one tile, no accumulator double-buffering, three 64 KB stages) was
     // measured 8-10 % slower on both the 512-D and the 2048-D shape
     const int blk = n_q < 128 ? n_q : 128;
-    return launch_scan(false, db, n_db, q, blk, D, MDIR_SCAN_DENSE, 0, 0, dense_out, dense_ld, nullptr, 0, nullptr, nullptr, 0, 0, stream, 1, 0, 0,
+    return launch_scan(kKindBf16, db, n_db, q, blk, D, MDIR_SCAN_DENSE, 0, 0, dense_out, dense_ld, nullptr, 0, nullptr, nullptr, 0, 0, stream, 1, 0, 0,
                        nullptr, nullptr, n_q > blk ? n_q : 0);
 }
 
@@ -803,7 +917,7 @@ extern "C" int mdir_sim_scan_wide_bf16(const uint16_t* db, int64_t n_db, const u
     // mdir_sim_scan_bf16 for 129 .. 1024 queries in one launch (DENSE: any number): blocks of 128 queries per work item
     MDIR_CHECK_ARG(n_q >= 1 && (mode == MDIR_SCAN_DENSE || n_q <= kMaxWideQ));
     const int blk = n_q < 128 ? n_q : 128;
-    return launch_scan(false, db, n_db, q, blk, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts, cap_s,
+    return launch_scan(kKindBf16, db, n_db, q, blk, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts, cap_s,
                        cap_l, stream, 1, 0, 0, nullptr, nullptr, n_q > blk ? n_q : 0);
 }
 
@@ -815,14 +929,22 @@ extern "C" int mdir_sim_scan_fused_bf16(const uint16_t* db, int64_t n_db, const 
                                         uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* ws,
                                         void* stream) {
     MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0);
-    return launch_scan(false, db, n_db, q, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
+    return launch_scan(kKindBf16, db, n_db, q, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
                        stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau);
+}
+
+extern "C" int mdir_sim_scan_fused_i8(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8, const float* q_scale,
+                                      int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
+                                      int cap_s, int cap_l, void* ws, void* stream) {
+    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0 && D % 128 == 0);
+    return launch_scan(kKindI8, db8, n_db, q8, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
+                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, row_scale, q_scale);
 }
 
 extern "C" int mdir_sim_scan_tf32(const float* db, int64_t n_db, const float* q, int n_q, int D, int mode, int sample_stride,
                                   int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
                                   uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* stream) {
-    return launch_scan(true, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+    return launch_scan(kKindTf32, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
                        cap_s, cap_l, stream);
 }
 
@@ -1025,7 +1147,7 @@ extern "C" int mdir_whiten_project_tc(const float* v, const float* m, int n, int
         center_split_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(v + (size_t)r0 * D, m, nb, D, vx3);
         MDIR_LAUNCH_CHECK();
         const int64_t split_stride = (int64_t)nb * dims;
-        int rc = launch_scan(true, Px3, dims, vx3, nb, 3 * D, MDIR_SCAN_DENSE, 0, 0, partial, dims, nullptr, 0, nullptr, nullptr, 0, 0,
+        int rc = launch_scan(kKindTf32, Px3, dims, vx3, nb, 3 * D, MDIR_SCAN_DENSE, 0, 0, partial, dims, nullptr, 0, nullptr, nullptr, 0, 0,
                              (void*)st, ks, split_stride);
         if (rc) return rc;
         // launch_scan may have reduced the split count; recompute it the same way

@@ -531,6 +531,8 @@ __device__ __forceinline__ void rescore_share(uint64_t* local_list, uint32_t rem
 // The answer is then PROVEN equal to the exact fp32 top k_out of the whole shard provided the candidate list
 // contains every row with bf16 score >= t - eps, i.e. the filter threshold tau[q] is not tighter than that bound
 // and nothing overflowed.  Otherwise status bit 1 (uncertified) is raised and the host widens the selection.
+// q_eps != NULL: the filter scores came from another encoding (the int8 scan) and q_eps[q] is that encoding's bound
+// for query q (mdir_pack_q_i8), used instead of the bf16 formula above.
 // status[q]: bit 0 = a candidate segment / the staging area overflowed, bit 1 = not certified.
 template <int CS>      // CS = CTAs per query (thread-block cluster size): rank 0 selects and sorts, all ranks share the fp32 re-scoring
 __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __restrict__ cand, int64_t cand_row,
@@ -540,7 +542,7 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
                                                              uint64_t* __restrict__ tau, int32_t* __restrict__ overflow,
                                                              const float* __restrict__ db32, int64_t n_db, uint32_t idx_base,
                                                              const float* __restrict__ q32, int D, int k_out,
-                                                             const float* __restrict__ db_stats) {
+                                                             const float* __restrict__ db_stats, const float* __restrict__ q_eps) {
     extern __shared__ uint64_t skeys[];
     __shared__ uint32_t hist[256];
     __shared__ uint64_t s_prefix;
@@ -731,7 +733,9 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
         __syncthreads();
         const uint64_t last16 = nk > 0 ? sl[nk - 1] : 0ull;          // worst bf16 key inside the shortlist
         float eps = 0.f;
-        if (db_stats) {
+        if (db_stats && q_eps) {
+            eps = q_eps[q];
+        } else if (db_stats) {
             // one block reduction for the three sums
             q2 = warp_sum(q2); qt2 = warp_sum(qt2); qf2 = warp_sum(qf2);
             const int wi = threadIdx.x >> 5;
@@ -959,7 +963,7 @@ extern "C" int mdir_select_kth(const float* scores, int64_t ld, int64_t n, int n
 static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0, int cap_l, int n_q,
                            int k, float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
                            const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D, int k_out, const float* db_stats,
-                           void* stream) {
+                           void* stream, const float* q_eps = nullptr) {
     MDIR_CHECK_ARG(cand && seg_counts && n_seg >= 1 && n_seg <= MDIR_CAND_SEGS && cap0 >= 0 && n_q >= 0 && k >= 1 && k <= 4096);
     MDIR_CHECK_ARG(n_seg == 1 || cap_l >= 1);
     MDIR_CHECK_ARG(cand_row >= (int64_t)cap0 + (int64_t)(n_seg - 1) * cap_l);
@@ -973,8 +977,14 @@ static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_
     // mdir_tune: a smaller staging area (two CTAs fit on an SM); a query with more candidates raises the overflow bit
     if (g_finalize_stage_cap > 0 && smem_cap > g_finalize_stage_cap) smem_cap = g_finalize_stage_cap;
     if (smem_cap < 2 * kpow2) smem_cap = 2 * kpow2;
-    // with re-scoring the selection area also takes the certified extension of the shortlist (as many keys again)
-    const int sl_cap = db32 ? 2 * kpow2 : kpow2;
+    // with re-scoring the selection area also takes the certified extension of the shortlist (as many keys again).  The
+    // int8 route's bound reaches ~5x as many rows: ~0.09 % of a unit-norm randn shard at D = 2048 against ~0.02 % for
+    // bf16, so its area grows with the shard -- room for 0.2 % of it, a power of two (the bitonic sorts), <= 2,048 keys
+    int sl_cap = db32 ? 2 * kpow2 : kpow2;
+    if (db32 && q_eps) {
+        const int64_t want = (int64_t)kpow2 + n_db / 512;
+        while (sl_cap < want && sl_cap < 2048) sl_cap <<= 1;
+    }
     size_t smem = (size_t)(smem_cap + sl_cap) * 8;
     if (db32) {
         MDIR_CHECK_ARG(q32 && D > 0 && D <= 8192 && k_out >= 1 && k_out <= k && n_db >= 0);
@@ -1008,13 +1018,13 @@ static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         MDIR_CUDA(cudaLaunchKernelEx(&cfg, topk_finalize_kernel<2>, cand, cand_row, seg_counts, n_seg, cap0, cap_l, k, smem_cap, sl_cap, out_scores,
-                                     out_idx, out_keys, tau, overflow, db32, n_db, idx_base, q32, D, k_out, db_stats));
+                                     out_idx, out_keys, tau, overflow, db32, n_db, idx_base, q32, D, k_out, db_stats, q_eps));
         MDIR_LAUNCH_CHECK();
         return 0;
     }
     topk_finalize_kernel<1><<<n_q, 1024, smem, (cudaStream_t)stream>>>(cand, cand_row, seg_counts, n_seg, cap0, cap_l, k, smem_cap, sl_cap,
                                                                         out_scores, out_idx, out_keys, tau, overflow, db32, n_db, idx_base,
-                                                                        q32, D, k_out, db_stats);
+                                                                        q32, D, k_out, db_stats, q_eps);
     MDIR_LAUNCH_CHECK();
     return 0;
 }
@@ -1033,6 +1043,16 @@ extern "C" int mdir_topk_finalize_rescore(const uint64_t* cand, int64_t cand_row
     MDIR_CHECK_ARG(db32 != nullptr);
     return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
                            db32, n_db, idx_base, q32, D, k_out, db_stats, stream);
+}
+
+extern "C" int mdir_topk_finalize_rescore_eps(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
+                                              int cap_l, int n_q, int shortlist, int k_out, const float* db32, int64_t n_db,
+                                              uint32_t idx_base, const float* q32, int D, const float* db_stats, const float* q_eps,
+                                              float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
+                                              void* stream) {
+    MDIR_CHECK_ARG(db32 != nullptr && db_stats != nullptr && q_eps != nullptr);
+    return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
+                           db32, n_db, idx_base, q32, D, k_out, db_stats, stream, q_eps);
 }
 
 // db_stats for the shortlist certificate: {max_r ||bf16(x_r) - x_r||^2, max_r ||x_r||^2} over the rows of a shard.
@@ -1071,6 +1091,149 @@ extern "C" int mdir_pack_stats(const float* db32, const uint16_t* db16, int64_t 
     const int64_t blocks = (n + 7) / 8;
     pack_stats_kernel<<<(unsigned)(blocks < 148 * 8 ? blocks : 148 * 8), 256, 0, (cudaStream_t)stream>>>(
         db32, reinterpret_cast<const __nv_bfloat16*>(db16), n, D, reinterpret_cast<uint32_t*>(stats));
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+// ---- int8 first pass of the certified serving scan (mdir_sim_scan_fused_i8) --------------------------------------
+// Symmetric quantisation of one value: v / s rounded to nearest even, clamped to the int8 range [-127, 127].
+namespace mdir {
+__device__ __forceinline__ float quant_i8(float v, float s) {
+    return s > 0.f ? fminf(fmaxf(rintf(__fdiv_rn(v, s)), -127.f), 127.f) : 0.f;
+}
+
+// One warp per database row: the int8 row x8_r with s_r = max_i |x_ri| / 127, and in the same pass the certificate's
+// database terms stats = {max_r ||bf16(x_r) - x_r||^2, max_r ||x_r||^2, max_r ||x_r - s_r x8_r||^2,
+// max_r ||x_r - s_r x8_r||^2 / ||x_r||^2} (the last one selects the route, see Index).
+__global__ void __launch_bounds__(256) pack_stats_i8_kernel(const float* __restrict__ db32, const __nv_bfloat16* __restrict__ db16, int64_t n,
+                                                            int D, uint32_t* __restrict__ stats, int8_t* __restrict__ db8,
+                                                            float* __restrict__ row_scale) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    float e_max = 0.f, x_max = 0.f, e8_max = 0.f, rel_max = 0.f;
+    for (int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); r < n; r += warps) {
+        const float* a = db32 + r * D;
+        const __nv_bfloat16* b = db16 + r * D;
+        float e2 = 0.f, x2 = 0.f, m = 0.f;
+        for (int i = lane; i < D; i += 32) {
+            const float x = a[i];
+            const float d = __bfloat162float(b[i]) - x;
+            e2 = fmaf(d, d, e2);
+            x2 = fmaf(x, x, x2);
+            m = fmaxf(m, fabsf(x));
+        }
+        e2 = warp_sum(e2);
+        x2 = warp_sum(x2);
+        const float s = __fdiv_rn(warp_max(m), 127.f);
+        float q2 = 0.f;
+        for (int i = lane * 4; i < D; i += 128) {          // D % 128 == 0: four int8 per lane and step
+            const float4 x = *reinterpret_cast<const float4*>(a + i);
+            const float c0 = quant_i8(x.x, s), c1 = quant_i8(x.y, s), c2 = quant_i8(x.z, s), c3 = quant_i8(x.w, s);
+            char4 o;
+            o.x = (signed char)c0; o.y = (signed char)c1; o.z = (signed char)c2; o.w = (signed char)c3;
+            *reinterpret_cast<char4*>(db8 + r * D + i) = o;
+            const float d0 = fmaf(-s, c0, x.x), d1 = fmaf(-s, c1, x.y), d2 = fmaf(-s, c2, x.z), d3 = fmaf(-s, c3, x.w);
+            q2 = fmaf(d0, d0, fmaf(d1, d1, fmaf(d2, d2, fmaf(d3, d3, q2))));
+        }
+        q2 = warp_sum(q2);
+        if (lane == 0) row_scale[r] = s;
+        e_max = fmaxf(e_max, e2);
+        x_max = fmaxf(x_max, x2);
+        e8_max = fmaxf(e8_max, q2);
+        if (x2 > 0.f) rel_max = fmaxf(rel_max, q2 / x2);
+    }
+    if (lane == 0) {
+        // head room for the order of the fp32 summations above (the int8 residual also for its fmaf rounding)
+        atomicMax(&stats[0], __float_as_uint(e_max * 1.0001f));
+        atomicMax(&stats[1], __float_as_uint(x_max * 1.0001f));
+        atomicMax(&stats[2], __float_as_uint(e8_max * 1.001f));
+        atomicMax(&stats[3], __float_as_uint(rel_max * 1.001f));
+    }
+}
+
+// One warp per query row of the int8 scan's B operand: q ~ s_hi * hi + s_lo * lo with hi = quant(q, s_hi),
+// lo = quant(q - s_hi * hi, s_lo) (two int8 planes: the query's own rounding nearly vanishes from the bound), and the
+// query's certificate bound for |int8-path score - fp32 score| over every row of the shard:
+//     eps = e8 ||q^|| + x ||q - q^||                          (Cauchy-Schwarz on the two rounding residuals)
+//         + 1.25 D 2^-24 x ||q||                               (fp32 accumulation of the exact re-score)
+//         + 8 2^-24 (x + e8) (||s_hi hi|| + ||s_lo lo||)     (s32 -> fp32 conversion and the scale products of the scan)
+// with e8 = max_r ||x_r - s_r x8_r||, x = max_r ||x_r|| (stats).  Rows n_q .. n_pad - 1 of the planes are zero.
+__global__ void __launch_bounds__(32) pack_q_i8_kernel(const float* __restrict__ q32, int n_q, int n_pad, int D, const float* __restrict__ stats,
+                                                       int8_t* __restrict__ q8, float* __restrict__ q_scale, float* __restrict__ q_eps) {
+    const int q = blockIdx.x, lane = threadIdx.x;
+    int8_t* hi_row = q8 + (int64_t)q * D;
+    int8_t* lo_row = q8 + (int64_t)(n_pad + q) * D;
+    if (q >= n_q) {
+        for (int i = lane * 4; i < D; i += 128) {
+            *reinterpret_cast<char4*>(hi_row + i) = make_char4(0, 0, 0, 0);
+            *reinterpret_cast<char4*>(lo_row + i) = make_char4(0, 0, 0, 0);
+        }
+        return;
+    }
+    const float* v = q32 + (int64_t)q * D;
+    float m = 0.f, q2 = 0.f;
+    for (int i = lane; i < D; i += 32) {
+        const float x = v[i];
+        m = fmaxf(m, fabsf(x));
+        q2 = fmaf(x, x, q2);
+    }
+    const float s_hi = __fdiv_rn(warp_max(m), 127.f);
+    float m2 = 0.f;
+    for (int i = lane; i < D; i += 32) m2 = fmaxf(m2, fabsf(fmaf(-s_hi, quant_i8(v[i], s_hi), v[i])));
+    const float s_lo = __fdiv_rn(warp_max(m2), 127.f);
+    float h2 = 0.f, l2 = 0.f, qh2 = 0.f, d2 = 0.f;
+    for (int i = lane * 4; i < D; i += 128) {
+        const float4 x = *reinterpret_cast<const float4*>(v + i);
+        const float xs[4] = {x.x, x.y, x.z, x.w};
+        signed char ho[4], lo[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const float h = quant_i8(xs[j], s_hi);
+            const float r = fmaf(-s_hi, h, xs[j]);
+            const float l = quant_i8(r, s_lo);
+            const float d = fmaf(-s_lo, l, r);                 // q - q^ (the residual's own rounding: within the 1.001 below)
+            const float qh = fmaf(s_lo, l, s_hi * h);
+            ho[j] = (signed char)h;
+            lo[j] = (signed char)l;
+            h2 = fmaf(h, h, h2);
+            l2 = fmaf(l, l, l2);
+            qh2 = fmaf(qh, qh, qh2);
+            d2 = fmaf(d, d, d2);
+        }
+        *reinterpret_cast<char4*>(hi_row + i) = make_char4(ho[0], ho[1], ho[2], ho[3]);
+        *reinterpret_cast<char4*>(lo_row + i) = make_char4(lo[0], lo[1], lo[2], lo[3]);
+    }
+    q2 = warp_sum(q2); h2 = warp_sum(h2); l2 = warp_sum(l2); qh2 = warp_sum(qh2); d2 = warp_sum(d2);
+    if (lane == 0) {
+        const float x_max = sqrtf(stats[1]), e8 = sqrtf(stats[2]);
+        const float u = 5.9604645e-8f;
+        float eps = e8 * sqrtf(qh2) + x_max * sqrtf(d2) + 1.25f * (float)D * u * x_max * sqrtf(q2) +
+                    8.f * u * (x_max + e8) * (s_hi * sqrtf(h2) + s_lo * sqrtf(l2));
+        q_scale[2 * q] = s_hi;
+        q_scale[2 * q + 1] = s_lo;
+        q_eps[q] = eps * 1.001f + 1e-7f;                       // slack for evaluating the bound itself in fp32
+    }
+}
+}  // namespace mdir
+
+extern "C" int mdir_pack_stats_i8(const float* db32, const uint16_t* db16, int64_t n, int D, float* stats, int8_t* db8, float* row_scale,
+                                  void* stream) {
+    MDIR_CHECK_ARG(db32 && db16 && stats && db8 && row_scale && n >= 0 && D > 0 && D % 128 == 0);
+    MDIR_CHECK_ARG((((uintptr_t)db32 | (uintptr_t)db8) & 15) == 0);
+    MDIR_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(float), (cudaStream_t)stream));
+    if (n == 0) return 0;
+    const int64_t blocks = (n + 7) / 8;
+    pack_stats_i8_kernel<<<(unsigned)(blocks < 148 * 8 ? blocks : 148 * 8), 256, 0, (cudaStream_t)stream>>>(
+        db32, reinterpret_cast<const __nv_bfloat16*>(db16), n, D, reinterpret_cast<uint32_t*>(stats), db8, row_scale);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_pack_q_i8(const float* q32, int n_q, int D, const float* stats, int8_t* q8, float* q_scale, float* q_eps, void* stream) {
+    MDIR_CHECK_ARG(q32 && stats && q8 && q_scale && q_eps && n_q >= 1 && n_q <= 128 && D > 0 && D % 128 == 0);
+    MDIR_CHECK_ARG((((uintptr_t)q32 | (uintptr_t)q8) & 15) == 0);
+    const int n_pad = (n_q + 15) & ~15;
+    pack_q_i8_kernel<<<n_pad, 32, 0, (cudaStream_t)stream>>>(q32, n_q, n_pad, D, stats, q8, q_scale, q_eps);
     MDIR_LAUNCH_CHECK();
     return 0;
 }

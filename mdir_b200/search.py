@@ -38,6 +38,20 @@ TARGET_CAND = 4500    # candidates per query the sampling plan aims for (kth * n
 
 STATUS_OVERFLOW, STATUS_UNCERTIFIED, STATUS_PEER_TIMEOUT = 1, 2, 4     # MDIR_STATUS_* (+ the exchange's own bit)
 MAX_KTH = 4096        # deepest selection the finalize kernel stages
+# int8 first pass (Index._i8_route): taken only when every row's int8 residual is small against the row,
+# max_r ||x_r - s_r x8_r|| / ||x_r|| below this.  Unit randn rows at D = 2048 measure 0.013, where the certified bound
+# (~0.013 on unit rows) keeps t - eps above the fused scan's in-kernel threshold for typical queries; a heavy-tailed
+# database (a few dimensions x20) measures several times more and stays on the bf16 first pass.
+I8_MAX_REL_RESIDUAL = 0.02
+# ... and only on shards of at least this many rows.  Both sides of the trade shrink with the shard, but not alike.
+# The scan saves n * D bytes.  The finalize re-scores ~5x as many rows in fp32, and that cost falls more slowly.  The
+# certified reach t - eps also narrows: t, the k-th best score, sits lower in a smaller shard's tail, while the fused
+# scan's threshold (the kth best of one sampled tile per CTA) sits higher, because the sample is a larger share.
+# Measured at D = 2048, 70 queries, top-100 on a B200 (tools/time_i8_shard.py, profiles/r03_i8_shard.log):
+#   125 k rows: int8 uncertified on every query;  250 k rows: 54 / 560 queries uncertified;
+#   500 k / 750 k rows: certified, but 0.424 / 0.525 ms per step against bf16's 0.363 / 0.515;
+#   1 M rows: 0.652 against 0.666.
+I8_MIN_ROWS = 900000
 
 
 def default_shortlist(k):
@@ -106,7 +120,9 @@ class Index:
             self.db32 = v.t().contiguous() if dxn else v
         self._ws = {}
         self._stats = None
-        self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0}
+        self.db8 = self.row_scale = None
+        self.route = None
+        self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0, "int8_blocks": 0, "int8_redone": 0}
 
     @classmethod
     def from_packed(cls, db16, db32=None, idx_base=0):
@@ -118,19 +134,34 @@ class Index:
         self.idx_base = int(idx_base)
         self._ws = {}
         self._stats = None
-        self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0}
+        self.db8 = self.row_scale = None
+        self.route = None
+        self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0, "int8_blocks": 0, "int8_redone": 0}
         return self
 
     def stats(self):
-        """Device float32[2] = {max_r ||bf16(x_r) - x_r||^2, max_r ||x_r||^2}: the database half of the shortlist
-        certificate's error bound (mdir_pack_stats; one pass over the shard, cached)."""
+        """Device float32[4] = {max_r ||bf16(x_r) - x_r||^2, max_r ||x_r||^2, max_r ||x_r - s_r x8_r||^2,
+        max_r ||x_r - s_r x8_r||^2 / ||x_r||^2}: the database half of the shortlist certificate's error bound (one pass
+        over the shard, cached).  When D % 128 == 0 and the shard has at least I8_MIN_ROWS rows the same pass builds the
+        int8 plane of the first pass (db8, row_scale: mdir_pack_stats_i8); it is kept only when the residuals qualify
+        for that route (I8_MAX_REL_RESIDUAL), which is read back to the host here, once per index.  Otherwise the last
+        two entries are 0."""
         if self._stats is None:
             if self.db32 is None:
                 raise _lib.MdirError("the shortlist certificate needs the fp32 master copy (keep_fp32=True)")
-            st = torch.zeros((2,), dtype=torch.float32, device=self.device)
+            st = torch.zeros((4,), dtype=torch.float32, device=self.device)
+            lib = _lib.lib()
             with torch.cuda.device(self.device):
-                _lib.check(_lib.lib().mdir_pack_stats(_lib.ptr(self.db32), _lib.ptr(self.db16), self.n, self.D, _lib.ptr(st), _lib.stream()),
-                           "mdir_pack_stats")
+                if self.D % 128 == 0 and self.n >= I8_MIN_ROWS:
+                    db8 = torch.empty((self.n, self.D), dtype=torch.int8, device=self.device)
+                    rs = torch.empty((self.n,), dtype=torch.float32, device=self.device)
+                    _lib.check(lib.mdir_pack_stats_i8(_lib.ptr(self.db32), _lib.ptr(self.db16), self.n, self.D, _lib.ptr(st), _lib.ptr(db8),
+                                                      _lib.ptr(rs), _lib.stream()), "mdir_pack_stats_i8")
+                    if float(st[3].item()) < I8_MAX_REL_RESIDUAL ** 2:
+                        self.db8, self.row_scale = db8, rs
+                else:
+                    _lib.check(lib.mdir_pack_stats(_lib.ptr(self.db32), _lib.ptr(self.db16), self.n, self.D, _lib.ptr(st), _lib.stream()),
+                               "mdir_pack_stats")
             self._stats = st
         return self._stats
 
@@ -174,6 +205,46 @@ class Index:
             return False
         return 1.25 * kth * n_tiles / (g * g) <= FUSED_CAP_L / 2
 
+    def _i8_route(self, kth, nq):
+        """The int8 first pass (mdir_pack_q_i8 -> mdir_sim_scan_fused_i8 -> mdir_topk_finalize_rescore_eps): half the
+        database bytes of the bf16 scan.  Taken for a certified fp32 search on the one-launch route when the shard
+        has an int8 plane (D % 128 == 0, at least I8_MIN_ROWS rows and small int8 residuals, see stats()).  Its bound is wider than bf16's, so it
+        never widens: a flagged block is redone through the bf16 route (Index._run_block)."""
+        if not (self.certify and self.db32 is not None and self.D % 128 == 0 and self._fused_ok(kth, nq)):
+            return False
+        self.stats()
+        return self.db8 is not None
+
+    def _fused_ws(self):
+        ws = self._ws.get("fused_ws")
+        if ws is None:                       # zeroed once; the kernel re-arms its arrival counters itself
+            ws = torch.zeros((_lib.lib().mdir_sim_scan_fused_workspace_bytes(MAX_Q) // 4,), dtype=torch.int32, device=self.device)
+            self._ws["fused_ws"] = ws
+        return ws
+
+    def _topk_block_i8(self, q32, kth, k_out, out_scores, out_idx, out_keys, ovf):
+        """The certified fp32 top-k_out of one block of <= 128 queries through the int8 first pass: three launches."""
+        lib = _lib.lib()
+        nq = q32.shape[0]
+        n_pad = -(-nq // 16) * 16
+        stats = self.stats()
+        q8 = self._buf("q8", (2 * n_pad, self.D), torch.int8)
+        qsc = self._buf("q8_scale", (nq, 2), torch.float32)
+        qeps = self._buf("q8_eps", (nq,), torch.float32)
+        _lib.check(lib.mdir_pack_q_i8(_lib.ptr(q32), nq, self.D, _lib.ptr(stats), _lib.ptr(q8), _lib.ptr(qsc), _lib.ptr(qeps), _lib.stream()),
+                   "mdir_pack_q_i8")
+        tau, cand, cnt = self._cand_bufs(nq)
+        ws = self._fused_ws()
+        prof = getattr(self, "prof", None)
+        if prof is not None:
+            prof.begin()
+        _lib.check(lib.mdir_sim_scan_fused_i8(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q8), _lib.ptr(qsc), nq, self.D, kth,
+                                              _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                              _lib.stream()), "mdir_sim_scan_fused_i8")
+        if prof is not None:
+            prof.end(self.n * self.D + 4 * self.n)       # int8 rows + their fp32 scales
+        self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, (q32, k_out), caps=(0, FUSED_CAP_L), q_eps=qeps)
+
     def _scan(self, q16, mode, stride, n_sample, dense, dense_ld, tau, cand, cnt):
         # more than 128 queries: one WIDE launch, work items = (tile, 128-query block) -- one kernel ramp, and a database
         # tile comes from HBM once for all the blocks (the tensor-bound regime: DBA, all-pairs)
@@ -187,14 +258,22 @@ class Index:
         return (self._buf("tau", (rows,), torch.int64), self._buf("cand", (rows, CAND_ROW), torch.int64),
                 self._buf("segcnt", (rows, N_SEGS), torch.int32))
 
-    def _finalize(self, cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore=None, caps=(CAP_S, CAP_L)):
-        """rescore = (q32_block, k_out): fused exact fp32 re-scoring of the kth-long bf16 shortlist."""
+    def _finalize(self, cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore=None, caps=(CAP_S, CAP_L), q_eps=None):
+        """rescore = (q32_block, k_out): fused exact fp32 re-scoring of the kth-long bf16 shortlist.
+        q_eps: per-query bounds of the int8 first pass (certified, instead of the bf16 bound)."""
         CAP_S, CAP_L = caps
         CAND_ROW = CAP_S + 148 * CAP_L            # the row stride the scan kernels derive from the two capacities
         if rescore is None:
             _lib.check(_lib.lib().mdir_topk_finalize(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth,
                                                      _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys), _lib.ptr(tau),
                                                      _lib.ptr(ovf), _lib.stream()), "mdir_topk_finalize")
+        elif q_eps is not None:
+            q32, k_out = rescore
+            _lib.check(_lib.lib().mdir_topk_finalize_rescore_eps(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth, k_out,
+                                                                 _lib.ptr(self.db32), self.n, self.idx_base, _lib.ptr(q32), self.D,
+                                                                 _lib.ptr(self.stats()), _lib.ptr(q_eps), _lib.ptr(out_scores), _lib.ptr(out_idx),
+                                                                 _lib.ptr(out_keys), _lib.ptr(tau), _lib.ptr(ovf), _lib.stream()),
+                       "mdir_topk_finalize_rescore_eps")
         else:
             q32, k_out = rescore
             stats = self.stats() if self.certify else None
@@ -226,10 +305,7 @@ class Index:
         tau, cand, cnt = self._cand_bufs(nq)     # the select / fused kernel (re)initialises every segment counter
         prof = getattr(self, "prof", None)       # bench.py: CUDA events around the dominant kernel, on its own stream
         if self._fused_ok(kth, nq):
-            ws = self._ws.get("fused_ws")
-            if ws is None:                       # zeroed once; the kernel re-arms its arrival counters itself
-                ws = torch.zeros((lib.mdir_sim_scan_fused_workspace_bytes(MAX_Q) // 4,), dtype=torch.int32, device=self.device)
-                self._ws["fused_ws"] = ws
+            ws = self._fused_ws()
             if prof is not None:
                 prof.begin()
             _lib.check(lib.mdir_sim_scan_fused_bf16(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, kth, _lib.ptr(tau),
@@ -288,7 +364,7 @@ class Index:
                 raise ValueError("precision must be 'fp32' or 'bf16'")
             if kth > 4096:
                 raise _lib.MdirError("k/shortlist %d too large for the fused path (max 4096); use ranks()" % kth)
-            q16 = pack_bf16(q32)
+            q16 = None                          # bf16 queries: packed on the first block that takes a bf16 route
             out_s = torch.empty((nq_all, k), dtype=torch.float32, device=self.device)
             out_i = torch.empty((nq_all, k), dtype=torch.int32, device=self.device)
             out_k = torch.empty((nq_all, k), dtype=torch.int64, device=self.device) if return_keys else None
@@ -302,6 +378,11 @@ class Index:
                 bk = out_k[q0:q1] if return_keys else None
                 rescore = (q32[q0:q1], k_eff) if precision == "fp32" else None
                 kk = kth if precision == "fp32" else k_eff
+                qb = None                       # None: the int8 first pass (_run_block)
+                if rescore is None or not self._i8_route(kk, nq):
+                    if q16 is None:
+                        q16 = pack_bf16(q32)
+                    qb = q16[q0:q1]
                 if k_eff < k:          # database smaller than k: pad the columns beyond it
                     bs.fill_(float("-inf")); bi.fill_(-1)
                     if bk is not None:
@@ -309,17 +390,32 @@ class Index:
                     tmp_s = torch.empty((nq, k_eff), dtype=torch.float32, device=self.device)
                     tmp_i = torch.empty((nq, k_eff), dtype=torch.int32, device=self.device)
                     tmp_k = torch.empty((nq, k_eff), dtype=torch.int64, device=self.device)
-                    self._run_block(q16[q0:q1], kk, tmp_s, tmp_i, tmp_k, ovf, check, rescore=rescore)
+                    self._run_block(qb, kk, tmp_s, tmp_i, tmp_k, ovf, check, rescore=rescore)
                     bs[:, :k_eff] = tmp_s; bi[:, :k_eff] = tmp_i
                     if bk is not None:
                         bk[:, :k_eff] = tmp_k
                 else:
-                    self._run_block(q16[q0:q1], kk, bs, bi, bk, ovf, check, rescore=rescore)
+                    self._run_block(qb, kk, bs, bi, bk, ovf, check, rescore=rescore)
             if return_keys:
                 return out_s, out_i, out_k
             return out_s, out_i
 
     def _run_block(self, q16, kth, out_s, out_i, out_k, ovf, check, rescore=None):
+        """q16 None: the int8 first pass (Index._i8_route); a block it flags (bit 0 or 1) is redone here through the
+        bf16 route when check=True -- the int8 pass never widens, recovery is the bf16 route's own."""
+        if q16 is None:
+            self.route = "int8"
+            self.cert["int8_blocks"] += 1
+            self._topk_block_i8(rescore[0], kth, rescore[1], out_s, out_i, out_k, ovf)
+            if not check:
+                return
+            st = ovf.cpu()
+            if not bool(st.any()):
+                self.cert["queries"] += int(st.numel())
+                return
+            self.cert["int8_redone"] += 1
+            q16 = pack_bf16(rescore[0])
+        self.route = "bf16"
         self._topk_block(q16, kth, out_s, out_i, out_k, ovf, rescore)
         if not check:
             return
@@ -883,11 +979,15 @@ class GraphedSearch:
             ovf = loc._buf("ovf", (max(nq, 1),), torch.int32)
         finally:
             loc._ws_tag = None
-        ws = loc._ws.get("fused_ws")
-        if ws is None:                           # zeroed once; the kernel re-arms its arrival counters itself
-            ws = torch.zeros((lib.mdir_sim_scan_fused_workspace_bytes(MAX_Q) // 4,), dtype=torch.int32, device=dev)
-            loc._ws["fused_ws"] = ws
-        self.q16 = torch.empty((nq, loc.D), dtype=torch.bfloat16, device=dev)
+        ws = loc._fused_ws()
+        i8 = loc._i8_route(self.kth, nq)         # the same route choice as Index.search
+        if i8:
+            stats = loc.stats()
+            self.q8 = torch.empty((2 * (-(-nq // 16) * 16), loc.D), dtype=torch.int8, device=dev)
+            self.q8_scale = torch.empty((nq, 2), dtype=torch.float32, device=dev)
+            self.q8_eps = torch.empty((nq,), dtype=torch.float32, device=dev)
+        else:
+            self.q16 = torch.empty((nq, loc.D), dtype=torch.bfloat16, device=dev)
         self.keys = torch.empty((nq, k), dtype=torch.int64, device=dev)
         self.local_out = (torch.empty((nq, k), dtype=torch.float32, device=dev), torch.empty((nq, k), dtype=torch.int32, device=dev))
         self.ovf = ovf[:nq]
@@ -898,18 +998,27 @@ class GraphedSearch:
             self.out, self.status = self.local_out, self.ovf
 
         def front():
-            _lib.check(lib.mdir_pack_bf16(_lib.ptr(self.q), nq, loc.D, 0, _lib.ptr(self.q16), _lib.stream()), "mdir_pack_bf16")
+            if i8:
+                _lib.check(lib.mdir_pack_q_i8(_lib.ptr(self.q), nq, loc.D, _lib.ptr(stats), _lib.ptr(self.q8), _lib.ptr(self.q8_scale),
+                                              _lib.ptr(self.q8_eps), _lib.stream()), "mdir_pack_q_i8")
+            else:
+                _lib.check(lib.mdir_pack_bf16(_lib.ptr(self.q), nq, loc.D, 0, _lib.ptr(self.q16), _lib.stream()), "mdir_pack_bf16")
             if prof is not None:
                 prof.begin()
             lib.mdir_tune(1, self.scan_ctas)
             try:
-                _lib.check(lib.mdir_sim_scan_fused_bf16(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
-                                                        loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                        _lib.stream()), "mdir_sim_scan_fused_bf16")
+                if i8:
+                    _lib.check(lib.mdir_sim_scan_fused_i8(_lib.ptr(loc.db8), _lib.ptr(loc.row_scale), loc.n, _lib.ptr(self.q8), _lib.ptr(self.q8_scale),
+                                                          nq, loc.D, self.kth, _lib.ptr(tau), loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0,
+                                                          FUSED_CAP_L, _lib.ptr(ws), _lib.stream()), "mdir_sim_scan_fused_i8")
+                else:
+                    _lib.check(lib.mdir_sim_scan_fused_bf16(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
+                                                            loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                                            _lib.stream()), "mdir_sim_scan_fused_bf16")
             finally:
                 lib.mdir_tune(1, 0)
             if prof is not None:
-                prof.end(loc.n * loc.D * 2)
+                prof.end(loc.n * loc.D + 4 * loc.n if i8 else loc.n * loc.D * 2)
 
         def back():
             chunk = self.fin_chunk if self.fin_chunk > 0 else nq
@@ -919,7 +1028,8 @@ class GraphedSearch:
                 for q0 in range(0, nq, chunk):
                     q1 = min(q0 + chunk, nq)
                     loc._finalize(cand[q0:q1], cnt[q0:q1], q1 - q0, self.kth, self.local_out[0][q0:q1], self.local_out[1][q0:q1],
-                                  self.keys[q0:q1], tau[q0:q1], self.ovf[q0:q1], (self.q[q0:q1], k), caps=(0, FUSED_CAP_L))
+                                  self.keys[q0:q1], tau[q0:q1], self.ovf[q0:q1], (self.q[q0:q1], k), caps=(0, FUSED_CAP_L),
+                                  q_eps=self.q8_eps[q0:q1] if i8 else None)
             finally:
                 lib.mdir_tune(2, 1)
                 lib.mdir_tune(3, 0)
