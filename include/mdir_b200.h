@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define MDIR_ABI_VERSION 2
+#define MDIR_ABI_VERSION 3
 
 #define MDIR_E_ARG      (-1)   /* invalid argument (shape/alignment/range) */
 #define MDIR_E_DRIVER   (-2)   /* driver entry point (cuTensorMapEncodeTiled) unavailable */
@@ -220,6 +220,38 @@ int mdir_sim_scan_tf32(const float* db, int64_t n_db, const float* q, int n_q, i
                        uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* stream);
 int mdir_split_tf32x3(const float* src, int64_t n, int D, int role, float* dst, void* stream);
 
+/* Live-row bitmap of a mutable database: bit (r & 31) of live[r >> 5] set = row r is live.  The _live
+ * variants of the scan and select entry points take it as their last argument before the stream; NULL
+ * means every row is live and is exactly the entry point without the suffix.  A dead row is scored like a
+ * row past the end of the database: it is never appended to a candidate list, SAMPLE / DENSE write -inf for
+ * it, and the fused launch's threshold sample skips it (the threshold is then the kth best of live rows, or
+ * "everything passes" when the sample holds fewer than kth of them: the candidate segments overflow and the
+ * caller's dense recovery answers exactly).  The bitmap covers whole 256-row tiles: ceil(n_db / 256) * 8
+ * words, those past n_db zero (mdir_select_kth_live reads them for the rows past the end of a sample).   */
+int mdir_sim_scan_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D,
+                            int mode, int sample_stride, int n_sample,
+                            float* dense_out, int64_t dense_ld,
+                            const uint64_t* tau, uint32_t idx_base,
+                            uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                            const uint32_t* live, void* stream);
+int mdir_sim_scan_wide_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode,
+                                 int sample_stride, int n_sample, float* dense_out, int64_t dense_ld,
+                                 const uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
+                                 int cap_s, int cap_l, const uint32_t* live, void* stream);
+int mdir_sim_scan_fused_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D,
+                                  int kth, uint64_t* tau, uint32_t idx_base,
+                                  uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                                  void* ws, const uint32_t* live, void* stream);
+int mdir_sim_scan_fused_i8_live(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8,
+                                const float* q_scale, int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base,
+                                uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                                void* ws, const uint32_t* live, void* stream);
+/* Sets (value != 0) or clears the live bits of ids[0 .. n_ids) in one launch (word-level atomics: repeated
+ * ids are harmless).  An id is a row index plus idx_base; ids outside [idx_base, idx_base + capacity) are
+ * ignored, so every shard of a sharded database can be given the same global list.                     */
+int mdir_live_update(uint32_t* live, int64_t capacity, uint32_t idx_base, const int64_t* ids, int64_t n_ids,
+                     int value, void* stream);
+
 /* key helpers exposed for tests: key = (~orderable(score) << 32) | index        */
 uint64_t mdir_make_key(float score, uint32_t index);
 float    mdir_key_score(uint64_t key);
@@ -237,6 +269,12 @@ int mdir_select_kth(const float* scores, int64_t ld, int64_t n, int n_q, int kth
                     int sample_stride, uint32_t idx_base,
                     uint64_t* tau, uint64_t* cand, int64_t cand_row, uint32_t* seg_counts, int n_seg,
                     int cap, int approx, void* stream);
+/* mdir_select_kth over the live rows only (live: see mdir_sim_scan_bf16_live; row = pos_to_idx(i) - idx_base).
+ * Fewer than kth live rows: tau[q] = all ones and every live row is appended.                           */
+int mdir_select_kth_live(const float* scores, int64_t ld, int64_t n, int n_q, int kth,
+                         int sample_stride, uint32_t idx_base,
+                         uint64_t* tau, uint64_t* cand, int64_t cand_row, uint32_t* seg_counts, int n_seg,
+                         int cap, int approx, const uint32_t* live, void* stream);
 
 /* For each query: gather the candidate keys of its n_seg segments (segment 0 holds up to
  * cap0 keys, the others cap_l each), emit the best k as (score fp32, index int32) rows of

@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmdir_b200.so")
 _lib = None
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class ImageDesc(C.Structure):
@@ -45,9 +45,15 @@ PROTOTYPES = {
     "mdir_sim_scan_fused_i8": (_i, [_vp, _vp, _i64, _vp, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp]),
     "mdir_sim_scan_tf32": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp]),
     "mdir_split_tf32x3": (_i, [_vp, _i64, _i, _i, _vp, _vp]),
+    "mdir_sim_scan_bf16_live": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp]),
+    "mdir_sim_scan_wide_bf16_live": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp]),
+    "mdir_sim_scan_fused_bf16_live": (_i, [_vp, _i64, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "mdir_sim_scan_fused_i8_live": (_i, [_vp, _vp, _i64, _vp, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "mdir_live_update": (_i, [_vp, _i64, _u32, _vp, _i64, _i, _vp]),
     "mdir_make_key": (_u64, [_f, _u32]),
     "mdir_key_score": (_f, [_u64]),
     "mdir_select_kth": (_i, [_vp, _i64, _i64, _i, _i, _i, _u32, _vp, _vp, _i64, _vp, _i, _i, _i, _vp]),
+    "mdir_select_kth_live": (_i, [_vp, _i64, _i64, _i, _i, _i, _u32, _vp, _vp, _i64, _vp, _i, _i, _i, _vp, _vp]),
     "mdir_topk_finalize": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_topk_finalize_rescore": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_topk_finalize_rescore_eps": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

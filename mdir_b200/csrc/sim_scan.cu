@@ -160,6 +160,9 @@ struct ScanParams {
     // (rows [0, n_pad) = hi, [n_pad, 2 n_pad) = lo of the B operand)
     const float* row_scale;      // s_r, n_db entries
     const float* q_scale;        // {s_hi, s_lo} per query
+    // live-row bitmap (NULL: every row < n_db is live): bit r & 31 of word r >> 5 set = row r is live.  A dead row
+    // is scored like a row past the end: never a candidate, -inf in the SAMPLE / DENSE outputs, no pass-A key.
+    const uint32_t* live;
 };
 
 constexpr int MDIR_SCAN_FUSED = 3;      // internal mode behind mdir_sim_scan_fused_bf16
@@ -457,6 +460,16 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                     if (row < p.n_db) s_rh[h] = __ldg(p.row_scale + row);
                 }
             }
+            // live bits of this lane's rows in both halves: the 32 rows of a warp and half are one aligned bitmap word, so
+            // this is one broadcast load per warp and half, also issued before the accumulator waits
+            uint32_t live_w[2] = {0xffffffffu, 0xffffffffu};
+            if (p.live) {
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int64_t row0 = (int64_t)tile * kBlockM + h * 128 + quarter * 32;
+                    live_w[h] = row0 < p.n_db ? __ldg(p.live + (row0 >> 5)) : 0u;
+                }
+            }
             // TMEM column of half h of this item's accumulators, and (int8) the barrier slot / phase of that half
             auto acc_col = [&](int h) -> uint32_t {
                 return I8 ? (uint32_t)((2 * it + h) % p.acc_bufs) * (uint32_t)p.acc_stride : (uint32_t)(b * 2 + h) * (uint32_t)p.acc_stride;
@@ -474,7 +487,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) {
                     const int64_t row = (int64_t)tile * kBlockM + h * 128 + quarter * 32 + lane;
-                    const bool row_ok = row < p.n_db;
+                    const bool row_ok = row < p.n_db && (((h ? live_w[1] : live_w[0]) >> lane) & 1u);
                     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc_col(h);
                     const float s_r = h ? s_rh[1] : s_rh[0];
 #pragma unroll 1
@@ -577,7 +590,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
             for (int h = 0; h < 2; ++h) {
                 const int r_in_tile = h * 128 + quarter * 32 + lane;
                 const int64_t row = (int64_t)tile * kBlockM + r_in_tile;
-                const bool row_ok = row < p.n_db;
+                const bool row_in = row < p.n_db;
+                const bool row_ok = row_in && (((h ? live_w[1] : live_w[0]) >> lane) & 1u);      // no dynamic index: no stack
                 if (I8) {
                     const int i = 2 * it + h;
                     mbar_wait(smem_u32(&tmem_full_bar[i % p.acc_bufs]), (uint32_t)(i / p.acc_bufs) & 1u);
@@ -592,7 +606,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                     float v[16];
                     acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qsc, v);
                     if (emode != MDIR_SCAN_FILTER) {
-                        // rows past the end of the database only exist in the compact SAMPLE buffer: mark them -inf
+                        // rows past the end of the database only exist in the compact SAMPLE buffer: mark them -inf, and
+                        // dead rows too
                         if (p.chain > 1) {
                             // chained chunk: running sum of this thread's row in shared memory (column-major, 128 rows
                             // per (half, column): conflict-free); only the last chunk touches dense_out
@@ -609,7 +624,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                                     if (c0 + i < p.n_q)
                                         dense_out[(int64_t)(c0 + i) * p.dense_ld + out_row] = __fadd_rn(sum[i * 128], v[i]);
                             }
-                        } else if (row_ok || p.mode == MDIR_SCAN_SAMPLE) {
+                        } else if (row_in || p.mode == MDIR_SCAN_SAMPLE) {
 #pragma unroll
                             for (int i = 0; i < 16; ++i)
                                 if (c0 + i < nq_here)
@@ -724,7 +739,7 @@ static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, in
                        float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base, uint64_t* cand,
                        uint32_t* seg_counts, int cap_s, int cap_l, void* stream, int k_split = 1, int64_t split_stride = 0,
                        int kth = 0, uint32_t* fused_ws = nullptr, uint64_t* tau_rw = nullptr, int n_q_total = 0,
-                       const float* row_scale = nullptr, const float* q_scale = nullptr) {
+                       const float* row_scale = nullptr, const float* q_scale = nullptr, const uint32_t* live = nullptr) {
     const bool tf32 = kind == kKindTf32, i8 = kind == kKindI8;
     const int esz = tf32 ? 4 : (i8 ? 1 : 2);
     MDIR_CHECK_ARG(db && q && n_db >= 1 && n_q >= 1 && n_q <= kMaxN && D >= 16 / esz && (D % (16 / esz)) == 0);
@@ -732,9 +747,11 @@ static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, in
     MDIR_CHECK_ARG(mode >= 0 && mode <= MDIR_SCAN_FUSED);
     MDIR_CHECK_ARG(n_db + (int64_t)idx_base <= ((int64_t)1 << 32));
     MDIR_CHECK_ARG(!i8 || (mode == MDIR_SCAN_FUSED && row_scale && q_scale));
+    MDIR_CHECK_ARG(!live || !tf32);
     ScanParams p;
     p.row_scale = row_scale;
     p.q_scale = q_scale;
+    p.live = live;
     p.n_db = n_db;
     p.n_q = n_q;
     p.n_pad = (n_q + 15) & ~15;
@@ -894,11 +911,18 @@ static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, in
     return 0;
 }
 
+extern "C" int mdir_sim_scan_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
+                                       int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
+                                       uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, const uint32_t* live, void* stream) {
+    return launch_scan(kKindBf16, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+                       cap_s, cap_l, stream, 1, 0, 0, nullptr, nullptr, 0, nullptr, nullptr, live);
+}
+
 extern "C" int mdir_sim_scan_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
                                   int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
                                   uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* stream) {
-    return launch_scan(kKindBf16, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
-                       cap_s, cap_l, stream);
+    return mdir_sim_scan_bf16_live(db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+                                   cap_s, cap_l, nullptr, stream);
 }
 
 extern "C" int mdir_sim_scan_dense_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, float* dense_out, int64_t dense_ld,
@@ -911,34 +935,54 @@ extern "C" int mdir_sim_scan_dense_bf16(const uint16_t* db, int64_t n_db, const 
                        nullptr, nullptr, n_q > blk ? n_q : 0);
 }
 
-extern "C" int mdir_sim_scan_wide_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
-                                       int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
-                                       uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* stream) {
+extern "C" int mdir_sim_scan_wide_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
+                                            int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
+                                            uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, const uint32_t* live, void* stream) {
     // mdir_sim_scan_bf16 for 129 .. 1024 queries in one launch (DENSE: any number): blocks of 128 queries per work item
     MDIR_CHECK_ARG(n_q >= 1 && (mode == MDIR_SCAN_DENSE || n_q <= kMaxWideQ));
     const int blk = n_q < 128 ? n_q : 128;
     return launch_scan(kKindBf16, db, n_db, q, blk, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts, cap_s,
-                       cap_l, stream, 1, 0, 0, nullptr, nullptr, n_q > blk ? n_q : 0);
+                       cap_l, stream, 1, 0, 0, nullptr, nullptr, n_q > blk ? n_q : 0, nullptr, nullptr, live);
+}
+
+extern "C" int mdir_sim_scan_wide_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
+                                       int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
+                                       uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* stream) {
+    return mdir_sim_scan_wide_bf16_live(db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+                                        cap_s, cap_l, nullptr, stream);
 }
 
 extern "C" size_t mdir_sim_scan_fused_workspace_bytes(int n_q) {
     return (4 + (size_t)(n_q > 0 ? n_q : 0) * kNumSMs * 16) * sizeof(uint32_t);
 }
 
+extern "C" int mdir_sim_scan_fused_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int kth, uint64_t* tau,
+                                             uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* ws,
+                                             const uint32_t* live, void* stream) {
+    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0);
+    return launch_scan(kKindBf16, db, n_db, q, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
+                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, nullptr, nullptr, live);
+}
+
 extern "C" int mdir_sim_scan_fused_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int kth, uint64_t* tau,
                                         uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* ws,
                                         void* stream) {
-    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0);
-    return launch_scan(kKindBf16, db, n_db, q, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
-                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau);
+    return mdir_sim_scan_fused_bf16_live(db, n_db, q, n_q, D, kth, tau, idx_base, cand, seg_counts, cap_s, cap_l, ws, nullptr, stream);
+}
+
+extern "C" int mdir_sim_scan_fused_i8_live(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8, const float* q_scale,
+                                           int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
+                                           int cap_s, int cap_l, void* ws, const uint32_t* live, void* stream) {
+    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0 && D % 128 == 0);
+    return launch_scan(kKindI8, db8, n_db, q8, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
+                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, row_scale, q_scale, live);
 }
 
 extern "C" int mdir_sim_scan_fused_i8(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8, const float* q_scale,
                                       int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
                                       int cap_s, int cap_l, void* ws, void* stream) {
-    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0 && D % 128 == 0);
-    return launch_scan(kKindI8, db8, n_db, q8, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
-                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, row_scale, q_scale);
+    return mdir_sim_scan_fused_i8_live(db8, row_scale, n_db, q8, q_scale, n_q, D, kth, tau, idx_base, cand, seg_counts, cap_s, cap_l, ws,
+                                       nullptr, stream);
 }
 
 extern "C" int mdir_sim_scan_tf32(const float* db, int64_t n_db, const float* q, int n_q, int D, int mode, int sample_stride,

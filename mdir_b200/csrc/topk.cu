@@ -14,6 +14,15 @@ __device__ __forceinline__ uint32_t sample_pos_to_idx(int64_t i, int sample_stri
     return idx_base + (uint32_t)(j * sample_stride * MDIR_SCAN_TILE_ROWS + r);
 }
 
+// Whether score position i < n of a selection row is a live database row (live == NULL: every row is).  The bitmap
+// covers whole 256-row tiles (mdir_select_kth_live), so the rows past the end of a compact sample's last tile read
+// zero words and are dead too: a dead row is neither counted nor appended, even when fewer than kth rows are live.
+__device__ __forceinline__ bool pos_live(const uint32_t* live, int64_t i, int sample_stride) {
+    if (!live) return true;
+    const uint32_t r = sample_pos_to_idx(i, sample_stride, 0u);
+    return (__ldg(live + (r >> 5)) >> (r & 31)) & 1u;
+}
+
 // kth smallest (1-based) of ONE 32-bit value per thread of a 1024-thread block (4 radix passes of
 // one element each).  Used to bound the selection: the kth smallest of the per-thread minima is an
 // upper bound B of the kth smallest key overall, so only the few keys <= B take part in the real
@@ -59,7 +68,7 @@ __device__ __forceinline__ uint32_t block_kth_of_thread_values(uint32_t val, uin
 __global__ void __launch_bounds__(1024) select_kth_kernel(const float* __restrict__ scores, int64_t ld, int64_t n, int kth,
                                                           int sample_stride, uint32_t idx_base, uint64_t* __restrict__ tau,
                                                           uint64_t* __restrict__ cand, int64_t cand_row, uint32_t* __restrict__ seg_counts,
-                                                          int n_seg, int cap) {
+                                                          int n_seg, int cap, const uint32_t* __restrict__ live) {
     __shared__ uint32_t hist[256];
     __shared__ uint32_t s_prefix;
     __shared__ uint32_t s_k;
@@ -85,8 +94,10 @@ __global__ void __launch_bounds__(1024) select_kth_kernel(const float* __restric
                     v[u] = i < n ? __ldg(sc + i) : 0.f;
                 }
 #pragma unroll
-                for (int u = 0; u < 8; ++u)
-                    if (base + u * 1024 + threadIdx.x < n) mymin = min(mymin, desc_key(v[u]));
+                for (int u = 0; u < 8; ++u) {
+                    const int64_t i = base + u * 1024 + threadIdx.x;
+                    if (i < n && pos_live(live, i, sample_stride)) mymin = min(mymin, desc_key(v[u]));
+                }
             }
             bound = block_kth_of_thread_values(mymin, (uint32_t)kth, hist, &s_prefix, &s_k);
         }
@@ -108,7 +119,7 @@ __global__ void __launch_bounds__(1024) select_kth_kernel(const float* __restric
 #pragma unroll
                 for (int u = 0; u < 8; ++u) {
                     const int64_t i = base + u * 1024 + threadIdx.x;
-                    const bool valid = i < n;
+                    const bool valid = i < n && pos_live(live, i, sample_stride);
                     const uint32_t key = desc_key(v[u]);
                     const bool hit = valid && key <= bound && ((key & himask) == prefix);
                     if (__any_sync(0xffffffffu, hit)) {
@@ -144,7 +155,7 @@ __global__ void __launch_bounds__(1024) select_kth_kernel(const float* __restric
                 const uint32_t himask = pass == 0 ? 0u : (0xffffffffu << (shift + 8));
                 for (int64_t base = 0; base < n_round; base += 1024) {
                     const int64_t i = base + threadIdx.x;
-                    const bool valid = i < n;
+                    const bool valid = i < n && pos_live(live, i, sample_stride);
                     const float v = valid ? __ldg(sc + i) : 0.f;
                     const uint32_t idx = sample_pos_to_idx(valid ? i : 0, sample_stride, idx_base);
                     const bool hit = valid && (desc_key(v) == result) && ((idx & himask) == prefix);
@@ -183,7 +194,7 @@ __global__ void __launch_bounds__(1024) select_kth_kernel(const float* __restric
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
                 const int64_t i = base + u * 1024 + threadIdx.x;
-                if (i < n && desc_key(v[u]) <= result) {
+                if (i < n && desc_key(v[u]) <= result && pos_live(live, i, sample_stride)) {
                     const uint64_t key = make_key(v[u], sample_pos_to_idx(i, sample_stride, idx_base));
                     if (key <= tau_key) {
                         const uint32_t pos = atomicAdd(&s_n, 1u);
@@ -203,7 +214,8 @@ __global__ void __launch_bounds__(1024) select_kth_kernel(const float* __restric
 __global__ void __launch_bounds__(1024, 1) select_kth_reg_kernel(const float* __restrict__ scores, int64_t ld, int n, int kth,
                                                                  int sample_stride, uint32_t idx_base, uint64_t* __restrict__ tau,
                                                                  uint64_t* __restrict__ cand, int64_t cand_row,
-                                                                 uint32_t* __restrict__ seg_counts, int n_seg, int cap, int approx) {
+                                                                 uint32_t* __restrict__ seg_counts, int n_seg, int cap, int approx,
+                                                                 const uint32_t* __restrict__ live) {
     __shared__ uint32_t hist[256];
     __shared__ uint32_t s_prefix, s_k, s_n, s_ties;
     const int q = blockIdx.x;
@@ -213,8 +225,11 @@ __global__ void __launch_bounds__(1024, 1) select_kth_reg_kernel(const float* __
 #pragma unroll
     for (int u = 0; u < 32; ++u) {
         const int i = u * 1024 + threadIdx.x;
-        key[u] = i < n ? desc_key(__ldg(sc + i)) : 0xffffffffu;     // padding sorts last (and is never valid)
+        key[u] = i < n && pos_live(live, i, sample_stride) ? desc_key(__ldg(sc + i)) : 0xffffffffu;     // padding sorts last (and is never valid)
     }
+    // position u * 1024 + threadIdx.x takes part: with a bitmap, dead rows carry the all-ones key (so does a NaN score,
+    // which ranks last anyway), which keeps the kernel within its 64 registers instead of a separate validity mask
+    auto valid = [&](int u) { return live ? key[u] != 0xffffffffu : u * 1024 + (int)threadIdx.x < n; };
     uint32_t result = 0xffffffffu, idx_limit = 0xffffffffu;
     if (kth <= n) {
         uint32_t bound = 0xffffffffu;
@@ -222,7 +237,7 @@ __global__ void __launch_bounds__(1024, 1) select_kth_reg_kernel(const float* __
             uint32_t mymin = 0xffffffffu;
 #pragma unroll
             for (int u = 0; u < 32; ++u)
-                if (u * 1024 + (int)threadIdx.x < n) mymin = min(mymin, key[u]);
+                if (valid(u)) mymin = min(mymin, key[u]);
             bound = block_kth_of_thread_values(mymin, (uint32_t)kth, hist, &s_prefix, &s_k);
         }
         // approx: the bound itself is a valid threshold (>= kth keys are <= it, typically ~7 % more than kth)
@@ -237,8 +252,7 @@ __global__ void __launch_bounds__(1024, 1) select_kth_reg_kernel(const float* __
             const uint32_t himask = pass == 0 ? 0u : (0xffffffffu << (shift + 8));
 #pragma unroll
             for (int u = 0; u < 32; ++u) {
-                const bool valid = u * 1024 + (int)threadIdx.x < n;
-                const bool hit = valid && key[u] <= bound && ((key[u] & himask) == prefix);
+                const bool hit = valid(u) && key[u] <= bound && ((key[u] & himask) == prefix);
                 if (__any_sync(0xffffffffu, hit)) {
                     const int d = (int)((key[u] >> shift) & 0xffu);
                     const unsigned peers = match_digit8(d, hit);
@@ -271,7 +285,7 @@ __global__ void __launch_bounds__(1024, 1) select_kth_reg_kernel(const float* __
                 for (int u = 0; u < 32; ++u) {
                     const int i = u * 1024 + threadIdx.x;
                     const uint32_t idx = sample_pos_to_idx(i, sample_stride, idx_base);
-                    const bool hit = i < n && key[u] == result && ((idx & himask) == prefix);
+                    const bool hit = valid(u) && key[u] == result && ((idx & himask) == prefix);
                     if (__any_sync(0xffffffffu, hit)) {
                         const int d = (int)((idx >> shift) & 0xffu);
                         const unsigned peers = match_digit8(d, hit);
@@ -300,7 +314,7 @@ __global__ void __launch_bounds__(1024, 1) select_kth_reg_kernel(const float* __
 #pragma unroll
         for (int u = 0; u < 32; ++u) {
             const int i = u * 1024 + threadIdx.x;
-            if (i < n && key[u] <= result) {
+            if (valid(u) && key[u] <= result) {
                 // key = (desc_key(score) << 32) | idx: the upper half is exactly the register key
                 const uint64_t k64 = ((uint64_t)key[u] << 32) | (uint64_t)sample_pos_to_idx(i, sample_stride, idx_base);
                 if (k64 <= tau_key) {
@@ -942,20 +956,53 @@ using namespace mdir;
 extern "C" uint64_t mdir_make_key(float score, uint32_t index) { return make_key(score, index); }
 extern "C" float mdir_key_score(uint64_t key) { return key_score(key); }
 
-extern "C" int mdir_select_kth(const float* scores, int64_t ld, int64_t n, int n_q, int kth, int sample_stride,
-                               uint32_t idx_base, uint64_t* tau, uint64_t* cand, int64_t cand_row, uint32_t* seg_counts, int n_seg,
-                               int cap, int approx, void* stream) {
+extern "C" int mdir_select_kth_live(const float* scores, int64_t ld, int64_t n, int n_q, int kth, int sample_stride,
+                                    uint32_t idx_base, uint64_t* tau, uint64_t* cand, int64_t cand_row, uint32_t* seg_counts, int n_seg,
+                                    int cap, int approx, const uint32_t* live, void* stream) {
     MDIR_CHECK_ARG(scores && tau && n >= 0 && n_q >= 0 && kth >= 1 && ld >= n);
     MDIR_CHECK_ARG(cand == nullptr || (seg_counts != nullptr && cap >= 1 && n_seg >= 1 && cand_row >= cap));
     if (n_q == 0) return 0;
     if (n <= 32 * 1024) {
         select_kth_reg_kernel<<<n_q, 1024, 0, (cudaStream_t)stream>>>(scores, ld, (int)n, kth, sample_stride, idx_base, tau, cand,
-                                                                      cand_row, seg_counts, n_seg, cap, approx);
+                                                                      cand_row, seg_counts, n_seg, cap, approx, live);
         MDIR_LAUNCH_CHECK();
         return 0;
     }
     select_kth_kernel<<<n_q, 1024, 0, (cudaStream_t)stream>>>(scores, ld, n, kth, sample_stride, idx_base, tau, cand, cand_row,
-                                                              seg_counts, n_seg, cap);
+                                                              seg_counts, n_seg, cap, live);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_select_kth(const float* scores, int64_t ld, int64_t n, int n_q, int kth, int sample_stride,
+                               uint32_t idx_base, uint64_t* tau, uint64_t* cand, int64_t cand_row, uint32_t* seg_counts, int n_seg,
+                               int cap, int approx, void* stream) {
+    return mdir_select_kth_live(scores, ld, n, n_q, kth, sample_stride, idx_base, tau, cand, cand_row, seg_counts, n_seg, cap, approx,
+                                nullptr, stream);
+}
+
+// Sets (value != 0) or clears bit id - idx_base of the live bitmap for every id of the list; ids outside
+// [idx_base, idx_base + capacity) are ignored, so every shard can be handed the same global list.  Word-level atomics:
+// duplicates and ids sharing a word are safe in one launch.
+namespace mdir {
+__global__ void __launch_bounds__(256) live_update_kernel(uint32_t* __restrict__ live, int64_t capacity, uint32_t idx_base,
+                                                          const int64_t* __restrict__ ids, int64_t n_ids, int value) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_ids) return;
+    const int64_t r = ids[i] - (int64_t)idx_base;
+    if (r < 0 || r >= capacity) return;
+    const uint32_t bit = 1u << (uint32_t)(r & 31);
+    if (value) atomicOr(live + (r >> 5), bit);
+    else atomicAnd(live + (r >> 5), ~bit);
+}
+}  // namespace mdir
+
+extern "C" int mdir_live_update(uint32_t* live, int64_t capacity, uint32_t idx_base, const int64_t* ids, int64_t n_ids, int value,
+                                void* stream) {
+    MDIR_CHECK_ARG(live && capacity >= 0 && n_ids >= 0 && (ids || n_ids == 0));
+    if (n_ids == 0) return 0;
+    MDIR_CHECK_ARG((n_ids + 255) / 256 <= 0x7fffffff);
+    live_update_kernel<<<(unsigned)((n_ids + 255) / 256), 256, 0, (cudaStream_t)stream>>>(live, capacity, idx_base, ids, n_ids, value);
     MDIR_LAUNCH_CHECK();
     return 0;
 }

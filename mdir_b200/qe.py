@@ -62,6 +62,7 @@ def dba(index, alpha=3.0, k_dba=10, rows=None):
     rows: augment only the first `rows` rows (the others are copied unchanged) -- bounded benchmarks."""
     if index.db32 is None:
         raise _lib.MdirError("DBA needs the fp32 master copy (keep_fp32=True)")
+    index._require_all_live("qe.dba()")
     n_aug = index.n if rows is None else min(int(rows), index.n)
     out = torch.empty_like(index.db32) if n_aug == index.n else index.db32.clone()
     for r0 in range(0, n_aug, DBA_BLOCK):
@@ -81,6 +82,7 @@ def dba_sharded(sharded, alpha=3.0, k_dba=10):
     local = sharded.local
     if local.db32 is None:
         raise _lib.MdirError("DBA needs the fp32 master copy (keep_fp32=True)")
+    local._require_all_live("qe.dba_sharded()")
     world = sharded.world
     if world == 1:
         out = dba(local, alpha, k_dba)

@@ -9,12 +9,16 @@ Replaces, for mdir's evaluation (mdir/components/optim/score/cirscore.py:65-70):
 * ``Index``                  -- a database resident in HBM as row-major bf16 (+ optional fp32
                                 master for exact re-scoring); ``search`` = tcgen05 scan with the
                                 top-k selection fused into the epilogue, ``scores`` / ``ranks``
-                                = the dense path.
+                                = the dense path.  Rows can be removed, restored and appended in
+                                place (``remove`` / ``restore`` / ``add``: a live-row bitmap the
+                                scan reads).
 * ``ShardedIndex``           -- rows sharded contiguously over the ranks of a torch.distributed
                                 group; local top-k + one all-gather of N_q*k keys + merge.
 * ``ranks_from_scores`` / ``topk_from_scores`` -- the sort/selection kernels fed an existing
                                 (N_db, N_q) score matrix (bit-exact vs the stable argsort).
 """
+import contextlib
+
 import numpy as np
 import torch
 
@@ -82,8 +86,9 @@ def _as_dev_f32(x, device):
     return x.contiguous()
 
 
-def pack_bf16(x, dxn=False):
-    """x fp32 cuda: (n, D) rows, or with dxn=True the reference's (D, n) -> (n, D) bf16 rows."""
+def pack_bf16(x, dxn=False, out=None):
+    """x fp32 cuda: (n, D) rows, or with dxn=True the reference's (D, n) -> (n, D) bf16 rows.
+    out: the first n rows of a preallocated contiguous (>= n, D) bf16 tensor to write (default: a new one)."""
     _lib.require_cuda(x, "descriptors")
     x = x.contiguous()
     if dxn:
@@ -92,32 +97,89 @@ def pack_bf16(x, dxn=False):
         n, D = x.shape
     if D % 8:
         raise _lib.MdirError("descriptor dimension must be a multiple of 8 (got %d)" % D)
-    out = torch.empty((n, D), dtype=torch.bfloat16, device=x.device)
+    if out is None:
+        out = torch.empty((n, D), dtype=torch.bfloat16, device=x.device)
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().mdir_pack_bf16(_lib.ptr(x), n, D, 1 if dxn else 0, _lib.ptr(out), _lib.stream()), "mdir_pack_bf16")
     return out
 
 
+def check_ids(ids, lo, hi):
+    """ids (host or device tensor, numpy array or sequence of integers) -> int64 numpy rows ids - lo; MdirError when
+    an id lies outside [lo, hi).  The host-side validation of Index.remove / restore."""
+    if isinstance(ids, torch.Tensor):
+        ids = ids.detach().cpu().numpy()
+    a = np.asarray(ids)
+    if a.size and not np.issubdtype(a.dtype, np.integer):
+        raise _lib.MdirError("ids must be integers (got %s)" % a.dtype)
+    a = a.astype(np.int64).ravel()
+    bad = (a < lo) | (a >= hi)
+    if bad.any():
+        raise _lib.MdirError("id %d is outside this index's ids [%d, %d)" % (int(a[bad][0]), lo, hi))
+    return a - lo
+
+
+def ids_for_rank(ids, ranges, rank):
+    """Global ids -> the int64 numpy ids that rank `rank` owns, ranges[r] = (first id, end id) of rank r (see
+    ShardedIndex.shard_bounds).  MdirError when an id lies in no rank's range."""
+    if isinstance(ids, torch.Tensor):
+        ids = ids.detach().cpu().numpy()
+    a = np.asarray(ids)
+    if a.size and not np.issubdtype(a.dtype, np.integer):
+        raise _lib.MdirError("ids must be integers (got %s)" % a.dtype)
+    a = a.astype(np.int64).ravel()
+    owned = np.zeros(a.shape, dtype=bool)
+    for lo, hi in ranges:
+        owned |= (a >= lo) & (a < hi)
+    if not owned.all():
+        raise _lib.MdirError("id %d is outside every shard of this index" % int(a[~owned][0]))
+    lo, hi = ranges[rank]
+    return a[(a >= lo) & (a < hi)]
+
+
 class Index:
-    """A (shard of a) descriptor database on one GPU."""
+    """A (shard of a) descriptor database on one GPU.
+
+    Mutable in place: ``remove(ids)`` hides rows from every later search, ``restore(ids)`` undoes that, and
+    ``add(vecs)`` writes new rows into free slots of a ``capacity`` larger than the initial database.  An id is
+    idx_base + slot; slots are never reused, so an id names one row for the life of the index.  Which rows are live
+    is one bitmap on the device (1 bit per slot) that every top-k route reads in the scan epilogue; CUDA graphs
+    captured over the index see every later mutation without re-capture.  The scan covers all ``capacity`` slots:
+    free and removed slots cost scan bandwidth like live rows."""
 
     fused = True      # allow the one-launch threshold + filter route (False: always sample -> select -> filter)
     certify = True    # precision="fp32": prove the shortlist complete (status bit 2 + widening when it cannot be)
     _sms = None
 
-    def __init__(self, vecs, dxn=False, device="cuda", keep_fp32=True, idx_base=0):
+    def __init__(self, vecs, dxn=False, device="cuda", keep_fp32=True, idx_base=0, capacity=None):
         """vecs: (n, D) fp32 rows (torch/numpy, host or device), or (D, n) with dxn=True
-        (the layout extract_vectors returns, cirtorch/networks/imageretrievalnet.py:291)."""
+        (the layout extract_vectors returns, cirtorch/networks/imageretrievalnet.py:291).
+        capacity (default n): slots allocated for rows; add() fills slots n, n + 1, ...  With capacity > n the bf16
+        rows, the fp32 master (a copy of vecs) and, once built, the int8 plane are allocated at capacity, the free
+        slots zero.  Every slot is scanned, free ones included.  idx_base + capacity must stay <= 2**32."""
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise _lib.MdirError("Index needs a CUDA device (no CPU path)")
         v = _as_dev_f32(vecs, self.device)
-        self.db16 = pack_bf16(v, dxn=dxn)
-        self.n, self.D = self.db16.shape
-        self.idx_base = int(idx_base)
-        self.db32 = None
-        if keep_fp32:
-            self.db32 = v.t().contiguous() if dxn else v
+        n, D = (v.shape[1], v.shape[0]) if dxn else (v.shape[0], v.shape[1])
+        cap = n if capacity is None else int(capacity)
+        if cap < n:
+            raise _lib.MdirError("capacity %d is smaller than the %d rows given" % (cap, n))
+        if int(idx_base) < 0 or int(idx_base) + cap > 1 << 32:
+            raise _lib.MdirError("idx_base + capacity must stay within [0, 2**32]")
+        with torch.cuda.device(self.device):
+            db16 = torch.zeros((cap, D), dtype=torch.bfloat16, device=self.device) if cap > n else None
+            self.db16 = pack_bf16(v, dxn=dxn, out=db16)
+            self.n, self.D = self.db16.shape
+            self.idx_base = int(idx_base)
+            self.db32 = None
+            if keep_fp32:
+                if cap == n:
+                    self.db32 = v.t().contiguous() if dxn else v
+                else:
+                    self.db32 = torch.zeros((cap, D), dtype=torch.float32, device=self.device)
+                    self.db32[:n].copy_(v.t() if dxn else v)
+            self._init_live(n)
         self._ws = {}
         self._stats = None
         self.db8 = self.row_scale = None
@@ -132,12 +194,110 @@ class Index:
         self.n, self.D = db16.shape
         self.db32 = db32
         self.idx_base = int(idx_base)
+        with torch.cuda.device(self.device):
+            self._init_live(self.n)
         self._ws = {}
         self._stats = None
         self.db8 = self.row_scale = None
         self.route = None
         self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0, "int8_blocks": 0, "int8_redone": 0}
         return self
+
+    # ------------------------------------------------------------------ live rows
+    def _init_live(self, n_used):
+        """The live bitmap: bit s & 31 of word s >> 5 = slot s is live; ones for the n_used filled slots, zeros for the
+        free tail.  It covers whole 256-row scan tiles (the select kernel reads the words of a sample's last tile past
+        the end) and is modified only in place, so a captured graph keeps reading the current version."""
+        words = -(-self.n // TILE) * (TILE // 32)
+        bits = np.zeros(words * 32, dtype=bool)
+        bits[:n_used] = True
+        host = np.packbits(bits, bitorder="little").view("<u4").view(np.int32)
+        self.live = torch.from_numpy(host.copy()).to(self.device)
+        self._live_host = bits[:self.n].copy()     # host mirror: id validation and n_live without a device read-back
+        self._n_used = int(n_used)
+
+    @property
+    def n_live(self):
+        """Number of live rows (filled and not removed)."""
+        return int(self._live_host.sum())
+
+    def _require_all_live(self, what):
+        if self.n_live != self.n:
+            raise _lib.MdirError("%s scores every slot and does not support an index with removed rows or free capacity "
+                                 "(%d of %d slots live); use search()" % (what, self.n_live, self.n))
+
+    def _set_live(self, rows, value):
+        rows = np.unique(rows)
+        rows = rows[self._live_host[rows] != bool(value)]          # repeated and no-op ids cost nothing
+        if rows.size == 0:
+            return
+        ids = torch.from_numpy(rows + self.idx_base).to(self.device)
+        _lib.check(_lib.lib().mdir_live_update(_lib.ptr(self.live), self.n, self.idx_base, _lib.ptr(ids), int(rows.size), int(value),
+                                               _lib.stream()), "mdir_live_update")
+        self._live_host[rows] = bool(value)
+
+    def remove(self, ids):
+        """Hide the rows with these ids (idx_base + slot) from every later search.  Stream-ordered on the current stream;
+        removing a removed id is a no-op; an id outside this index raises MdirError."""
+        rows = check_ids(ids, self.idx_base, self.idx_base + self.n)
+        with torch.cuda.device(self.device):
+            self._set_live(rows, 0)
+
+    def restore(self, ids):
+        """Undo remove() for these ids (the rows' data never left their slots).  An id of a slot that add() never
+        filled, or outside this index, raises MdirError."""
+        rows = check_ids(ids, self.idx_base, self.idx_base + self.n)
+        if rows.size and int(rows.max()) >= self._n_used:
+            raise _lib.MdirError("id %d names a slot that was never filled" % (int(rows.max()) + self.idx_base))
+        with torch.cuda.device(self.device):
+            self._set_live(rows, 1)
+
+    def add(self, vecs):
+        """Append (m, D) fp32 rows to the next free slots; returns their ids (idx_base + slot, int64 host tensor).
+        In stream order: bf16 rows, fp32 master rows, int8 rows + certificate stats (when built), then the live bits,
+        so a search queued after this call sees the new rows and one queued before it does not.  New rows can only
+        widen the certificate's bounds: the first-pass route chosen earlier stays and stays exact.  MdirError when the
+        rows do not fit the capacity."""
+        lib = _lib.lib()
+        with torch.cuda.device(self.device):
+            v = _as_dev_f32(vecs, self.device)
+            if v.dim() != 2 or v.shape[1] != self.D:
+                raise _lib.MdirError("add() expects (m, %d) rows, got %s" % (self.D, tuple(v.shape)))
+            m, s0 = int(v.shape[0]), self._n_used
+            if s0 + m > self.n:
+                raise _lib.MdirError("index is full: %d free slots, %d rows given" % (self.n - s0, m))
+            if m == 0:
+                return torch.empty((0,), dtype=torch.int64)
+            s1 = s0 + m
+            pack_bf16(v, out=self.db16[s0:s1])
+            if self.db32 is not None:
+                self.db32[s0:s1].copy_(v)
+            if self._stats is not None:
+                # the stats of the new rows merged into the live ones by max: the same values as one pass over every row
+                st = torch.zeros((4,), dtype=torch.float32, device=self.device)
+                if self.db8 is not None:
+                    _lib.check(lib.mdir_pack_stats_i8(_lib.ptr(self.db32[s0:s1]), _lib.ptr(self.db16[s0:s1]), m, self.D, _lib.ptr(st),
+                                                      _lib.ptr(self.db8[s0:s1]), _lib.ptr(self.row_scale[s0:s1]), _lib.stream()),
+                               "mdir_pack_stats_i8")
+                else:
+                    _lib.check(lib.mdir_pack_stats(_lib.ptr(self.db32[s0:s1]), _lib.ptr(self.db16[s0:s1]), m, self.D, _lib.ptr(st),
+                                                   _lib.stream()), "mdir_pack_stats")
+                torch.maximum(self._stats, st, out=self._stats)
+            self._n_used = s1
+            self._set_live(np.arange(s0, s1, dtype=np.int64), 1)
+            return torch.arange(self.idx_base + s0, self.idx_base + s1, dtype=torch.int64)
+
+    @contextlib.contextmanager
+    def _live_version(self, live):
+        """Searches inside the block read `live` (an earlier copy of the bitmap) instead of the current one."""
+        if live is None:
+            yield
+            return
+        cur, self.live = self.live, live
+        try:
+            yield
+        finally:
+            self.live = cur
 
     def stats(self):
         """Device float32[4] = {max_r ||bf16(x_r) - x_r||^2, max_r ||x_r||^2, max_r ||x_r - s_r x8_r||^2,
@@ -238,9 +398,9 @@ class Index:
         prof = getattr(self, "prof", None)
         if prof is not None:
             prof.begin()
-        _lib.check(lib.mdir_sim_scan_fused_i8(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q8), _lib.ptr(qsc), nq, self.D, kth,
-                                              _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                              _lib.stream()), "mdir_sim_scan_fused_i8")
+        _lib.check(lib.mdir_sim_scan_fused_i8_live(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q8), _lib.ptr(qsc), nq, self.D,
+                                                   kth, _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                                   _lib.ptr(self.live), _lib.stream()), "mdir_sim_scan_fused_i8_live")
         if prof is not None:
             prof.end(self.n * self.D + 4 * self.n)       # int8 rows + their fp32 scales
         self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, (q32, k_out), caps=(0, FUSED_CAP_L), q_eps=qeps)
@@ -248,10 +408,10 @@ class Index:
     def _scan(self, q16, mode, stride, n_sample, dense, dense_ld, tau, cand, cnt):
         # more than 128 queries: one WIDE launch, work items = (tile, 128-query block) -- one kernel ramp, and a database
         # tile comes from HBM once for all the blocks (the tensor-bound regime: DBA, all-pairs)
-        fn = _lib.lib().mdir_sim_scan_wide_bf16 if q16.shape[0] > MAX_Q else _lib.lib().mdir_sim_scan_bf16
+        fn = _lib.lib().mdir_sim_scan_wide_bf16_live if q16.shape[0] > MAX_Q else _lib.lib().mdir_sim_scan_bf16_live
         _lib.check(fn(_lib.ptr(self.db16), self.n, _lib.ptr(q16), q16.shape[0], self.D, mode, stride,
                       n_sample, _lib.ptr(dense), dense_ld, _lib.ptr(tau), self.idx_base, _lib.ptr(cand),
-                      _lib.ptr(cnt), CAP_S, CAP_L, _lib.stream()), "mdir_sim_scan_bf16")
+                      _lib.ptr(cnt), CAP_S, CAP_L, _lib.ptr(self.live), _lib.stream()), "mdir_sim_scan_bf16_live")
 
     def _cand_bufs(self, nq=MAX_Q_WIDE):
         rows = MAX_Q_WIDE if nq <= MAX_Q_WIDE else WIDE_Q
@@ -291,8 +451,8 @@ class Index:
         tau, cand, cnt = self._cand_bufs(nq)     # the select kernel (re)initialises every segment counter
         dense = self._buf("dense", (MAX_Q if nq <= MAX_Q else (MAX_Q_WIDE if nq <= MAX_Q_WIDE else WIDE_Q), max(self.n, 1)), torch.float32)
         self._scan(q16, 0, 0, 0, dense, self.n, None, None, None)
-        _lib.check(lib.mdir_select_kth(_lib.ptr(dense), self.n, self.n, nq, kth, 0, self.idx_base, _lib.ptr(tau),
-                                       _lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, 0, _lib.stream()), "mdir_select_kth")
+        _lib.check(lib.mdir_select_kth_live(_lib.ptr(dense), self.n, self.n, nq, kth, 0, self.idx_base, _lib.ptr(tau), _lib.ptr(cand),
+                                            CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, 0, _lib.ptr(self.live), _lib.stream()), "mdir_select_kth_live")
         self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore)
 
     def _topk_block(self, q16, kth, out_scores, out_idx, out_keys, ovf, rescore=None):
@@ -308,9 +468,9 @@ class Index:
             ws = self._fused_ws()
             if prof is not None:
                 prof.begin()
-            _lib.check(lib.mdir_sim_scan_fused_bf16(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, kth, _lib.ptr(tau),
-                                                    self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                    _lib.stream()), "mdir_sim_scan_fused_bf16")
+            _lib.check(lib.mdir_sim_scan_fused_bf16_live(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, kth, _lib.ptr(tau),
+                                                         self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                                         _lib.ptr(self.live), _lib.stream()), "mdir_sim_scan_fused_bf16_live")
             if prof is not None:
                 prof.end(self.n * self.D * 2)
             return self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore, caps=(0, FUSED_CAP_L))
@@ -323,8 +483,8 @@ class Index:
             sample = self._buf("sample_wide", (WIDE_Q, rows), torch.float32)
             ld = rows
         self._scan(q16, 1, stride, n_sample, sample, ld, None, None, None)
-        _lib.check(lib.mdir_select_kth(_lib.ptr(sample), ld, rows, nq, kth, stride, self.idx_base, _lib.ptr(tau),
-                                       _lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, 1, _lib.stream()), "mdir_select_kth")
+        _lib.check(lib.mdir_select_kth_live(_lib.ptr(sample), ld, rows, nq, kth, stride, self.idx_base, _lib.ptr(tau), _lib.ptr(cand),
+                                            CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, 1, _lib.ptr(self.live), _lib.stream()), "mdir_select_kth_live")
         if prof is not None:
             prof.begin()
         self._scan(q16, 2, stride, n_sample, None, 0, tau, cand, cnt)
@@ -466,7 +626,9 @@ class Index:
         precision "bf16": bf16 operands, fp32 accumulate (|err| <~ 1e-3 on unit vectors);
                   "tf32": fp32 operands consumed as TF32 by the tensor cores;
                   "fp32": 3xTF32 split (hi*hi + hi*lo + lo*hi) = fp32-faithful (|err| ~ 1e-6);
-        tf32 / fp32 need the fp32 master copy (keep_fp32=True); fp32 caches a 3x-wide split of it."""
+        tf32 / fp32 need the fp32 master copy (keep_fp32=True); fp32 caches a 3x-wide split of it.
+        Every slot is scored, so an index with removed rows or free capacity raises MdirError."""
+        self._require_all_live("Index.scores()")
         lib = _lib.lib()
         with torch.cuda.device(self.device):
             q32 = _as_dev_f32(q, self.device)
@@ -505,7 +667,9 @@ class Index:
     def ranks(self, q, max_pairs=1 << 28, precision="bf16"):
         """Full ranking: (N_db, N_q) int64 C-order on the device (== np.argsort(-scores, axis=0,
         kind='stable') of this index's scores at the given precision, see scores()).  Queries are processed in chunks of at most
-        max_pairs // N_db to bound the sort workspace (~30 B per pair)."""
+        max_pairs // N_db to bound the sort workspace (~30 B per pair).  An index with removed rows or free capacity
+        raises MdirError."""
+        self._require_all_live("Index.ranks()")
         lib = _lib.lib()
         with torch.cuda.device(self.device):
             q32 = _as_dev_f32(q, self.device)
@@ -743,6 +907,34 @@ class ShardedIndex:
         per = (n_total + world - 1) // world
         lo = min(rank * per, n_total)
         return lo, min(lo + per, n_total)
+
+    def _id_ranges(self):
+        """(first id, end id) of every rank's shard, gathered once: a collective, like remove() / restore()."""
+        if getattr(self, "_ranges", None) is None:
+            loc = self.local
+            if self.world == 1:
+                self._ranges = [(loc.idx_base, loc.idx_base + loc.n)]
+            else:
+                dev = self.device if self.dist.get_backend(self.group) == "nccl" else torch.device("cpu")
+                mine = torch.tensor([loc.idx_base, loc.idx_base + loc.n], dtype=torch.int64, device=dev)
+                allr = torch.empty((self.world * 2,), dtype=torch.int64, device=dev)
+                self.dist.all_gather_into_tensor(allr, mine, group=self.group)
+                r = allr.cpu().tolist()
+                self._ranges = [(int(r[2 * i]), int(r[2 * i + 1])) for i in range(self.world)]
+        return self._ranges
+
+    def _local_ids(self, ids):
+        rank = self.dist.get_rank(self.group) if self.world > 1 else 0
+        return ids_for_rank(ids, self._id_ranges(), rank)
+
+    def remove(self, ids):
+        """Index.remove with GLOBAL ids: every rank makes the same call with the same list and applies the ids its shard
+        owns.  An id in no rank's shard raises MdirError (on every rank)."""
+        self.local.remove(self._local_ids(ids))
+
+    def restore(self, ids):
+        """Index.restore with GLOBAL ids, called by every rank with the same list (see remove())."""
+        self.local.restore(self._local_ids(ids))
 
     def search(self, q, k, precision="fp32", shortlist=None, check=True, exchange="sync"):
         """exchange="sync": the merged global top-k of THIS call.  exchange="deferred" (peer-memory route only, at most
@@ -1008,13 +1200,14 @@ class GraphedSearch:
             lib.mdir_tune(1, self.scan_ctas)
             try:
                 if i8:
-                    _lib.check(lib.mdir_sim_scan_fused_i8(_lib.ptr(loc.db8), _lib.ptr(loc.row_scale), loc.n, _lib.ptr(self.q8), _lib.ptr(self.q8_scale),
-                                                          nq, loc.D, self.kth, _lib.ptr(tau), loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0,
-                                                          FUSED_CAP_L, _lib.ptr(ws), _lib.stream()), "mdir_sim_scan_fused_i8")
+                    _lib.check(lib.mdir_sim_scan_fused_i8_live(_lib.ptr(loc.db8), _lib.ptr(loc.row_scale), loc.n, _lib.ptr(self.q8),
+                                                               _lib.ptr(self.q8_scale), nq, loc.D, self.kth, _lib.ptr(tau), loc.idx_base, _lib.ptr(cand),
+                                                               _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws), _lib.ptr(loc.live), _lib.stream()),
+                               "mdir_sim_scan_fused_i8_live")
                 else:
-                    _lib.check(lib.mdir_sim_scan_fused_bf16(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
-                                                            loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                            _lib.stream()), "mdir_sim_scan_fused_bf16")
+                    _lib.check(lib.mdir_sim_scan_fused_bf16_live(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
+                                                                 loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                                                 _lib.ptr(loc.live), _lib.stream()), "mdir_sim_scan_fused_bf16_live")
             finally:
                 lib.mdir_tune(1, 0)
             if prof is not None:
@@ -1095,7 +1288,8 @@ class SearchPipeline:
     `depth` CUDA graphs (one static query buffer and output set each) replay back to back on one
     compute stream; uploads and downloads run on their own streams, ordered by events only.  A step
     whose candidate lists overflowed is transparently redone through index.search() (exact recovery).
-    With a ShardedIndex every rank must submit the same sequence (the all-gather is inside the graphs)."""
+    With a ShardedIndex every rank must submit the same sequence (the all-gather is inside the graphs).
+    remove() / restore() / add() mutate the index between tickets without re-capturing the graphs."""
 
     def __init__(self, index, n_q, k, depth=None, precision="fp32", shortlist=None, prof=None, deferred=None, overlap=None, split=True,
                  scan_ctas=None):
@@ -1141,7 +1335,7 @@ class SearchPipeline:
                     "idx": torch.empty((self.n_q, self.k), dtype=torch.int32).pin_memory(),
                     "ovf": torch.zeros((self.n_q,), dtype=torch.int32).pin_memory(),
                     "up": torch.cuda.Event(), "done": torch.cuda.Event(), "down": torch.cuda.Event(), "local": torch.cuda.Event(),
-                    "q": None, "pending": False, "merged": False, "used": False})
+                    "q": None, "pending": False, "merged": False, "used": False, "live": None})
             if self.deferred:
                 self.drain_out = (torch.empty((self.n_q, self.k), dtype=torch.float32, device=dev),
                                   torch.empty((self.n_q, self.k), dtype=torch.int32, device=dev))
@@ -1151,6 +1345,39 @@ class SearchPipeline:
             torch.cuda.synchronize(dev)
         self.n_submitted = 0
         self.n_recovered = 0          # steps redone exactly because a status word was raised
+
+    def _mutate(self, fn):
+        """Run a mutation of the index on the compute stream, after every replay already queued there (and, in overlap
+        mode, after the finalize / exchange queued on the exchange stream, which read the rows and stats that add()
+        writes).  Tickets in flight keep a device copy of the live bitmap they were submitted with: a ticket redone by
+        result()'s recovery path then sees the same rows as its replay did.  A copy is dropped when its last ticket is
+        collected."""
+        dev = self.local.device
+        with torch.cuda.device(dev):
+            if self.overlap:
+                self.compute.wait_stream(self.exch)
+            with torch.cuda.stream(self.compute):
+                waiting = [sl for sl in self.slots if sl["pending"] and sl["live"] is None]
+                if waiting:
+                    snap = self.local.live.clone()
+                    for sl in waiting:
+                        sl["live"] = snap
+                return fn()
+
+    def remove(self, ids):
+        """index.remove(ids) between tickets: tickets submitted before this call do not see it, later ones do.  With a
+        ShardedIndex, ids are global and every rank makes the same call at the same point of its ticket sequence."""
+        self._mutate(lambda: self.index.remove(ids))
+
+    def restore(self, ids):
+        """index.restore(ids) between tickets (see remove())."""
+        self._mutate(lambda: self.index.restore(ids))
+
+    def add(self, vecs):
+        """index.add(vecs) between tickets (see remove()); returns the new ids.  Single-GPU Index only."""
+        if isinstance(self.index, ShardedIndex):
+            raise _lib.MdirError("SearchPipeline.add() needs an Index: ShardedIndex has no add()")
+        return self._mutate(lambda: self.index.add(vecs))
 
     def _download(self, slot, src, status):
         """Queue the D2H of a merged result and its status words into `slot`'s pinned buffers (ordered after the compute
@@ -1227,7 +1454,8 @@ class SearchPipeline:
             # exact recovery, ordered after everything already queued on the compute stream (shared workspaces)
             if self.overlap:
                 self.compute.wait_stream(self.exch)
-            with torch.cuda.stream(self.compute):
+            # with the live rows this ticket was submitted with (a mutation may have been queued since)
+            with torch.cuda.stream(self.compute), self.local._live_version(slot["live"]):
                 if sharded:
                     s, i = self.index.search_collective_recovery(slot["q"], self.k, precision=self.precision, shortlist=self.shortlist)
                 else:
@@ -1235,7 +1463,7 @@ class SearchPipeline:
                 slot["scores"].copy_(s)
                 slot["idx"].copy_(i)
             self.compute.synchronize()
-        slot["q"] = None
+        slot["q"], slot["live"] = None, None
         return slot["scores"].numpy(), slot["idx"].numpy()
 
     def map(self, batches):
