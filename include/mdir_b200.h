@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define MDIR_ABI_VERSION 3
+#define MDIR_ABI_VERSION 4
 
 #define MDIR_E_ARG      (-1)   /* invalid argument (shape/alignment/range) */
 #define MDIR_E_DRIVER   (-2)   /* driver entry point (cuTensorMapEncodeTiled) unavailable */
@@ -246,6 +246,30 @@ int mdir_sim_scan_fused_i8_live(const int8_t* db8, const float* row_scale, int64
                                 const float* q_scale, int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base,
                                 uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
                                 void* ws, const uint32_t* live, void* stream);
+/* Scan extent of a compacted database: the _extent variants take a device int64 n_scan after the bitmap.
+ * The FILTER and fused launches (bf16 and int8) scan only rows [0, min(n_db, *n_scan)), read at kernel
+ * start, so a captured graph follows the value the database writes in stream order; tiles past it are
+ * never loaded.  The fused launch places its sample tiles on that extent: CTA c samples tile
+ * c * max(1, T / grid) of the T used tiles when that is below T, otherwise it publishes no sample keys.
+ * SAMPLE and DENSE launches ignore n_scan.  NULL is exactly the _live entry point.                   */
+int mdir_sim_scan_bf16_extent(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D,
+                              int mode, int sample_stride, int n_sample,
+                              float* dense_out, int64_t dense_ld,
+                              const uint64_t* tau, uint32_t idx_base,
+                              uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                              const uint32_t* live, const int64_t* n_scan, void* stream);
+int mdir_sim_scan_wide_bf16_extent(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode,
+                                   int sample_stride, int n_sample, float* dense_out, int64_t dense_ld,
+                                   const uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
+                                   int cap_s, int cap_l, const uint32_t* live, const int64_t* n_scan, void* stream);
+int mdir_sim_scan_fused_bf16_extent(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D,
+                                    int kth, uint64_t* tau, uint32_t idx_base,
+                                    uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                                    void* ws, const uint32_t* live, const int64_t* n_scan, void* stream);
+int mdir_sim_scan_fused_i8_extent(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8,
+                                  const float* q_scale, int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base,
+                                  uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                                  void* ws, const uint32_t* live, const int64_t* n_scan, void* stream);
 /* Sets (value != 0) or clears the live bits of ids[0 .. n_ids) in one launch (word-level atomics: repeated
  * ids are harmless).  An id is a row index plus idx_base; ids outside [idx_base, idx_base + capacity) are
  * ignored, so every shard of a sharded database can be given the same global list.                     */
@@ -312,6 +336,40 @@ int mdir_topk_finalize_rescore_eps(const uint64_t* cand, int64_t cand_row, const
                                    const float* db_stats, const float* q_eps,
                                    float* out_scores, int32_t* out_idx, uint64_t* out_keys,
                                    uint64_t* tau, int32_t* overflow, void* stream);
+/* The finalize entry points with an id map: slot_id (NULL = identity) maps a slot (candidate index minus
+ * idx_base) to the id emitted in out_idx / out_keys.  Re-scoring still addresses db32 by slot.  The map must
+ * be strictly increasing over the slots that can be candidates, so the order of the output is unchanged.   */
+int mdir_topk_finalize_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg,
+                           int cap0, int cap_l, int n_q, int k,
+                           float* out_scores, int32_t* out_idx, uint64_t* out_keys,
+                           uint64_t* tau, int32_t* overflow, uint32_t idx_base, const uint32_t* slot_id, void* stream);
+int mdir_topk_finalize_rescore_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg,
+                                   int cap0, int cap_l, int n_q, int shortlist, int k_out,
+                                   const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D,
+                                   const float* db_stats,
+                                   float* out_scores, int32_t* out_idx, uint64_t* out_keys,
+                                   uint64_t* tau, int32_t* overflow, const uint32_t* slot_id, void* stream);
+int mdir_topk_finalize_rescore_eps_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg,
+                                       int cap0, int cap_l, int n_q, int shortlist, int k_out,
+                                       const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D,
+                                       const float* db_stats, const float* q_eps,
+                                       float* out_scores, int32_t* out_idx, uint64_t* out_keys,
+                                       uint64_t* tau, int32_t* overflow, const uint32_t* slot_id, void* stream);
+
+/* In-place compaction of a mutable database (Index.compact).  mdir_compact_prefix: word_prefix[w] = live
+ * slots in bitmap words [0, w), word_prefix[n_words] = all.  mdir_compact_move: the live slots of [lo, hi)
+ * move, in order, to slots dst0 .. dst0 + n_dst - 1 of every plane given (db16 and slot_id always; db32,
+ * db8 + row_scale optional); dst0 + n_dst <= hi.  scratch NULL: one launch, needs dst0 + n_dst <= lo;
+ * otherwise the rows are staged in scratch (mdir_compact_scratch_bytes(n_dst, ...) bytes): two launches.
+ * Chunks must be moved in ascending order.  mdir_compact_finish: zero rows [n_live, n_used) of every plane
+ * (slot_id: 0xffffffff), bitmap = ones on [0, n_live), *n_scan = n_live.                                 */
+size_t mdir_compact_scratch_bytes(int64_t rows, int D, int has_fp32, int has_i8);
+int mdir_compact_prefix(const uint32_t* live, int64_t n_words, int64_t* word_prefix, void* stream);
+int mdir_compact_move(uint16_t* db16, float* db32, int8_t* db8, float* row_scale, uint32_t* slot_id, int64_t capacity,
+                      int D, const uint32_t* live, const int64_t* word_prefix, int64_t lo, int64_t hi, int64_t dst0,
+                      int64_t n_dst, void* scratch, size_t scratch_bytes, void* stream);
+int mdir_compact_finish(uint16_t* db16, float* db32, int8_t* db8, float* row_scale, uint32_t* slot_id, int D,
+                        uint32_t* live, int64_t n_words, int64_t n_live, int64_t n_used, int64_t* n_scan, void* stream);
 #define MDIR_STATUS_OVERFLOW    1
 #define MDIR_STATUS_UNCERTIFIED 2
 
@@ -345,6 +403,11 @@ int mdir_rescore_f32(const float* db32, int64_t n_db, uint32_t idx_base, const f
  * combine with an all-reduce);  mdir_add_l2n: out = (a + b) / ||a + b||, b may be NULL.   */
 int mdir_qe_accumulate(const float* db32, int64_t n_db, uint32_t idx_base, int D, const int32_t* idx,
                        const float* scores, int n_q, int n_qe, float alpha, float* acc, void* stream);
+/* mdir_qe_accumulate for a compacted database: idx holds ids, looked up by binary search in the strictly
+ * increasing slot -> id map slot_id[0 .. n_used) (NULL = identity, exactly mdir_qe_accumulate).         */
+int mdir_qe_accumulate_ids(const float* db32, int64_t n_db, uint32_t idx_base, int D, const int32_t* idx,
+                           const float* scores, int n_q, int n_qe, float alpha, float* acc,
+                           const uint32_t* slot_id, int64_t n_used, void* stream);
 int mdir_add_l2n(const float* a, const float* b, int n, int D, float* out, void* stream);
 
 /* Full per-query ranking of a score matrix given in the REFERENCE layout

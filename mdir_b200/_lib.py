@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmdir_b200.so")
 _lib = None
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 
 class ImageDesc(C.Structure):
@@ -49,6 +49,10 @@ PROTOTYPES = {
     "mdir_sim_scan_wide_bf16_live": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp]),
     "mdir_sim_scan_fused_bf16_live": (_i, [_vp, _i64, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "mdir_sim_scan_fused_i8_live": (_i, [_vp, _vp, _i64, _vp, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "mdir_sim_scan_bf16_extent": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "mdir_sim_scan_wide_bf16_extent": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _i64, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "mdir_sim_scan_fused_bf16_extent": (_i, [_vp, _i64, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
+    "mdir_sim_scan_fused_i8_extent": (_i, [_vp, _vp, _i64, _vp, _vp, _i, _i, _i, _vp, _u32, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "mdir_live_update": (_i, [_vp, _i64, _u32, _vp, _i64, _i, _vp]),
     "mdir_make_key": (_u64, [_f, _u32]),
     "mdir_key_score": (_f, [_u64]),
@@ -57,11 +61,21 @@ PROTOTYPES = {
     "mdir_topk_finalize": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_topk_finalize_rescore": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_topk_finalize_rescore_eps": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mdir_topk_finalize_ids": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _u32, _vp, _vp]),
+    "mdir_topk_finalize_rescore_ids": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                            _vp]),
+    "mdir_topk_finalize_rescore_eps_ids": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                _vp, _vp, _vp]),
+    "mdir_compact_scratch_bytes": (_sz, [_i64, _i, _i, _i]),
+    "mdir_compact_prefix": (_i, [_vp, _i64, _vp, _vp]),
+    "mdir_compact_move": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _sz, _vp]),
+    "mdir_compact_finish": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
     "mdir_pack_stats": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
     "mdir_pack_stats_i8": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "mdir_pack_q_i8": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "mdir_rescore_f32": (_i, [_vp, _i64, _u32, _vp, _i, _i, _vp, _i, _vp, _vp]),
     "mdir_qe_accumulate": (_i, [_vp, _i64, _u32, _i, _vp, _vp, _i, _i, _f, _vp, _vp]),
+    "mdir_qe_accumulate_ids": (_i, [_vp, _i64, _u32, _i, _vp, _vp, _i, _i, _f, _vp, _vp, _i64, _vp]),
     "mdir_add_l2n": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "mdir_map_workspace_bytes": (_sz, [_i64, _i]),
     "mdir_compute_ap": (_i, [_vp, _i64, _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp, _vp]),

@@ -163,6 +163,9 @@ struct ScanParams {
     // live-row bitmap (NULL: every row < n_db is live): bit r & 31 of word r >> 5 set = row r is live.  A dead row
     // is scored like a row past the end: never a candidate, -inf in the SAMPLE / DENSE outputs, no pass-A key.
     const uint32_t* live;
+    // device-side scan extent (NULL: n_db): FILTER and FUSED launches scan only rows [0, min(n_db, *n_scan)), read once
+    // per CTA at kernel start.  SAMPLE and DENSE ignore it (they cover n_db; rows past the extent are dead by `live`).
+    const int64_t* n_scan;
 };
 
 constexpr int MDIR_SCAN_FUSED = 3;      // internal mode behind mdir_sim_scan_fused_bf16
@@ -171,9 +174,41 @@ struct WorkItem {
     int tile, ks, kb0, nkb, j, chunk, last, qb;
 };
 
-__device__ __forceinline__ int tile_of_work(const ScanParams& p, int j);
+// The part of the work list that depends on the scan extent, identical in the producer, the MMA issuer and the epilogue
+// of a CTA.  Without an extent below n_db these are the host's values.  With one (T_used = used tiles):
+// FILTER keeps the sample tiles planned on n_db and walks only the non-sample tiles below T_used; FUSED places its
+// sample tiles on the extent: CTA c samples tile c * max(1, T_used / grid) when that is below T_used, otherwise it owns
+// no sample tile (sample_tile = -1: its item 0 loads tile 0 and counts no row, so it publishes all-ones pass-A keys).
+struct Span {
+    int64_t n_end;           // rows [0, n_end) are scanned
+    int n_work, n_sample, sample_stride, sample_tile;
+};
 
-__device__ __forceinline__ WorkItem decode_work(const ScanParams& p, int j) {
+__device__ __forceinline__ Span make_span(const ScanParams& p, int64_t n_end) {
+    Span s;
+    s.n_end = n_end;
+    s.n_work = p.n_work;
+    s.n_sample = p.n_sample;
+    s.sample_stride = p.sample_stride;
+    s.sample_tile = (int)blockIdx.x * p.sample_stride;
+    if (n_end < p.n_db) {                 // only FILTER / FUSED launches with an extent get here
+        const int t_used = (int)((n_end + kBlockM - 1) / kBlockM);
+        if (p.mode == MDIR_SCAN_FUSED) {
+            s.sample_stride = max(1, t_used / (int)gridDim.x);
+            s.n_sample = min((int)gridDim.x, (t_used + s.sample_stride - 1) / s.sample_stride);
+            s.sample_tile = (int)blockIdx.x < s.n_sample ? (int)blockIdx.x * s.sample_stride : -1;
+            s.n_work = t_used - s.n_sample;
+        } else {
+            const int n_s = p.n_sample == 0 ? 0 : min(p.n_sample, (t_used + p.sample_stride - 1) / p.sample_stride);
+            s.n_work = (t_used - n_s) * p.n_qblocks;
+        }
+    }
+    return s;
+}
+
+__device__ __forceinline__ int tile_of_work(const ScanParams& p, const Span& s, int j);
+
+__device__ __forceinline__ WorkItem decode_work(const ScanParams& p, const Span& s, int j) {
     WorkItem w;
     w.qb = 0;
     if (p.mode == MDIR_SCAN_DENSE && p.k_split > 1) {
@@ -185,7 +220,7 @@ __device__ __forceinline__ WorkItem decode_work(const ScanParams& p, int j) {
         // wide launch: work item = (tile-level item, query block), the blocks of a tile adjacent in the round-robin
         const int jt = j / p.n_qblocks;
         w.qb = j - jt * p.n_qblocks;
-        w.tile = tile_of_work(p, jt);
+        w.tile = tile_of_work(p, s, jt);
         w.ks = 0;
         w.kb0 = 0;
         w.nkb = p.num_k_blocks;
@@ -194,7 +229,7 @@ __device__ __forceinline__ WorkItem decode_work(const ScanParams& p, int j) {
         w.last = 1;
         return w;
     } else {
-        w.tile = tile_of_work(p, j);
+        w.tile = tile_of_work(p, s, j);
         w.ks = 0;
         w.kb0 = 0;
         w.nkb = p.num_k_blocks;
@@ -207,7 +242,7 @@ __device__ __forceinline__ WorkItem decode_work(const ScanParams& p, int j) {
 
 // The it-th work item of this CTA (persistent round-robin); false when the CTA is done.  In FUSED mode item 0 is
 // the CTA's own sample tile and the rest walk the non-sample tiles exactly like FILTER mode.
-__device__ __forceinline__ bool next_item(const ScanParams& p, int it, WorkItem& w) {
+__device__ __forceinline__ bool next_item(const ScanParams& p, const Span& s, int it, WorkItem& w) {
     if (p.chain > 1) {                    // DENSE, chained chunks: chunk c of the CTA's (it / chain)-th tile
         const int t = it / p.chain, c = it - t * p.chain;
         const int tile = (int)blockIdx.x + t * (int)gridDim.x;
@@ -225,7 +260,7 @@ __device__ __forceinline__ bool next_item(const ScanParams& p, int it, WorkItem&
     int j = (int)blockIdx.x + it * (int)gridDim.x;
     if (p.mode == MDIR_SCAN_FUSED) {
         if (it == 0) {
-            w.tile = (int)blockIdx.x * p.sample_stride;
+            w.tile = s.sample_tile >= 0 ? s.sample_tile : 0;
             w.ks = 0;
             w.qb = 0;
             w.kb0 = 0;
@@ -237,8 +272,8 @@ __device__ __forceinline__ bool next_item(const ScanParams& p, int it, WorkItem&
         }
         j -= (int)gridDim.x;
     }
-    if (j >= p.n_work) return false;
-    w = decode_work(p, j);
+    if (j >= s.n_work) return false;
+    w = decode_work(p, s, j);
     return true;
 }
 
@@ -253,18 +288,18 @@ __device__ __forceinline__ bool spin_until(const uint32_t* ctr, uint32_t target)
     return false;
 }
 
-__device__ __forceinline__ int tile_of_work(const ScanParams& p, int j) {
+__device__ __forceinline__ int tile_of_work(const ScanParams& p, const Span& s, int j) {
     if (p.mode == MDIR_SCAN_DENSE) return j;
     if (p.mode == MDIR_SCAN_SAMPLE) return j * p.sample_stride;
-    // FILTER: every tile that is not a sample tile
-    if (p.n_sample == 0) return j;
-    const int per = p.sample_stride - 1;
-    const int in_groups = p.n_sample * per;
+    // FILTER: every tile that is not a sample tile, in ascending order (per = 0: the sample tiles are the first n_sample)
+    if (s.n_sample == 0) return j;
+    const int per = s.sample_stride - 1;
+    const int in_groups = s.n_sample * per;
     if (j < in_groups) {
         const int g = j / per;
-        return g * p.sample_stride + 1 + (j - g * per);
+        return g * s.sample_stride + 1 + (j - g * per);
     }
-    return p.n_sample * p.sample_stride + (j - in_groups);
+    return s.n_sample * s.sample_stride + (j - in_groups);
 }
 
 // 16 scores (columns c0 .. c0 + 15 of this warp's TMEM lanes) of one accumulator.  int8: the hi plane's s32 sums sit in
@@ -356,10 +391,20 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
             cand_n[c] = 0u;
         }
     }
+    __shared__ int64_t n_end_s;
+    if (threadIdx.x == 96) {            // an epilogue thread: its load overlaps the barrier setup and the TMEM allocation
+        int64_t e = p.n_db;
+        if (p.n_scan && (p.mode == MDIR_SCAN_FILTER || p.mode == MDIR_SCAN_FUSED)) {
+            const int64_t x = *p.n_scan;
+            e = x < 0 ? 0 : (x < e ? x : e);
+        }
+        n_end_s = e;
+    }
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_s;
+    const Span sp = make_span(p, n_end_s);
 
     if (warp == 0) {
         // ------------------------------------------------------------ TMA producer
@@ -367,7 +412,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
             int stage = 0;
             uint32_t phase = 0;
             WorkItem w;
-            for (int it = 0; next_item(p, it, w); ++it) {
+            for (int it = 0; next_item(p, sp, it, w); ++it) {
                 const int row0 = w.tile * kBlockM;
                 for (int kb = w.kb0; kb < w.kb0 + w.nkb; ++kb) {
                     mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1u);
@@ -393,7 +438,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
             int stage = 0;
             uint32_t phase = 0;
             WorkItem w;
-            for (int it = 0; next_item(p, it, w); ++it) {
+            for (int it = 0; next_item(p, sp, it, w); ++it) {
                 const int b = it % p.acc_bufs;
                 const uint32_t acc_phase = (uint32_t)(it / p.acc_bufs) & 1u;
                 uint32_t d_half[2];
@@ -444,7 +489,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
         const int emode = p.mode == MDIR_SCAN_FUSED ? MDIR_SCAN_FILTER : p.mode;
         float* chain_sum = reinterpret_cast<float*>(smem_raw + (smem_base - smem_u32(smem_raw)) + (uint32_t)p.num_stages * stage_bytes);
         WorkItem w;
-        for (int it = 0; next_item(p, it, w); ++it) {
+        for (int it = 0; next_item(p, sp, it, w); ++it) {
             const int b = it % p.acc_bufs;
             const uint32_t acc_phase = (uint32_t)(it / p.acc_bufs) & 1u;
             const int tile = w.tile;
@@ -481,13 +526,15 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                 }
                 tc_fence_after();
             }
+            // FUSED item 0 of a CTA without a sample tile (extent below grid tiles): nothing of it is counted
+            const bool item_rows = !(p.mode == MDIR_SCAN_FUSED && it == 0 && sp.sample_tile < 0);
             if (p.mode == MDIR_SCAN_FUSED && it == 0) {
                 // ---- pass A over the sample tile: best two keys of each 32-row group (this warp x half), per query
                 const int et = (int)threadIdx.x - 64;
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) {
                     const int64_t row = (int64_t)tile * kBlockM + h * 128 + quarter * 32 + lane;
-                    const bool row_ok = row < p.n_db && (((h ? live_w[1] : live_w[0]) >> lane) & 1u);
+                    const bool row_ok = item_rows && row < sp.n_end && (((h ? live_w[1] : live_w[0]) >> lane) & 1u);
                     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc_col(h);
                     const float s_r = h ? s_rh[1] : s_rh[0];
 #pragma unroll 1
@@ -590,8 +637,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
             for (int h = 0; h < 2; ++h) {
                 const int r_in_tile = h * 128 + quarter * 32 + lane;
                 const int64_t row = (int64_t)tile * kBlockM + r_in_tile;
-                const bool row_in = row < p.n_db;
-                const bool row_ok = row_in && (((h ? live_w[1] : live_w[0]) >> lane) & 1u);      // no dynamic index: no stack
+                const bool row_in = row < sp.n_end;
+                const bool row_ok = item_rows && row_in && (((h ? live_w[1] : live_w[0]) >> lane) & 1u);      // no dynamic index: no stack
                 if (I8) {
                     const int i = 2 * it + h;
                     mbar_wait(smem_u32(&tmem_full_bar[i % p.acc_bufs]), (uint32_t)(i / p.acc_bufs) & 1u);
@@ -739,7 +786,8 @@ static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, in
                        float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base, uint64_t* cand,
                        uint32_t* seg_counts, int cap_s, int cap_l, void* stream, int k_split = 1, int64_t split_stride = 0,
                        int kth = 0, uint32_t* fused_ws = nullptr, uint64_t* tau_rw = nullptr, int n_q_total = 0,
-                       const float* row_scale = nullptr, const float* q_scale = nullptr, const uint32_t* live = nullptr) {
+                       const float* row_scale = nullptr, const float* q_scale = nullptr, const uint32_t* live = nullptr,
+                       const int64_t* n_scan = nullptr) {
     const bool tf32 = kind == kKindTf32, i8 = kind == kKindI8;
     const int esz = tf32 ? 4 : (i8 ? 1 : 2);
     MDIR_CHECK_ARG(db && q && n_db >= 1 && n_q >= 1 && n_q <= kMaxN && D >= 16 / esz && (D % (16 / esz)) == 0);
@@ -752,6 +800,7 @@ static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, in
     p.row_scale = row_scale;
     p.q_scale = q_scale;
     p.live = live;
+    p.n_scan = n_scan;
     p.n_db = n_db;
     p.n_q = n_q;
     p.n_pad = (n_q + 15) & ~15;
@@ -911,11 +960,19 @@ static int launch_scan(int kind, const void* db, int64_t n_db, const void* q, in
     return 0;
 }
 
+extern "C" int mdir_sim_scan_bf16_extent(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
+                                         int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
+                                         uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, const uint32_t* live,
+                                         const int64_t* n_scan, void* stream) {
+    return launch_scan(kKindBf16, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+                       cap_s, cap_l, stream, 1, 0, 0, nullptr, nullptr, 0, nullptr, nullptr, live, n_scan);
+}
+
 extern "C" int mdir_sim_scan_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
                                        int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
                                        uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, const uint32_t* live, void* stream) {
-    return launch_scan(kKindBf16, db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
-                       cap_s, cap_l, stream, 1, 0, 0, nullptr, nullptr, 0, nullptr, nullptr, live);
+    return mdir_sim_scan_bf16_extent(db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts,
+                                     cap_s, cap_l, live, nullptr, stream);
 }
 
 extern "C" int mdir_sim_scan_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
@@ -935,14 +992,22 @@ extern "C" int mdir_sim_scan_dense_bf16(const uint16_t* db, int64_t n_db, const 
                        nullptr, nullptr, n_q > blk ? n_q : 0);
 }
 
-extern "C" int mdir_sim_scan_wide_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
-                                            int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
-                                            uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, const uint32_t* live, void* stream) {
+extern "C" int mdir_sim_scan_wide_bf16_extent(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode,
+                                              int sample_stride, int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau,
+                                              uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l,
+                                              const uint32_t* live, const int64_t* n_scan, void* stream) {
     // mdir_sim_scan_bf16 for 129 .. 1024 queries in one launch (DENSE: any number): blocks of 128 queries per work item
     MDIR_CHECK_ARG(n_q >= 1 && (mode == MDIR_SCAN_DENSE || n_q <= kMaxWideQ));
     const int blk = n_q < 128 ? n_q : 128;
     return launch_scan(kKindBf16, db, n_db, q, blk, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand, seg_counts, cap_s,
-                       cap_l, stream, 1, 0, 0, nullptr, nullptr, n_q > blk ? n_q : 0, nullptr, nullptr, live);
+                       cap_l, stream, 1, 0, 0, nullptr, nullptr, n_q > blk ? n_q : 0, nullptr, nullptr, live, n_scan);
+}
+
+extern "C" int mdir_sim_scan_wide_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
+                                            int n_sample, float* dense_out, int64_t dense_ld, const uint64_t* tau, uint32_t idx_base,
+                                            uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, const uint32_t* live, void* stream) {
+    return mdir_sim_scan_wide_bf16_extent(db, n_db, q, n_q, D, mode, sample_stride, n_sample, dense_out, dense_ld, tau, idx_base, cand,
+                                          seg_counts, cap_s, cap_l, live, nullptr, stream);
 }
 
 extern "C" int mdir_sim_scan_wide_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int mode, int sample_stride,
@@ -956,12 +1021,18 @@ extern "C" size_t mdir_sim_scan_fused_workspace_bytes(int n_q) {
     return (4 + (size_t)(n_q > 0 ? n_q : 0) * kNumSMs * 16) * sizeof(uint32_t);
 }
 
+extern "C" int mdir_sim_scan_fused_bf16_extent(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int kth, uint64_t* tau,
+                                               uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* ws,
+                                               const uint32_t* live, const int64_t* n_scan, void* stream) {
+    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0);
+    return launch_scan(kKindBf16, db, n_db, q, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
+                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, nullptr, nullptr, live, n_scan);
+}
+
 extern "C" int mdir_sim_scan_fused_bf16_live(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int kth, uint64_t* tau,
                                              uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts, int cap_s, int cap_l, void* ws,
                                              const uint32_t* live, void* stream) {
-    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0);
-    return launch_scan(kKindBf16, db, n_db, q, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
-                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, nullptr, nullptr, live);
+    return mdir_sim_scan_fused_bf16_extent(db, n_db, q, n_q, D, kth, tau, idx_base, cand, seg_counts, cap_s, cap_l, ws, live, nullptr, stream);
 }
 
 extern "C" int mdir_sim_scan_fused_bf16(const uint16_t* db, int64_t n_db, const uint16_t* q, int n_q, int D, int kth, uint64_t* tau,
@@ -970,12 +1041,19 @@ extern "C" int mdir_sim_scan_fused_bf16(const uint16_t* db, int64_t n_db, const 
     return mdir_sim_scan_fused_bf16_live(db, n_db, q, n_q, D, kth, tau, idx_base, cand, seg_counts, cap_s, cap_l, ws, nullptr, stream);
 }
 
+extern "C" int mdir_sim_scan_fused_i8_extent(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8, const float* q_scale,
+                                             int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
+                                             int cap_s, int cap_l, void* ws, const uint32_t* live, const int64_t* n_scan, void* stream) {
+    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0 && D % 128 == 0);
+    return launch_scan(kKindI8, db8, n_db, q8, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
+                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, row_scale, q_scale, live, n_scan);
+}
+
 extern "C" int mdir_sim_scan_fused_i8_live(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8, const float* q_scale,
                                            int n_q, int D, int kth, uint64_t* tau, uint32_t idx_base, uint64_t* cand, uint32_t* seg_counts,
                                            int cap_s, int cap_l, void* ws, const uint32_t* live, void* stream) {
-    MDIR_CHECK_ARG(ws && (((uintptr_t)ws) & 15) == 0 && D % 128 == 0);
-    return launch_scan(kKindI8, db8, n_db, q8, n_q, D, MDIR_SCAN_FUSED, 0, 0, nullptr, 0, nullptr, idx_base, cand, seg_counts, cap_s, cap_l,
-                       stream, 1, 0, kth, static_cast<uint32_t*>(ws), tau, 0, row_scale, q_scale, live);
+    return mdir_sim_scan_fused_i8_extent(db8, row_scale, n_db, q8, q_scale, n_q, D, kth, tau, idx_base, cand, seg_counts, cap_s, cap_l, ws,
+                                         live, nullptr, stream);
 }
 
 extern "C" int mdir_sim_scan_fused_i8(const int8_t* db8, const float* row_scale, int64_t n_db, const int8_t* q8, const float* q_scale,

@@ -548,6 +548,9 @@ __device__ __forceinline__ void rescore_share(uint64_t* local_list, uint32_t rem
 // q_eps != NULL: the filter scores came from another encoding (the int8 scan) and q_eps[q] is that encoding's bound
 // for query q (mdir_pack_q_i8), used instead of the bf16 formula above.
 // status[q]: bit 0 = a candidate segment / the staging area overflowed, bit 1 = not certified.
+// slot_id != NULL: the candidate keys carry slots (idx_base + slot, which re-scoring addresses db32 by); the emitted
+// indices and keys carry slot_id[slot] instead.  The map is strictly increasing over the used slots, so the sorted order
+// and the (score desc, index asc) tie-break are the same either way.
 template <int CS>      // CS = CTAs per query (thread-block cluster size): rank 0 selects and sorts, all ranks share the fp32 re-scoring
 __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __restrict__ cand, int64_t cand_row,
                                                              const uint32_t* __restrict__ seg_counts, int n_seg, int cap0, int cap_l,
@@ -556,7 +559,8 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
                                                              uint64_t* __restrict__ tau, int32_t* __restrict__ overflow,
                                                              const float* __restrict__ db32, int64_t n_db, uint32_t idx_base,
                                                              const float* __restrict__ q32, int D, int k_out,
-                                                             const float* __restrict__ db_stats, const float* __restrict__ q_eps) {
+                                                             const float* __restrict__ db_stats, const float* __restrict__ q_eps,
+                                                             const uint32_t* __restrict__ slot_id) {
     extern __shared__ uint64_t skeys[];
     __shared__ uint32_t hist[256];
     __shared__ uint64_t s_prefix;
@@ -836,8 +840,9 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
     }
     if (threadIdx.x == 0 && overflow) overflow[q] = status;
     for (int j = threadIdx.x; j < k_emit; j += blockDim.x) {
-        const uint64_t key = j < nres ? res[j] : ~0ull;
+        uint64_t key = j < nres ? res[j] : ~0ull;
         const bool ok = j < nres && key != ~0ull;
+        if (ok && slot_id) key = (key & 0xffffffff00000000ull) | slot_id[(uint32_t)key - idx_base];
         if (out_scores) out_scores[(int64_t)q * k_emit + j] = ok ? key_score(key) : -INFINITY;
         if (out_idx) out_idx[(int64_t)q * k_emit + j] = ok ? (int32_t)(uint32_t)key : -1;
         if (out_keys) out_keys[(int64_t)q * k_emit + j] = ok ? key : ~0ull;
@@ -912,15 +917,27 @@ __global__ void __launch_bounds__(256) pack_bf16_transpose_kernel(const float* _
 
 // alpha-QE / DBA accumulation (NOT in the reference; SURVEY.md App. E).  One CTA per query:
 // acc[q, :] = sum_j max(s_j, 0)^alpha * db32[idx_j - idx_base, :] over the entries this shard owns.
+// slot_id != NULL (a compacted index): idx holds ids, found by binary search in the strictly increasing slot -> id map
+// over the n_used used slots; an id the map does not hold belongs to another shard (or was purged).
 __global__ void __launch_bounds__(256) qe_accumulate_kernel(const float* __restrict__ db32, int64_t n_db, uint32_t idx_base, int D,
                                                             const int32_t* __restrict__ idx, const float* __restrict__ scores,
-                                                            int n_qe, float alpha, float* __restrict__ acc) {
+                                                            int n_qe, float alpha, float* __restrict__ acc,
+                                                            const uint32_t* __restrict__ slot_id, int64_t n_used) {
     __shared__ float w_s[256];
     __shared__ int64_t row_s[256];
     const int q = blockIdx.x;
     for (int j = threadIdx.x; j < n_qe; j += blockDim.x) {
         const int32_t gi = idx[(int64_t)q * n_qe + j];
-        const int64_t row = (int64_t)(uint32_t)gi - (int64_t)idx_base;
+        int64_t row = (int64_t)(uint32_t)gi - (int64_t)idx_base;
+        if (slot_id && gi >= 0) {
+            int64_t lo = 0, hi = n_used;                    // first slot whose id is >= gi
+            while (lo < hi) {
+                const int64_t mid = (lo + hi) >> 1;
+                if (slot_id[mid] < (uint32_t)gi) lo = mid + 1;
+                else hi = mid;
+            }
+            row = lo < n_used && slot_id[lo] == (uint32_t)gi ? lo : -1;
+        }
         const bool own = gi >= 0 && row >= 0 && row < n_db;
         row_s[j] = own ? row : -1;
         w_s[j] = own ? powf(fmaxf(scores[(int64_t)q * n_qe + j], 0.f), alpha) : 0.f;
@@ -1010,7 +1027,7 @@ extern "C" int mdir_live_update(uint32_t* live, int64_t capacity, uint32_t idx_b
 static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0, int cap_l, int n_q,
                            int k, float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
                            const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D, int k_out, const float* db_stats,
-                           void* stream, const float* q_eps = nullptr) {
+                           void* stream, const float* q_eps = nullptr, const uint32_t* slot_id = nullptr) {
     MDIR_CHECK_ARG(cand && seg_counts && n_seg >= 1 && n_seg <= MDIR_CAND_SEGS && cap0 >= 0 && n_q >= 0 && k >= 1 && k <= 4096);
     MDIR_CHECK_ARG(n_seg == 1 || cap_l >= 1);
     MDIR_CHECK_ARG(cand_row >= (int64_t)cap0 + (int64_t)(n_seg - 1) * cap_l);
@@ -1065,13 +1082,13 @@ static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         MDIR_CUDA(cudaLaunchKernelEx(&cfg, topk_finalize_kernel<2>, cand, cand_row, seg_counts, n_seg, cap0, cap_l, k, smem_cap, sl_cap, out_scores,
-                                     out_idx, out_keys, tau, overflow, db32, n_db, idx_base, q32, D, k_out, db_stats, q_eps));
+                                     out_idx, out_keys, tau, overflow, db32, n_db, idx_base, q32, D, k_out, db_stats, q_eps, slot_id));
         MDIR_LAUNCH_CHECK();
         return 0;
     }
     topk_finalize_kernel<1><<<n_q, 1024, smem, (cudaStream_t)stream>>>(cand, cand_row, seg_counts, n_seg, cap0, cap_l, k, smem_cap, sl_cap,
                                                                         out_scores, out_idx, out_keys, tau, overflow, db32, n_db, idx_base,
-                                                                        q32, D, k_out, db_stats, q_eps);
+                                                                        q32, D, k_out, db_stats, q_eps, slot_id);
     MDIR_LAUNCH_CHECK();
     return 0;
 }
@@ -1083,13 +1100,39 @@ extern "C" int mdir_topk_finalize(const uint64_t* cand, int64_t cand_row, const 
                            0, nullptr, 0, 0, nullptr, stream);
 }
 
+extern "C" int mdir_topk_finalize_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0, int cap_l,
+                                      int n_q, int k, float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau,
+                                      int32_t* overflow, uint32_t idx_base, const uint32_t* slot_id, void* stream) {
+    return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, k, out_scores, out_idx, out_keys, tau, overflow, nullptr, 0,
+                           idx_base, nullptr, 0, 0, nullptr, stream, nullptr, slot_id);
+}
+
+extern "C" int mdir_topk_finalize_rescore_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
+                                              int cap_l, int n_q, int shortlist, int k_out, const float* db32, int64_t n_db,
+                                              uint32_t idx_base, const float* q32, int D, const float* db_stats, float* out_scores,
+                                              int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
+                                              const uint32_t* slot_id, void* stream) {
+    MDIR_CHECK_ARG(db32 != nullptr);
+    return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
+                           db32, n_db, idx_base, q32, D, k_out, db_stats, stream, nullptr, slot_id);
+}
+
 extern "C" int mdir_topk_finalize_rescore(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
                                           int cap_l, int n_q, int shortlist, int k_out, const float* db32, int64_t n_db,
                                           uint32_t idx_base, const float* q32, int D, const float* db_stats, float* out_scores,
                                           int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow, void* stream) {
-    MDIR_CHECK_ARG(db32 != nullptr);
+    return mdir_topk_finalize_rescore_ids(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, k_out, db32, n_db, idx_base, q32, D,
+                                          db_stats, out_scores, out_idx, out_keys, tau, overflow, nullptr, stream);
+}
+
+extern "C" int mdir_topk_finalize_rescore_eps_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
+                                                  int cap_l, int n_q, int shortlist, int k_out, const float* db32, int64_t n_db,
+                                                  uint32_t idx_base, const float* q32, int D, const float* db_stats, const float* q_eps,
+                                                  float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
+                                                  const uint32_t* slot_id, void* stream) {
+    MDIR_CHECK_ARG(db32 != nullptr && db_stats != nullptr && q_eps != nullptr);
     return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
-                           db32, n_db, idx_base, q32, D, k_out, db_stats, stream);
+                           db32, n_db, idx_base, q32, D, k_out, db_stats, stream, q_eps, slot_id);
 }
 
 extern "C" int mdir_topk_finalize_rescore_eps(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
@@ -1097,9 +1140,8 @@ extern "C" int mdir_topk_finalize_rescore_eps(const uint64_t* cand, int64_t cand
                                               uint32_t idx_base, const float* q32, int D, const float* db_stats, const float* q_eps,
                                               float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
                                               void* stream) {
-    MDIR_CHECK_ARG(db32 != nullptr && db_stats != nullptr && q_eps != nullptr);
-    return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
-                           db32, n_db, idx_base, q32, D, k_out, db_stats, stream, q_eps);
+    return mdir_topk_finalize_rescore_eps_ids(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, k_out, db32, n_db, idx_base, q32,
+                                              D, db_stats, q_eps, out_scores, out_idx, out_keys, tau, overflow, nullptr, stream);
 }
 
 // db_stats for the shortlist certificate: {max_r ||bf16(x_r) - x_r||^2, max_r ||x_r||^2} over the rows of a shard.
@@ -1315,13 +1357,19 @@ extern "C" int mdir_pack_bf16(const float* src, int64_t n, int D, int src_is_Dxn
     return 0;
 }
 
-extern "C" int mdir_qe_accumulate(const float* db32, int64_t n_db, uint32_t idx_base, int D, const int32_t* idx, const float* scores,
-                                  int n_q, int n_qe, float alpha, float* acc, void* stream) {
+extern "C" int mdir_qe_accumulate_ids(const float* db32, int64_t n_db, uint32_t idx_base, int D, const int32_t* idx, const float* scores,
+                                      int n_q, int n_qe, float alpha, float* acc, const uint32_t* slot_id, int64_t n_used, void* stream) {
     MDIR_CHECK_ARG(db32 && idx && scores && acc && n_db >= 0 && D > 0 && n_q >= 0 && n_qe >= 1 && n_qe <= 256);
+    MDIR_CHECK_ARG(!slot_id || (n_used >= 0 && n_used <= n_db));
     if (n_q == 0) return 0;
-    qe_accumulate_kernel<<<n_q, 256, 0, (cudaStream_t)stream>>>(db32, n_db, idx_base, D, idx, scores, n_qe, alpha, acc);
+    qe_accumulate_kernel<<<n_q, 256, 0, (cudaStream_t)stream>>>(db32, n_db, idx_base, D, idx, scores, n_qe, alpha, acc, slot_id, n_used);
     MDIR_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int mdir_qe_accumulate(const float* db32, int64_t n_db, uint32_t idx_base, int D, const int32_t* idx, const float* scores,
+                                  int n_q, int n_qe, float alpha, float* acc, void* stream) {
+    return mdir_qe_accumulate_ids(db32, n_db, idx_base, D, idx, scores, n_q, n_qe, alpha, acc, nullptr, 0, stream);
 }
 
 extern "C" int mdir_add_l2n(const float* a, const float* b, int n, int D, float* out, void* stream) {

@@ -22,9 +22,10 @@ def _accumulate(index, idx, scores, alpha):
     n_q, n_qe = idx.shape
     acc = torch.empty((n_q, index.D), dtype=torch.float32, device=index.device)
     with torch.cuda.device(index.device):
-        _lib.check(_lib.lib().mdir_qe_accumulate(_lib.ptr(index.db32), index.n, index.idx_base, index.D, _lib.ptr(idx.contiguous()),
-                                                 _lib.ptr(scores.contiguous()), n_q, n_qe, float(alpha), _lib.ptr(acc), _lib.stream()),
-                   "mdir_qe_accumulate")
+        # idx holds ids: the slot -> id map of the index finds their rows (after compact() they are no longer id - idx_base)
+        _lib.check(_lib.lib().mdir_qe_accumulate_ids(_lib.ptr(index.db32), index.n, index.idx_base, index.D, _lib.ptr(idx.contiguous()),
+                                                     _lib.ptr(scores.contiguous()), n_q, n_qe, float(alpha), _lib.ptr(acc),
+                                                     _lib.ptr(index.slot_id), index._n_used, _lib.stream()), "mdir_qe_accumulate_ids")
     return acc
 
 

@@ -11,7 +11,8 @@ Replaces, for mdir's evaluation (mdir/components/optim/score/cirscore.py:65-70):
                                 top-k selection fused into the epilogue, ``scores`` / ``ranks``
                                 = the dense path.  Rows can be removed, restored and appended in
                                 place (``remove`` / ``restore`` / ``add``: a live-row bitmap the
-                                scan reads).
+                                scan reads); ``compact`` purges removed rows and shrinks the scan to the
+                                live ones, ids unchanged.
 * ``ShardedIndex``           -- rows sharded contiguously over the ranks of a torch.distributed
                                 group; local top-k + one all-gather of N_q*k keys + merge.
 * ``ranks_from_scores`` / ``topk_from_scores`` -- the sort/selection kernels fed an existing
@@ -119,6 +120,26 @@ def check_ids(ids, lo, hi):
     return a - lo
 
 
+def compaction_schedule(live, chunk):
+    """The in-place move of Index.compact: live (bool per used slot) -> [(lo, hi, dst0, n_dst, staged)], chunks of at most
+    `chunk` slots in ascending order from the first dead slot.  The n_dst live slots of [lo, hi) go, in order, to
+    [dst0, dst0 + n_dst); dst0 = live slots before lo, so a chunk only overwrites slots below hi, which this or an
+    earlier chunk has already read.  staged = the destinations reach into the chunk itself (dst0 + n_dst > lo): its
+    rows are gathered into scratch first; otherwise reads and writes are disjoint and the chunk moves directly."""
+    live = np.asarray(live, dtype=bool)
+    dead = np.flatnonzero(~live)
+    if dead.size == 0:
+        return []
+    cum = np.concatenate([[0], np.cumsum(live, dtype=np.int64)])
+    out = []
+    for lo in range(int(dead[0]), live.size, int(chunk)):
+        hi = min(lo + int(chunk), live.size)
+        dst0, n_dst = int(cum[lo]), int(cum[hi] - cum[lo])
+        if n_dst:
+            out.append((lo, hi, dst0, n_dst, dst0 + n_dst > lo))
+    return out
+
+
 def ids_for_rank(ids, ranges, rank):
     """Global ids -> the int64 numpy ids that rank `rank` owns, ranges[r] = (first id, end id) of rank r (see
     ShardedIndex.shard_bounds).  MdirError when an id lies in no rank's range."""
@@ -141,13 +162,16 @@ class Index:
     """A (shard of a) descriptor database on one GPU.
 
     Mutable in place: ``remove(ids)`` hides rows from every later search, ``restore(ids)`` undoes that, and
-    ``add(vecs)`` writes new rows into free slots of a ``capacity`` larger than the initial database.  An id is
-    idx_base + slot; slots are never reused, so an id names one row for the life of the index.  Which rows are live
-    is one bitmap on the device (1 bit per slot) that every top-k route reads in the scan epilogue; CUDA graphs
-    captured over the index see every later mutation without re-capture.  The scan covers all ``capacity`` slots:
-    free and removed slots cost scan bandwidth like live rows."""
+    ``add(vecs)`` writes new rows into free slots of a ``capacity`` larger than the initial database.  An id names
+    one row for the life of the index and is never reused; until the first ``compact()`` it is idx_base + slot.
+    Which rows are live is one bitmap on the device (1 bit per slot) that every top-k route reads in the scan
+    epilogue.  The scan covers the used slots [0, n_used), a device-side extent: removed rows cost scan bandwidth like
+    live ones until ``compact()`` moves the live rows to the front (stably), purges the removed ones and shrinks the
+    extent; a slot -> id map keeps the ids.  CUDA graphs captured over the index see every later mutation and
+    compaction without re-capture."""
 
     fused = True      # allow the one-launch threshold + filter route (False: always sample -> select -> filter)
+    compact_chunk = 16384   # slots per chunk of compact()'s in-place move (its scratch holds one chunk's live rows)
     certify = True    # precision="fp32": prove the shortlist complete (status bit 2 + widening when it cannot be)
     _sms = None
 
@@ -156,7 +180,7 @@ class Index:
         (the layout extract_vectors returns, cirtorch/networks/imageretrievalnet.py:291).
         capacity (default n): slots allocated for rows; add() fills slots n, n + 1, ...  With capacity > n the bf16
         rows, the fp32 master (a copy of vecs) and, once built, the int8 plane are allocated at capacity, the free
-        slots zero.  Every slot is scanned, free ones included.  idx_base + capacity must stay <= 2**32."""
+        slots zero.  The scan covers the filled slots.  idx_base + capacity must stay <= 2**32."""
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise _lib.MdirError("Index needs a CUDA device (no CPU path)")
@@ -215,6 +239,13 @@ class Index:
         self.live = torch.from_numpy(host.copy()).to(self.device)
         self._live_host = bits[:self.n].copy()     # host mirror: id validation and n_live without a device read-back
         self._n_used = int(n_used)
+        # the scan extent (slots [0, n_used) are scanned) and the slot -> id map (uint32 ids, identity until compact()),
+        # both on the device for the kernels and captured graphs, updated in place in stream order
+        self.n_scan = torch.tensor([self._n_used], dtype=torch.int64, device=self.device)
+        ident = np.arange(self.idx_base, self.idx_base + self.n, dtype=np.int64)
+        self.slot_id = torch.from_numpy(ident.astype(np.uint32).view(np.int32)).to(self.device)
+        self._ids = ident[:self._n_used].copy()    # host mirror over the used slots, strictly increasing
+        self._next_id = self._n_used               # ids idx_base .. idx_base + _next_id - 1 have been issued
 
     @property
     def n_live(self):
@@ -236,28 +267,42 @@ class Index:
                                                _lib.stream()), "mdir_live_update")
         self._live_host[rows] = bool(value)
 
+    def _slots(self, ids):
+        """ids -> (ids int64, their slots, found): searchsorted in the monotone slot -> id map.  An id outside
+        [idx_base, idx_base + max(capacity, ids issued)) raises MdirError; found is False for an id no used slot holds
+        (never issued, or purged by compact())."""
+        a = check_ids(ids, self.idx_base, self.idx_base + max(self.n, self._next_id)) + self.idx_base
+        pos = np.searchsorted(self._ids, a)
+        found = pos < self._ids.size
+        found[found] = self._ids[pos[found]] == a[found]
+        return a, pos, found
+
     def remove(self, ids):
-        """Hide the rows with these ids (idx_base + slot) from every later search.  Stream-ordered on the current stream;
-        removing a removed id is a no-op; an id outside this index raises MdirError."""
-        rows = check_ids(ids, self.idx_base, self.idx_base + self.n)
+        """Hide the rows with these ids from every later search.  Stream-ordered on the current stream; removing a
+        removed (or purged) id is a no-op; an id outside this index raises MdirError."""
+        _, pos, found = self._slots(ids)
         with torch.cuda.device(self.device):
-            self._set_live(rows, 0)
+            self._set_live(pos[found], 0)
 
     def restore(self, ids):
-        """Undo remove() for these ids (the rows' data never left their slots).  An id of a slot that add() never
-        filled, or outside this index, raises MdirError."""
-        rows = check_ids(ids, self.idx_base, self.idx_base + self.n)
-        if rows.size and int(rows.max()) >= self._n_used:
-            raise _lib.MdirError("id %d names a slot that was never filled" % (int(rows.max()) + self.idx_base))
+        """Undo remove() for these ids (the rows' data never left the device).  An id that compact() purged, one that
+        add() never issued, or one outside this index raises MdirError."""
+        a, pos, found = self._slots(ids)
+        if not found.all():
+            bad = int(a[~found][0])
+            if bad < self.idx_base + self._next_id:
+                raise _lib.MdirError("id %d was removed and then purged by compact(); it cannot be restored" % bad)
+            raise _lib.MdirError("id %d names a slot that was never filled" % bad)
         with torch.cuda.device(self.device):
-            self._set_live(rows, 1)
+            self._set_live(pos, 1)
 
     def add(self, vecs):
-        """Append (m, D) fp32 rows to the next free slots; returns their ids (idx_base + slot, int64 host tensor).
-        In stream order: bf16 rows, fp32 master rows, int8 rows + certificate stats (when built), then the live bits,
-        so a search queued after this call sees the new rows and one queued before it does not.  New rows can only
-        widen the certificate's bounds: the first-pass route chosen earlier stays and stays exact.  MdirError when the
-        rows do not fit the capacity."""
+        """Append (m, D) fp32 rows to the next free slots; returns their ids (int64 host tensor), which continue from the
+        highest id ever issued (idx_base + slot until the first compact()); idx_base + ids issued must stay <= 2**32.
+        In stream order: bf16 rows, fp32 master rows, int8 rows + certificate stats (when built), the id map and scan
+        extent, then the live bits, so a search queued after this call sees the new rows and one queued before it does
+        not.  New rows can only widen the certificate's bounds: the first-pass route chosen earlier stays and stays
+        exact.  MdirError when the rows do not fit the capacity."""
         lib = _lib.lib()
         with torch.cuda.device(self.device):
             v = _as_dev_f32(vecs, self.device)
@@ -268,6 +313,8 @@ class Index:
                 raise _lib.MdirError("index is full: %d free slots, %d rows given" % (self.n - s0, m))
             if m == 0:
                 return torch.empty((0,), dtype=torch.int64)
+            if self.idx_base + self._next_id + m > 1 << 32:
+                raise _lib.MdirError("ids would pass 2**32: %d issued from idx_base %d" % (self._next_id, self.idx_base))
             s1 = s0 + m
             pack_bf16(v, out=self.db16[s0:s1])
             if self.db32 is not None:
@@ -283,9 +330,57 @@ class Index:
                     _lib.check(lib.mdir_pack_stats(_lib.ptr(self.db32[s0:s1]), _lib.ptr(self.db16[s0:s1]), m, self.D, _lib.ptr(st),
                                                    _lib.stream()), "mdir_pack_stats")
                 torch.maximum(self._stats, st, out=self._stats)
-            self._n_used = s1
+            ids = self._issue_ids(m)
+            self.slot_id[s0:s1].copy_(torch.from_numpy(ids.astype(np.uint32).view(np.int32)))
+            self.n_scan.fill_(s1)
             self._set_live(np.arange(s0, s1, dtype=np.int64), 1)
-            return torch.arange(self.idx_base + s0, self.idx_base + s1, dtype=torch.int64)
+            return torch.from_numpy(ids)
+
+    def _issue_ids(self, m):
+        """Host bookkeeping of add(): the ids of m rows appended at slot _n_used, continuing from the highest id issued."""
+        ids = np.arange(self.idx_base + self._next_id, self.idx_base + self._next_id + m, dtype=np.int64)
+        self._ids = np.concatenate([self._ids, ids])
+        self._next_id += m
+        self._n_used += m
+        return ids
+
+    def _compacted_mirrors(self, keep):
+        """Host bookkeeping of compact(): the used slots `keep` (ascending) are now slots [0, len(keep))."""
+        self._ids = self._ids[keep]
+        self._live_host[:] = False
+        self._live_host[:keep.size] = True
+        self._n_used = int(keep.size)
+
+    def compact(self):
+        """Move the live rows to slots [0, n_live), keeping their order, in every plane (bf16 rows, fp32 master, int8
+        rows and scales, the slot -> id map); zero the freed slots; shrink the scan extent to n_live.  Removed rows are
+        purged: their data is gone from the device, restore() of their ids raises, and add() refills the freed slots with
+        new ids.  Ids of live rows do not change.  Returns the number of rows purged (0: nothing launched).  Stream-ordered
+        on the current stream; the certificate stats are kept (maxima over a superset of the rows: still a bound).  An Index
+        built from a device fp32 tensor with capacity == n keeps that tensor as its master copy, so this rewrites it."""
+        used = self._live_host[:self._n_used]
+        keep = np.flatnonzero(used)
+        purged = self._n_used - keep.size
+        if purged == 0:
+            return 0
+        lib = _lib.lib()
+        sched = compaction_schedule(used, self.compact_chunk)
+        with torch.cuda.device(self.device):
+            n_words = self.live.numel()
+            prefix = torch.empty((n_words + 1,), dtype=torch.int64, device=self.device)
+            _lib.check(lib.mdir_compact_prefix(_lib.ptr(self.live), n_words, _lib.ptr(prefix), _lib.stream()), "mdir_compact_prefix")
+            staged = max([c[3] for c in sched if c[4]], default=0)
+            sbytes = lib.mdir_compact_scratch_bytes(staged, self.D, int(self.db32 is not None), int(self.db8 is not None)) if staged else 0
+            scratch = torch.empty((sbytes,), dtype=torch.uint8, device=self.device) if staged else None
+            planes = (_lib.ptr(self.db16), _lib.ptr(self.db32), _lib.ptr(self.db8), _lib.ptr(self.row_scale), _lib.ptr(self.slot_id))
+            for lo, hi, dst0, n_dst, st in sched:
+                _lib.check(lib.mdir_compact_move(*planes, self.n, self.D, _lib.ptr(self.live), _lib.ptr(prefix), lo, hi, dst0, n_dst,
+                                                 _lib.ptr(scratch if st else None), sbytes if st else 0, _lib.stream()), "mdir_compact_move")
+            _lib.check(lib.mdir_compact_finish(*planes, self.D, _lib.ptr(self.live), n_words, keep.size, self._n_used, _lib.ptr(self.n_scan),
+                                               _lib.stream()), "mdir_compact_finish")
+        self._compacted_mirrors(keep)
+        self._db_x3 = None                         # scores(precision="fp32") split of the old layout
+        return int(purged)
 
     @contextlib.contextmanager
     def _live_version(self, live):
@@ -398,9 +493,10 @@ class Index:
         prof = getattr(self, "prof", None)
         if prof is not None:
             prof.begin()
-        _lib.check(lib.mdir_sim_scan_fused_i8_live(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q8), _lib.ptr(qsc), nq, self.D,
-                                                   kth, _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                   _lib.ptr(self.live), _lib.stream()), "mdir_sim_scan_fused_i8_live")
+        _lib.check(lib.mdir_sim_scan_fused_i8_extent(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q8), _lib.ptr(qsc), nq,
+                                                     self.D, kth, _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L,
+                                                     _lib.ptr(ws), _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream()),
+                   "mdir_sim_scan_fused_i8_extent")
         if prof is not None:
             prof.end(self.n * self.D + 4 * self.n)       # int8 rows + their fp32 scales
         self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, (q32, k_out), caps=(0, FUSED_CAP_L), q_eps=qeps)
@@ -408,10 +504,10 @@ class Index:
     def _scan(self, q16, mode, stride, n_sample, dense, dense_ld, tau, cand, cnt):
         # more than 128 queries: one WIDE launch, work items = (tile, 128-query block) -- one kernel ramp, and a database
         # tile comes from HBM once for all the blocks (the tensor-bound regime: DBA, all-pairs)
-        fn = _lib.lib().mdir_sim_scan_wide_bf16_live if q16.shape[0] > MAX_Q else _lib.lib().mdir_sim_scan_bf16_live
+        fn = _lib.lib().mdir_sim_scan_wide_bf16_extent if q16.shape[0] > MAX_Q else _lib.lib().mdir_sim_scan_bf16_extent
         _lib.check(fn(_lib.ptr(self.db16), self.n, _lib.ptr(q16), q16.shape[0], self.D, mode, stride,
                       n_sample, _lib.ptr(dense), dense_ld, _lib.ptr(tau), self.idx_base, _lib.ptr(cand),
-                      _lib.ptr(cnt), CAP_S, CAP_L, _lib.ptr(self.live), _lib.stream()), "mdir_sim_scan_bf16_live")
+                      _lib.ptr(cnt), CAP_S, CAP_L, _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream()), "mdir_sim_scan_bf16_extent")
 
     def _cand_bufs(self, nq=MAX_Q_WIDE):
         rows = MAX_Q_WIDE if nq <= MAX_Q_WIDE else WIDE_Q
@@ -424,23 +520,24 @@ class Index:
         CAP_S, CAP_L = caps
         CAND_ROW = CAP_S + 148 * CAP_L            # the row stride the scan kernels derive from the two capacities
         if rescore is None:
-            _lib.check(_lib.lib().mdir_topk_finalize(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth,
-                                                     _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys), _lib.ptr(tau),
-                                                     _lib.ptr(ovf), _lib.stream()), "mdir_topk_finalize")
+            _lib.check(_lib.lib().mdir_topk_finalize_ids(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth,
+                                                         _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys), _lib.ptr(tau),
+                                                         _lib.ptr(ovf), self.idx_base, _lib.ptr(self.slot_id), _lib.stream()), "mdir_topk_finalize_ids")
         elif q_eps is not None:
             q32, k_out = rescore
-            _lib.check(_lib.lib().mdir_topk_finalize_rescore_eps(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth, k_out,
-                                                                 _lib.ptr(self.db32), self.n, self.idx_base, _lib.ptr(q32), self.D,
-                                                                 _lib.ptr(self.stats()), _lib.ptr(q_eps), _lib.ptr(out_scores), _lib.ptr(out_idx),
-                                                                 _lib.ptr(out_keys), _lib.ptr(tau), _lib.ptr(ovf), _lib.stream()),
-                       "mdir_topk_finalize_rescore_eps")
+            _lib.check(_lib.lib().mdir_topk_finalize_rescore_eps_ids(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth, k_out,
+                                                                     _lib.ptr(self.db32), self.n, self.idx_base, _lib.ptr(q32), self.D,
+                                                                     _lib.ptr(self.stats()), _lib.ptr(q_eps), _lib.ptr(out_scores),
+                                                                     _lib.ptr(out_idx), _lib.ptr(out_keys), _lib.ptr(tau), _lib.ptr(ovf),
+                                                                     _lib.ptr(self.slot_id), _lib.stream()), "mdir_topk_finalize_rescore_eps_ids")
         else:
             q32, k_out = rescore
             stats = self.stats() if self.certify else None
-            _lib.check(_lib.lib().mdir_topk_finalize_rescore(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth, k_out,
-                                                             _lib.ptr(self.db32), self.n, self.idx_base, _lib.ptr(q32), self.D,
-                                                             _lib.ptr(stats), _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys),
-                                                             _lib.ptr(tau), _lib.ptr(ovf), _lib.stream()), "mdir_topk_finalize_rescore")
+            _lib.check(_lib.lib().mdir_topk_finalize_rescore_ids(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth, k_out,
+                                                                 _lib.ptr(self.db32), self.n, self.idx_base, _lib.ptr(q32), self.D,
+                                                                 _lib.ptr(stats), _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys),
+                                                                 _lib.ptr(tau), _lib.ptr(ovf), _lib.ptr(self.slot_id), _lib.stream()),
+                       "mdir_topk_finalize_rescore_ids")
 
     def _dense_block(self, q16, kth, out_scores, out_idx, out_keys, ovf, rescore=None):
         """All scores of the block -> exact kth-key select -> sort.  The route for small databases
@@ -468,9 +565,10 @@ class Index:
             ws = self._fused_ws()
             if prof is not None:
                 prof.begin()
-            _lib.check(lib.mdir_sim_scan_fused_bf16_live(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, kth, _lib.ptr(tau),
-                                                         self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                         _lib.ptr(self.live), _lib.stream()), "mdir_sim_scan_fused_bf16_live")
+            _lib.check(lib.mdir_sim_scan_fused_bf16_extent(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, kth, _lib.ptr(tau),
+                                                           self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                                           _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream()),
+                       "mdir_sim_scan_fused_bf16_extent")
             if prof is not None:
                 prof.end(self.n * self.D * 2)
             return self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore, caps=(0, FUSED_CAP_L))
@@ -936,6 +1034,11 @@ class ShardedIndex:
         """Index.restore with GLOBAL ids, called by every rank with the same list (see remove())."""
         self.local.restore(self._local_ids(ids))
 
+    def compact(self):
+        """Index.compact of this rank's shard, called by every rank at the same point of its sequence (like remove()).
+        The ids and every rank's id range are unchanged.  Returns the rows this shard purged."""
+        return self.local.compact()
+
     def search(self, q, k, precision="fp32", shortlist=None, check=True, exchange="sync"):
         """exchange="sync": the merged global top-k of THIS call.  exchange="deferred" (peer-memory route only, at most
         128 queries): pushes this call's keys and returns the merged result of the PREVIOUS deferred call with the same
@@ -1200,14 +1303,15 @@ class GraphedSearch:
             lib.mdir_tune(1, self.scan_ctas)
             try:
                 if i8:
-                    _lib.check(lib.mdir_sim_scan_fused_i8_live(_lib.ptr(loc.db8), _lib.ptr(loc.row_scale), loc.n, _lib.ptr(self.q8),
-                                                               _lib.ptr(self.q8_scale), nq, loc.D, self.kth, _lib.ptr(tau), loc.idx_base, _lib.ptr(cand),
-                                                               _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws), _lib.ptr(loc.live), _lib.stream()),
-                               "mdir_sim_scan_fused_i8_live")
+                    _lib.check(lib.mdir_sim_scan_fused_i8_extent(_lib.ptr(loc.db8), _lib.ptr(loc.row_scale), loc.n, _lib.ptr(self.q8),
+                                                                 _lib.ptr(self.q8_scale), nq, loc.D, self.kth, _lib.ptr(tau), loc.idx_base,
+                                                                 _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws), _lib.ptr(loc.live),
+                                                                 _lib.ptr(loc.n_scan), _lib.stream()), "mdir_sim_scan_fused_i8_extent")
                 else:
-                    _lib.check(lib.mdir_sim_scan_fused_bf16_live(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
-                                                                 loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                                 _lib.ptr(loc.live), _lib.stream()), "mdir_sim_scan_fused_bf16_live")
+                    _lib.check(lib.mdir_sim_scan_fused_bf16_extent(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
+                                                                   loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
+                                                                   _lib.ptr(loc.live), _lib.ptr(loc.n_scan), _lib.stream()),
+                               "mdir_sim_scan_fused_bf16_extent")
             finally:
                 lib.mdir_tune(1, 0)
             if prof is not None:
@@ -1289,7 +1393,7 @@ class SearchPipeline:
     compute stream; uploads and downloads run on their own streams, ordered by events only.  A step
     whose candidate lists overflowed is transparently redone through index.search() (exact recovery).
     With a ShardedIndex every rank must submit the same sequence (the all-gather is inside the graphs).
-    remove() / restore() / add() mutate the index between tickets without re-capturing the graphs."""
+    remove() / restore() / add() / compact() mutate the index between tickets without re-capturing the graphs."""
 
     def __init__(self, index, n_q, k, depth=None, precision="fp32", shortlist=None, prof=None, deferred=None, overlap=None, split=True,
                  scan_ctas=None):
@@ -1378,6 +1482,17 @@ class SearchPipeline:
         if isinstance(self.index, ShardedIndex):
             raise _lib.MdirError("SearchPipeline.add() needs an Index: ShardedIndex has no add()")
         return self._mutate(lambda: self.index.add(vecs))
+
+    def compact(self):
+        """index.compact() on the compute stream, after the replays and exchanges already queued.  A maintenance step:
+        collect every ticket first -- MdirError while one is pending, because the live-row copy a ticket keeps for its
+        recovery path describes the slot layout compaction changes.  The graphs keep working without re-capture, and
+        tickets submitted afterwards see the compacted index.  With a ShardedIndex every rank calls it at the same point.
+        Returns the rows purged (on this rank)."""
+        pending = [sl for sl in self.slots if sl["pending"]]
+        if pending:
+            raise _lib.MdirError("SearchPipeline.compact(): collect the %d pending ticket(s) first" % len(pending))
+        return self._mutate(self.index.compact)
 
     def _download(self, slot, src, status):
         """Queue the D2H of a merged result and its status words into `slot`'s pinned buffers (ordered after the compute
