@@ -373,6 +373,39 @@ int mdir_compact_finish(uint16_t* db16, float* db32, int8_t* db8, float* row_sca
 #define MDIR_STATUS_OVERFLOW    1
 #define MDIR_STATUS_UNCERTIFIED 2
 
+/* Range search (Index.range_search): every live row whose score is >= min_score[q] (device fp32, one per query).
+ * mdir_range_tau: tau[q] = the FILTER key of min_score[q] (db_stats NULL: bf16 scores), or, for exact fp32 scores,
+ *   of min_score[q] - eps_q rounded down, eps_q the certified bound of mdir_topk_finalize_rescore from db_stats
+ *   (mdir_pack_stats) and q32 (n_q, D): every row whose fp32 score is >= min_score[q] passes the scan.
+ * The scan is mdir_sim_scan_bf16_extent(MDIR_SCAN_FILTER, n_sample 0, cap_s 0, cap_l) on zeroed seg_counts
+ *   (n_q, MDIR_CAND_SEGS); its candidate rows are cand_row = 148 * cap_l keys.
+ * mdir_range_gather: per (chunk of MDIR_RANGE_CHUNK candidate slots, query): the candidates, re-scored in fp32 from
+ *   db32 (NULL: the bf16 keys as they are) and kept when score >= min_score[q], go unsorted to surv
+ *   (n_q, n_chunks, MDIR_RANGE_CHUNK) keys, n_chunks = mdir_range_chunks(cand_row); run_len (n_q, n_chunks) = how
+ *   many per chunk; max_seg[q] = the largest raw segment count (> cap_l: a segment overflowed, the clamped
+ *   candidates are still processed).
+ * mdir_range_emit: every query with count = lims[q + 1] - lims[q] in [1, stage_cap] (a power of two <= 16384):
+ *   its survivors (chunk c at run_off[q, c] within the query) sorted by key into out_scores / out_ids[lims[q] ..],
+ *   ids through the slot -> id map slot_id (NULL: idx_base + slot).
+ * mdir_range_sort_runs + mdir_range_merge: the queries rows[0 .. n_rows) with more survivors: each group of
+ *   MDIR_RANGE_GROUP chunks is sorted in place, then every key is written at lims[q] + its rank among the query's. */
+#define MDIR_RANGE_CHUNK 1024
+#define MDIR_RANGE_GROUP 16
+int64_t mdir_range_chunks(int64_t cand_row);
+int mdir_range_tau(const float* q32, int n_q, int D, const float* min_score, const float* db_stats, uint64_t* tau,
+                   void* stream);
+int mdir_range_gather(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int cap_l, int n_q,
+                      const float* min_score, const float* db32, int64_t n_db, uint32_t idx_base, const float* q32,
+                      int D, uint64_t* surv, int n_chunks, int32_t* run_len, int32_t* max_seg, void* stream);
+int mdir_range_emit(const uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* run_off,
+                    const int64_t* lims, int n_q, int stage_cap, uint32_t idx_base, const uint32_t* slot_id,
+                    float* out_scores, int32_t* out_ids, void* stream);
+int mdir_range_sort_runs(uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* rows, int n_rows,
+                         void* stream);
+int mdir_range_merge(const uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* rows, int n_rows,
+                     const int64_t* lims, uint32_t idx_base, const uint32_t* slot_id, float* out_scores,
+                     int32_t* out_ids, void* stream);
+
 /* stats[2] (device) = {max_r ||bf16(x_r) - x_r||_2^2, max_r ||x_r||_2^2} over the n rows of a shard:
  * the database half of the certificate's error bound.  db16 = mdir_pack_bf16(db32).            */
 int mdir_pack_stats(const float* db32, const uint16_t* db16, int64_t n, int D, float* stats, void* stream);

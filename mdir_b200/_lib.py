@@ -70,6 +70,12 @@ PROTOTYPES = {
     "mdir_compact_prefix": (_i, [_vp, _i64, _vp, _vp]),
     "mdir_compact_move": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _sz, _vp]),
     "mdir_compact_finish": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _i64, _i64, _vp, _vp]),
+    "mdir_range_chunks": (_i64, [_i64]),
+    "mdir_range_tau": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp]),
+    "mdir_range_gather": (_i, [_vp, _i64, _vp, _i, _i, _vp, _vp, _i64, _u32, _vp, _i, _vp, _i, _vp, _vp, _vp]),
+    "mdir_range_emit": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _u32, _vp, _vp, _vp, _vp]),
+    "mdir_range_sort_runs": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
+    "mdir_range_merge": (_i, [_vp, _i, _vp, _vp, _i, _vp, _u32, _vp, _vp, _vp, _vp]),
     "mdir_pack_stats": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
     "mdir_pack_stats_i8": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "mdir_pack_q_i8": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),

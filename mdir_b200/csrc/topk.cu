@@ -1379,3 +1379,305 @@ extern "C" int mdir_add_l2n(const float* a, const float* b, int n, int D, float*
     MDIR_LAUNCH_CHECK();
     return 0;
 }
+
+// ---- range search (Index.range_search): every live row whose score reaches a per-query threshold -----------------
+// The scan is the FILTER epilogue with the threshold below (no sample tiles, cap_s = 0): its per-(query, CTA) counts
+// keep counting past the segment capacity, so a row that passes is either stored or visible as an overflow.  The
+// gather re-scores and filters the candidates in chunks of MDIR_RANGE_CHUNK slots spread over the grid; the emit
+// sorts each query's survivors in shared memory (<= 16,384 of them) and writes them at the query's CSR offset.  A
+// query with more survivors is sorted by groups of MDIR_RANGE_GROUP chunks, then every key is placed at its rank
+// among all of the query's keys (keys are unique: the slot breaks score ties).
+namespace mdir {
+constexpr int kRangeChunk = MDIR_RANGE_CHUNK;
+constexpr int kRangeGroup = MDIR_RANGE_GROUP;
+constexpr int kRangeStage = kRangeChunk * kRangeGroup;      // 16,384 keys: the emit's shared-memory sort
+static_assert(kRangeStage == 16384, "a chunk group is one shared-memory sort");
+
+// tau[q] = the FILTER key that passes every row with score >= lim: (desc_key(lim) << 32) | all index bits.
+// db_stats != NULL: lim = min_score - eps rounded down, eps the certified bound of topk_finalize_kernel, so every row
+// whose fp32 score is >= min_score has a bf16 score >= lim.
+__global__ void __launch_bounds__(256) range_tau_kernel(const float* __restrict__ q32, int D, const float* __restrict__ min_score,
+                                                        const float* __restrict__ db_stats, uint64_t* __restrict__ tau) {
+    __shared__ float red[32];
+    const int q = blockIdx.x;
+    float lim = min_score[q];
+    if (db_stats) {
+        float q2 = 0.f, qt2 = 0.f, qf2 = 0.f;
+        for (int i = threadIdx.x; i < D; i += blockDim.x) {
+            const float v = q32[(int64_t)q * D + i];
+            const float vt = __bfloat162float(__float2bfloat16_rn(v));
+            q2 = fmaf(v, v, q2);
+            qt2 = fmaf(vt, vt, qt2);
+            qf2 = fmaf(v - vt, v - vt, qf2);
+        }
+        q2 = block_sum(q2, red);
+        qt2 = block_sum(qt2, red);
+        qf2 = block_sum(qf2, red);
+        const float e_max = sqrtf(db_stats[0]), x_max = sqrtf(db_stats[1]);
+        float eps = e_max * sqrtf(qt2) + x_max * sqrtf(qf2) + 1.25f * (float)D * 5.9604645e-8f * x_max * sqrtf(q2);
+        eps = eps * 1.001f + 1e-7f;
+        lim = __fsub_rd(lim, eps);
+    }
+    if (threadIdx.x == 0) tau[q] = ((uint64_t)desc_key(lim) << 32) | 0xffffffffull;
+}
+
+// One CTA per (chunk c of kRangeChunk candidate slots, query q).  The candidate slots of q are its scan segments
+// (segment s at cand[q * cand_row + s * cap_l], seg_counts column 1 + s) concatenated after clamping to cap_l.
+// db32 != NULL: each candidate is re-scored in fp32 (one warp per row, always in rescore_row2's summation order) and
+// kept when that score is >= min_score[q].  search's finalize sums a row it re-scores in a pair in that order too, but a
+// row it re-scores alone in rescore_row's; for D > 384 the two orders can differ in the last bits, so a range score is
+// search's bit for bit on paired rows and within a few ulps on the others.  db32 ==
+// NULL: the bf16 keys are kept as they are (the scan threshold was min_score itself).  Survivors go, unsorted, to
+// chunk c of q's survivor row; run_len = their number.  max_seg[q] = the largest raw segment count (> cap_l: overflow).
+__global__ void __launch_bounds__(512) range_gather_kernel(const uint64_t* __restrict__ cand, int64_t cand_row, const uint32_t* __restrict__ seg_counts,
+                                                           int cap_l, const float* __restrict__ min_score, const float* __restrict__ db32,
+                                                           int64_t n_db, uint32_t idx_base, const float* __restrict__ q32, int D,
+                                                           uint64_t* __restrict__ surv, int n_chunks, int32_t* __restrict__ run_len,
+                                                           int32_t* __restrict__ max_seg) {
+    extern __shared__ uint64_t rkeys[];           // kRangeChunk keys, then the query (fp32) when re-scoring
+    __shared__ int s_off[kNumSMs + 1];
+    __shared__ uint32_t s_max, s_n;
+    const int c = blockIdx.x, q = blockIdx.y;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+    if (threadIdx.x < 32) {
+        constexpr int kRounds = (kNumSMs + 31) / 32;
+        int run = 0;
+        uint32_t mx = 0u;
+#pragma unroll
+        for (int i = 0; i < kRounds; ++i) {
+            const int sg = i * 32 + lane;
+            const uint32_t raw = sg < kNumSMs ? seg_counts[(int64_t)q * MDIR_CAND_SEGS + 1 + sg] : 0u;
+            mx = max(mx, raw);
+            const int cl = (int)min(raw, (uint32_t)cap_l);
+            int incl = cl;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int t = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += t;
+            }
+            if (sg < kNumSMs) s_off[sg] = run + incl - cl;
+            run += __shfl_sync(0xffffffffu, incl, 31);
+        }
+        mx = __reduce_max_sync(0xffffffffu, mx);
+        if (lane == 0) { s_off[kNumSMs] = run; s_max = mx; s_n = 0u; }
+    }
+    __syncthreads();
+    if (c == 0 && threadIdx.x == 0) max_seg[q] = (int32_t)min(s_max, 0x7fffffffu);
+    const int lo = c * kRangeChunk;
+    const int n = min(kRangeChunk, s_off[kNumSMs] - lo);
+    if (n <= 0) {
+        if (threadIdx.x == 0) run_len[(int64_t)q * n_chunks + c] = 0;
+        return;
+    }
+    const uint64_t* row = cand + (int64_t)q * cand_row;
+    for (int p = threadIdx.x; p < n; p += blockDim.x) {
+        const int slot = lo + p;
+        int a = 0, b = kNumSMs;                                   // last segment with s_off[sg] <= slot
+        while (b - a > 1) {
+            const int mid = (a + b) >> 1;
+            if (s_off[mid] <= slot) a = mid; else b = mid;
+        }
+        rkeys[p] = row[(int64_t)a * cap_l + (slot - s_off[a])];
+    }
+    if (db32) {
+        float* qs = reinterpret_cast<float*>(rkeys + kRangeChunk);
+        for (int i = threadIdx.x; i < D; i += blockDim.x) qs[i] = q32[(int64_t)q * D + i];
+        __syncthreads();
+        const float m = min_score[q];
+        for (int j = 2 * warp; j < n; j += 2 * n_warps) {
+            const bool two = j + 1 < n;
+            const uint64_t k0 = rkeys[j], k1 = two ? rkeys[j + 1] : k0;
+            const uint32_t g0 = (uint32_t)k0, g1 = (uint32_t)k1;
+            const int64_t r0 = (int64_t)g0 - (int64_t)idx_base, r1 = (int64_t)g1 - (int64_t)idx_base;
+            const bool ok0 = r0 >= 0 && r0 < n_db, ok1 = r1 >= 0 && r1 < n_db;
+            float s0, s1;
+            rescore_row2(db32 + (ok0 ? r0 : 0) * D, db32 + (ok1 ? r1 : 0) * D, qs, D, lane, s0, s1);
+            __syncwarp();
+            if (lane == 0) {
+                rkeys[j] = ok0 && s0 >= m ? make_key(s0, g0) : ~0ull;
+                if (two) rkeys[j + 1] = ok1 && s1 >= m ? make_key(s1, g1) : ~0ull;
+            }
+        }
+    }
+    __syncthreads();
+    uint64_t* out = surv + ((int64_t)q * n_chunks + c) * kRangeChunk;
+    for (int p = threadIdx.x; p < n; p += blockDim.x) {
+        const uint64_t key = rkeys[p];
+        if (key != ~0ull) out[atomicAdd(&s_n, 1u)] = key;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) run_len[(int64_t)q * n_chunks + c] = (int32_t)s_n;
+}
+
+__device__ __forceinline__ void range_write(uint64_t key, int64_t pos, uint32_t idx_base, const uint32_t* __restrict__ slot_id,
+                                            float* __restrict__ out_scores, int32_t* __restrict__ out_ids) {
+    const uint32_t id = slot_id ? slot_id[(uint32_t)key - idx_base] : (uint32_t)key;
+    out_scores[pos] = key_score(key);
+    out_ids[pos] = (int32_t)id;
+}
+
+// One CTA per query whose survivor count lims[q + 1] - lims[q] is in [1, stage_cap]: its chunks' survivors (at
+// run_off within the query) are staged in shared memory, sorted and written to [lims[q], lims[q + 1]).
+__global__ void __launch_bounds__(1024) range_emit_kernel(const uint64_t* __restrict__ surv, int n_chunks, const int32_t* __restrict__ run_len,
+                                                          const int32_t* __restrict__ run_off, const int64_t* __restrict__ lims, int stage_cap,
+                                                          uint32_t idx_base, const uint32_t* __restrict__ slot_id, float* __restrict__ out_scores,
+                                                          int32_t* __restrict__ out_ids) {
+    extern __shared__ uint64_t ekeys[];
+    const int q = blockIdx.x;
+    const int64_t o0 = lims[q];
+    const int cnt = (int)(lims[q + 1] - o0);
+    if (cnt <= 0 || cnt > stage_cap) return;
+    const int lane = threadIdx.x & 31;
+    for (int c = threadIdx.x >> 5; c < n_chunks; c += 32) {
+        const int64_t rc = (int64_t)q * n_chunks + c;
+        const int n = run_len[rc], off = run_off[rc];
+        for (int i = lane; i < n; i += 32) ekeys[off + i] = surv[rc * kRangeChunk + i];
+    }
+    int n2 = 32;
+    while (n2 < cnt) n2 <<= 1;
+    for (int i = cnt + threadIdx.x; i < n2; i += blockDim.x) ekeys[i] = ~0ull;
+    __syncthreads();
+    if (cnt <= 1024) {
+        // rank counting (keys are unique)
+        uint64_t mine = ~0ull;
+        int r = 0;
+        if ((int)threadIdx.x < cnt) {
+            mine = ekeys[threadIdx.x];
+            for (int j = 0; j < cnt; ++j) r += ekeys[j] < mine ? 1 : 0;
+        }
+        __syncthreads();
+        if ((int)threadIdx.x < cnt) ekeys[r] = mine;
+        __syncthreads();
+    } else {
+        bitonic_sort_smem(ekeys, n2);
+    }
+    for (int j = threadIdx.x; j < cnt; j += blockDim.x) range_write(ekeys[j], o0 + j, idx_base, slot_id, out_scores, out_ids);
+}
+
+// One CTA per (group of kRangeGroup chunks, query rows[y]): the group's survivors (<= kRangeStage) sorted in place,
+// contiguous from the group's first chunk.
+__global__ void __launch_bounds__(1024) range_sort_runs_kernel(uint64_t* __restrict__ surv, int n_chunks, const int32_t* __restrict__ run_len,
+                                                               const int32_t* __restrict__ rows) {
+    extern __shared__ uint64_t gkeys[];
+    __shared__ int s_goff[kRangeGroup + 1];
+    const int q = rows[blockIdx.y];
+    const int c0 = blockIdx.x * kRangeGroup, nc = min(kRangeGroup, n_chunks - c0);
+    const int64_t r0 = (int64_t)q * n_chunks + c0;
+    if (threadIdx.x == 0) {
+        int acc = 0;
+        for (int i = 0; i < nc; ++i) { s_goff[i] = acc; acc += run_len[r0 + i]; }
+        s_goff[nc] = acc;
+    }
+    __syncthreads();
+    const int n = s_goff[nc];
+    if (n == 0) return;
+    const int lane = threadIdx.x & 31;
+    for (int i = threadIdx.x >> 5; i < nc; i += 32) {
+        const int len = s_goff[i + 1] - s_goff[i];
+        for (int j = lane; j < len; j += 32) gkeys[s_goff[i] + j] = surv[(r0 + i) * kRangeChunk + j];
+    }
+    int n2 = 32;
+    while (n2 < n) n2 <<= 1;
+    for (int i = n + threadIdx.x; i < n2; i += blockDim.x) gkeys[i] = ~0ull;
+    __syncthreads();
+    bitonic_sort_smem(gkeys, n2);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) surv[r0 * kRangeChunk + i] = gkeys[i];
+}
+
+// One CTA per (group g, query rows[y]) after range_sort_runs_kernel: every key of group g goes to lims[q] + (its index
+// in g) + (keys smaller than it in every other group, by binary search).
+__global__ void __launch_bounds__(256) range_merge_kernel(const uint64_t* __restrict__ surv, int n_chunks, const int32_t* __restrict__ run_len,
+                                                          const int32_t* __restrict__ rows, const int64_t* __restrict__ lims, uint32_t idx_base,
+                                                          const uint32_t* __restrict__ slot_id, float* __restrict__ out_scores,
+                                                          int32_t* __restrict__ out_ids) {
+    extern __shared__ int glen[];
+    const int q = rows[blockIdx.y], g = blockIdx.x;
+    const int n_groups = (n_chunks + kRangeGroup - 1) / kRangeGroup;
+    for (int h = threadIdx.x; h < n_groups; h += blockDim.x) {
+        int acc = 0;
+        for (int c = h * kRangeGroup; c < min(n_chunks, (h + 1) * kRangeGroup); ++c) acc += run_len[(int64_t)q * n_chunks + c];
+        glen[h] = acc;
+    }
+    __syncthreads();
+    const uint64_t* base = surv + (int64_t)q * n_chunks * kRangeChunk;
+    const uint64_t* mine = base + (int64_t)g * kRangeStage;
+    const int64_t o0 = lims[q];
+    for (int i = threadIdx.x; i < glen[g]; i += blockDim.x) {
+        const uint64_t key = mine[i];
+        int64_t r = i;
+        for (int h = 0; h < n_groups; ++h) {
+            if (h == g) continue;
+            const uint64_t* run = base + (int64_t)h * kRangeStage;
+            int a = 0, b = glen[h];                              // keys of run h below `key`
+            while (a < b) {
+                const int mid = (a + b) >> 1;
+                if (run[mid] < key) a = mid + 1; else b = mid;
+            }
+            r += a;
+        }
+        range_write(key, o0 + r, idx_base, slot_id, out_scores, out_ids);
+    }
+}
+}  // namespace mdir
+
+extern "C" int64_t mdir_range_chunks(int64_t cand_row) { return cand_row <= 0 ? 0 : (cand_row + kRangeChunk - 1) / kRangeChunk; }
+
+extern "C" int mdir_range_tau(const float* q32, int n_q, int D, const float* min_score, const float* db_stats, uint64_t* tau, void* stream) {
+    MDIR_CHECK_ARG(min_score && tau && n_q >= 0 && (!db_stats || (q32 && D > 0)));
+    if (n_q == 0) return 0;
+    range_tau_kernel<<<n_q, 256, 0, (cudaStream_t)stream>>>(q32, D, min_score, db_stats, tau);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_range_gather(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int cap_l, int n_q, const float* min_score,
+                                 const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D, uint64_t* surv, int n_chunks,
+                                 int32_t* run_len, int32_t* max_seg, void* stream) {
+    MDIR_CHECK_ARG(cand && seg_counts && min_score && surv && run_len && max_seg && cap_l >= 1 && n_q >= 0 && n_q <= 65535);
+    MDIR_CHECK_ARG(cand_row == (int64_t)kNumSMs * cap_l && n_chunks == mdir_range_chunks(cand_row));
+    MDIR_CHECK_ARG(!db32 || (q32 && n_db >= 0 && D > 0 && D <= 8192 && ((((uintptr_t)db32 | (uintptr_t)q32) & 15) == 0)));
+    if (n_q == 0) return 0;
+    const size_t smem = (size_t)kRangeChunk * 8 + (db32 ? (size_t)D * 4 : 0);
+    static PerDeviceOnce once;
+    if (once.first() != 0) MDIR_CUDA(cudaFuncSetAttribute(range_gather_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRangeChunk * 8 + 8192 * 4));
+    range_gather_kernel<<<dim3(n_chunks, n_q), 512, smem, (cudaStream_t)stream>>>(cand, cand_row, seg_counts, cap_l, min_score, db32, n_db, idx_base,
+                                                                                  q32, D, surv, n_chunks, run_len, max_seg);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_range_emit(const uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* run_off, const int64_t* lims, int n_q,
+                               int stage_cap, uint32_t idx_base, const uint32_t* slot_id, float* out_scores, int32_t* out_ids, void* stream) {
+    MDIR_CHECK_ARG(surv && run_len && run_off && lims && out_scores && out_ids && n_chunks >= 1 && n_q >= 0);
+    MDIR_CHECK_ARG(stage_cap >= 32 && stage_cap <= kRangeStage && (stage_cap & (stage_cap - 1)) == 0);
+    if (n_q == 0) return 0;
+    static PerDeviceOnce once;
+    if (once.first() != 0) MDIR_CUDA(cudaFuncSetAttribute(range_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRangeStage * 8));
+    range_emit_kernel<<<n_q, 1024, (size_t)stage_cap * 8, (cudaStream_t)stream>>>(surv, n_chunks, run_len, run_off, lims, stage_cap, idx_base, slot_id,
+                                                                                 out_scores, out_ids);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_range_sort_runs(uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* rows, int n_rows, void* stream) {
+    MDIR_CHECK_ARG(surv && run_len && rows && n_chunks >= 1 && n_rows >= 0 && n_rows <= 65535);
+    if (n_rows == 0) return 0;
+    static PerDeviceOnce once;
+    if (once.first() != 0) MDIR_CUDA(cudaFuncSetAttribute(range_sort_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRangeStage * 8));
+    const int n_groups = (n_chunks + kRangeGroup - 1) / kRangeGroup;
+    range_sort_runs_kernel<<<dim3(n_groups, n_rows), 1024, (size_t)kRangeStage * 8, (cudaStream_t)stream>>>(surv, n_chunks, run_len, rows);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_range_merge(const uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* rows, int n_rows, const int64_t* lims,
+                                uint32_t idx_base, const uint32_t* slot_id, float* out_scores, int32_t* out_ids, void* stream) {
+    MDIR_CHECK_ARG(surv && run_len && rows && lims && out_scores && out_ids && n_chunks >= 1 && n_rows >= 0 && n_rows <= 65535);
+    const int n_groups = (n_chunks + kRangeGroup - 1) / kRangeGroup;
+    MDIR_CHECK_ARG(n_groups <= 12288);                  // group lengths in the default 48 KB of shared memory
+    if (n_rows == 0) return 0;
+    range_merge_kernel<<<dim3(n_groups, n_rows), 256, (size_t)n_groups * 4, (cudaStream_t)stream>>>(surv, n_chunks, run_len, rows, lims, idx_base,
+                                                                                                   slot_id, out_scores, out_ids);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}

@@ -12,7 +12,8 @@ Replaces, for mdir's evaluation (mdir/components/optim/score/cirscore.py:65-70):
                                 = the dense path.  Rows can be removed, restored and appended in
                                 place (``remove`` / ``restore`` / ``add``: a live-row bitmap the
                                 scan reads); ``compact`` purges removed rows and shrinks the scan to the
-                                live ones, ids unchanged.
+                                live ones, ids unchanged.  ``range_search`` = every live row whose
+                                score reaches a per-query threshold (CSR output, exact fp32).
 * ``ShardedIndex``           -- rows sharded contiguously over the ranks of a torch.distributed
                                 group; local top-k + one all-gather of N_q*k keys + merge.
 * ``ranks_from_scores`` / ``topk_from_scores`` -- the sort/selection kernels fed an existing
@@ -57,6 +58,16 @@ I8_MAX_REL_RESIDUAL = 0.02
 #   500 k / 750 k rows: certified, but 0.424 / 0.525 ms per step against bf16's 0.363 / 0.515;
 #   1 M rows: 0.652 against 0.666.
 I8_MIN_ROWS = 900000
+# range_search: initial capacity of each scan CTA's candidate segment.  At 10,000 fp32 matches per query in 1 M rows the
+# scan passes ~14,000 candidates (the certified bound lowers its threshold), ~92 per segment on average; a block whose
+# segments still overflow is re-scanned once at the exact capacity the counts report.
+RANGE_CAP_L = 192
+RANGE_CHUNK = 1024      # MDIR_RANGE_CHUNK: candidate slots per CTA of mdir_range_gather
+RANGE_STAGE = 16384     # survivors of one query that mdir_range_emit sorts in shared memory; more take the group merge
+# bytes of candidate + survivor keys (8 B each, 148 * cap_l + chunks * RANGE_CHUNK per query) one re-scan may hold: a
+# block whose exact counts need more is re-scanned in smaller query groups (min_score = -inf over 1 M rows needs ~16 MB
+# per query, so 32 queries per group)
+RANGE_BUDGET = 1 << 29
 
 
 def default_shortlist(k):
@@ -140,6 +151,51 @@ def compaction_schedule(live, chunk):
     return out
 
 
+def range_thresholds(min_score, nq):
+    """min_score (a float, or one per query: tensor / array / sequence of nq) -> (nq,) float32 numpy.  A float64 value is
+    rounded UP to float32, so that an fp32 score passes the float32 threshold exactly when it is >= the value given.
+    MdirError on NaN or a wrong length."""
+    if isinstance(min_score, torch.Tensor):
+        min_score = min_score.detach().cpu().numpy()
+    a = np.asarray(min_score, dtype=np.float64)
+    if a.ndim == 0:
+        a = np.full((nq,), float(a))
+    if a.shape != (nq,):
+        raise _lib.MdirError("min_score must be a float or hold one value per query (%d), got shape %s" % (nq, a.shape))
+    if np.isnan(a).any():
+        raise _lib.MdirError("min_score is NaN for query %d" % int(np.flatnonzero(np.isnan(a))[0]))
+    a32 = a.astype(np.float32)
+    low = a32.astype(np.float64) < a
+    a32[low] = np.nextafter(a32[low], np.float32(np.inf))
+    return a32
+
+
+def range_chunks(cap_l):
+    """mdir_range_chunks: gather chunks covering one candidate row of 148 segments of cap_l keys."""
+    return -(-148 * int(cap_l) // RANGE_CHUNK)
+
+
+def range_csr(run_len):
+    """run_len (nq, n_chunks): survivors of every gather chunk -> (counts (nq,) int64, lims (nq + 1,) int64 -- the CSR
+    offsets, query i at [lims[i], lims[i + 1]) --, run_off (nq, n_chunks) int32: survivors of the query before chunk c)."""
+    run_len = np.asarray(run_len, dtype=np.int64)
+    counts = run_len.sum(axis=1)
+    lims = np.zeros((run_len.shape[0] + 1,), dtype=np.int64)
+    np.cumsum(counts, out=lims[1:])
+    run_off = np.ascontiguousarray(np.cumsum(run_len, axis=1) - run_len, dtype=np.int32)
+    return counts, lims, run_off
+
+
+def range_rescan_plan(max_seg, budget=RANGE_BUDGET):
+    """After a range scan overflowed: (cap_l, group) = the segment capacity that holds the largest count any segment
+    reported (rounded up to 32), and how many queries one re-scan takes so that its candidate + survivor keys stay
+    within `budget` bytes (at least one)."""
+    max_seg = np.asarray(max_seg, dtype=np.int64)
+    cap = max(32, -(-int(max_seg.max()) // 32) * 32)
+    per_query = 8 * (148 * cap + range_chunks(cap) * RANGE_CHUNK)
+    return cap, int(max(1, min(max_seg.size, budget // per_query)))
+
+
 def ids_for_rank(ids, ranges, rank):
     """Global ids -> the int64 numpy ids that rank `rank` owns, ranges[r] = (first id, end id) of rank r (see
     ShardedIndex.shard_bounds).  MdirError when an id lies in no rank's range."""
@@ -209,6 +265,7 @@ class Index:
         self.db8 = self.row_scale = None
         self.route = None
         self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0, "int8_blocks": 0, "int8_redone": 0}
+        self.range_stats = {"queries": 0, "blocks": 0, "rescans": 0, "rescan_groups": 0, "large_sorts": 0}
 
     @classmethod
     def from_packed(cls, db16, db32=None, idx_base=0):
@@ -225,6 +282,7 @@ class Index:
         self.db8 = self.row_scale = None
         self.route = None
         self.cert = {"queries": 0, "flagged": 0, "widened_blocks": 0, "uncertified": 0, "int8_blocks": 0, "int8_redone": 0}
+        self.range_stats = {"queries": 0, "blocks": 0, "rescans": 0, "rescan_groups": 0, "large_sorts": 0}
         return self
 
     # ------------------------------------------------------------------ live rows
@@ -711,6 +769,151 @@ class Index:
     def status(self):
         """Per-query status words of the last search (0 = exact and, for precision='fp32', certified)."""
         return self._ovf
+
+    def range_search(self, q, min_score, precision="fp32", check=True):
+        """Every live row whose score against query i is >= min_score (a float, or a (N_q,) tensor: one per query).
+        q: (N_q, D) fp32 (host or device).  Returns (lims (N_q + 1,) int64, scores fp32, ids int32), all on the device, in
+        the CSR layout of FAISS range_search: the results of query i are scores / ids[lims[i]:lims[i + 1]], ordered by
+        (score desc, id asc) as search() orders them; ids go through the slot -> id map.
+
+        precision="fp32": the exact fp32 score (one fixed summation order: the one search(precision="fp32") uses for the
+                          rows it re-scores in pairs, e.g. its whole shortlist at k = 100; a row search re-scores alone
+                          is summed in another order and can differ from the range score in the last bits when
+                          D > 384).  The bf16 scan
+                          passes every row within the certified bound eps of min_score; those rows are re-scored in fp32
+                          and filtered, so the result is complete by construction (no threshold to guess, no widening).
+        precision="bf16": the bf16-input / fp32-accumulate scan score, as search(precision="bf16") reports it.
+        One scan per block of 128 queries.  A candidate segment that overflowed is visible in the scan's exact counts;
+        check=True re-scans that block once with segments sized from them (in smaller query groups when they exceed
+        RANGE_BUDGET; range_stats counts both), check=False returns the block as it is with status bit 0 raised for the
+        truncated queries (status() / check_overflow()).  NaN in min_score raises MdirError."""
+        lib = _lib.lib()
+        with torch.cuda.device(self.device):
+            q32 = _as_dev_f32(q, self.device)
+            if q32.dim() != 2 or q32.shape[1] != self.D:
+                raise _lib.MdirError("range_search expects (N_q, %d) queries, got %s" % (self.D, tuple(q32.shape)))
+            if precision == "fp32":
+                if self.db32 is None:
+                    raise _lib.MdirError("precision='fp32' needs keep_fp32=True")
+            elif precision != "bf16":
+                raise ValueError("precision must be 'fp32' or 'bf16'")
+            nq_all = q32.shape[0]
+            m_host = range_thresholds(min_score, nq_all)
+            parts = []                          # (counts, scores, ids, status) of consecutive query groups
+            if nq_all and self._n_used:       # an index with every row removed scans and returns nothing
+                m_all = torch.from_numpy(m_host).to(self.device)
+                stats = self.stats() if precision == "fp32" else None
+                q16 = pack_bf16(q32)
+                tau = torch.empty((nq_all,), dtype=torch.int64, device=self.device)
+                _lib.check(lib.mdir_range_tau(_lib.ptr(q32), nq_all, self.D, _lib.ptr(m_all), _lib.ptr(stats), _lib.ptr(tau), _lib.stream()),
+                           "mdir_range_tau")
+                for q0 in range(0, nq_all, MAX_Q):
+                    q1 = min(q0 + MAX_Q, nq_all)
+                    parts += self._range_block(q16[q0:q1], q32[q0:q1], m_all[q0:q1], tau[q0:q1], stats, check)
+                self.range_stats["queries"] += nq_all
+            else:
+                parts.append((np.zeros((nq_all,), dtype=np.int64), torch.empty((0,), dtype=torch.float32, device=self.device),
+                              torch.empty((0,), dtype=torch.int32, device=self.device), np.zeros((nq_all,), dtype=np.int32), None))
+            status = np.concatenate([p[3] for p in parts])
+            self._ovf = torch.from_numpy(status).to(self.device) if status.any() else torch.zeros((nq_all,), dtype=torch.int32, device=self.device)
+            if len(parts) == 1:
+                out_s, out_i, lims = parts[0][1], parts[0][2], parts[0][4]
+            else:
+                out_s, out_i, lims = torch.cat([p[1] for p in parts]), torch.cat([p[2] for p in parts]), None
+            if lims is None:                    # several groups (or nothing to emit): offsets of the concatenation
+                lims_h = np.zeros((nq_all + 1,), dtype=np.int64)
+                np.cumsum(np.concatenate([p[0] for p in parts]), out=lims_h[1:])
+                lims = torch.from_numpy(lims_h).to(self.device)
+            return lims, out_s, out_i
+
+    def _range_block(self, q16, q32, m, tau, stats, check):
+        """One block of <= 128 queries -> [(counts, scores, ids, status, lims)] for consecutive groups of its queries."""
+        nq = q16.shape[0]
+        self.range_stats["blocks"] += 1
+        bufs = self._range_bufs(RANGE_CAP_L, MAX_Q, cached=True)
+        run_len, max_seg = self._range_pass(q16, q32, m, tau, stats, RANGE_CAP_L, bufs)
+        over = max_seg > RANGE_CAP_L
+        if not check or not over.any():
+            return [self._range_emit(bufs, run_len, over)]
+        # the exact counts say how deep every segment has to be: one re-scan, in query groups that fit the budget
+        self.range_stats["rescans"] += 1
+        cap, group = range_rescan_plan(max_seg)
+        out = []
+        for g0 in range(0, nq, group):
+            g1 = min(g0 + group, nq)
+            self.range_stats["rescan_groups"] += 1
+            bufs = self._range_bufs(cap, g1 - g0, cached=False)
+            run_len, max_seg = self._range_pass(q16[g0:g1], q32[g0:g1], m[g0:g1], tau[g0:g1], stats, cap, bufs)
+            if (max_seg > cap).any():
+                raise _lib.MdirError("range_search re-scan overflowed its exact capacity (internal error)")
+            out.append(self._range_emit(bufs, run_len, max_seg > cap))
+        return out
+
+    def _range_bufs(self, cap_l, rows, cached):
+        """Candidate rows, segment counts, survivors and the gather's per-chunk counts + max segment counts of a range
+        scan with segment capacity cap_l.  The default capacity's buffers are kept (through _buf, apart from search()'s
+        candidate buffers, so a range call never changes a later search); a re-scan's are freed with the call."""
+        n_chunks = range_chunks(cap_l)
+        shapes = (("range_cand", (rows, 148 * cap_l), torch.int64), ("range_segcnt", (rows, N_SEGS), torch.int32),
+                  ("range_surv", (rows, n_chunks * RANGE_CHUNK), torch.int64), ("range_runs", (rows * (n_chunks + 1),), torch.int32))
+        if cached:
+            return tuple(self._buf(n, sh, dt) for n, sh, dt in shapes)
+        return tuple(torch.empty(sh, dtype=dt, device=self.device) for _, sh, dt in shapes)
+
+    def _range_pass(self, q16, q32, m, tau, stats, cap_l, bufs):
+        """FILTER scan of every used slot at threshold tau, then the gather -> (run_len (nq, n_chunks), max_seg (nq,)),
+        read back in one copy (the call's synchronisation point).  stats None: bf16 scores, no re-scoring."""
+        lib = _lib.lib()
+        nq = q16.shape[0]
+        cand, cnt, surv, runs = bufs
+        n_chunks = range_chunks(cap_l)
+        cnt[:nq].zero_()                    # the scan writes the segments of the CTAs it launches; the rest stay empty
+        prof = getattr(self, "prof", None)
+        if prof is not None:
+            prof.begin()
+        _lib.check(lib.mdir_sim_scan_bf16_extent(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, 2, 0, 0, None, 0, _lib.ptr(tau),
+                                                 self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, cap_l, _lib.ptr(self.live),
+                                                 _lib.ptr(self.n_scan), _lib.stream()), "mdir_sim_scan_bf16_extent")
+        if prof is not None:
+            prof.end(self._n_used * self.D * 2)
+        run_len, max_seg = runs[:nq * n_chunks], runs[nq * n_chunks:nq * (n_chunks + 1)]
+        _lib.check(lib.mdir_range_gather(_lib.ptr(cand), 148 * cap_l, _lib.ptr(cnt), cap_l, nq, _lib.ptr(m),
+                                         _lib.ptr(self.db32 if stats is not None else None), self.n, self.idx_base, _lib.ptr(q32), self.D,
+                                         _lib.ptr(surv), n_chunks, _lib.ptr(run_len), _lib.ptr(max_seg), _lib.stream()), "mdir_range_gather")
+        host = runs[:nq * (n_chunks + 1)].cpu().numpy()
+        return host[:nq * n_chunks].reshape(nq, n_chunks), host[nq * n_chunks:]
+
+    def _range_emit(self, bufs, run_len, over):
+        """Sorted CSR output of one range pass -> (counts, scores, ids, status, lims on the device or None) of its queries."""
+        lib = _lib.lib()
+        _, _, surv, runs = bufs
+        nq, n_chunks = run_len.shape
+        counts, lims, run_off = range_csr(run_len)
+        total = int(lims[-1])
+        scores = torch.empty((total,), dtype=torch.float32, device=self.device)
+        ids = torch.empty((total,), dtype=torch.int32, device=self.device)
+        lims_d = None
+        if total:
+            lims_d = torch.from_numpy(lims).to(self.device)
+            small = counts[(counts > 0) & (counts <= RANGE_STAGE)]
+            if small.size:
+                stage = 32
+                while stage < int(small.max()):
+                    stage *= 2
+                off_d = torch.from_numpy(run_off).to(self.device)
+                _lib.check(lib.mdir_range_emit(_lib.ptr(surv), n_chunks, _lib.ptr(runs), _lib.ptr(off_d), _lib.ptr(lims_d), nq, stage, self.idx_base,
+                                               _lib.ptr(self.slot_id), _lib.ptr(scores), _lib.ptr(ids), _lib.stream()), "mdir_range_emit")
+            big = np.flatnonzero(counts > RANGE_STAGE).astype(np.int32)
+            if big.size:
+                self.range_stats["large_sorts"] += int(big.size)
+                rows = torch.from_numpy(big).to(self.device)
+                _lib.check(lib.mdir_range_sort_runs(_lib.ptr(surv), n_chunks, _lib.ptr(runs), _lib.ptr(rows), int(big.size), _lib.stream()),
+                           "mdir_range_sort_runs")
+                _lib.check(lib.mdir_range_merge(_lib.ptr(surv), n_chunks, _lib.ptr(runs), _lib.ptr(rows), int(big.size), _lib.ptr(lims_d),
+                                                self.idx_base, _lib.ptr(self.slot_id), _lib.ptr(scores), _lib.ptr(ids), _lib.stream()),
+                           "mdir_range_merge")
+        status = np.where(np.asarray(over, dtype=bool), STATUS_OVERFLOW, 0).astype(np.int32)
+        return counts, scores, ids, status, lims_d
 
     def _split3(self, x, role):
         """(n, D) fp32 -> (n, 3D) fp32 [hi|hi|lo] (role 0) / [hi|lo|hi] (role 1) for the 3xTF32 scan."""
