@@ -405,6 +405,16 @@ int mdir_range_sort_runs(uint64_t* surv, int n_chunks, const int32_t* run_len, c
 int mdir_range_merge(const uint64_t* surv, int n_chunks, const int32_t* run_len, const int32_t* rows, int n_rows,
                      const int64_t* lims, uint32_t idx_base, const uint32_t* slot_id, float* out_scores,
                      int32_t* out_ids, void* stream);
+/* mdir_range_offsets: the CSR offsets of a range step on the device, from the gather's run_len (n_q, n_chunks) and
+ *   max_seg (n_q,), without a host round trip (captured range steps).  run_off (n_q, n_chunks) = survivors of the
+ *   query before each chunk.  A query is emitted when its survivors are <= max_results (1 .. 16384) and
+ *   max_seg[q] <= cap_l; any other query counts 0, with status[q] = MDIR_STATUS_OVERFLOW (a segment overflowed)
+ *   and/or MDIR_STATUS_RANGE_FULL (more survivors than max_results), else 0.  lims (n_q + 1) = exclusive prefix
+ *   sum of the emitted counts, at most n_q * max_results.  One CTA: 1 <= n_q <= 1024.  Feed mdir_range_emit with
+ *   stage_cap = max_results rounded up to a power of two (at least 32).                                          */
+#define MDIR_STATUS_RANGE_FULL  8
+int mdir_range_offsets(const int32_t* run_len, const int32_t* max_seg, int n_q, int n_chunks, int cap_l,
+                       int max_results, int64_t* lims, int32_t* run_off, int32_t* status, void* stream);
 
 /* stats[2] (device) = {max_r ||bf16(x_r) - x_r||_2^2, max_r ||x_r||_2^2} over the n rows of a shard:
  * the database half of the certificate's error bound.  db16 = mdir_pack_bf16(db32).            */

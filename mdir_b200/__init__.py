@@ -16,7 +16,8 @@ from ._lib import MdirError, lib  # noqa: F401
 from .layers import GeM, MAC, SPoC, L2N, POOLING, gem, mac, spoc, l2n  # noqa: F401
 from .wrappers import CirMultiscaleAggregation, CirtorchWhiten, RetrievalHead, whitenapply  # noqa: F401
 from .clahe import clahe_u8, image_clahe, ChannelClahe, ImageClahe, ApplyClahe, AddClaheFromRgb, CreateClahedImage  # noqa: F401
-from .search import Index, ShardedIndex, GraphedSearch, SearchPipeline, rank, ranks_from_scores, topk_from_scores  # noqa: F401
+from .search import (Index, ShardedIndex, GraphedSearch, SearchPipeline, GraphedRangeSearch, RangePipeline, rank,  # noqa: F401
+                     ranks_from_scores, topk_from_scores)
 from .extract import extract_vectors, extract_from_tensors  # noqa: F401
 from .evaluate import compute_map, compute_map_and_print  # noqa: F401
 from .score import install  # noqa: F401

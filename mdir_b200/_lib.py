@@ -76,6 +76,7 @@ PROTOTYPES = {
     "mdir_range_emit": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _u32, _vp, _vp, _vp, _vp]),
     "mdir_range_sort_runs": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "mdir_range_merge": (_i, [_vp, _i, _vp, _vp, _i, _vp, _u32, _vp, _vp, _vp, _vp]),
+    "mdir_range_offsets": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "mdir_pack_stats": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
     "mdir_pack_stats_i8": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "mdir_pack_q_i8": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),

@@ -1618,6 +1618,51 @@ __global__ void __launch_bounds__(256) range_merge_kernel(const uint64_t* __rest
         range_write(key, o0 + r, idx_base, slot_id, out_scores, out_ids);
     }
 }
+
+// One CTA, thread q = query q (n_q <= 1024): the CSR offsets of a captured range step, computed where the gather left
+// its counts (the eager route reads them back and builds them on the host).  run_off[q, c] = survivors of q before chunk
+// c.  A query is emitted when its survivors fit max_results and no segment overflowed cap_l; any other query counts 0 and
+// gets MDIR_STATUS_OVERFLOW and/or MDIR_STATUS_RANGE_FULL.  lims = exclusive prefix sum of the emitted counts, so the
+// output never exceeds n_q * max_results.
+__global__ void __launch_bounds__(1024) range_offsets_kernel(const int32_t* __restrict__ run_len, const int32_t* __restrict__ max_seg, int n_q,
+                                                             int n_chunks, int cap_l, int max_results, int64_t* __restrict__ lims,
+                                                             int32_t* __restrict__ run_off, int32_t* __restrict__ status) {
+    __shared__ int warp_tot[32];
+    const int q = threadIdx.x, lane = q & 31, warp = q >> 5;
+    int count = 0;
+    if (q < n_q) {
+        int acc = 0;
+        for (int c = 0; c < n_chunks; ++c) {
+            run_off[(int64_t)q * n_chunks + c] = acc;
+            acc += run_len[(int64_t)q * n_chunks + c];
+        }
+        const int st = (max_seg[q] > cap_l ? MDIR_STATUS_OVERFLOW : 0) | (acc > max_results ? MDIR_STATUS_RANGE_FULL : 0);
+        status[q] = st;
+        count = st ? 0 : acc;
+    }
+    int incl = count;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) warp_tot[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        const int w = lane < (int)(blockDim.x >> 5) ? warp_tot[lane] : 0;
+        int wi = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, wi, o);
+            if (lane >= o) wi += t;
+        }
+        warp_tot[lane] = wi - w;
+    }
+    __syncthreads();
+    const int64_t excl = (int64_t)warp_tot[warp] + incl - count;
+    if (q < n_q) lims[q] = excl;
+    if (q == n_q - 1) lims[n_q] = excl + count;
+}
 }  // namespace mdir
 
 extern "C" int64_t mdir_range_chunks(int64_t cand_row) { return cand_row <= 0 ? 0 : (cand_row + kRangeChunk - 1) / kRangeChunk; }
@@ -1678,6 +1723,16 @@ extern "C" int mdir_range_merge(const uint64_t* surv, int n_chunks, const int32_
     if (n_rows == 0) return 0;
     range_merge_kernel<<<dim3(n_groups, n_rows), 256, (size_t)n_groups * 4, (cudaStream_t)stream>>>(surv, n_chunks, run_len, rows, lims, idx_base,
                                                                                                    slot_id, out_scores, out_ids);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_range_offsets(const int32_t* run_len, const int32_t* max_seg, int n_q, int n_chunks, int cap_l, int max_results,
+                                  int64_t* lims, int32_t* run_off, int32_t* status, void* stream) {
+    MDIR_CHECK_ARG(run_len && max_seg && lims && run_off && status && n_q >= 1 && n_q <= 1024 && n_chunks >= 1 && cap_l >= 1);
+    MDIR_CHECK_ARG(max_results >= 1 && max_results <= kRangeStage);
+    range_offsets_kernel<<<1, (n_q + 31) / 32 * 32, 0, (cudaStream_t)stream>>>(run_len, max_seg, n_q, n_chunks, cap_l, max_results, lims,
+                                                                               run_off, status);
     MDIR_LAUNCH_CHECK();
     return 0;
 }

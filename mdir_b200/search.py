@@ -43,6 +43,7 @@ TARGET_CAND = 4500    # candidates per query the sampling plan aims for (kth * n
 
 
 STATUS_OVERFLOW, STATUS_UNCERTIFIED, STATUS_PEER_TIMEOUT = 1, 2, 4     # MDIR_STATUS_* (+ the exchange's own bit)
+STATUS_RANGE_FULL = 8     # MDIR_STATUS_RANGE_FULL: a captured range step found more survivors than max_results
 MAX_KTH = 4096        # deepest selection the finalize kernel stages
 # int8 first pass (Index._i8_route): taken only when every row's int8 residual is small against the row,
 # max_r ||x_r - s_r x8_r|| / ||x_r|| below this.  Unit randn rows at D = 2048 measure 0.013, where the certified bound
@@ -194,6 +195,43 @@ def range_rescan_plan(max_seg, budget=RANGE_BUDGET):
     cap = max(32, -(-int(max_seg.max()) // 32) * 32)
     per_query = 8 * (148 * cap + range_chunks(cap) * RANGE_CHUNK)
     return cap, int(max(1, min(max_seg.size, budget // per_query)))
+
+
+def range_stage_cap(max_results):
+    """mdir_range_emit's stage_cap for a captured range step: max_results rounded up to a power of two, at least 32."""
+    stage = 32
+    while stage < int(max_results):
+        stage *= 2
+    return stage
+
+
+def range_splice(lims, scores, ids, flagged, sub_lims, sub_scores, sub_ids):
+    """Replace the results of the queries `flagged` (ascending query numbers) in the CSR (lims, scores, ids) by the CSR
+    (sub_lims, sub_scores, sub_ids) of those queries, in the same order -> a new packed CSR (lims, scores, ids), numpy.
+    RangePipeline's recovery: the flagged queries of a captured step redone by Index.range_search."""
+    lims, sub_lims = np.asarray(lims, dtype=np.int64), np.asarray(sub_lims, dtype=np.int64)
+    flagged = np.asarray(flagged, dtype=np.int64).ravel()
+    nq = lims.size - 1
+    if flagged.size and (flagged[0] < 0 or flagged[-1] >= nq or (np.diff(flagged) <= 0).any()):
+        raise _lib.MdirError("range_splice: flagged must be ascending query numbers in [0, %d)" % nq)
+    if sub_lims.size != flagged.size + 1:
+        raise _lib.MdirError("range_splice: %d flagged queries need %d sub_lims, got %d" % (flagged.size, flagged.size + 1, sub_lims.size))
+    sub_of = np.full((nq,), -1, dtype=np.int64)
+    sub_of[flagged] = np.arange(flagged.size)
+    counts = np.diff(lims)
+    counts[flagged] = np.diff(sub_lims)
+    out_lims = np.zeros((nq + 1,), dtype=np.int64)
+    np.cumsum(counts, out=out_lims[1:])
+    out_s = np.empty((int(out_lims[-1]),), dtype=np.asarray(scores).dtype)
+    out_i = np.empty((int(out_lims[-1]),), dtype=np.asarray(ids).dtype)
+    for j in range(nq):
+        a, b = out_lims[j], out_lims[j + 1]
+        if sub_of[j] < 0:
+            out_s[a:b], out_i[a:b] = scores[lims[j]:lims[j + 1]], ids[lims[j]:lims[j + 1]]
+        else:
+            k = sub_of[j]
+            out_s[a:b], out_i[a:b] = sub_scores[sub_lims[k]:sub_lims[k + 1]], sub_ids[sub_lims[k]:sub_lims[k + 1]]
+    return out_lims, out_s, out_i
 
 
 def ids_for_rank(ids, ranges, rank):
@@ -861,8 +899,18 @@ class Index:
         return tuple(torch.empty(sh, dtype=dt, device=self.device) for _, sh, dt in shapes)
 
     def _range_pass(self, q16, q32, m, tau, stats, cap_l, bufs):
-        """FILTER scan of every used slot at threshold tau, then the gather -> (run_len (nq, n_chunks), max_seg (nq,)),
-        read back in one copy (the call's synchronisation point).  stats None: bf16 scores, no re-scoring."""
+        """_range_launch, then run_len (nq, n_chunks) and max_seg (nq,) read back in one copy (the call's synchronisation
+        point)."""
+        nq = q16.shape[0]
+        n_chunks = range_chunks(cap_l)
+        self._range_launch(q16, q32, m, tau, stats, cap_l, bufs)
+        host = bufs[3][:nq * (n_chunks + 1)].cpu().numpy()
+        return host[:nq * n_chunks].reshape(nq, n_chunks), host[nq * n_chunks:]
+
+    def _range_launch(self, q16, q32, m, tau, stats, cap_l, bufs):
+        """FILTER scan of every used slot at threshold tau, then the gather -> device views (run_len (nq * n_chunks,),
+        max_seg (nq,)) of bufs' runs.  No host synchronisation (GraphedRangeSearch captures it).  stats None: bf16
+        scores, no re-scoring."""
         lib = _lib.lib()
         nq = q16.shape[0]
         cand, cnt, surv, runs = bufs
@@ -880,8 +928,7 @@ class Index:
         _lib.check(lib.mdir_range_gather(_lib.ptr(cand), 148 * cap_l, _lib.ptr(cnt), cap_l, nq, _lib.ptr(m),
                                          _lib.ptr(self.db32 if stats is not None else None), self.n, self.idx_base, _lib.ptr(q32), self.D,
                                          _lib.ptr(surv), n_chunks, _lib.ptr(run_len), _lib.ptr(max_seg), _lib.stream()), "mdir_range_gather")
-        host = runs[:nq * (n_chunks + 1)].cpu().numpy()
-        return host[:nq * n_chunks].reshape(nq, n_chunks), host[nq * n_chunks:]
+        return run_len, max_seg
 
     def _range_emit(self, bufs, run_len, over):
         """Sorted CSR output of one range pass -> (counts, scores, ids, status, lims on the device or None) of its queries."""
@@ -1582,7 +1629,83 @@ class GraphedSearch:
         return bool(self.status.any().item())
 
 
-class SearchPipeline:
+class _Pipeline:
+    """The ticket slots and the mutation ordering that SearchPipeline and RangePipeline share.  A subclass sets index,
+    local, depth, overlap, the streams compute / d2h (and exch when overlap) and self.slots: one dict per slot with at
+    least "pending" (a ticket is in flight) and "live" (the bitmap copy its recovery reads, None: the current one)."""
+
+    def _mutate(self, fn):
+        """Run a mutation of the index on the compute stream, after every replay already queued there (and, in overlap
+        mode, after the finalize / exchange queued on the exchange stream, which read the rows and stats that add()
+        writes).  Tickets in flight keep a device copy of the live bitmap they were submitted with: a ticket redone by
+        result()'s recovery path then sees the same rows as its replay did.  A copy is dropped when its last ticket is
+        collected."""
+        dev = self.local.device
+        with torch.cuda.device(dev):
+            if self.overlap:
+                self.compute.wait_stream(self.exch)
+            with torch.cuda.stream(self.compute):
+                waiting = [sl for sl in self.slots if sl["pending"] and sl["live"] is None]
+                if waiting:
+                    snap = self.local.live.clone()
+                    for sl in waiting:
+                        sl["live"] = snap
+                return fn()
+
+    def remove(self, ids):
+        """index.remove(ids) between tickets: tickets submitted before this call do not see it, later ones do.  With a
+        ShardedIndex, ids are global and every rank makes the same call at the same point of its ticket sequence."""
+        self._mutate(lambda: self.index.remove(ids))
+
+    def restore(self, ids):
+        """index.restore(ids) between tickets (see remove())."""
+        self._mutate(lambda: self.index.restore(ids))
+
+    def add(self, vecs):
+        """index.add(vecs) between tickets (see remove()); returns the new ids.  Single-GPU Index only."""
+        if isinstance(self.index, ShardedIndex):
+            raise _lib.MdirError("%s.add() needs an Index: ShardedIndex has no add()" % type(self).__name__)
+        return self._mutate(lambda: self.index.add(vecs))
+
+    def compact(self):
+        """index.compact() on the compute stream, after the replays and exchanges already queued.  A maintenance step:
+        collect every ticket first -- MdirError while one is pending, because the live-row copy a ticket keeps for its
+        recovery path describes the slot layout compaction changes.  The graphs keep working without re-capture, and
+        tickets submitted afterwards see the compacted index.  With a ShardedIndex every rank calls it at the same point.
+        Returns the rows purged (on this rank)."""
+        pending = [sl for sl in self.slots if sl["pending"]]
+        if pending:
+            raise _lib.MdirError("%s.compact(): collect the %d pending ticket(s) first" % (type(self).__name__, len(pending)))
+        return self._mutate(self.index.compact)
+
+    def _free_slot(self, ticket):
+        """The slot of a ticket about to be submitted; MdirError while the ticket `depth` before it is uncollected."""
+        slot = self.slots[ticket % self.depth]
+        if slot["pending"]:
+            raise _lib.MdirError("%s: collect result() of ticket %d before submitting more" % (type(self).__name__, ticket - self.depth))
+        return slot
+
+    def _pending_slot(self, ticket):
+        """The slot of a ticket in flight whose result has not been collected; MdirError otherwise."""
+        if not (self.n_submitted - self.depth <= ticket < self.n_submitted):
+            raise _lib.MdirError("%s: ticket %d is not in flight" % (type(self).__name__, ticket))
+        slot = self.slots[ticket % self.depth]
+        if not slot["pending"]:
+            raise _lib.MdirError("%s: result(%d) was already collected" % (type(self).__name__, ticket))
+        return slot
+
+    def _map(self, batches, submit):
+        """Generator of result()s over `batches`, each passed to submit, keeping `depth` tickets in flight."""
+        tickets = []
+        for b in batches:
+            if len(tickets) == self.depth:
+                yield self.result(tickets.pop(0))
+            tickets.append(submit(b))
+        for t in tickets:
+            yield self.result(t)
+
+
+class SearchPipeline(_Pipeline):
     """Host-facing serving loop: query batches arrive in (pinned) host memory, results go back to
     pinned host memory, and the copies of one step overlap the scan of its neighbours.
 
@@ -1653,50 +1776,6 @@ class SearchPipeline:
         self.n_submitted = 0
         self.n_recovered = 0          # steps redone exactly because a status word was raised
 
-    def _mutate(self, fn):
-        """Run a mutation of the index on the compute stream, after every replay already queued there (and, in overlap
-        mode, after the finalize / exchange queued on the exchange stream, which read the rows and stats that add()
-        writes).  Tickets in flight keep a device copy of the live bitmap they were submitted with: a ticket redone by
-        result()'s recovery path then sees the same rows as its replay did.  A copy is dropped when its last ticket is
-        collected."""
-        dev = self.local.device
-        with torch.cuda.device(dev):
-            if self.overlap:
-                self.compute.wait_stream(self.exch)
-            with torch.cuda.stream(self.compute):
-                waiting = [sl for sl in self.slots if sl["pending"] and sl["live"] is None]
-                if waiting:
-                    snap = self.local.live.clone()
-                    for sl in waiting:
-                        sl["live"] = snap
-                return fn()
-
-    def remove(self, ids):
-        """index.remove(ids) between tickets: tickets submitted before this call do not see it, later ones do.  With a
-        ShardedIndex, ids are global and every rank makes the same call at the same point of its ticket sequence."""
-        self._mutate(lambda: self.index.remove(ids))
-
-    def restore(self, ids):
-        """index.restore(ids) between tickets (see remove())."""
-        self._mutate(lambda: self.index.restore(ids))
-
-    def add(self, vecs):
-        """index.add(vecs) between tickets (see remove()); returns the new ids.  Single-GPU Index only."""
-        if isinstance(self.index, ShardedIndex):
-            raise _lib.MdirError("SearchPipeline.add() needs an Index: ShardedIndex has no add()")
-        return self._mutate(lambda: self.index.add(vecs))
-
-    def compact(self):
-        """index.compact() on the compute stream, after the replays and exchanges already queued.  A maintenance step:
-        collect every ticket first -- MdirError while one is pending, because the live-row copy a ticket keeps for its
-        recovery path describes the slot layout compaction changes.  The graphs keep working without re-capture, and
-        tickets submitted afterwards see the compacted index.  With a ShardedIndex every rank calls it at the same point.
-        Returns the rows purged (on this rank)."""
-        pending = [sl for sl in self.slots if sl["pending"]]
-        if pending:
-            raise _lib.MdirError("SearchPipeline.compact(): collect the %d pending ticket(s) first" % len(pending))
-        return self._mutate(self.index.compact)
-
     def _download(self, slot, src, status):
         """Queue the D2H of a merged result and its status words into `slot`'s pinned buffers (ordered after the compute
         stream's last event)."""
@@ -1711,9 +1790,7 @@ class SearchPipeline:
         """q: (n_q, D) fp32, pinned host memory for a truly asynchronous upload (device tensors work too).
         Returns a ticket for result().  The caller keeps q unchanged until result(ticket) returned."""
         t_new = self.n_submitted
-        slot, gs = self.slots[t_new % self.depth], self.graphs[t_new % self.depth]
-        if slot["pending"]:
-            raise _lib.MdirError("SearchPipeline: collect result() of ticket %d before submitting more" % (t_new - self.depth))
+        slot, gs = self._free_slot(t_new), self.graphs[t_new % self.depth]
         q = torch.as_tensor(q)
         if tuple(q.shape) != tuple(gs.q.shape):
             raise _lib.MdirError("SearchPipeline expects query batches of shape %s" % (tuple(gs.q.shape),))
@@ -1745,11 +1822,7 @@ class SearchPipeline:
 
     def result(self, ticket):
         """Blocks until step `ticket` is in host memory; returns (scores (n_q, k) fp32, idx (n_q, k) int32) numpy views."""
-        if not (self.n_submitted - self.depth <= ticket < self.n_submitted):
-            raise _lib.MdirError("SearchPipeline: ticket %d is not in flight" % ticket)
-        slot = self.slots[ticket % self.depth]
-        if not slot["pending"]:
-            raise _lib.MdirError("SearchPipeline: result(%d) was already collected" % ticket)
+        slot = self._pending_slot(ticket)
         if not slot["merged"]:
             # deferred exchange and nothing was submitted after this ticket: merge it now (every rank does the same)
             if ticket != self.n_submitted - 1:
@@ -1786,10 +1859,204 @@ class SearchPipeline:
 
     def map(self, batches):
         """Generator over an iterable of query batches, keeping `depth` steps in flight."""
-        tickets = []
-        for q in batches:
-            if len(tickets) == self.depth:
-                yield self.result(tickets.pop(0))
-            tickets.append(self.submit(q))
-        for t in tickets:
-            yield self.result(t)
+        return self._map(batches, self.submit)
+
+
+class GraphedRangeSearch:
+    """One range step (Index.range_search) captured in a CUDA graph: static queries (n_q, D) fp32 and thresholds
+    min_score (n_q,) fp32 in, a CSR of static size out -- lims (n_q + 1,) int64, scores / ids arenas of
+    n_q * max_results entries (query i at [lims[i], lims[i + 1])) and status (n_q,) int32.
+
+        gr = GraphedRangeSearch(index, n_q=70, max_results=1024)
+        lims, scores, ids = gr(q, min_score)      # min_score: a float or one value per query
+        gr.check_overflow()                        # after a sync: True -> redo the flagged queries with range_search
+
+    The chain (pack, threshold keys, FILTER scan at RANGE_CAP_L, gather, device CSR offsets, emit) runs without a host
+    synchronisation, so the step has no variable-size output.  A query is emitted when its survivors fit max_results
+    and no candidate segment overflowed; any other query gets no rows and a status word: STATUS_OVERFLOW (a segment
+    overflowed: the graph has no re-scan) and/or STATUS_RANGE_FULL (more than max_results matches).  Whoever owns the
+    graph redoes those queries eagerly (RangePipeline does).  Emitted queries are bit for bit those of range_search.
+    The graph works in a workspace of its own, so eager calls between replays and replays leave each other unchanged;
+    it reads the live bitmap, the scan extent, the slot -> id map and the certificate stats from device memory, so
+    remove / restore / add / compact need no re-capture."""
+
+    def __init__(self, index, n_q, max_results=1024, precision="fp32"):
+        if isinstance(index, ShardedIndex):
+            raise _lib.MdirError("GraphedRangeSearch needs an Index: ShardedIndex has no range_search")
+        self.n_q, self.max_results, self.precision = int(n_q), int(max_results), precision
+        if not 1 <= self.n_q <= MAX_Q:
+            raise _lib.MdirError("GraphedRangeSearch: n_q must be in [1, %d] (got %d)" % (MAX_Q, self.n_q))
+        if not 1 <= self.max_results <= RANGE_STAGE:
+            raise _lib.MdirError("GraphedRangeSearch: max_results must be in [1, %d] (got %d)" % (RANGE_STAGE, self.max_results))
+        if precision == "fp32":
+            if index.db32 is None:
+                raise _lib.MdirError("precision='fp32' needs keep_fp32=True")
+        elif precision != "bf16":
+            raise ValueError("precision must be 'fp32' or 'bf16'")
+        self.index = loc = index
+        dev, nq, D = loc.device, self.n_q, loc.D
+        lib = _lib.lib()
+        n_chunks = range_chunks(RANGE_CAP_L)
+        stage = range_stage_cap(self.max_results)
+        with torch.cuda.device(dev):
+            stats = loc.stats() if precision == "fp32" else None     # its one read-back happens here, never in the graph
+            self.q = torch.zeros((nq, D), dtype=torch.float32, device=dev)
+            self.min_score = torch.full((nq,), float("inf"), dtype=torch.float32, device=dev)
+            self.lims = torch.zeros((nq + 1,), dtype=torch.int64, device=dev)
+            self.scores = torch.empty((nq * self.max_results,), dtype=torch.float32, device=dev)
+            self.ids = torch.empty((nq * self.max_results,), dtype=torch.int32, device=dev)
+            self.status = torch.zeros((nq,), dtype=torch.int32, device=dev)
+            # the graph's other buffers: held by this object (a tensor only the capture used would be freed and its
+            # memory handed to later allocations while the graph still writes it)
+            self._q16 = q16 = torch.empty((nq, D), dtype=torch.bfloat16, device=dev)
+            self._tau = tau = torch.empty((nq,), dtype=torch.int64, device=dev)
+            self._run_off = run_off = torch.empty((nq, n_chunks), dtype=torch.int32, device=dev)
+            loc._ws_tag = ("range_graph", id(self))
+            try:
+                self._bufs = bufs = loc._range_bufs(RANGE_CAP_L, nq, cached=True)
+            finally:
+                loc._ws_tag = None
+            runs = bufs[3]
+
+            def step():
+                _lib.check(lib.mdir_pack_bf16(_lib.ptr(self.q), nq, D, 0, _lib.ptr(q16), _lib.stream()), "mdir_pack_bf16")
+                _lib.check(lib.mdir_range_tau(_lib.ptr(self.q), nq, D, _lib.ptr(self.min_score), _lib.ptr(stats), _lib.ptr(tau), _lib.stream()),
+                           "mdir_range_tau")
+                run_len, max_seg = loc._range_launch(q16, self.q, self.min_score, tau, stats, RANGE_CAP_L, bufs)
+                _lib.check(lib.mdir_range_offsets(_lib.ptr(run_len), _lib.ptr(max_seg), nq, n_chunks, RANGE_CAP_L, self.max_results,
+                                                  _lib.ptr(self.lims), _lib.ptr(run_off), _lib.ptr(self.status), _lib.stream()),
+                           "mdir_range_offsets")
+                _lib.check(lib.mdir_range_emit(_lib.ptr(bufs[2]), n_chunks, _lib.ptr(runs), _lib.ptr(run_off), _lib.ptr(self.lims), nq, stage,
+                                               loc.idx_base, _lib.ptr(loc.slot_id), _lib.ptr(self.scores), _lib.ptr(self.ids), _lib.stream()),
+                           "mdir_range_emit")
+
+            prof, loc.prof = getattr(loc, "prof", None), None            # no timing events inside the graph
+            try:
+                side = torch.cuda.Stream(device=dev)
+                side.wait_stream(torch.cuda.current_stream(dev))
+                with torch.cuda.stream(side):                             # warm-up: per-device kernel attributes
+                    step()
+                torch.cuda.current_stream(dev).wait_stream(side)
+                torch.cuda.synchronize(dev)
+                self.graph = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(self.graph):
+                    step()
+            finally:
+                loc.prof = prof
+
+    def __call__(self, q=None, min_score=None):
+        """Replay on the current stream.  q: (n_q, D) fp32 (host, pinned for an asynchronous copy, or device) copied into
+        the static input; min_score: a float or one value per query (range_thresholds).  None keeps the previous value.
+        Returns the static (lims, scores, ids): the result is scores / ids[:lims[n_q]]."""
+        if q is not None:
+            self.q.copy_(q, non_blocking=True)
+        if min_score is not None:
+            self.min_score.copy_(torch.from_numpy(range_thresholds(min_score, self.n_q)))
+        self.graph.replay()
+        return self.lims, self.scores, self.ids
+
+    def check_overflow(self):
+        """True when some query of the last replay was flagged (STATUS_OVERFLOW / STATUS_RANGE_FULL) and has no rows:
+        redo those queries through index.range_search()."""
+        return bool(self.status.any().item())
+
+
+class RangePipeline(_Pipeline):
+    """Host-facing range serving: query batches and thresholds go up from pinned host buffers, GraphedRangeSearch
+    replays back to back on one compute stream, and each ticket's CSR comes back in pinned buffers of static size (the
+    whole max_results arena per query), copies and replays ordered by events only.
+
+        pipe = RangePipeline(index, n_q=70, max_results=1024)
+        t0 = pipe.submit(q_0, 0.4)                 # min_score: a float or one value per query
+        t1 = pipe.submit(q_1, m_1)
+        lims, scores, ids = pipe.result(t0)        # numpy: query i at [lims[i], lims[i + 1])
+
+    result() is the complete exact answer of range_search(check=True) for every query: a query the graph flagged (a
+    candidate segment overflowed, or more than max_results matches) is redone eagerly, with the live rows its ticket
+    was submitted with, and spliced into the ticket's CSR (range_splice).  remove() / restore() / add() / compact()
+    mutate the index between tickets without re-capturing the graphs."""
+
+    def __init__(self, index, n_q, max_results=1024, depth=2, precision="fp32"):
+        if isinstance(index, ShardedIndex):
+            raise _lib.MdirError("RangePipeline needs an Index: ShardedIndex has no range_search")
+        if int(depth) < 1:
+            raise _lib.MdirError("RangePipeline: depth must be at least 1 (got %d)" % int(depth))
+        self.graphs = [GraphedRangeSearch(index, n_q, max_results=max_results, precision=precision) for _ in range(int(depth))]
+        self.index = self.local = index
+        self.n_q, self.max_results, self.precision = int(n_q), int(max_results), precision
+        self.depth, self.overlap = int(depth), False
+        dev = index.device
+        arena = self.n_q * self.max_results
+        with torch.cuda.device(dev):
+            self.compute, self.h2d, self.d2h = (torch.cuda.Stream(device=dev) for _ in range(3))
+            self.slots = [{
+                "q": torch.empty((self.n_q, index.D), dtype=torch.float32).pin_memory(),
+                "m": torch.empty((self.n_q,), dtype=torch.float32).pin_memory(),
+                "lims": torch.empty((self.n_q + 1,), dtype=torch.int64).pin_memory(),
+                "status": torch.empty((self.n_q,), dtype=torch.int32).pin_memory(),
+                "scores": torch.empty((arena,), dtype=torch.float32).pin_memory(),
+                "ids": torch.empty((arena,), dtype=torch.int32).pin_memory(),
+                "up": torch.cuda.Event(), "done": torch.cuda.Event(), "down": torch.cuda.Event(),
+                "pending": False, "live": None} for _ in range(self.depth)]
+            torch.cuda.synchronize(dev)
+        self.n_submitted = 0
+        self.n_recovered = 0            # tickets with at least one query redone eagerly
+        self.recovered = {"overflow": 0, "range_full": 0}     # queries redone, by status bit (a query may count in both)
+
+    def submit(self, q, min_score):
+        """q: (n_q, D) fp32 (host or device), min_score: a float or one value per query.  Both are copied into the
+        slot's pinned staging buffers here, so the caller may reuse them at once.  Returns a ticket for result()."""
+        t_new = self.n_submitted
+        slot, gr = self._free_slot(t_new), self.graphs[t_new % self.depth]
+        q = torch.as_tensor(q)
+        if tuple(q.shape) != tuple(gr.q.shape):
+            raise _lib.MdirError("RangePipeline expects query batches of shape %s" % (tuple(gr.q.shape),))
+        m = range_thresholds(min_score, self.n_q)
+        slot["q"].copy_(q)
+        slot["m"].copy_(torch.from_numpy(m))
+        with torch.cuda.device(self.local.device):
+            with torch.cuda.stream(self.h2d):              # this slot's previous replay was collected by result()
+                gr.q.copy_(slot["q"], non_blocking=True)
+                gr.min_score.copy_(slot["m"], non_blocking=True)
+                slot["up"].record()
+            with torch.cuda.stream(self.compute):
+                self.compute.wait_event(slot["up"])
+                gr.graph.replay()
+                slot["done"].record()
+            with torch.cuda.stream(self.d2h):
+                self.d2h.wait_event(slot["done"])
+                for name, src in (("lims", gr.lims), ("status", gr.status), ("scores", gr.scores), ("ids", gr.ids)):
+                    slot[name].copy_(src, non_blocking=True)
+                slot["down"].record()
+        slot["pending"] = True
+        self.n_submitted += 1
+        return t_new
+
+    def result(self, ticket):
+        """Blocks until ticket's CSR is in host memory -> (lims (n_q + 1,) int64, scores fp32, ids int32) numpy.  Views of
+        the pinned buffers, valid until `depth` more submits, unless a query was redone: then fresh arrays."""
+        slot = self._pending_slot(ticket)
+        slot["down"].synchronize()
+        slot["pending"] = False
+        lims = slot["lims"].numpy()
+        n = int(lims[-1])
+        out = (lims, slot["scores"].numpy()[:n], slot["ids"].numpy()[:n])
+        status = slot["status"].numpy()
+        flagged = np.flatnonzero(status)
+        if flagged.size:
+            self.n_recovered += 1
+            self.recovered["overflow"] += int(((status & STATUS_OVERFLOW) != 0).sum())
+            self.recovered["range_full"] += int(((status & STATUS_RANGE_FULL) != 0).sum())
+            rows = torch.from_numpy(flagged)
+            dev = self.local.device
+            # on the compute stream (after every replay queued there), with the live rows this ticket was submitted with
+            with torch.cuda.device(dev), torch.cuda.stream(self.compute), self.local._live_version(slot["live"]):
+                sub = self.index.range_search(slot["q"][rows], slot["m"][rows], precision=self.precision, check=True)
+                sub = tuple(t.cpu().numpy() for t in sub)
+            out = range_splice(*out, flagged, *sub)
+        slot["live"] = None
+        return out
+
+    def map(self, batches):
+        """Generator over an iterable of (q, min_score) pairs, keeping `depth` tickets in flight."""
+        return self._map(batches, lambda b: self.submit(*b))
