@@ -416,6 +416,30 @@ int mdir_range_merge(const uint64_t* surv, int n_chunks, const int32_t* run_len,
 int mdir_range_offsets(const int32_t* run_len, const int32_t* max_seg, int n_q, int n_chunks, int cap_l,
                        int max_results, int64_t* lims, int32_t* run_off, int32_t* status, void* stream);
 
+/* Diffusion re-ranking (mdir_b200.Diffusion; Iscen et al., CVPR 2017; tests/diffusion_reference.py).
+ * mdir_diffusion_graph: knn_ids / knn_s (n_used, k + 1) = Index.search(rows of slots 0 .. n_used, k + 1, fp32): ids
+ *   (-1 padding) and scores, row r = slot r; slot_id the slot -> id map of the index.  N(i) = slot i's list without i,
+ *   or without its last entry when i is not in it.  Out, per slot: nbr (n_used, k) int32 = the mutual neighbours' slots
+ *   in N(i) order, then -1; w (n_used, k) = max(s, 0)^gamma with s from the lower slot's list (0 padding); deg (n_used,)
+ *   = sum of w in N(i) order.  1 <= k <= 255.
+ * mdir_diffusion_normalize: S[i, e] = w[i, e] / (sqrtf(deg[i]) sqrtf(deg[nbr[i, e]])), 0 where w is 0 or nbr -1
+ *   (S may alias w).
+ * mdir_diffusion_solve: per query q, L = the ids L_ids[q, 0 .. n) before the first -1 of its (n_q, trunc) shortlist,
+ *   L_s their scores; y_u = max(L_s[u], 0)^gamma for u < k_q, else 0; f = CG (fp64 arithmetic on the fp32 S) on
+ *   (I - alpha S_LL) f = y from 0, stopped
+ *   when ||r|| < rtol ||y|| (tested first in each of at most iters iterations) or r = 0.  f_out / ids_out (n_q, k_out) =
+ *   the top k_out of L by (f desc, position asc), -inf / -1 padding.  1 <= k_q, k_out <= trunc <= 2048,
+ *   0 < alpha < 1, 1 <= iters <= 1000, rtol >= 0; ws = mdir_diffusion_solve_workspace_bytes(n_q, trunc, k) bytes.
+ *   Bit-identical for a query alone or in any batch.                                                                */
+int mdir_diffusion_graph(const int32_t* knn_ids, const float* knn_s, int64_t n_used, int k, const uint32_t* slot_id,
+                         float gamma, int32_t* nbr, float* w, float* deg, void* stream);
+int mdir_diffusion_normalize(const int32_t* nbr, const float* w, const float* deg, int64_t n_used, int k, float* S,
+                             void* stream);
+size_t mdir_diffusion_solve_workspace_bytes(int n_q, int trunc, int k);
+int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int n_q, int trunc, const uint32_t* slot_id, int64_t n_used,
+                         const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
+                         int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, void* stream);
+
 /* stats[2] (device) = {max_r ||bf16(x_r) - x_r||_2^2, max_r ||x_r||_2^2} over the n rows of a shard:
  * the database half of the certificate's error bound.  db16 = mdir_pack_bf16(db32).            */
 int mdir_pack_stats(const float* db32, const uint16_t* db16, int64_t n, int D, float* stats, void* stream);

@@ -77,6 +77,10 @@ PROTOTYPES = {
     "mdir_range_sort_runs": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "mdir_range_merge": (_i, [_vp, _i, _vp, _vp, _i, _vp, _u32, _vp, _vp, _vp, _vp]),
     "mdir_range_offsets": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "mdir_diffusion_graph": (_i, [_vp, _vp, _i64, _i, _vp, _f, _vp, _vp, _vp, _vp]),
+    "mdir_diffusion_normalize": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _vp]),
+    "mdir_diffusion_solve_workspace_bytes": (_sz, [_i, _i, _i]),
+    "mdir_diffusion_solve": (_i, [_vp, _vp, _i, _i, _vp, _i64, _vp, _vp, _i, _i, _f, _d, _i, _d, _i, _vp, _sz, _vp, _vp, _vp]),
     "mdir_pack_stats": (_i, [_vp, _vp, _i64, _i, _vp, _vp]),
     "mdir_pack_stats_i8": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "mdir_pack_q_i8": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),

@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmdir_b200.so")
-SOURCES = ["api.cu", "pool_head.cu", "clahe.cu", "topk.cu", "ranks.cu", "sim_scan.cu", "evaluate.cu", "colorspace.cu", "mining.cu", "gemm_f64.cu", "shard_merge.cu", "composite.cu", "compact.cu"]
+SOURCES = ["api.cu", "pool_head.cu", "clahe.cu", "topk.cu", "ranks.cu", "sim_scan.cu", "evaluate.cu", "colorspace.cu", "mining.cu", "gemm_f64.cu", "shard_merge.cu", "composite.cu", "compact.cu", "diffusion.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -268,6 +268,7 @@ class Index:
     compact_chunk = 16384   # slots per chunk of compact()'s in-place move (its scratch holds one chunk's live rows)
     certify = True    # precision="fp32": prove the shortlist complete (status bit 2 + widening when it cannot be)
     _sms = None
+    _mutations = 0    # remove / restore / add / compact calls that changed the index (Diffusion's graph goes stale)
 
     def __init__(self, vecs, dxn=False, device="cuda", keep_fp32=True, idx_base=0, capacity=None):
         """vecs: (n, D) fp32 rows (torch/numpy, host or device), or (D, n) with dxn=True
@@ -358,6 +359,7 @@ class Index:
         rows = rows[self._live_host[rows] != bool(value)]          # repeated and no-op ids cost nothing
         if rows.size == 0:
             return
+        self._mutations += 1
         ids = torch.from_numpy(rows + self.idx_base).to(self.device)
         _lib.check(_lib.lib().mdir_live_update(_lib.ptr(self.live), self.n, self.idx_base, _lib.ptr(ids), int(rows.size), int(value),
                                                _lib.stream()), "mdir_live_update")
@@ -459,6 +461,7 @@ class Index:
         purged = self._n_used - keep.size
         if purged == 0:
             return 0
+        self._mutations += 1
         lib = _lib.lib()
         sched = compaction_schedule(used, self.compact_chunk)
         with torch.cuda.device(self.device):
