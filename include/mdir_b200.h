@@ -538,7 +538,9 @@ int mdir_compute_ap(const int64_t* ranks, int64_t n_db, int n_q, const int64_t* 
  *   out_scores / out_idx (n_q, k), out_keys (n_q, k) or NULL, overflow (n_q) int32 status words
  *   (MDIR_STATUS_*).  k <= n_db.
  *   ws: mdir_sim_topk_workspace_bytes(D) bytes (~115 MB), contents irrelevant.
- *   mdir_topk_plan exposes the route choice (0 dense / 1 one-launch / 2 three-launch + its sampling plan).
+ *   mdir_topk_plan exposes the route choice (0 dense / 1 one-launch / 2 three-launch) and the three-launch
+ *   sampling plan (n_sample tiles at stride), reported on routes 1 and 2 (the fallback of a caller that may not
+ *   take the one-launch route, e.g. more than 128 queries); zeros on route 0.  The planner of Index.search too.
  * mdir_gem_head: pooling -> L2N -> multi-scale aggregation -> [Lw centre, project, renormalise] for
  *   n_img images x S scales (maps image-major, scale-minor; off/hw as in mdir_pool).  P (>= dims, C)
  *   and/or Px3 = mdir_split_tf32x3(P, role 0) select the projection (both NULL: out is (n_img, C));

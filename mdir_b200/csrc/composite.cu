@@ -59,8 +59,10 @@ extern "C" size_t mdir_sim_topk_workspace_bytes(int D) {
 }
 
 // Host-only: which route a top-k over n_db rows with selection depth kth takes on a device with sm_count SMs.
-// route 0 = dense (every score, exact select), 1 = one-launch threshold + filter scan, 2 = sample / select / filter with
-// n_sample tiles at the given stride.  No CUDA call.
+// route 0 = dense (every score, exact select), 1 = one-launch threshold + filter scan, 2 = sample / select / filter.
+// n_sample / stride = the three-launch sampling plan (n_sample tiles at that stride), reported on routes 1 and 2: a
+// caller that may not take the one-launch route (more than 128 queries, or the route disabled) falls back to it.  Zero
+// only when no three-launch plan exists (route 0).  No CUDA call.
 extern "C" int mdir_topk_plan(int64_t n_db, int kth, int sm_count, int* route, int* n_sample, int* stride) {
     MDIR_CHECK_ARG(route && n_sample && stride && n_db >= 0 && kth >= 1 && sm_count >= 1);
     *route = 0;
@@ -68,13 +70,6 @@ extern "C" int mdir_topk_plan(int64_t n_db, int kth, int sm_count, int* route, i
     *stride = 0;
     const int64_t n_tiles = (n_db + kTile - 1) / kTile;
     if (n_tiles < 64) return 0;
-    int64_t g = sm_count < 148 ? sm_count : 148;
-    if (g > n_tiles / 2) g = n_tiles / 2;
-    g = balanced_grid(n_tiles, (int)g);          // the grid mdir_sim_scan_fused_bf16 launches
-    if (g * 16 >= 2 * (int64_t)kth && 1.25 * kth * (double)n_tiles / ((double)g * (double)g) <= kFusedCapL / 2.0) {
-        *route = 1;
-        return 0;
-    }
     int64_t want = ((int64_t)kth * n_tiles + kTargetCand - 1) / kTargetCand;
     if (want > 148) want = (want + 147) / 148 * 148;
     int64_t ns = want < n_tiles / 4 ? want : n_tiles / 4;
@@ -86,6 +81,10 @@ extern "C" int mdir_topk_plan(int64_t n_db, int kth, int sm_count, int* route, i
         *n_sample = (int)ns;
         *stride = (int)st;
     }
+    int64_t g = sm_count < 148 ? sm_count : 148;
+    if (g > n_tiles / 2) g = n_tiles / 2;
+    g = balanced_grid(n_tiles, (int)g);          // the grid mdir_sim_scan_fused_bf16 launches
+    if (g * 16 >= 2 * (int64_t)kth && 1.25 * kth * (double)n_tiles / ((double)g * (double)g) <= kFusedCapL / 2.0) *route = 1;
     return 0;
 }
 
@@ -107,7 +106,7 @@ extern "C" int mdir_sim_topk_bf16(const uint16_t* db16, const float* db32, const
     if (rc) return rc;
     const int64_t n_tiles = (n_db + kTile - 1) / kTile;
 
-    // route planning (the same rules as mdir_b200/search.py:Index._plan / _fused_ok; tests/test_cpu_boundary.py compares them)
+    // route planning: the planner Index.search uses too (search.py:Index._route); only route 2 reads the sampling plan
     const int sm_count = device_sm_count();
     MDIR_CHECK_ARG(sm_count > 0);
     int plan_route = 0, n_sample = 0, stride = 0;

@@ -20,6 +20,8 @@ Replaces, for mdir's evaluation (mdir/components/optim/score/cirscore.py:65-70):
                                 (N_db, N_q) score matrix (bit-exact vs the stable argsort).
 """
 import contextlib
+import ctypes as C
+import functools
 
 import numpy as np
 import torch
@@ -39,7 +41,7 @@ CAND_ROW = CAP_S + 148 * CAP_L
 STAGE_CAP = 16384     # keys mdir_topk_finalize can stage in shared memory
 MAX_SAMPLE_TILES = 512
 FUSED_CAP_L = CAND_ROW // 148   # one-launch route: no select segment, so each CTA segment gets the whole row's share
-TARGET_CAND = 4500    # candidates per query the sampling plan aims for (kth * n_tiles / n_sample), ~30 per CTA segment
+DENSE_ROUTE = (0, 0, 0)   # Index._route's (route, n_sample, stride) of the dense route
 
 
 STATUS_OVERFLOW, STATUS_UNCERTIFIED, STATUS_PEER_TIMEOUT = 1, 2, 4     # MDIR_STATUS_* (+ the exchange's own bit)
@@ -79,14 +81,15 @@ def default_shortlist(k):
     return -(-(-(-5 * int(k) // 4)) // 64) * 64
 
 
-def balanced_grid(n_work, max_ctas):
-    """common.cuh:balanced_grid -- the smallest persistent grid that needs as many rounds as max_ctas CTAs would."""
-    if n_work <= 0 or max_ctas <= 0:
-        return 1
-    if n_work <= max_ctas:
-        return int(n_work)
-    rounds = -(-n_work // max_ctas)
-    return int(-(-n_work // rounds))
+@functools.lru_cache(maxsize=4096)
+def topk_plan(n_db, kth, sm_count):
+    """mdir_topk_plan: (route, n_sample, stride) of a top-k over n_db rows at selection depth kth on sm_count SMs (the
+    rules live in composite.cu only; see Index._route).  Host-only: no CUDA call; cached, so that eager search() pays
+    no ctypes call per block."""
+    route, n_sample, stride = C.c_int(), C.c_int(), C.c_int()
+    _lib.check(_lib.lib().mdir_topk_plan(int(n_db), int(kth), int(sm_count), C.byref(route), C.byref(n_sample), C.byref(stride)),
+               "mdir_topk_plan")
+    return route.value, n_sample.value, stride.value
 
 
 def _as_dev_f32(x, device):
@@ -520,44 +523,31 @@ class Index:
         return self._stats
 
     # ------------------------------------------------------------------ helpers
-    def _buf(self, name, shape, dtype):
-        key = (getattr(self, "_ws_tag", None), name, tuple(shape), dtype)      # _ws_tag: a private workspace set (GraphedSearch(split=True))
-        b = self._ws.get(key)
+    def _buf(self, name, shape, dtype, ws=None):
+        """The device buffer (name, shape, dtype) of workspace ws (a dict; default: the index's own), allocated once."""
+        ws = self._ws if ws is None else ws
+        key = (name, tuple(shape), dtype)
+        b = ws.get(key)
         if b is None:
-            b = torch.empty(shape, dtype=dtype, device=self.device)
-            self._ws[key] = b
+            b = ws[key] = torch.empty(shape, dtype=dtype, device=self.device)
         return b
 
-    def _plan(self, kth):
-        """Sampling plan for the threshold pass: (n_sample, stride) or None for the dense route.
-        The threshold is the kth best of n_sample*256 sampled rows, so about kth * n_tiles / n_sample
-        rows survive the filter pass; n_sample is sized to keep that near TARGET_CAND."""
-        n_tiles = (self.n + TILE - 1) // TILE
-        if n_tiles < 64:
-            return None
-        want = -(-kth * n_tiles // TARGET_CAND)                     # ceil
-        if want > 148:                                              # whole waves of the 148 persistent CTAs
-            want = -(-want // 148) * 148
-        n_sample = max(32, min(MAX_SAMPLE_TILES, n_tiles // 4, want))
-        stride = n_tiles // n_sample
-        if n_sample * TILE < 2 * kth or stride < 2:
-            return None
-        return n_sample, stride
-
-    def _fused_ok(self, kth, nq=1):
-        """One-launch route (mdir_sim_scan_fused_bf16): each of the g persistent CTAs samples one tile, so the
-        threshold is about the kth best of g*256 rows and ~1.25 * kth * n_tiles / g rows survive, spread over g
-        segments.  Taken when that keeps the segments at most half full; larger k or databases use the
-        three-launch route, whose sample grows with the database."""
-        if not self.fused or nq > MAX_Q:
-            return False
-        n_tiles = (self.n + TILE - 1) // TILE
+    def _route(self, kth, nq):
+        """The top-k first pass of a block of nq queries at selection depth kth -> (route, n_sample, stride):
+        mdir_topk_plan on the capacity and this device's SM count.  Route 0 = dense, 1 = one-launch (each persistent CTA
+        samples one tile; taken while the candidate segments stay at most half full), 2 = sample / select / filter with
+        n_sample tiles at that stride (a sample that grows with the database: larger k or databases).  The one-launch
+        route is demoted to the three-launch plan (dense when there is none) when `fused` is off or nq > MAX_Q."""
         if self._sms is None:
             self._sms = torch.cuda.get_device_properties(self.device).multi_processor_count
-        g = balanced_grid(n_tiles, min(148, self._sms, n_tiles // 2))
-        if n_tiles < 64 or g * 16 < 2 * kth:
-            return False
-        return 1.25 * kth * n_tiles / (g * g) <= FUSED_CAP_L / 2
+        route, n_sample, stride = topk_plan(self.n, kth, self._sms)
+        if route == 1 and (not self.fused or nq > MAX_Q):
+            route = 2 if n_sample else 0
+        return route, n_sample, stride
+
+    def _fused_ok(self, kth, nq=1):
+        """True when a block of nq queries at selection depth kth takes the one-launch route."""
+        return self._route(kth, nq)[0] == 1
 
     def _i8_route(self, kth, nq):
         """The int8 first pass (mdir_pack_q_i8 -> mdir_sim_scan_fused_i8 -> mdir_topk_finalize_rescore_eps): half the
@@ -576,29 +566,17 @@ class Index:
             self._ws["fused_ws"] = ws
         return ws
 
-    def _topk_block_i8(self, q32, kth, k_out, out_scores, out_idx, out_keys, ovf):
-        """The certified fp32 top-k_out of one block of <= 128 queries through the int8 first pass: three launches."""
-        lib = _lib.lib()
+    def _pack_q_i8(self, q32, ws=None):
+        """q32 (nq, D) fp32 -> the int8 first pass's query operand (q8 = two int8 planes, their scales) and the per-query
+        bounds q_eps of its certificate (mdir_pack_q_i8), in workspace ws."""
         nq = q32.shape[0]
         n_pad = -(-nq // 16) * 16
-        stats = self.stats()
-        q8 = self._buf("q8", (2 * n_pad, self.D), torch.int8)
-        qsc = self._buf("q8_scale", (nq, 2), torch.float32)
-        qeps = self._buf("q8_eps", (nq,), torch.float32)
-        _lib.check(lib.mdir_pack_q_i8(_lib.ptr(q32), nq, self.D, _lib.ptr(stats), _lib.ptr(q8), _lib.ptr(qsc), _lib.ptr(qeps), _lib.stream()),
-                   "mdir_pack_q_i8")
-        tau, cand, cnt = self._cand_bufs(nq)
-        ws = self._fused_ws()
-        prof = getattr(self, "prof", None)
-        if prof is not None:
-            prof.begin()
-        _lib.check(lib.mdir_sim_scan_fused_i8_extent(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q8), _lib.ptr(qsc), nq,
-                                                     self.D, kth, _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L,
-                                                     _lib.ptr(ws), _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream()),
-                   "mdir_sim_scan_fused_i8_extent")
-        if prof is not None:
-            prof.end(self.n * self.D + 4 * self.n)       # int8 rows + their fp32 scales
-        self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, (q32, k_out), caps=(0, FUSED_CAP_L), q_eps=qeps)
+        q8 = self._buf("q8", (2 * n_pad, self.D), torch.int8, ws)
+        qsc = self._buf("q8_scale", (nq, 2), torch.float32, ws)
+        qeps = self._buf("q8_eps", (nq,), torch.float32, ws)
+        _lib.check(_lib.lib().mdir_pack_q_i8(_lib.ptr(q32), nq, self.D, _lib.ptr(self.stats()), _lib.ptr(q8), _lib.ptr(qsc), _lib.ptr(qeps),
+                                             _lib.stream()), "mdir_pack_q_i8")
+        return (q8, qsc), qeps
 
     def _scan(self, q16, mode, stride, n_sample, dense, dense_ld, tau, cand, cnt):
         # more than 128 queries: one WIDE launch, work items = (tile, 128-query block) -- one kernel ramp, and a database
@@ -608,10 +586,61 @@ class Index:
                       n_sample, _lib.ptr(dense), dense_ld, _lib.ptr(tau), self.idx_base, _lib.ptr(cand),
                       _lib.ptr(cnt), CAP_S, CAP_L, _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream()), "mdir_sim_scan_bf16_extent")
 
-    def _cand_bufs(self, nq=MAX_Q_WIDE):
+    def _cand_bufs(self, nq=MAX_Q_WIDE, ws=None):
         rows = MAX_Q_WIDE if nq <= MAX_Q_WIDE else WIDE_Q
-        return (self._buf("tau", (rows,), torch.int64), self._buf("cand", (rows, CAND_ROW), torch.int64),
-                self._buf("segcnt", (rows, N_SEGS), torch.int32))
+        return (self._buf("tau", (rows,), torch.int64, ws), self._buf("cand", (rows, CAND_ROW), torch.int64, ws),
+                self._buf("segcnt", (rows, N_SEGS), torch.int32, ws))
+
+    def _first_pass(self, route, q, kth, nq, ws=None):
+        """The first pass of the top-kth of one block of nq queries, into the candidate buffers of workspace ws ->
+        (tau, cand, cnt, caps) for _finalize.  route = (route, n_sample, stride) of _route; q = the bf16 queries (nq, D),
+        or on the one-launch route the int8 operand of _pack_q_i8.
+        Dense (route 0): every score -> exact kth-key select; the route for small databases and the recovery after a
+        candidate segment overflowed (the select emits exactly kth keys, so nothing can overflow here).  Three-launch
+        (route 2): SAMPLE scan -> select the threshold -> FILTER scan; one WIDE launch each beyond MAX_Q queries.
+        One-launch (route 1): threshold and filter inside the bf16 or int8 scan.
+        self.prof (bench.py: CUDA events on the launch stream) brackets the dominant kernel with its algorithmic bytes."""
+        lib = _lib.lib()
+        r, n_sample, stride = route
+        tau, cand, cnt = self._cand_bufs(nq, ws)     # the select / fused kernel (re)initialises every segment counter
+        prof = getattr(self, "prof", None)
+        if r == 1:
+            rest = (kth, _lib.ptr(tau), self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(self._fused_ws()),
+                    _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream())
+            if prof is not None:
+                prof.begin()
+            if isinstance(q, tuple):
+                _lib.check(lib.mdir_sim_scan_fused_i8_extent(_lib.ptr(self.db8), _lib.ptr(self.row_scale), self.n, _lib.ptr(q[0]), _lib.ptr(q[1]),
+                                                             nq, self.D, *rest), "mdir_sim_scan_fused_i8_extent")
+                nbytes = self.n * self.D + 4 * self.n       # int8 rows + their fp32 scales
+            else:
+                _lib.check(lib.mdir_sim_scan_fused_bf16_extent(_lib.ptr(self.db16), self.n, _lib.ptr(q), nq, self.D, *rest),
+                           "mdir_sim_scan_fused_bf16_extent")
+                nbytes = self.n * self.D * 2
+            if prof is not None:
+                prof.end(nbytes)
+            return tau, cand, cnt, (0, FUSED_CAP_L)
+        # scores of every row (dense) or of the sampled tiles (SAMPLE mode 1) -> the select kernel
+        sampled = int(r == 2)
+        if not sampled:
+            rows = ld = self.n
+            scores = self._buf("dense", (MAX_Q if nq <= MAX_Q else (MAX_Q_WIDE if nq <= MAX_Q_WIDE else WIDE_Q), max(self.n, 1)), torch.float32, ws)
+        elif nq <= MAX_Q_WIDE:
+            rows, ld = n_sample * TILE, MAX_SAMPLE_TILES * TILE
+            scores = self._buf("sample", (MAX_Q if nq <= MAX_Q else MAX_Q_WIDE, ld), torch.float32, ws)
+        else:
+            rows = ld = n_sample * TILE
+            scores = self._buf("sample_wide", (WIDE_Q, rows), torch.float32, ws)
+        self._scan(q, sampled, stride, n_sample, scores, ld, None, None, None)
+        _lib.check(lib.mdir_select_kth_live(_lib.ptr(scores), ld, rows, nq, kth, stride, self.idx_base, _lib.ptr(tau), _lib.ptr(cand),
+                                            CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, sampled, _lib.ptr(self.live), _lib.stream()), "mdir_select_kth_live")
+        if sampled:
+            if prof is not None:
+                prof.begin()
+            self._scan(q, 2, stride, n_sample, None, 0, tau, cand, cnt)
+            if prof is not None:
+                prof.end((self.n - rows) * self.D * 2)
+        return tau, cand, cnt, (CAP_S, CAP_L)
 
     def _finalize(self, cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore=None, caps=(CAP_S, CAP_L), q_eps=None):
         """rescore = (q32_block, k_out): fused exact fp32 re-scoring of the kth-long bf16 shortlist.
@@ -637,57 +666,6 @@ class Index:
                                                                  _lib.ptr(stats), _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys),
                                                                  _lib.ptr(tau), _lib.ptr(ovf), _lib.ptr(self.slot_id), _lib.stream()),
                        "mdir_topk_finalize_rescore_ids")
-
-    def _dense_block(self, q16, kth, out_scores, out_idx, out_keys, ovf, rescore=None):
-        """All scores of the block -> exact kth-key select -> sort.  The route for small databases
-        and the guaranteed-terminating recovery when a candidate segment overflowed (the select
-        emits exactly kth keys, so nothing can overflow here)."""
-        lib = _lib.lib()
-        nq = q16.shape[0]
-        tau, cand, cnt = self._cand_bufs(nq)     # the select kernel (re)initialises every segment counter
-        dense = self._buf("dense", (MAX_Q if nq <= MAX_Q else (MAX_Q_WIDE if nq <= MAX_Q_WIDE else WIDE_Q), max(self.n, 1)), torch.float32)
-        self._scan(q16, 0, 0, 0, dense, self.n, None, None, None)
-        _lib.check(lib.mdir_select_kth_live(_lib.ptr(dense), self.n, self.n, nq, kth, 0, self.idx_base, _lib.ptr(tau), _lib.ptr(cand),
-                                            CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, 0, _lib.ptr(self.live), _lib.stream()), "mdir_select_kth_live")
-        self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore)
-
-    def _topk_block(self, q16, kth, out_scores, out_idx, out_keys, ovf, rescore=None):
-        """Exact top-kth of one block of <= 128 queries by bf16-input/fp32-accumulate scores."""
-        lib = _lib.lib()
-        nq = q16.shape[0]
-        plan = self._plan(kth)
-        if plan is None:
-            return self._dense_block(q16, kth, out_scores, out_idx, out_keys, ovf, rescore)
-        tau, cand, cnt = self._cand_bufs(nq)     # the select / fused kernel (re)initialises every segment counter
-        prof = getattr(self, "prof", None)       # bench.py: CUDA events around the dominant kernel, on its own stream
-        if self._fused_ok(kth, nq):
-            ws = self._fused_ws()
-            if prof is not None:
-                prof.begin()
-            _lib.check(lib.mdir_sim_scan_fused_bf16_extent(_lib.ptr(self.db16), self.n, _lib.ptr(q16), nq, self.D, kth, _lib.ptr(tau),
-                                                           self.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                           _lib.ptr(self.live), _lib.ptr(self.n_scan), _lib.stream()),
-                       "mdir_sim_scan_fused_bf16_extent")
-            if prof is not None:
-                prof.end(self.n * self.D * 2)
-            return self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore, caps=(0, FUSED_CAP_L))
-        n_sample, stride = plan
-        rows = n_sample * TILE
-        if nq <= MAX_Q_WIDE:
-            sample = self._buf("sample", (MAX_Q if nq <= MAX_Q else MAX_Q_WIDE, MAX_SAMPLE_TILES * TILE), torch.float32)
-            ld = MAX_SAMPLE_TILES * TILE
-        else:
-            sample = self._buf("sample_wide", (WIDE_Q, rows), torch.float32)
-            ld = rows
-        self._scan(q16, 1, stride, n_sample, sample, ld, None, None, None)
-        _lib.check(lib.mdir_select_kth_live(_lib.ptr(sample), ld, rows, nq, kth, stride, self.idx_base, _lib.ptr(tau), _lib.ptr(cand),
-                                            CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, 1, _lib.ptr(self.live), _lib.stream()), "mdir_select_kth_live")
-        if prof is not None:
-            prof.begin()
-        self._scan(q16, 2, stride, n_sample, None, 0, tau, cand, cnt)
-        if prof is not None:
-            prof.end((self.n - rows) * self.D * 2)
-        self._finalize(cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore)
 
     # ------------------------------------------------------------------ public
     def search(self, q, k, precision="fp32", shortlist=None, check=True, return_keys=False, block_q=MAX_Q):
@@ -758,12 +736,20 @@ class Index:
             return out_s, out_i
 
     def _run_block(self, q16, kth, out_s, out_i, out_k, ovf, check, rescore=None):
-        """q16 None: the int8 first pass (Index._i8_route); a block it flags (bit 0 or 1) is redone here through the
-        bf16 route when check=True -- the int8 pass never widens, recovery is the bf16 route's own."""
+        """The top-kth of one block: the first pass _route chooses, then _finalize.  q16 None: the int8 first pass
+        (Index._i8_route); a block it flags (bit 0 or 1) is redone here through the bf16 route when check=True -- the
+        int8 pass never widens, recovery is the bf16 route's own."""
+        nq = ovf.shape[0]
+
+        def topk(route, q, kth, q_eps=None):
+            tau, cand, cnt, caps = self._first_pass(route, q, kth, nq)
+            self._finalize(cand, cnt, nq, kth, out_s, out_i, out_k, tau, ovf, rescore, caps, q_eps)
+
         if q16 is None:
             self.route = "int8"
             self.cert["int8_blocks"] += 1
-            self._topk_block_i8(rescore[0], kth, rescore[1], out_s, out_i, out_k, ovf)
+            q8, q_eps = self._pack_q_i8(rescore[0])
+            topk(self._route(kth, nq), q8, kth, q_eps)
             if not check:
                 return
             st = ovf.cpu()
@@ -773,14 +759,14 @@ class Index:
             self.cert["int8_redone"] += 1
             q16 = pack_bf16(rescore[0])
         self.route = "bf16"
-        self._topk_block(q16, kth, out_s, out_i, out_k, ovf, rescore)
+        topk(self._route(kth, nq), q16, kth)
         if not check:
             return
         st = ovf.cpu()
         self.cert["queries"] += int(st.numel())
         if bool((st & STATUS_OVERFLOW).any()):
             # a candidate segment overflowed (adversarial row order / massive ties): exact dense route
-            self._dense_block(q16, kth, out_s, out_i, out_k, ovf, rescore)
+            topk(DENSE_ROUTE, q16, kth)
             st = ovf.cpu()
             if bool((st & STATUS_OVERFLOW).any()):
                 raise _lib.MdirError("dense recovery overflowed (internal error)")
@@ -793,10 +779,10 @@ class Index:
         while bool((st & STATUS_UNCERTIFIED).any()) and kth < k_max:
             kth = min(2 * kth, k_max)
             self.cert["widened_blocks"] += 1
-            self._topk_block(q16, kth, out_s, out_i, out_k, ovf, rescore)
+            topk(self._route(kth, nq), q16, kth)
             st = ovf.cpu()
             if bool((st & STATUS_OVERFLOW).any()):
-                self._dense_block(q16, kth, out_s, out_i, out_k, ovf, rescore)
+                topk(DENSE_ROUTE, q16, kth)
                 st = ovf.cpu()
         # still flagged: more than ~MAX_KTH rows lie within the error bound of the k-th score (massive near-ties).
         # The best-effort answer stands; the flag stays raised in status() and the counter records it.
@@ -871,7 +857,7 @@ class Index:
         """One block of <= 128 queries -> [(counts, scores, ids, status, lims)] for consecutive groups of its queries."""
         nq = q16.shape[0]
         self.range_stats["blocks"] += 1
-        bufs = self._range_bufs(RANGE_CAP_L, MAX_Q, cached=True)
+        bufs = self._range_bufs(RANGE_CAP_L, MAX_Q)
         run_len, max_seg = self._range_pass(q16, q32, m, tau, stats, RANGE_CAP_L, bufs)
         over = max_seg > RANGE_CAP_L
         if not check or not over.any():
@@ -883,23 +869,21 @@ class Index:
         for g0 in range(0, nq, group):
             g1 = min(g0 + group, nq)
             self.range_stats["rescan_groups"] += 1
-            bufs = self._range_bufs(cap, g1 - g0, cached=False)
+            bufs = self._range_bufs(cap, g1 - g0, {})         # a workspace of its own: freed with the call
             run_len, max_seg = self._range_pass(q16[g0:g1], q32[g0:g1], m[g0:g1], tau[g0:g1], stats, cap, bufs)
             if (max_seg > cap).any():
                 raise _lib.MdirError("range_search re-scan overflowed its exact capacity (internal error)")
             out.append(self._range_emit(bufs, run_len, max_seg > cap))
         return out
 
-    def _range_bufs(self, cap_l, rows, cached):
+    def _range_bufs(self, cap_l, rows, ws=None):
         """Candidate rows, segment counts, survivors and the gather's per-chunk counts + max segment counts of a range
-        scan with segment capacity cap_l.  The default capacity's buffers are kept (through _buf, apart from search()'s
-        candidate buffers, so a range call never changes a later search); a re-scan's are freed with the call."""
+        scan with segment capacity cap_l, from workspace ws (default: the index's own, under names apart from search()'s
+        candidate buffers, so a range call never changes a later search)."""
         n_chunks = range_chunks(cap_l)
-        shapes = (("range_cand", (rows, 148 * cap_l), torch.int64), ("range_segcnt", (rows, N_SEGS), torch.int32),
-                  ("range_surv", (rows, n_chunks * RANGE_CHUNK), torch.int64), ("range_runs", (rows * (n_chunks + 1),), torch.int32))
-        if cached:
-            return tuple(self._buf(n, sh, dt) for n, sh, dt in shapes)
-        return tuple(torch.empty(sh, dtype=dt, device=self.device) for _, sh, dt in shapes)
+        return (self._buf("range_cand", (rows, 148 * cap_l), torch.int64, ws), self._buf("range_segcnt", (rows, N_SEGS), torch.int32, ws),
+                self._buf("range_surv", (rows, n_chunks * RANGE_CHUNK), torch.int64, ws),
+                self._buf("range_runs", (rows * (n_chunks + 1),), torch.int32, ws))
 
     def _range_pass(self, q16, q32, m, tau, stats, cap_l, bufs):
         """_range_launch, then run_len (nq, n_chunks) and max_seg (nq,) read back in one copy (the call's synchronisation
@@ -1521,24 +1505,14 @@ class GraphedSearch:
     def _init_split(self, prof):
         loc, dev, nq, k = self.local, self.local.device, self.n_q, self.k
         lib = _lib.lib()
-        loc._ws_tag = ("graph", id(self))
-        try:
-            tau, cand, cnt = loc._cand_bufs(nq)
-            ovf = loc._buf("ovf", (max(nq, 1),), torch.int32)
-        finally:
-            loc._ws_tag = None
-        ws = loc._fused_ws()
+        # the graphs' own candidate, status and query buffers: eager searches between replays leave them alone (the fused
+        # scan's arrival counters are shared: zeroed once, re-armed by the kernel itself)
+        self._ws = ws = {}
+        route = loc._route(self.kth, nq)
         i8 = loc._i8_route(self.kth, nq)         # the same route choice as Index.search
-        if i8:
-            stats = loc.stats()
-            self.q8 = torch.empty((2 * (-(-nq // 16) * 16), loc.D), dtype=torch.int8, device=dev)
-            self.q8_scale = torch.empty((nq, 2), dtype=torch.float32, device=dev)
-            self.q8_eps = torch.empty((nq,), dtype=torch.float32, device=dev)
-        else:
-            self.q16 = torch.empty((nq, loc.D), dtype=torch.bfloat16, device=dev)
         self.keys = torch.empty((nq, k), dtype=torch.int64, device=dev)
         self.local_out = (torch.empty((nq, k), dtype=torch.float32, device=dev), torch.empty((nq, k), dtype=torch.int32, device=dev))
-        self.ovf = ovf[:nq]
+        self.ovf = loc._buf("ovf", (max(nq, 1),), torch.int32, ws)[:nq]
         if self._has_exchange:
             self.out = (torch.empty((nq, k), dtype=torch.float32, device=dev), torch.empty((nq, k), dtype=torch.int32, device=dev))
             self.status = torch.zeros((nq,), dtype=torch.int32, device=dev)
@@ -1546,31 +1520,19 @@ class GraphedSearch:
             self.out, self.status = self.local_out, self.ovf
 
         def front():
+            q_eps = None
             if i8:
-                _lib.check(lib.mdir_pack_q_i8(_lib.ptr(self.q), nq, loc.D, _lib.ptr(stats), _lib.ptr(self.q8), _lib.ptr(self.q8_scale),
-                                              _lib.ptr(self.q8_eps), _lib.stream()), "mdir_pack_q_i8")
+                q, q_eps = loc._pack_q_i8(self.q, ws)
             else:
-                _lib.check(lib.mdir_pack_bf16(_lib.ptr(self.q), nq, loc.D, 0, _lib.ptr(self.q16), _lib.stream()), "mdir_pack_bf16")
-            if prof is not None:
-                prof.begin()
+                q = pack_bf16(self.q, out=loc._buf("q16", (nq, loc.D), torch.bfloat16, ws))
             lib.mdir_tune(1, self.scan_ctas)
             try:
-                if i8:
-                    _lib.check(lib.mdir_sim_scan_fused_i8_extent(_lib.ptr(loc.db8), _lib.ptr(loc.row_scale), loc.n, _lib.ptr(self.q8),
-                                                                 _lib.ptr(self.q8_scale), nq, loc.D, self.kth, _lib.ptr(tau), loc.idx_base,
-                                                                 _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws), _lib.ptr(loc.live),
-                                                                 _lib.ptr(loc.n_scan), _lib.stream()), "mdir_sim_scan_fused_i8_extent")
-                else:
-                    _lib.check(lib.mdir_sim_scan_fused_bf16_extent(_lib.ptr(loc.db16), loc.n, _lib.ptr(self.q16), nq, loc.D, self.kth, _lib.ptr(tau),
-                                                                   loc.idx_base, _lib.ptr(cand), _lib.ptr(cnt), 0, FUSED_CAP_L, _lib.ptr(ws),
-                                                                   _lib.ptr(loc.live), _lib.ptr(loc.n_scan), _lib.stream()),
-                               "mdir_sim_scan_fused_bf16_extent")
+                return loc._first_pass(route, q, self.kth, nq, ws), q_eps
             finally:
                 lib.mdir_tune(1, 0)
-            if prof is not None:
-                prof.end(loc.n * loc.D + 4 * loc.n if i8 else loc.n * loc.D * 2)
 
-        def back():
+        def back(first):
+            (tau, cand, cnt, caps), q_eps = first
             chunk = self.fin_chunk if self.fin_chunk > 0 else nq
             lib.mdir_tune(2, 0 if self.fin_chunk > 0 else 1)
             lib.mdir_tune(3, self.fin_stage)
@@ -1578,8 +1540,8 @@ class GraphedSearch:
                 for q0 in range(0, nq, chunk):
                     q1 = min(q0 + chunk, nq)
                     loc._finalize(cand[q0:q1], cnt[q0:q1], q1 - q0, self.kth, self.local_out[0][q0:q1], self.local_out[1][q0:q1],
-                                  self.keys[q0:q1], tau[q0:q1], self.ovf[q0:q1], (self.q[q0:q1], k), caps=(0, FUSED_CAP_L),
-                                  q_eps=self.q8_eps[q0:q1] if i8 else None)
+                                  self.keys[q0:q1], tau[q0:q1], self.ovf[q0:q1], (self.q[q0:q1], k), caps=caps,
+                                  q_eps=None if q_eps is None else q_eps[q0:q1])
             finally:
                 lib.mdir_tune(2, 1)
                 lib.mdir_tune(3, 0)
@@ -1588,19 +1550,20 @@ class GraphedSearch:
                 self.index._exchange(self.keys, nq, k, 0, self.out[0], self.out[1], self.ovf, self.status)
 
         with torch.cuda.device(dev):
+            loc.prof = prof                      # the scan's event pair: recorded in the warm-up too, captured in `graph`
             side = torch.cuda.Stream(device=dev)
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):
                 for _ in range(2):
-                    front()
-                    back()
+                    back(front())
             torch.cuda.current_stream(dev).wait_stream(side)
             torch.cuda.synchronize(dev)
             self.graph, self.back = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
-                front()
+                first = front()
             with torch.cuda.graph(self.back):
-                back()
+                back(first)
+            loc.prof = None
             self.local_done, self.done = torch.cuda.Event(), torch.cuda.Event()
 
     def exchange(self):
@@ -1914,11 +1877,8 @@ class GraphedRangeSearch:
             self._q16 = q16 = torch.empty((nq, D), dtype=torch.bfloat16, device=dev)
             self._tau = tau = torch.empty((nq,), dtype=torch.int64, device=dev)
             self._run_off = run_off = torch.empty((nq, n_chunks), dtype=torch.int32, device=dev)
-            loc._ws_tag = ("range_graph", id(self))
-            try:
-                self._bufs = bufs = loc._range_bufs(RANGE_CAP_L, nq, cached=True)
-            finally:
-                loc._ws_tag = None
+            self._ws = {}
+            self._bufs = bufs = loc._range_bufs(RANGE_CAP_L, nq, self._ws)
             runs = bufs[3]
 
             def step():

@@ -150,9 +150,43 @@ def test_install_patches_registries():
     assert isinstance(comp.wrappers[0], mdir_b200.CirMultiscaleAggregation)
 
 
+def _balanced_grid(n_work, max_ctas):
+    """common.cuh:balanced_grid -- the smallest persistent grid that needs as many rounds as max_ctas CTAs would."""
+    if n_work <= 0 or max_ctas <= 0:
+        return 1
+    if n_work <= max_ctas:
+        return int(n_work)
+    rounds = -(-n_work // max_ctas)
+    return int(-(-n_work // rounds))
+
+
+def _topk_plan_restatement(n_db, kth, sms):
+    """The top-k route rules in Python, the reference mdir_topk_plan is checked against -> (route, n_sample, stride).
+    Three-launch sampling plan: the threshold is the kth best of n_sample * 256 sampled rows, so about
+    kth * n_tiles / n_sample rows survive the filter pass; n_sample is sized to keep that near 4,500 (None: no plan,
+    dense).  One-launch route: each of the g persistent CTAs samples one tile, so the threshold is about the kth best
+    of g * 256 rows and ~1.25 * kth * n_tiles / g rows survive, spread over g segments; taken when that keeps the
+    segments at most half full.  Route 1 reports the three-launch plan too (the fallback of more than 128 queries)."""
+    from mdir_b200 import search
+    n_tiles = (n_db + search.TILE - 1) // search.TILE
+    if n_tiles < 64:
+        return 0, 0, 0
+    want = -(-kth * n_tiles // 4500)                            # ceil
+    if want > 148:                                              # whole waves of the 148 persistent CTAs
+        want = -(-want // 148) * 148
+    n_sample = max(32, min(search.MAX_SAMPLE_TILES, n_tiles // 4, want))
+    stride = n_tiles // n_sample
+    plan = (0, 0, 0) if n_sample * search.TILE < 2 * kth or stride < 2 else (2, n_sample, stride)
+    g = _balanced_grid(n_tiles, min(148, sms, n_tiles // 2))
+    if g * 16 >= 2 * kth and 1.25 * kth * n_tiles / (g * g) <= search.FUSED_CAP_L / 2:
+        return (1,) + plan[1:]
+    return plan
+
+
 def test_topk_route_planner_c_equals_python(libpath):
-    """The route rules exist twice: search.py (Index._plan / _fused_ok, used by the Python face) and composite.cu
-    (mdir_topk_plan, used by mdir_sim_topk_bf16).  They must agree for every database size / depth / SM count."""
+    """mdir_topk_plan (composite.cu), the one planner of Index.search and mdir_sim_topk_bf16, equals the Python
+    statement of the route rules for every database size / depth / SM count, sampling plan included; Index._route
+    demotes the one-launch route to that plan when the route is disabled or a block has more than 128 queries."""
     import ctypes as C
     from mdir_b200 import search
     l = C.CDLL(libpath)
@@ -160,16 +194,23 @@ def test_topk_route_planner_c_equals_python(libpath):
     rs = np.random.RandomState(0)
     sizes = [1, 255, 16383, 16384, 16385, 20000, 32768, 75000, 125126, 250251, 1001001, 2600000, 4000000, 20000000]
     sizes += [int(x) for x in rs.randint(1, 5_000_000, 60)]
+    routes = set()
     for n_db in sizes:
         for kth in (1, 10, 100, 132, 200, 384, 700, 1184, 1185, 2048, 4096):
             for sms in (148, 132, 60):
-                idx = search.Index.__new__(search.Index)
-                idx.n, idx._sms, idx.fused = n_db, sms, True
-                plan = idx._plan(kth)
-                want = (0, 0, 0) if plan is None else ((1, 0, 0) if idx._fused_ok(kth) else (2, plan[0], plan[1]))
+                want = _topk_plan_restatement(n_db, kth, sms)
                 r, ns, st = C.c_int(-1), C.c_int(-1), C.c_int(-1)
                 assert l.mdir_topk_plan(n_db, kth, sms, C.byref(r), C.byref(ns), C.byref(st)) == 0
                 assert (r.value, ns.value, st.value) == want, (n_db, kth, sms, want, (r.value, ns.value, st.value))
+                routes.add(want[0])
+                idx = search.Index.__new__(search.Index)
+                idx.n, idx._sms, idx.fused = n_db, sms, True
+                assert idx._route(kth, 128) == want and idx._fused_ok(kth) == (want[0] == 1)
+                demoted = want if want[0] != 1 else ((2,) + want[1:] if want[1] else (0, 0, 0))
+                assert idx._route(kth, 129) == demoted
+                idx.fused = False
+                assert idx._route(kth, 1) == demoted and not idx._fused_ok(kth)
+    assert routes == {0, 1, 2}
 
 
 def test_tune_knobs_and_workspace_sizes_are_host_only(libpath):

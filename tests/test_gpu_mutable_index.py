@@ -92,9 +92,9 @@ def _check_route(m, index, name, precision, k, nq):
     """The route the case is meant to exercise is the one search() takes."""
     kth = k if precision == "bf16" else max(k, m.search.default_shortlist(k))
     if name == "dense":
-        assert index._plan(kth) is None
+        assert index._route(kth, min(nq, 128))[0] == 0
     elif name in ("three", "three_large_k"):
-        assert index._plan(kth) is not None and not index._fused_ok(kth, min(nq, 128))
+        assert index._route(kth, min(nq, 128))[0] == 2
     elif name == "fused":
         assert index._fused_ok(kth, nq)
 
