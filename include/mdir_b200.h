@@ -355,6 +355,15 @@ int mdir_topk_finalize_rescore_eps_ids(const uint64_t* cand, int64_t cand_row, c
                                        const float* db_stats, const float* q_eps,
                                        float* out_scores, int32_t* out_idx, uint64_t* out_keys,
                                        uint64_t* tau, int32_t* overflow, const uint32_t* slot_id, void* stream);
+/* mdir_topk_finalize_rescore_eps_ids with the bf16 rows db16 (the same slots as db32): the certified
+ * extension is re-scored from db16 first, and only its rows inside the bf16 bound (computed from db_stats
+ * and the query norm) are re-scored from db32.  Same output, status words included; fewer fp32 rows gathered. */
+int mdir_topk_finalize_rescore_tiered_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg,
+                                          int cap0, int cap_l, int n_q, int shortlist, int k_out,
+                                          const float* db32, const uint16_t* db16, int64_t n_db, uint32_t idx_base,
+                                          const float* q32, int D, const float* db_stats, const float* q_eps,
+                                          float* out_scores, int32_t* out_idx, uint64_t* out_keys,
+                                          uint64_t* tau, int32_t* overflow, const uint32_t* slot_id, void* stream);
 
 /* In-place compaction of a mutable database (Index.compact).  mdir_compact_prefix: word_prefix[w] = live
  * slots in bitmap words [0, w), word_prefix[n_words] = all.  mdir_compact_move: the live slots of [lo, hi)

@@ -66,6 +66,8 @@ PROTOTYPES = {
                                             _vp]),
     "mdir_topk_finalize_rescore_eps_ids": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp,
                                                 _vp, _vp, _vp]),
+    "mdir_topk_finalize_rescore_tiered_ids": (_i, [_vp, _i64, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _i64, _u32, _vp, _i, _vp, _vp, _vp,
+                                                   _vp, _vp, _vp, _vp, _vp, _vp]),
     "mdir_compact_scratch_bytes": (_sz, [_i64, _i, _i, _i]),
     "mdir_compact_prefix": (_i, [_vp, _i64, _vp, _vp]),
     "mdir_compact_move": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _sz, _vp]),

@@ -359,28 +359,30 @@ __device__ __forceinline__ int cluster_ld_s32(uint32_t a) {
     return v;
 }
 
-// fp32 dot product of one database row with the query staged in shared memory, one warp per row
+// fp32 dot product of one database row with the query staged in shared memory, one warp per row.  The summation order
+// is that of each row of rescore_row2, so a row's fp32 score does not depend on whether it was re-scored alone or as
+// one of a pair: every finalize path and range_gather_kernel give the same bits for the same row.
 __device__ __forceinline__ float rescore_row(const float* __restrict__ a, const float* qs, int D, int lane) {
     float acc = 0.f;
     if ((D & 3) == 0) {
         const float4* a4 = reinterpret_cast<const float4*>(a);
         const float4* b4 = reinterpret_cast<const float4*>(qs);
         const int n4 = D >> 2;
-        float acc1 = 0.f, acc2 = 0.f, acc3 = 0.f;
+        float sa = 0.f, sb = 0.f;
         int i = lane;
         for (; i + 96 < n4; i += 128) {            // 4 independent 128-bit loads in flight per lane
             const float4 x0 = __ldg(a4 + i), x1 = __ldg(a4 + i + 32), x2 = __ldg(a4 + i + 64), x3 = __ldg(a4 + i + 96);
             const float4 y0 = b4[i], y1 = b4[i + 32], y2 = b4[i + 64], y3 = b4[i + 96];
-            acc = fmaf(x0.x, y0.x, acc); acc = fmaf(x0.y, y0.y, acc); acc = fmaf(x0.z, y0.z, acc); acc = fmaf(x0.w, y0.w, acc);
-            acc1 = fmaf(x1.x, y1.x, acc1); acc1 = fmaf(x1.y, y1.y, acc1); acc1 = fmaf(x1.z, y1.z, acc1); acc1 = fmaf(x1.w, y1.w, acc1);
-            acc2 = fmaf(x2.x, y2.x, acc2); acc2 = fmaf(x2.y, y2.y, acc2); acc2 = fmaf(x2.z, y2.z, acc2); acc2 = fmaf(x2.w, y2.w, acc2);
-            acc3 = fmaf(x3.x, y3.x, acc3); acc3 = fmaf(x3.y, y3.y, acc3); acc3 = fmaf(x3.z, y3.z, acc3); acc3 = fmaf(x3.w, y3.w, acc3);
+            sa = fmaf(x0.x, y0.x, sa); sa = fmaf(x0.y, y0.y, sa); sa = fmaf(x0.z, y0.z, sa); sa = fmaf(x0.w, y0.w, sa);
+            sb = fmaf(x1.x, y1.x, sb); sb = fmaf(x1.y, y1.y, sb); sb = fmaf(x1.z, y1.z, sb); sb = fmaf(x1.w, y1.w, sb);
+            sa = fmaf(x2.x, y2.x, sa); sa = fmaf(x2.y, y2.y, sa); sa = fmaf(x2.z, y2.z, sa); sa = fmaf(x2.w, y2.w, sa);
+            sb = fmaf(x3.x, y3.x, sb); sb = fmaf(x3.y, y3.y, sb); sb = fmaf(x3.z, y3.z, sb); sb = fmaf(x3.w, y3.w, sb);
         }
         for (; i < n4; i += 32) {
             const float4 x = __ldg(a4 + i), y = b4[i];
-            acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc); acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
+            sa = fmaf(x.x, y.x, sa); sa = fmaf(x.y, y.y, sa); sa = fmaf(x.z, y.z, sa); sa = fmaf(x.w, y.w, sa);
         }
-        acc = (acc + acc1) + (acc2 + acc3);
+        acc = sa + sb;
     } else {
         for (int i = lane; i < D; i += 32) acc = fmaf(a[i], qs[i], acc);
     }
@@ -495,12 +497,65 @@ __device__ __forceinline__ void rescore_row2(const float* __restrict__ a0, const
     r1 = warp_sum(s1a + s1b);
 }
 
+// fp32 dot products of TWO bf16 database rows (bf16 -> fp32, fp32 FMA) with the staged fp32 query: tier 2 of the int8
+// certificate (topk_finalize_kernel).  D % 8 == 0.  4 + 4 16-byte loads per lane in flight, the register budget of
+// the 1,024-thread finalize (64 per thread): two rounds per row pair at D = 2048, where the fp32 pair takes four.
+__device__ __forceinline__ float dot_bf16x8(uint4 x, float4 ya, float4 yb, float acc) {
+    acc = fmaf(__uint_as_float(x.x << 16), ya.x, acc); acc = fmaf(__uint_as_float(x.x & 0xffff0000u), ya.y, acc);
+    acc = fmaf(__uint_as_float(x.y << 16), ya.z, acc); acc = fmaf(__uint_as_float(x.y & 0xffff0000u), ya.w, acc);
+    acc = fmaf(__uint_as_float(x.z << 16), yb.x, acc); acc = fmaf(__uint_as_float(x.z & 0xffff0000u), yb.y, acc);
+    acc = fmaf(__uint_as_float(x.w << 16), yb.z, acc); acc = fmaf(__uint_as_float(x.w & 0xffff0000u), yb.w, acc);
+    return acc;
+}
+__device__ __forceinline__ void rescore_row2_bf16(const __nv_bfloat16* __restrict__ a0, const __nv_bfloat16* __restrict__ a1, const float* qs,
+                                                  int D, int lane, float& r0, float& r1) {
+    const uint4* p0 = reinterpret_cast<const uint4*>(a0);
+    const uint4* p1 = reinterpret_cast<const uint4*>(a1);
+    const float4* b4 = reinterpret_cast<const float4*>(qs);
+    const int n8 = D >> 3;
+    float s0 = 0.f, s1 = 0.f;
+    int i = lane;
+    for (; i + 96 < n8; i += 128) {
+        const uint4 x0 = __ldg(p0 + i), x1 = __ldg(p0 + i + 32), x2 = __ldg(p0 + i + 64), x3 = __ldg(p0 + i + 96);
+        const uint4 z0 = __ldg(p1 + i), z1 = __ldg(p1 + i + 32), z2 = __ldg(p1 + i + 64), z3 = __ldg(p1 + i + 96);
+        float4 ya = b4[2 * i], yb = b4[2 * i + 1];
+        s0 = dot_bf16x8(x0, ya, yb, s0); s1 = dot_bf16x8(z0, ya, yb, s1);
+        ya = b4[2 * i + 64]; yb = b4[2 * i + 65];
+        s0 = dot_bf16x8(x1, ya, yb, s0); s1 = dot_bf16x8(z1, ya, yb, s1);
+        ya = b4[2 * i + 128]; yb = b4[2 * i + 129];
+        s0 = dot_bf16x8(x2, ya, yb, s0); s1 = dot_bf16x8(z2, ya, yb, s1);
+        ya = b4[2 * i + 192]; yb = b4[2 * i + 193];
+        s0 = dot_bf16x8(x3, ya, yb, s0); s1 = dot_bf16x8(z3, ya, yb, s1);
+    }
+    for (; i < n8; i += 32) {
+        const uint4 x = __ldg(p0 + i), z = __ldg(p1 + i);
+        const float4 ya = b4[2 * i], yb = b4[2 * i + 1];
+        s0 = dot_bf16x8(x, ya, yb, s0); s1 = dot_bf16x8(z, ya, yb, s1);
+    }
+    r0 = warp_sum(s0);
+    r1 = warp_sum(s1);
+}
+
+// the scores of one warp's row pair from the fp32 master (a lone row in the same order: rescore_row) or, for tier 2 of
+// the int8 certificate, from the bf16 rows (a lone row is paired with itself; its order does not matter there)
+__device__ __forceinline__ void rescore_pair(const float* __restrict__ db32, int64_t row0, int64_t row1, bool ok0, bool ok1,
+                                             const float* qs, int D, int lane, float& s0, float& s1) {
+    if (ok0 && ok1) rescore_row2(db32 + row0 * D, db32 + row1 * D, qs, D, lane, s0, s1);
+    else if (ok0) s0 = rescore_row(db32 + row0 * D, qs, D, lane);
+    else if (ok1) s1 = rescore_row(db32 + row1 * D, qs, D, lane);
+}
+__device__ __forceinline__ void rescore_pair(const __nv_bfloat16* __restrict__ db16, int64_t row0, int64_t row1, bool ok0, bool ok1,
+                                             const float* qs, int D, int lane, float& s0, float& s1) {
+    if (ok0 || ok1) rescore_row2_bf16(db16 + (ok0 ? row0 : row1) * D, db16 + (ok1 ? row1 : row0) * D, qs, D, lane, s0, s1);
+}
+
 // Rescore entries [j0, j0 + n) of the key list at shared-memory address `list` of cluster rank 0 (DSMEM when this
 // CTA is a helper): one warp per row, rows interleaved over the CS CTAs of the cluster, two rows of a warp in flight
-// together (a row is 4 * D bytes gathered from HBM: latency, not bandwidth, is what a warp waits for).
-template <int CS>
+// together (a row is 4 * D bytes gathered from HBM: latency, not bandwidth, is what a warp waits for).  T = float:
+// the fp32 master db32; T = __nv_bfloat16: the bf16 rows (tier 2 of the int8 certificate).
+template <int CS, typename T>
 __device__ __forceinline__ void rescore_share(uint64_t* local_list, uint32_t remote_list, bool remote, int j0, int n, int crank,
-                                              const float* __restrict__ db32, int64_t n_db, uint32_t idx_base, const float* qs, int D) {
+                                              const T* __restrict__ db, int64_t n_db, uint32_t idx_base, const float* qs, int D) {
     const int lane = threadIdx.x & 31;
     for (int j = (threadIdx.x >> 5) * CS + crank; j < n; j += 64 * CS) {
         const int jb = j + 32 * CS;                       // this warp's second row of the round
@@ -511,9 +566,7 @@ __device__ __forceinline__ void rescore_share(uint64_t* local_list, uint32_t rem
         const int64_t row0 = (int64_t)g0 - (int64_t)idx_base, row1 = (int64_t)g1 - (int64_t)idx_base;
         const bool ok0 = key0 != ~0ull && row0 >= 0 && row0 < n_db, ok1 = key1 != ~0ull && row1 >= 0 && row1 < n_db;
         float s0 = 0.f, s1 = 0.f;
-        if (ok0 && ok1) rescore_row2(db32 + row0 * D, db32 + row1 * D, qs, D, lane, s0, s1);
-        else if (ok0) s0 = rescore_row(db32 + row0 * D, qs, D, lane);
-        else if (ok1) s1 = rescore_row(db32 + row1 * D, qs, D, lane);
+        rescore_pair(db, row0, row1, ok0, ok1, qs, D, lane, s0, s1);
         const uint64_t n0 = ok0 ? make_key(s0, g0) : ~0ull, n1 = ok1 ? make_key(s1, g1) : ~0ull;
         __syncwarp();
         if (lane == 0) {
@@ -547,6 +600,11 @@ __device__ __forceinline__ void rescore_share(uint64_t* local_list, uint32_t rem
 // and nothing overflowed.  Otherwise status bit 1 (uncertified) is raised and the host widens the selection.
 // q_eps != NULL: the filter scores came from another encoding (the int8 scan) and q_eps[q] is that encoding's bound
 // for query q (mdir_pack_q_i8), used instead of the bf16 formula above.
+// db16 != NULL as well (three tiers): the extension E is first re-scored from the bf16 rows against the fp32 query
+// (s16), and only the rows F of E with s16 >= t - eps16 (eps16: the tier-2 bound, see pack_q_i8_kernel) are re-scored
+// in fp32; the answer is the top k_out of the shortlist and F.  A row of E \ F has an fp32 score below t, and the
+// shortlist holds k_out rows at or above t, so the answer is the two-tier one, bit for bit (every fp32 re-score uses
+// one summation order, rescore_row).
 // status[q]: bit 0 = a candidate segment / the staging area overflowed, bit 1 = not certified.
 // slot_id != NULL: the candidate keys carry slots (idx_base + slot, which re-scoring addresses db32 by); the emitted
 // indices and keys carry slot_id[slot] instead.  The map is strictly increasing over the used slots, so the sorted order
@@ -560,14 +618,14 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
                                                              const float* __restrict__ db32, int64_t n_db, uint32_t idx_base,
                                                              const float* __restrict__ q32, int D, int k_out,
                                                              const float* __restrict__ db_stats, const float* __restrict__ q_eps,
-                                                             const uint32_t* __restrict__ slot_id) {
+                                                             const uint32_t* __restrict__ slot_id, const __nv_bfloat16* __restrict__ db16) {
     extern __shared__ uint64_t skeys[];
     __shared__ uint32_t hist[256];
     __shared__ uint64_t s_prefix;
     __shared__ uint32_t s_k, s_done, s_out;
     __shared__ int s_off[MDIR_CAND_SEGS + 1];
     __shared__ int s_ovf;
-    __shared__ int s_hdr[3];                      // rank 0 -> helpers: {shortlist length, offset of the list in skeys, extension length}
+    __shared__ int s_hdr[4];                      // rank 0 -> helpers: {shortlist length, offset of the list in skeys, extension length, |F|}
     __shared__ uint64_t s_tkey;
     __shared__ float s_red[96];
     __shared__ uint32_t hist_sel[1024];
@@ -590,6 +648,15 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
         cluster_sync_all();                                            // (2) every share is back in rank 0
         cluster_sync_all();                                            // (3) extension ready
         const int n_ext = cluster_ld_s32(cluster_map(&s_hdr[2], 0));
+        if (db16) {
+            rescore_share<CS>(nullptr, rk0, true, nk, n_ext, crank, db16, n_db, idx_base, qs, D);
+            cluster_sync_all();                                        // (4) bf16 shares are back
+            cluster_sync_all();                                        // (5) F ready
+            const int n_f = cluster_ld_s32(cluster_map(&s_hdr[3], 0));
+            rescore_share<CS>(nullptr, rk0, true, nk, n_f, crank, db32, n_db, idx_base, qs, D);
+            cluster_sync_all();                                        // (6) F shares are back
+            return;
+        }
         rescore_share<CS>(nullptr, rk0, true, nk, n_ext, crank, db32, n_db, idx_base, qs, D);
         cluster_sync_all();                                            // (4) extension shares are back
         return;
@@ -750,9 +817,18 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
         if (threadIdx.x == 0) { s_hdr[0] = nk; s_hdr[1] = (int)(sl - skeys); s_hdr[2] = 0; s_out = 0u; s_tkey = ~0ull; }
         __syncthreads();
         const uint64_t last16 = nk > 0 ? sl[nk - 1] : 0ull;          // worst bf16 key inside the shortlist
-        float eps = 0.f;
+        float eps = 0.f, eps16 = 0.f;
         if (db_stats && q_eps) {
             eps = q_eps[q];
+            if (db16) {                                              // the tier-2 bound (pack_q_i8_kernel)
+                q2 = warp_sum(q2);
+                if (lane == 0) s_red[threadIdx.x >> 5] = q2;
+                __syncthreads();
+                const float qn = sqrtf(warp_sum(s_red[lane]));
+                const float e_max = sqrtf(db_stats[0]), x_max = sqrtf(db_stats[1]), acc = 1.25f * (float)D * 5.9604645e-8f;
+                eps16 = e_max * qn + acc * (x_max + e_max) * qn + acc * x_max * qn;
+                eps16 = eps16 * 1.001f + 1e-7f;
+            }
         } else if (db_stats) {
             // one block reduction for the three sums
             q2 = warp_sum(q2); qt2 = warp_sum(qt2); qf2 = warp_sum(qf2);
@@ -770,6 +846,7 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
         if (CS > 1) cluster_sync_all();                                // (2) helpers' shares have landed
         __syncthreads();
         int n_ext = 0;
+        uint64_t bound16 = ~0ull;
         if (db_stats) {
             // t = k_out-th best re-scored key (rank counting; the in-place bitonic sort when the shortlist is long)
             if (nk >= k_out) {
@@ -794,6 +871,7 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
             const uint64_t tkey = s_tkey;
             // every row whose bf16 score is >= t - eps must be re-scored: bound key B (all index bits set)
             const uint64_t bound = tkey == ~0ull ? ~0ull : ((uint64_t)desc_key(key_score(tkey) - eps) << 32) | 0xffffffffull;
+            if (tkey != ~0ull) bound16 = ((uint64_t)desc_key(key_score(tkey) - eps16) << 32) | 0xffffffffull;
             const int ext_cap = sl_cap - nk;
             for (int i = threadIdx.x; i < cnt; i += blockDim.x) {
                 const uint64_t key = skeys[i];
@@ -810,8 +888,39 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
             __syncthreads();
         }
         if (CS > 1) cluster_sync_all();                                // (3) helpers may read the extension
+        if (db16) {
+            // tier 2: E from the bf16 rows; tier 3: F = {s16 >= t - eps16} compacted in place (stably, 1,024 keys per
+            // round: a key moves only to a lower position, after the round's reads) and re-scored in fp32
+            rescore_share<CS>(sl, 0u, false, nk, n_ext, 0, db16, n_db, idx_base, qs, D);
+            if (CS > 1) cluster_sync_all();                            // (4) bf16 shares have landed
+            __syncthreads();
+            uint32_t* s_wcnt = reinterpret_cast<uint32_t*>(s_red);
+            const int wi = threadIdx.x >> 5;
+            int n_f = 0;
+            for (int c = 0; c < n_ext; c += blockDim.x) {
+                const int i = c + (int)threadIdx.x;
+                const uint64_t key = i < n_ext ? sl[nk + i] : ~0ull;
+                const bool keep = key != ~0ull && key <= bound16;
+                const uint32_t m = __ballot_sync(0xffffffffu, keep);
+                if (lane == 0) s_wcnt[wi] = (uint32_t)__popc(m);
+                __syncthreads();
+                int pre = 0, tot = 0;
+                for (int j = 0; j < 32; ++j) {
+                    const int cj = (int)s_wcnt[j];
+                    pre += j < wi ? cj : 0;
+                    tot += cj;
+                }
+                if (keep) sl[nk + n_f + pre + __popc(m & ((1u << lane) - 1u))] = key;
+                n_f += tot;
+                __syncthreads();
+            }
+            n_ext = n_f;
+            if (threadIdx.x == 0) s_hdr[3] = n_f;
+            __syncthreads();
+            if (CS > 1) cluster_sync_all();                            // (5) helpers may read F
+        }
         rescore_share<CS>(sl, 0u, false, nk, n_ext, 0, db32, n_db, idx_base, qs, D);
-        if (CS > 1) cluster_sync_all();                                // (4) extension shares have landed
+        if (CS > 1) cluster_sync_all();                                // (4) extension shares have landed ((6) with db16)
         __syncthreads();
         const int n_all = nk + n_ext;
         if (n_all <= 1024) {
@@ -1027,7 +1136,8 @@ extern "C" int mdir_live_update(uint32_t* live, int64_t capacity, uint32_t idx_b
 static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0, int cap_l, int n_q,
                            int k, float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau, int32_t* overflow,
                            const float* db32, int64_t n_db, uint32_t idx_base, const float* q32, int D, int k_out, const float* db_stats,
-                           void* stream, const float* q_eps = nullptr, const uint32_t* slot_id = nullptr) {
+                           void* stream, const float* q_eps = nullptr, const uint32_t* slot_id = nullptr,
+                           const __nv_bfloat16* db16 = nullptr) {
     MDIR_CHECK_ARG(cand && seg_counts && n_seg >= 1 && n_seg <= MDIR_CAND_SEGS && cap0 >= 0 && n_q >= 0 && k >= 1 && k <= 4096);
     MDIR_CHECK_ARG(n_seg == 1 || cap_l >= 1);
     MDIR_CHECK_ARG(cand_row >= (int64_t)cap0 + (int64_t)(n_seg - 1) * cap_l);
@@ -1054,6 +1164,7 @@ static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_
         MDIR_CHECK_ARG(q32 && D > 0 && D <= 8192 && k_out >= 1 && k_out <= k && n_db >= 0);
         MDIR_CHECK_ARG((((uintptr_t)db32 | (uintptr_t)q32) & 15) == 0);
         MDIR_CHECK_ARG(db_stats == nullptr || tau != nullptr);          // the certificate compares against the filter threshold
+        MDIR_CHECK_ARG(db16 == nullptr || (q_eps != nullptr && D % 8 == 0 && ((uintptr_t)db16 & 15) == 0));
         smem += (size_t)D * 4;
     }
     // 227 KB per CTA minus the kernel's static arrays: the deepest selection (4096-row shortlist) leaves room for D <= 7168
@@ -1082,13 +1193,13 @@ static int launch_finalize(const uint64_t* cand, int64_t cand_row, const uint32_
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         MDIR_CUDA(cudaLaunchKernelEx(&cfg, topk_finalize_kernel<2>, cand, cand_row, seg_counts, n_seg, cap0, cap_l, k, smem_cap, sl_cap, out_scores,
-                                     out_idx, out_keys, tau, overflow, db32, n_db, idx_base, q32, D, k_out, db_stats, q_eps, slot_id));
+                                     out_idx, out_keys, tau, overflow, db32, n_db, idx_base, q32, D, k_out, db_stats, q_eps, slot_id, db16));
         MDIR_LAUNCH_CHECK();
         return 0;
     }
     topk_finalize_kernel<1><<<n_q, 1024, smem, (cudaStream_t)stream>>>(cand, cand_row, seg_counts, n_seg, cap0, cap_l, k, smem_cap, sl_cap,
                                                                         out_scores, out_idx, out_keys, tau, overflow, db32, n_db, idx_base,
-                                                                        q32, D, k_out, db_stats, q_eps, slot_id);
+                                                                        q32, D, k_out, db_stats, q_eps, slot_id, db16);
     MDIR_LAUNCH_CHECK();
     return 0;
 }
@@ -1133,6 +1244,19 @@ extern "C" int mdir_topk_finalize_rescore_eps_ids(const uint64_t* cand, int64_t 
     MDIR_CHECK_ARG(db32 != nullptr && db_stats != nullptr && q_eps != nullptr);
     return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
                            db32, n_db, idx_base, q32, D, k_out, db_stats, stream, q_eps, slot_id);
+}
+
+// mdir_topk_finalize_rescore_eps_ids with the bf16 rows db16 (same slots as db32): the three-tier re-score (the
+// extension is screened on db16 and only the rows inside the tier-2 bound are gathered from db32), same output
+extern "C" int mdir_topk_finalize_rescore_tiered_ids(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
+                                                     int cap_l, int n_q, int shortlist, int k_out, const float* db32, const uint16_t* db16,
+                                                     int64_t n_db, uint32_t idx_base, const float* q32, int D, const float* db_stats,
+                                                     const float* q_eps, float* out_scores, int32_t* out_idx, uint64_t* out_keys, uint64_t* tau,
+                                                     int32_t* overflow, const uint32_t* slot_id, void* stream) {
+    MDIR_CHECK_ARG(db32 != nullptr && db16 != nullptr && db_stats != nullptr && q_eps != nullptr);
+    return launch_finalize(cand, cand_row, seg_counts, n_seg, cap0, cap_l, n_q, shortlist, out_scores, out_idx, out_keys, tau, overflow,
+                           db32, n_db, idx_base, q32, D, k_out, db_stats, stream, q_eps, slot_id,
+                           reinterpret_cast<const __nv_bfloat16*>(db16));
 }
 
 extern "C" int mdir_topk_finalize_rescore_eps(const uint64_t* cand, int64_t cand_row, const uint32_t* seg_counts, int n_seg, int cap0,
@@ -1247,6 +1371,12 @@ __global__ void __launch_bounds__(256) pack_stats_i8_kernel(const float* __restr
 //         + 1.25 D 2^-24 x ||q||                               (fp32 accumulation of the exact re-score)
 //         + 8 2^-24 (x + e8) (||s_hi hi|| + ||s_lo lo||)     (s32 -> fp32 conversion and the scale products of the scan)
 // with e8 = max_r ||x_r - s_r x8_r||, x = max_r ||x_r|| (stats).  Rows n_q .. n_pad - 1 of the planes are zero.
+// Tier 2 of the finalize (db16 given) re-scores the extension as s16 = fp32 sum of bf16(x_r) . q; its bound, computed
+// there per query from the same stats (e = max_r ||bf16(x_r) - x_r||):
+//     eps16 = e ||q||                                          (Cauchy-Schwarz on the row's bf16 rounding)
+//           + 1.25 D 2^-24 (x + e) ||q||                       (fp32 accumulation of s16: ||bf16(x_r)|| <= x + e)
+//           + 1.25 D 2^-24 x ||q||                             (fp32 accumulation of the exact re-score)
+// times 1.001, plus 1e-7, as here.
 __global__ void __launch_bounds__(32) pack_q_i8_kernel(const float* __restrict__ q32, int n_q, int n_pad, int D, const float* __restrict__ stats,
                                                        int8_t* __restrict__ q8, float* __restrict__ q_scale, float* __restrict__ q_eps) {
     const int q = blockIdx.x, lane = threadIdx.x;
@@ -1423,11 +1553,9 @@ __global__ void __launch_bounds__(256) range_tau_kernel(const float* __restrict_
 
 // One CTA per (chunk c of kRangeChunk candidate slots, query q).  The candidate slots of q are its scan segments
 // (segment s at cand[q * cand_row + s * cap_l], seg_counts column 1 + s) concatenated after clamping to cap_l.
-// db32 != NULL: each candidate is re-scored in fp32 (one warp per row, always in rescore_row2's summation order) and
-// kept when that score is >= min_score[q].  search's finalize sums a row it re-scores in a pair in that order too, but a
-// row it re-scores alone in rescore_row's; for D > 384 the two orders can differ in the last bits, so a range score is
-// search's bit for bit on paired rows and within a few ulps on the others.  db32 ==
-// NULL: the bf16 keys are kept as they are (the scan threshold was min_score itself).  Survivors go, unsorted, to
+// db32 != NULL: each candidate is re-scored in fp32 (one warp per pair of rows, rescore_row2) and kept when that score
+// is >= min_score[q].  search's finalize sums every row in the same order (rescore_row), so a range score is search's
+// bit for bit.  db32 == NULL: the bf16 keys are kept as they are (the scan threshold was min_score itself).  Survivors go, unsorted, to
 // chunk c of q's survivor row; run_len = their number.  max_seg[q] = the largest raw segment count (> cap_l: overflow).
 __global__ void __launch_bounds__(512) range_gather_kernel(const uint64_t* __restrict__ cand, int64_t cand_row, const uint32_t* __restrict__ seg_counts,
                                                            int cap_l, const float* __restrict__ min_score, const float* __restrict__ db32,

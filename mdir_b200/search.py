@@ -270,6 +270,7 @@ class Index:
     fused = True      # allow the one-launch threshold + filter route (False: always sample -> select -> filter)
     compact_chunk = 16384   # slots per chunk of compact()'s in-place move (its scratch holds one chunk's live rows)
     certify = True    # precision="fp32": prove the shortlist complete (status bit 2 + widening when it cannot be)
+    tiered = True     # int8 route: screen the certified extension on the bf16 rows before the fp32 gather (same output)
     _sms = None
     _mutations = 0    # remove / restore / add / compact calls that changed the index (Diffusion's graph goes stale)
 
@@ -644,13 +645,22 @@ class Index:
 
     def _finalize(self, cand, cnt, nq, kth, out_scores, out_idx, out_keys, tau, ovf, rescore=None, caps=(CAP_S, CAP_L), q_eps=None):
         """rescore = (q32_block, k_out): fused exact fp32 re-scoring of the kth-long bf16 shortlist.
-        q_eps: per-query bounds of the int8 first pass (certified, instead of the bf16 bound)."""
+        q_eps: per-query bounds of the int8 first pass (certified, instead of the bf16 bound); with `tiered` its
+        extension is re-scored from the bf16 rows first and only the rows inside their bound from fp32."""
         CAP_S, CAP_L = caps
         CAND_ROW = CAP_S + 148 * CAP_L            # the row stride the scan kernels derive from the two capacities
         if rescore is None:
             _lib.check(_lib.lib().mdir_topk_finalize_ids(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth,
                                                          _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys), _lib.ptr(tau),
                                                          _lib.ptr(ovf), self.idx_base, _lib.ptr(self.slot_id), _lib.stream()), "mdir_topk_finalize_ids")
+        elif q_eps is not None and self.tiered:
+            q32, k_out = rescore
+            _lib.check(_lib.lib().mdir_topk_finalize_rescore_tiered_ids(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth,
+                                                                        k_out, _lib.ptr(self.db32), _lib.ptr(self.db16), self.n, self.idx_base,
+                                                                        _lib.ptr(q32), self.D, _lib.ptr(self.stats()), _lib.ptr(q_eps),
+                                                                        _lib.ptr(out_scores), _lib.ptr(out_idx), _lib.ptr(out_keys), _lib.ptr(tau),
+                                                                        _lib.ptr(ovf), _lib.ptr(self.slot_id), _lib.stream()),
+                       "mdir_topk_finalize_rescore_tiered_ids")
         elif q_eps is not None:
             q32, k_out = rescore
             _lib.check(_lib.lib().mdir_topk_finalize_rescore_eps_ids(_lib.ptr(cand), CAND_ROW, _lib.ptr(cnt), N_SEGS, CAP_S, CAP_L, nq, kth, k_out,
@@ -803,10 +813,8 @@ class Index:
         the CSR layout of FAISS range_search: the results of query i are scores / ids[lims[i]:lims[i + 1]], ordered by
         (score desc, id asc) as search() orders them; ids go through the slot -> id map.
 
-        precision="fp32": the exact fp32 score (one fixed summation order: the one search(precision="fp32") uses for the
-                          rows it re-scores in pairs, e.g. its whole shortlist at k = 100; a row search re-scores alone
-                          is summed in another order and can differ from the range score in the last bits when
-                          D > 384).  The bf16 scan
+        precision="fp32": the exact fp32 score, in the one summation order search(precision="fp32") uses for every
+                          row, so a row's range score is its search score bit for bit.  The bf16 scan
                           passes every row within the certified bound eps of min_score; those rows are re-scored in fp32
                           and filtered, so the result is complete by construction (no threshold to guess, no widening).
         precision="bf16": the bf16-input / fp32-accumulate scan score, as search(precision="bf16") reports it.
