@@ -303,9 +303,10 @@ __device__ __forceinline__ int tile_of_work(const ScanParams& p, const Span& s, 
 }
 
 // 16 scores (columns c0 .. c0 + 15 of this warp's TMEM lanes) of one accumulator.  int8: the hi plane's s32 sums sit in
-// columns [0, n_pad), the lo plane's in [n_pad, 2 n_pad); s_r is this lane's row scale and qsc the per-query scales.
+// columns [0, n_pad), the lo plane's in [n_pad, 2 n_pad); s_r is this lane's row scale and qrec the per-query records
+// {s_hi, s_lo, tau_f, 0}, read with one 16-byte load per query; t = their tau_f (int8 only).
 template <int KIND>
-__device__ __forceinline__ void acc_scores16(uint32_t taddr, int c0, int n_pad, float s_r, const float* qsc, float (&s)[16]) {
+__device__ __forceinline__ void acc_scores16(uint32_t taddr, int c0, int n_pad, float s_r, const float* qrec, float (&s)[16], float (&t)[16]) {
     uint32_t v[16];
     tmem_ld16(taddr + (uint32_t)c0, v);
     if (KIND == kKindI8) {
@@ -314,8 +315,9 @@ __device__ __forceinline__ void acc_scores16(uint32_t taddr, int c0, int n_pad, 
         tmem_ld_wait();
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
-            const float2 sc = *reinterpret_cast<const float2*>(qsc + 2 * (c0 + i));
-            s[i] = __fmul_rn(__fmaf_rn((float)(int)v[i], sc.x, __fmul_rn((float)(int)lo[i], sc.y)), s_r);
+            const float4 r = *reinterpret_cast<const float4*>(qrec + 4 * (c0 + i));
+            s[i] = __fmul_rn(__fmaf_rn((float)(int)v[i], r.x, __fmul_rn((float)(int)lo[i], r.y)), s_r);
+            t[i] = r.z;
         }
     } else {
         tmem_ld_wait();
@@ -342,7 +344,9 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
     __shared__ uint64_t tau_s0[kMaxN];
     __shared__ float tau_f0[kMaxN];
     __shared__ uint32_t cand_n0[kMaxN];    // candidates this CTA has appended per query (CTA-private list: no global atomics)
-    __shared__ __align__(8) float qsc[I8 ? 2 * 128 : 2];    // int8: {s_hi, s_lo} per query
+    // int8: {s_hi, s_lo, tau_f, 0} per query (tau_f once the threshold exchange has published it), so that the epilogue's
+    // filter reads one 16-byte record per query from shared memory instead of an 8-byte and a 4-byte one
+    __shared__ __align__(I8 ? 16 : 8) float qrec[I8 ? 4 * 128 : 2];
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -382,7 +386,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
     if (p.mode == MDIR_SCAN_FUSED) {
         for (int c = threadIdx.x; c < kMaxN; c += kThreads) cand_n[c] = 0u;
         if (I8)
-            for (int c = threadIdx.x; c < 2 * p.n_pad; c += kThreads) qsc[c] = c < 2 * p.n_q ? p.q_scale[c] : 0.f;
+            for (int c = threadIdx.x; c < 4 * p.n_pad; c += kThreads)
+                qrec[c] = ((c & 3) < 2 && (c >> 2) < p.n_q) ? p.q_scale[2 * (c >> 2) + (c & 3)] : 0.f;
     } else if (p.mode == MDIR_SCAN_FILTER) {
         for (int c = threadIdx.x; c < n_state; c += kThreads) {
             uint64_t t = c < p.n_q_total ? p.tau[c] : 0ull;
@@ -539,8 +544,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                     const float s_r = h ? s_rh[1] : s_rh[0];
 #pragma unroll 1
                     for (int c0 = 0; c0 < p.n_pad; c0 += 16) {
-                        float v[16];
-                        acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qsc, v);
+                        float v[16], t_unused[16];
+                        acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qrec, v, t_unused);
                         uint32_t m1 = 0xffffffffu, m2 = 0xffffffffu;
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
@@ -629,6 +634,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                     const uint64_t tq = (ok && et < p.n_q) ? __ldcg(reinterpret_cast<const unsigned long long*>(p.tau_rw) + et) : 0ull;
                     tau_s[et] = tq;
                     tau_f[et] = ((uint32_t)(tq >> 32) == 0xffffffffu) ? -INFINITY : key_score(tq);
+                    if (I8) qrec[4 * et + 2] = tau_f[et];
                     if (!ok) cand_n[et] = (uint32_t)p.cap_l + 1u;        // barrier timed out: report overflow, never hang
                 }
                 asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -650,8 +656,8 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
                 const uint32_t gidx = p.idx_base + (uint32_t)row;
 #pragma unroll 1
                 for (int c0 = 0; c0 < p.n_pad; c0 += 16) {
-                    float v[16];
-                    acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qsc, v);
+                    float v[16], tv[16];
+                    acc_scores16<KIND>(taddr, c0, p.n_pad, s_r, qrec, v, tv);
                     if (emode != MDIR_SCAN_FILTER) {
                         // rows past the end of the database only exist in the compact SAMPLE buffer: mark them -inf, and
                         // dead rows too
@@ -682,7 +688,7 @@ __global__ void __launch_bounds__(kThreads, 1) sim_scan_kernel(const __grid_cons
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
                             const float s = v[i];
-                            if (s >= tau_f[qo + i] && c0 + i < nq_here) {
+                            if (s >= (I8 ? tv[i] : tau_f[qo + i]) && c0 + i < nq_here) {
                                 const uint64_t key = make_key(s, gidx);
                                 if (key <= tau_s[qo + i]) {
                                     const uint32_t pos = atomicAdd(&cand_n[qo + i], 1u);      // shared memory, rare
