@@ -449,6 +449,29 @@ int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int n_q, int tr
                          const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
                          int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, void* stream);
 
+/* Incremental update of the raw lists (Diffusion.add / restore / remove; DESIGN 2.2e).  A list entry's key is
+ * mdir_make_key(score, id), smaller = better, all ones for padding; T_i = the key of entry k of slot i's list.
+ * mdir_diffusion_batch_eps: eps[j] = the certified bf16 bound of row j of q32 (n_q, D) taken as a query (the formula of
+ *   mdir_range_tau), db_stats = Index.stats() covering those rows.
+ * mdir_diffusion_merge: merges a batch B of nb rows (slots bslot[0 .. nb)) into the lists of the target slots: the
+ *   slots of [col0, col0 + n_cols) whose bit in `live` is set.  plane (nb, ld) fp32 = mdir_sim_scan_dense_bf16 of B's
+ *   bf16 rows against the bf16 rows of those slots.  Slots are taken in tiles of 32 (tile t = slots [32 t, 32 t + 32),
+ *   col0 % 32 == 0): all tiles of the range, or (tiles != NULL) the n_tiles listed.  Pair (i, j) passes the screen
+ *   when plane >= fsub_rd(score(T_i), eps[j]) (always when T_i is padding) and is re-scored in fp32 with slot i's row
+ *   as the query (the summation order of every search finalize); key(s_ij, slot_id[j]) < T_i enters i's list, which
+ *   keeps its first k + 1 keys.  B's ids must be in no target list.  cnt[t] = pairs of tile t that passed, exact; a
+ *   tile with cnt[t] > cap changes no list (re-run it with cap >= cnt[t]); rep[t] = list entries replaced in tile t.
+ *   seg: 2 * cap uint64 per launched tile.  knn_ids / knn_s (capacity, k + 1) are updated in place; 1 <= k <= 255.
+ * mdir_diffusion_stale_rows: per used slot i < n_used, one warp: a slot whose bit in `live` is clear gets a padding
+ *   list (-1, -inf) and flag 0; a live slot gets flag 1 iff its list holds an id that no live used slot holds.     */
+int mdir_diffusion_batch_eps(const float* q32, int n_q, int D, const float* db_stats, float* eps, void* stream);
+int mdir_diffusion_merge(const float* plane, int64_t ld, int nb, int64_t col0, int64_t n_cols, const int32_t* tiles, int n_tiles,
+                         const uint32_t* live, const float* eps, const int64_t* bslot, const float* db32, int D,
+                         const uint32_t* slot_id, int32_t* knn_ids, float* knn_s, int k, uint64_t* seg, int cap, int32_t* cnt,
+                         int32_t* rep, void* stream);
+int mdir_diffusion_stale_rows(int32_t* knn_ids, float* knn_s, int64_t n_used, int k, const uint32_t* slot_id,
+                              const uint32_t* live, uint8_t* flag, void* stream);
+
 /* stats[2] (device) = {max_r ||bf16(x_r) - x_r||_2^2, max_r ||x_r||_2^2} over the n rows of a shard:
  * the database half of the certificate's error bound.  db16 = mdir_pack_bf16(db32).            */
 int mdir_pack_stats(const float* db32, const uint16_t* db16, int64_t n, int D, float* stats, void* stream);

@@ -156,6 +156,47 @@ __device__ __forceinline__ int find_bin_warp0(const uint32_t* hist, uint32_t k, 
     return bin;
 }
 
+// fp32 dot product of one database row with a query (in shared or global memory), one warp per row.  The summation
+// order is that of each row of rescore_row2 (topk.cu), so a row's fp32 score does not depend on whether it was
+// re-scored alone or as one of a pair: every finalize path, range_gather_kernel and the diffusion graph update give the
+// same bits for the same row.
+__device__ __forceinline__ float rescore_row(const float* __restrict__ a, const float* qs, int D, int lane) {
+    float acc = 0.f;
+    if ((D & 3) == 0) {
+        const float4* a4 = reinterpret_cast<const float4*>(a);
+        const float4* b4 = reinterpret_cast<const float4*>(qs);
+        const int n4 = D >> 2;
+        float sa = 0.f, sb = 0.f;
+        int i = lane;
+        for (; i + 96 < n4; i += 128) {            // 4 independent 128-bit loads in flight per lane
+            const float4 x0 = __ldg(a4 + i), x1 = __ldg(a4 + i + 32), x2 = __ldg(a4 + i + 64), x3 = __ldg(a4 + i + 96);
+            const float4 y0 = b4[i], y1 = b4[i + 32], y2 = b4[i + 64], y3 = b4[i + 96];
+            sa = fmaf(x0.x, y0.x, sa); sa = fmaf(x0.y, y0.y, sa); sa = fmaf(x0.z, y0.z, sa); sa = fmaf(x0.w, y0.w, sa);
+            sb = fmaf(x1.x, y1.x, sb); sb = fmaf(x1.y, y1.y, sb); sb = fmaf(x1.z, y1.z, sb); sb = fmaf(x1.w, y1.w, sb);
+            sa = fmaf(x2.x, y2.x, sa); sa = fmaf(x2.y, y2.y, sa); sa = fmaf(x2.z, y2.z, sa); sa = fmaf(x2.w, y2.w, sa);
+            sb = fmaf(x3.x, y3.x, sb); sb = fmaf(x3.y, y3.y, sb); sb = fmaf(x3.z, y3.z, sb); sb = fmaf(x3.w, y3.w, sb);
+        }
+        for (; i < n4; i += 32) {
+            const float4 x = __ldg(a4 + i), y = b4[i];
+            sa = fmaf(x.x, y.x, sa); sa = fmaf(x.y, y.y, sa); sa = fmaf(x.z, y.z, sa); sa = fmaf(x.w, y.w, sa);
+        }
+        acc = sa + sb;
+    } else {
+        for (int i = lane; i < D; i += 32) acc = fmaf(a[i], qs[i], acc);
+    }
+    return warp_sum(acc);
+}
+
+// The certified bound on |bf16-path score - fp32 score| of any database row against a query q (topk_finalize_kernel
+// derives it): q2 = ||q||^2, qt2 = ||bf16(q)||^2, qf2 = ||q - bf16(q)||^2, db_stats = {max_r ||bf16(x_r) - x_r||^2,
+// max_r ||x_r||^2} (mdir_pack_stats).  The bound is symmetric in the two rows when db_stats covers q's row as well.
+__device__ __forceinline__ float bf16_eps(const float* __restrict__ db_stats, float q2, float qt2, float qf2, int D) {
+    const float e_max = sqrtf(db_stats[0]), x_max = sqrtf(db_stats[1]);
+    float eps = e_max * sqrtf(qt2) + x_max * sqrtf(qf2) + 1.25f * (float)D * 5.9604645e-8f * x_max * sqrtf(q2);
+    eps = eps * 1.001f + 1e-7f;                              // slack for evaluating the bound itself in fp32
+    return eps;
+}
+
 __device__ __forceinline__ void bitonic_sort_smem(uint64_t* a, int n) {
     for (int kk = 2; kk <= n; kk <<= 1) {
         for (int j = kk >> 1; j > 0; j >>= 1) {

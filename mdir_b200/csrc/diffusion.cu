@@ -11,6 +11,8 @@
 // Solve.  One CTA per query (a persistent grid over the queries); CG in fp64 on the fp32 graph weights.  Every step's arithmetic depends only on the query's
 // own shortlist and the graph, and every reduction runs in a fixed order (per-thread strided sums, an xor-shuffle tree
 // per warp, the warp partials summed in warp order), so a query's result is the same bits alone or in any batch.
+#include <cuda_bf16.h>
+
 #include <cfloat>
 
 #include "common.cuh"
@@ -243,6 +245,238 @@ __global__ void __launch_bounds__(kDiffThreads) diffusion_solve_kernel(
 
 constexpr size_t kDiffSmem = (size_t)kDiffMaxTrunc * (8 + 4 * 8 + 2);   // keys, x / r / p / Ap, counts: 84 KB
 
+// ---- incremental graph update (Diffusion.add / restore / remove) ---------------------------------------------------
+// Raw lists hold (k + 1) entries per slot; an entry's key is make_key(score, id) (smaller = better), ~0 for padding.
+constexpr int kMergeCols = 32;            // target rows per CTA of diffusion_merge_kernel
+constexpr int kMergeWarps = 8;
+constexpr int kMergeStage = 128;          // new keys a warp stages before merging them into its row's list
+
+__device__ __forceinline__ uint64_t diff_entry_key(const int32_t* ids, const float* s, int64_t e) {
+    const int32_t id = ids[e];
+    return id == -1 ? ~0ull : make_key(s[e], (uint32_t)id);
+}
+__device__ __forceinline__ bool diff_live(const uint32_t* __restrict__ live, int64_t slot) {
+    return (live[slot >> 5] >> (slot & 31)) & 1u;
+}
+
+// eps[j] = bf16_eps of row j of q32 (n_q, D) taken as a query: range_tau_kernel's norms and bound.
+__global__ void __launch_bounds__(256) diffusion_batch_eps_kernel(const float* __restrict__ q32, int D, const float* __restrict__ db_stats,
+                                                                  float* __restrict__ eps) {
+    __shared__ float red[32];
+    const int q = blockIdx.x;
+    float q2 = 0.f, qt2 = 0.f, qf2 = 0.f;
+    for (int i = threadIdx.x; i < D; i += blockDim.x) {
+        const float v = q32[(int64_t)q * D + i];
+        const float vt = __bfloat162float(__float2bfloat16_rn(v));
+        q2 = fmaf(v, v, q2);
+        qt2 = fmaf(vt, vt, qt2);
+        qf2 = fmaf(v - vt, v - vt, qf2);
+    }
+    q2 = block_sum(q2, red);
+    qt2 = block_sum(qt2, red);
+    qf2 = block_sum(qf2, red);
+    if (threadIdx.x == 0) eps[q] = bf16_eps(db_stats, q2, qt2, qf2, D);
+}
+
+// The reverse merge of a batch B into the raw lists of the target rows i (rows of the plane's chunk whose bit in `live`
+// is set), one CTA per tile of kMergeCols rows, in two kernels on the same grid.  plane (nb, ld) fp32 = the bf16 scores
+// of B (queries) against the chunk's rows.
+// (1) diffusion_screen_kernel: pair (i, j) passes when its bf16 score >= fsub_rd(score(T_i), eps[j]), T_i the key of
+//     entry k of i's list (every pair passes when that entry is padding).  Passing pairs go to the CTA's segment through a
+//     warp-aggregated shared-memory counter; cnt[tile] is exact even past `cap`, so that the host re-runs an overflowed
+//     tile with room.
+// (2) diffusion_merge_kernel, for a tile with cnt <= cap: one warp per passing pair re-scores it with rescore_row, row i
+//     as the query (the build's roles and summation order), and accepts key(s_ij, id_j) < T_i; then one warp per target
+//     row stages its accepted keys and rank-merges them into the sorted list (keys are unique: B's ids are in no target
+//     list), keeping the first k + 1.  rep[tile] = list entries replaced (0 when the tile overflowed: no list touched).
+// T_i and the screen limit of the tile's kMergeCols target rows (s_ts NaN: row i is not a target, nothing passes)
+__device__ __forceinline__ void diff_tile_thresholds(int64_t row0, int64_t n_rows, const uint32_t* __restrict__ live, const int32_t* knn_ids,
+                                                     const float* knn_s, int k, uint64_t* s_T, float* s_ts) {
+    if (threadIdx.x < kMergeCols) {
+        const int64_t i = row0 + threadIdx.x;
+        const bool ok = threadIdx.x < n_rows && diff_live(live, i);
+        const uint64_t T = ok ? diff_entry_key(knn_ids, knn_s, i * (k + 1) + k) : 0ull;     // 0: no key is smaller
+        s_T[threadIdx.x] = T;
+        s_ts[threadIdx.x] = !ok ? NAN : T == ~0ull ? -INFINITY : key_score(T);
+    }
+    __syncthreads();
+}
+
+__global__ void __launch_bounds__(kMergeWarps * 32) diffusion_screen_kernel(
+        const float* __restrict__ plane, int64_t ld, int nb, int64_t col0, int64_t n_cols, const int32_t* __restrict__ tiles,
+        const uint32_t* __restrict__ live, const float* __restrict__ eps, const int32_t* __restrict__ knn_ids, const float* __restrict__ knn_s,
+        int k, uint64_t* __restrict__ seg, int cap, int32_t* __restrict__ cnt) {
+    __shared__ uint64_t s_T[kMergeCols];
+    __shared__ float s_ts[kMergeCols];
+    __shared__ int s_cnt;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t tile = tiles ? (int64_t)tiles[blockIdx.x] : col0 / kMergeCols + blockIdx.x;
+    const int64_t c_lo = tile * kMergeCols - col0;             // the tile's first column of the plane
+    uint64_t* ent = seg + (int64_t)blockIdx.x * 2 * cap;        // (column << 32 | batch row)
+    if (threadIdx.x == 0) s_cnt = 0;
+    diff_tile_thresholds(col0 + c_lo, n_cols - c_lo, live, knn_ids, knn_s, k, s_T, s_ts);
+    // (1) screen: warp w reads batch rows w, w + 8, ...; lane = column (coalesced 128-byte rows of the plane)
+    const float ts = s_ts[lane];
+    if (__any_sync(0xffffffffu, ts == ts)) {
+        const float* col = plane + c_lo + lane;
+        for (int j0 = warp; j0 < nb; j0 += 4 * kMergeWarps) {
+            float v[4];                                         // four rows' loads in flight per lane
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int j = j0 + u * kMergeWarps;
+                v[u] = ts == ts && j < nb ? __ldg(col + (int64_t)j * ld) : 0.f;
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int j = j0 + u * kMergeWarps;
+                const bool pass = ts == ts && j < nb && v[u] >= __fsub_rd(ts, __ldg(eps + min(j, nb - 1)));
+                const unsigned bal = __ballot_sync(0xffffffffu, pass);
+                if (bal) {
+                    int base = 0;
+                    if (lane == 0) base = atomicAdd(&s_cnt, __popc(bal));
+                    base = __shfl_sync(0xffffffffu, base, 0);
+                    const int o = base + __popc(bal & ((1u << lane) - 1u));
+                    if (pass && o < cap) ent[o] = ((uint64_t)lane << 32) | (uint32_t)j;
+                }
+            }
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) cnt[tile] = s_cnt;
+}
+
+// Runs after diffusion_screen_kernel on the same grid: a tile whose count exceeds cap is left as it is.
+__global__ void __launch_bounds__(kMergeWarps * 32, 1) diffusion_merge_kernel(
+        int64_t col0, int64_t n_cols, const int32_t* __restrict__ tiles, const uint32_t* __restrict__ live, const int64_t* __restrict__ bslot,
+        const float* __restrict__ db32, int D, const uint32_t* __restrict__ slot_id, int32_t* __restrict__ knn_ids, float* __restrict__ knn_s,
+        int k, uint64_t* __restrict__ seg, int cap, const int32_t* __restrict__ cnt, int32_t* __restrict__ rep) {
+    __shared__ uint64_t s_T[kMergeCols];
+    __shared__ float s_ts[kMergeCols];
+    __shared__ uint64_t s_lst[kMergeWarps][kDiffMaxK + 1], s_out[kMergeWarps][kDiffMaxK + 1], s_stage[kMergeWarps][kMergeStage];
+    __shared__ int s_rep;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int kr = k + 1;
+    const int64_t tile = tiles ? (int64_t)tiles[blockIdx.x] : col0 / kMergeCols + blockIdx.x;
+    const int64_t c_lo = tile * kMergeCols - col0;
+    const int n = cnt[tile];
+    if (n > cap) {
+        if (threadIdx.x == 0) rep[tile] = 0;
+        return;
+    }
+    uint64_t* ent = seg + (int64_t)blockIdx.x * 2 * cap;        // (column << 32 | batch row), then the accepted keys
+    uint64_t* acc = ent + cap;
+    if (threadIdx.x == 0) s_rep = 0;
+    diff_tile_thresholds(col0 + c_lo, n_cols - c_lo, live, knn_ids, knn_s, k, s_T, s_ts);
+    // (2) re-score every passing pair in fp32
+    for (int e = warp; e < n; e += kMergeWarps) {
+        const uint64_t en = ent[e];
+        const int c = (int)(en >> 32);
+        const int64_t i = col0 + c_lo + c, j = bslot[(uint32_t)en];
+        const float s = rescore_row(db32 + j * D, db32 + i * D, D, lane);
+        const uint64_t key = make_key(s, slot_id[j]);
+        if (lane == 0) acc[e] = key < s_T[c] ? key : ~0ull;
+    }
+    __syncthreads();
+    // (3) merge, one warp per target row
+    uint64_t* lst = s_lst[warp];
+    uint64_t* out = s_out[warp];
+    uint64_t* stage = s_stage[warp];
+    int replaced = 0;
+    for (int c = warp; c < kMergeCols; c += kMergeWarps) {
+        if (s_ts[c] != s_ts[c]) continue;
+        const int64_t i = col0 + c_lo + c;
+        for (int p = lane; p < kr; p += 32) lst[p] = diff_entry_key(knn_ids, knn_s, i * kr + p);
+        int ns = 0, n_new = 0;
+        for (int e0 = 0; e0 < n; e0 += 32) {
+            const int e = e0 + lane;
+            const uint64_t key = e < n && (int)(ent[e] >> 32) == c ? acc[e] : ~0ull;
+            const unsigned bal = __ballot_sync(0xffffffffu, key != ~0ull);
+            if (key != ~0ull) stage[ns + __popc(bal & ((1u << lane) - 1u))] = key;
+            ns += __popc(bal);
+            n_new += __popc(bal);
+            if (ns > kMergeStage - 32 || (e0 + 32 >= n && ns > 0)) {
+                __syncwarp();
+                // ranks in the union: old entry p -> p + #(staged keys below it); staged key -> #(staged below) + #(old below)
+                for (int p = lane; p < kr; p += 32) {
+                    const uint64_t a = lst[p];
+                    int r = p;
+                    for (int t = 0; t < ns; ++t) r += stage[t] < a;
+                    if (r < kr) out[r] = a;
+                }
+                for (int t = lane; t < ns; t += 32) {
+                    const uint64_t b = stage[t];
+                    int r = 0;
+                    for (int u = 0; u < ns; ++u) r += stage[u] < b;
+                    int lo = 0, hi = kr;
+                    while (lo < hi) {
+                        const int mid = (lo + hi) >> 1;
+                        if (lst[mid] < b) lo = mid + 1;
+                        else hi = mid;
+                    }
+                    r += lo;
+                    if (r < kr) out[r] = b;
+                }
+                __syncwarp();
+                for (int p = lane; p < kr; p += 32) lst[p] = out[p];
+                __syncwarp();
+                ns = 0;
+            }
+        }
+        if (n_new == 0) continue;
+        // entries of the merged list that were not in the old one, then the list written back
+        for (int p = lane; p < kr; p += 32) {
+            const uint64_t key = lst[p];
+            if (key == ~0ull) continue;
+            int lo = 0, hi = kr;
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (diff_entry_key(knn_ids, knn_s, i * kr + mid) < key) lo = mid + 1;
+                else hi = mid;
+            }
+            replaced += !(lo < kr && diff_entry_key(knn_ids, knn_s, i * kr + lo) == key);
+        }
+        __syncwarp();
+        for (int p = lane; p < kr; p += 32) {
+            const uint64_t key = lst[p];
+            knn_ids[i * kr + p] = key == ~0ull ? -1 : (int32_t)(uint32_t)key;
+            knn_s[i * kr + p] = key == ~0ull ? -INFINITY : key_score(key);
+        }
+        __syncwarp();
+    }
+    replaced = warp_sum_int(replaced);
+    if (lane == 0 && replaced) atomicAdd(&s_rep, replaced);
+    __syncthreads();
+    if (threadIdx.x == 0) rep[tile] = s_rep;
+}
+
+// One warp per used slot: a removed slot's list becomes padding; a live slot whose list holds an id that is no longer
+// live (or no longer held by any used slot) gets flag 1, else 0.
+__global__ void __launch_bounds__(256) diffusion_stale_kernel(int32_t* __restrict__ knn_ids, float* __restrict__ knn_s, int64_t n_used, int k,
+                                                              const uint32_t* __restrict__ slot_id, const uint32_t* __restrict__ live,
+                                                              uint8_t* __restrict__ flag) {
+    const int lane = threadIdx.x & 31;
+    const int64_t i = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (i >= n_used) return;
+    const int kr = k + 1;
+    if (!diff_live(live, i)) {
+        for (int p = lane; p < kr; p += 32) {
+            knn_ids[i * kr + p] = -1;
+            knn_s[i * kr + p] = -INFINITY;
+        }
+        if (lane == 0) flag[i] = 0;
+        return;
+    }
+    bool stale = false;
+    for (int p = lane; p < kr; p += 32) {
+        const int32_t id = knn_ids[i * kr + p];
+        if (id == -1) continue;
+        const int64_t s = diff_slot_of(slot_id, n_used, id);
+        stale |= s < 0 || !diff_live(live, s);
+    }
+    stale = __any_sync(0xffffffffu, stale);
+    if (lane == 0) flag[i] = stale ? 1 : 0;
+}
+
 }  // namespace mdir
 
 using namespace mdir;
@@ -264,6 +498,42 @@ extern "C" int mdir_diffusion_normalize(const int32_t* nbr, const float* w, cons
     const int64_t n = n_used * k;
     if (n == 0) return 0;
     diffusion_normalize_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(nbr, w, deg, n_used, k, S);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_diffusion_batch_eps(const float* q32, int n_q, int D, const float* db_stats, float* eps, void* stream) {
+    MDIR_CHECK_ARG(q32 && db_stats && eps && n_q >= 0 && D >= 1);
+    if (n_q == 0) return 0;
+    diffusion_batch_eps_kernel<<<n_q, 256, 0, (cudaStream_t)stream>>>(q32, D, db_stats, eps);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_diffusion_merge(const float* plane, int64_t ld, int nb, int64_t col0, int64_t n_cols, const int32_t* tiles, int n_tiles,
+                                    const uint32_t* live, const float* eps, const int64_t* bslot, const float* db32, int D,
+                                    const uint32_t* slot_id, int32_t* knn_ids, float* knn_s, int k, uint64_t* seg, int cap, int32_t* cnt,
+                                    int32_t* rep, void* stream) {
+    MDIR_CHECK_ARG(plane && live && eps && bslot && db32 && slot_id && knn_ids && knn_s && seg && cnt && rep);
+    MDIR_CHECK_ARG(nb >= 1 && n_cols >= 0 && ld >= n_cols && col0 >= 0 && col0 % kMergeCols == 0 && D >= 1 && k >= 1 && k <= kDiffMaxK);
+    MDIR_CHECK_ARG(cap >= 1 && (tiles == nullptr || n_tiles >= 0));
+    const int64_t grid = tiles ? n_tiles : (n_cols + kMergeCols - 1) / kMergeCols;
+    if (grid == 0) return 0;
+    MDIR_CHECK_ARG(grid < ((int64_t)1 << 31));
+    diffusion_screen_kernel<<<(unsigned)grid, kMergeWarps * 32, 0, (cudaStream_t)stream>>>(plane, ld, nb, col0, n_cols, tiles, live, eps, knn_ids,
+                                                                                           knn_s, k, seg, cap, cnt);
+    MDIR_LAUNCH_CHECK();
+    diffusion_merge_kernel<<<(unsigned)grid, kMergeWarps * 32, 0, (cudaStream_t)stream>>>(col0, n_cols, tiles, live, bslot, db32, D, slot_id, knn_ids,
+                                                                                          knn_s, k, seg, cap, cnt, rep);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_diffusion_stale_rows(int32_t* knn_ids, float* knn_s, int64_t n_used, int k, const uint32_t* slot_id, const uint32_t* live,
+                                         uint8_t* flag, void* stream) {
+    MDIR_CHECK_ARG(knn_ids && knn_s && slot_id && live && flag && n_used >= 0 && k >= 1 && k <= kDiffMaxK);
+    if (n_used == 0) return 0;
+    diffusion_stale_kernel<<<(unsigned)((n_used + 7) / 8), 256, 0, (cudaStream_t)stream>>>(knn_ids, knn_s, n_used, k, slot_id, live, flag);
     MDIR_LAUNCH_CHECK();
     return 0;
 }

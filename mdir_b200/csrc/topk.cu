@@ -359,35 +359,7 @@ __device__ __forceinline__ int cluster_ld_s32(uint32_t a) {
     return v;
 }
 
-// fp32 dot product of one database row with the query staged in shared memory, one warp per row.  The summation order
-// is that of each row of rescore_row2, so a row's fp32 score does not depend on whether it was re-scored alone or as
-// one of a pair: every finalize path and range_gather_kernel give the same bits for the same row.
-__device__ __forceinline__ float rescore_row(const float* __restrict__ a, const float* qs, int D, int lane) {
-    float acc = 0.f;
-    if ((D & 3) == 0) {
-        const float4* a4 = reinterpret_cast<const float4*>(a);
-        const float4* b4 = reinterpret_cast<const float4*>(qs);
-        const int n4 = D >> 2;
-        float sa = 0.f, sb = 0.f;
-        int i = lane;
-        for (; i + 96 < n4; i += 128) {            // 4 independent 128-bit loads in flight per lane
-            const float4 x0 = __ldg(a4 + i), x1 = __ldg(a4 + i + 32), x2 = __ldg(a4 + i + 64), x3 = __ldg(a4 + i + 96);
-            const float4 y0 = b4[i], y1 = b4[i + 32], y2 = b4[i + 64], y3 = b4[i + 96];
-            sa = fmaf(x0.x, y0.x, sa); sa = fmaf(x0.y, y0.y, sa); sa = fmaf(x0.z, y0.z, sa); sa = fmaf(x0.w, y0.w, sa);
-            sb = fmaf(x1.x, y1.x, sb); sb = fmaf(x1.y, y1.y, sb); sb = fmaf(x1.z, y1.z, sb); sb = fmaf(x1.w, y1.w, sb);
-            sa = fmaf(x2.x, y2.x, sa); sa = fmaf(x2.y, y2.y, sa); sa = fmaf(x2.z, y2.z, sa); sa = fmaf(x2.w, y2.w, sa);
-            sb = fmaf(x3.x, y3.x, sb); sb = fmaf(x3.y, y3.y, sb); sb = fmaf(x3.z, y3.z, sb); sb = fmaf(x3.w, y3.w, sb);
-        }
-        for (; i < n4; i += 32) {
-            const float4 x = __ldg(a4 + i), y = b4[i];
-            sa = fmaf(x.x, y.x, sa); sa = fmaf(x.y, y.y, sa); sa = fmaf(x.z, y.z, sa); sa = fmaf(x.w, y.w, sa);
-        }
-        acc = sa + sb;
-    } else {
-        for (int i = lane; i < D; i += 32) acc = fmaf(a[i], qs[i], acc);
-    }
-    return warp_sum(acc);
-}
+// rescore_row (common.cuh): the fp32 dot product of one row with the staged query, one warp per row.
 
 // The k smallest of the cnt unique keys in skeys[0, cnt) (1024-thread block), sorted ascending into out[0, min(k, cnt))
 // (padded with ~0 up to kpow2), without the 8 MSB radix passes: candidates of one query share sign and exponent, so
@@ -836,9 +808,7 @@ __global__ void __launch_bounds__(1024) topk_finalize_kernel(const uint64_t* __r
             if (lane == 0) { s_red[wi] = q2; s_red[32 + wi] = qt2; s_red[64 + wi] = qf2; }
             __syncthreads();
             q2 = warp_sum(s_red[lane]); qt2 = warp_sum(s_red[32 + lane]); qf2 = warp_sum(s_red[64 + lane]);
-            const float e_max = sqrtf(db_stats[0]), x_max = sqrtf(db_stats[1]);
-            eps = e_max * sqrtf(qt2) + x_max * sqrtf(qf2) + 1.25f * (float)D * 5.9604645e-8f * x_max * sqrtf(q2);
-            eps = eps * 1.001f + 1e-7f;                              // slack for evaluating the bound itself in fp32
+            eps = bf16_eps(db_stats, q2, qt2, qf2, D);
         }
         __syncthreads();
         if (CS > 1) cluster_sync_all();                                // (1) helpers may read the shortlist
@@ -1543,10 +1513,7 @@ __global__ void __launch_bounds__(256) range_tau_kernel(const float* __restrict_
         q2 = block_sum(q2, red);
         qt2 = block_sum(qt2, red);
         qf2 = block_sum(qf2, red);
-        const float e_max = sqrtf(db_stats[0]), x_max = sqrtf(db_stats[1]);
-        float eps = e_max * sqrtf(qt2) + x_max * sqrtf(qf2) + 1.25f * (float)D * 5.9604645e-8f * x_max * sqrtf(q2);
-        eps = eps * 1.001f + 1e-7f;
-        lim = __fsub_rd(lim, eps);
+        lim = __fsub_rd(lim, bf16_eps(db_stats, q2, qt2, qf2, D));
     }
     if (threadIdx.x == 0) tau[q] = ((uint64_t)desc_key(lim) << 32) | 0xffffffffull;
 }

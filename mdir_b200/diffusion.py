@@ -1,11 +1,14 @@
 """Diffusion re-ranking on a mutual kNN graph of the database (Iscen, Tolias, Avrithis, Furon, Chum, CVPR 2017).
 
 NOT in the reference (parity unpinned, like qe.py): the semantics are restated in tests/diffusion_reference.py:diffusion_graph
-/ diffusion_search.  The graph is built once per index from the certified fp32 top-(k+1) of every row; a query's
+/ diffusion_search.  The graph is built once per index from the certified fp32 top-(k+1) of every row and kept exact
+through add / remove / restore / compact made through the Diffusion (DESIGN 2.2e); a query's
 certified fp32 shortlist L is re-ranked by f, the truncated CG solution of (I - alpha S_LL) f = y, where y holds the
 query's top k_q scores raised to gamma.  The graph kernels and the per-query solve are mdir_b200/csrc/diffusion.cu."""
+import contextlib
 import math
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -14,6 +17,12 @@ from .search import Index, ShardedIndex, WIDE_Q, _as_dev_f32
 
 MAX_K = 255          # neighbours per database row
 MAX_TRUNC = 2048     # shortlist rows per query the solve kernel holds in shared memory
+MERGE_TILE = 32      # target rows per CTA of mdir_diffusion_merge
+MERGE_CAP = 1024     # candidate pairs one tile of the reverse merge holds; a tile with more is re-run with exactly the room it needs
+# bytes of the (batch, row chunk) fp32 bf16-score plane of the reverse merge: 1,024 added rows screen 256 Ki rows per
+# dense scan, 10,000 rows 26 Ki.  At R1M on a B200 (1,000 W) the 10,000-row scan in 38 chunks ran at ~1,020 TFLOP/s and
+# the 1,024-row scan in 4 chunks at ~1,100 (profiles/r12_diffusion_update_1gpu.log); other sizes were not measured.
+SCREEN_PLANE_BYTES = 1 << 30
 
 
 def check_graph_params(k, gamma):
@@ -44,10 +53,19 @@ class Diffusion:
 
         g = Diffusion(index, k=50, gamma=3.0)      # the graph: one wide search pass per 1,024 rows
         f, ids = g.search(q, k=100, trunc=1000, k_q=10, alpha=0.99, iters=20, rtol=1e-6)
+        ids = g.add(vecs); g.remove(ids); g.restore(ids); g.compact()     # the index changes, the graph follows
 
     The index needs the fp32 master copy and no removed rows among its used slots (call compact() first; a free
-    capacity tail is fine).  A later remove / restore / add / compact makes the graph stale: search() then raises
-    until a new Diffusion is built."""
+    capacity tail is fine).  add / remove / restore / compact through the Diffusion mutate the index and keep the graph
+    exactly what a new Diffusion over the live rows would build (DESIGN 2.2e); a mutation made on the Index directly
+    makes the graph stale, and search() then raises until a new Diffusion is built.
+
+    State, allocated at the index's capacity (padding past the used slots): the raw lists knn_i / knn_s (the certified
+    fp32 top-(k+1) of every slot, -1 / -inf padding for a removed slot), 8 (k + 1) bytes per slot, and the graph nbr /
+    S / deg, 8 k + 4 bytes per slot.  update_stats counts, over the life of the object: rows re-searched, pairs passed by
+    the bf16 screen, pairs re-scored in fp32, list entries replaced and screen tiles re-run after an overflow."""
+
+    timed = False               # True: update_time gets each update's device time per phase (CUDA events)
 
     def __init__(self, index, k=50, gamma=3.0):
         check_graph_params(k, gamma)
@@ -62,32 +80,227 @@ class Diffusion:
         self.index, self.k, self.gamma = index, int(k), float(gamma)
         self._version = index._mutations
         self._status = None
-        dev = index.device
+        self.update_stats = {"rows_searched": 0, "screen_passed": 0, "rescored": 0, "replaced": 0, "screen_reruns": 0}
+        self.update_time = {}
+        self._events = []
+        cap, dev = index.n, index.device
         with torch.cuda.device(dev):
-            knn_i = torch.empty((n_used, self.k + 1), dtype=torch.int32, device=dev)
-            knn_s = torch.empty((n_used, self.k + 1), dtype=torch.float32, device=dev)
-            for r0 in range(0, n_used, DBA_BLOCK):
-                r1 = min(r0 + DBA_BLOCK, n_used)
-                s, i = index.search(index.db32[r0:r1], self.k + 1, precision="fp32", block_q=WIDE_Q)
-                knn_s[r0:r1] = s
-                knn_i[r0:r1] = i
-            self.nbr = torch.empty((n_used, self.k), dtype=torch.int32, device=dev)
-            self.S = torch.empty((n_used, self.k), dtype=torch.float32, device=dev)
-            self.deg = torch.empty((n_used,), dtype=torch.float32, device=dev)
-            lib = _lib.lib()
-            _lib.check(lib.mdir_diffusion_graph(_lib.ptr(knn_i), _lib.ptr(knn_s), n_used, self.k, _lib.ptr(index.slot_id), self.gamma,
-                                                _lib.ptr(self.nbr), _lib.ptr(self.S), _lib.ptr(self.deg), _lib.stream()), "mdir_diffusion_graph")
-            _lib.check(lib.mdir_diffusion_normalize(_lib.ptr(self.nbr), _lib.ptr(self.S), _lib.ptr(self.deg), n_used, self.k, _lib.ptr(self.S),
-                                                    _lib.stream()), "mdir_diffusion_normalize")
+            self.knn_i = torch.full((cap, self.k + 1), -1, dtype=torch.int32, device=dev)
+            self.knn_s = torch.full((cap, self.k + 1), float("-inf"), dtype=torch.float32, device=dev)
+            self.nbr = torch.full((cap, self.k), -1, dtype=torch.int32, device=dev)
+            self.S = torch.zeros((cap, self.k), dtype=torch.float32, device=dev)
+            self.deg = torch.zeros((cap,), dtype=torch.float32, device=dev)
+            self._search_rows(torch.arange(n_used, dtype=torch.int64, device=dev))
+            self._build_graph()
+        self.update_stats["rows_searched"] = 0              # the counters cover the updates
 
     def graph(self):
         """(nbr (n_used, k) int32 neighbour slots, mutual ones first and -1 padding; S (n_used, k) fp32 normalised
         weights aligned with nbr; deg (n_used,) fp32 degrees), on the device."""
-        return self.nbr, self.S, self.deg
+        n = self.index._n_used
+        return self.nbr[:n], self.S[:n], self.deg[:n]
 
     def status(self):
         """Per-query status words of the last search()'s shortlist search (Index.status(): 0 = exact and certified)."""
         return self._status
+
+    def _check_current(self):
+        if self.index._mutations != self._version:
+            raise _lib.MdirError("the index was mutated (remove / restore / add / compact) after the diffusion graph was built: "
+                                 "build a new Diffusion")
+
+    @contextlib.contextmanager
+    def _phase(self, name):
+        """Brackets one phase of an update with CUDA events when `timed` is set."""
+        if not self.timed:
+            yield
+            return
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        yield
+        b.record()
+        self._events.append((name, a, b))
+
+    def _finish(self):
+        """End of an update: the graph is current again; with `timed`, update_time = ms per phase of this update."""
+        self._version = self.index._mutations
+        if self.timed:
+            torch.cuda.current_stream().synchronize()
+            self.update_time = {}
+            for name, a, b in self._events:
+                self.update_time[name] = self.update_time.get(name, 0.0) + a.elapsed_time(b)
+            self._events = []
+
+    def _search_rows(self, slots):
+        """The raw lists of these slots (a device int64 tensor), with the build's own call: the certified fp32
+        top-(k+1) of each row against the index, DBA_BLOCK rows per search, wide passes."""
+        index = self.index
+        self.update_stats["rows_searched"] += int(slots.numel())
+        with self._phase("search"):
+            for r0 in range(0, slots.numel(), DBA_BLOCK):
+                b = slots[r0:r0 + DBA_BLOCK]
+                s, i = index.search(index.db32[b], self.k + 1, precision="fp32", block_q=WIDE_Q)
+                self.knn_s[b] = s
+                self.knn_i[b] = i
+
+    def _build_graph(self):
+        """nbr / S / deg over the used slots from the raw lists (the build's kernels; padding rows give empty rows)."""
+        n_used, lib = self.index._n_used, _lib.lib()
+        with self._phase("graph"):
+            _lib.check(lib.mdir_diffusion_graph(_lib.ptr(self.knn_i), _lib.ptr(self.knn_s), n_used, self.k, _lib.ptr(self.index.slot_id),
+                                                self.gamma, _lib.ptr(self.nbr), _lib.ptr(self.S), _lib.ptr(self.deg), _lib.stream()),
+                       "mdir_diffusion_graph")
+            _lib.check(lib.mdir_diffusion_normalize(_lib.ptr(self.nbr), _lib.ptr(self.S), _lib.ptr(self.deg), n_used, self.k, _lib.ptr(self.S),
+                                                    _lib.stream()), "mdir_diffusion_normalize")
+
+    def _merge_batch(self, bslot, live0, n_target):
+        """The reverse merge: the rows of slots bslot (device int64) into the lists of the slots [0, n_target) that are
+        set in live0 (the bitmap before the mutation, so the batch itself is no target).  One dense bf16 scan of the
+        batch against SCREEN_PLANE_BYTES-sized row chunks, then mdir_diffusion_merge per chunk; the tiles' counts are
+        read back once, and a tile that overflowed MERGE_CAP is re-run with exactly the room its count asks for."""
+        index, lib = self.index, _lib.lib()
+        nb, D = int(bslot.numel()), index.D
+        if nb == 0 or n_target == 0:
+            return
+        dev = index.device
+        stats = index.stats()                              # covers every row, the batch included (add merges its stats)
+        q16 = index.db16[bslot]
+        eps = torch.empty((nb,), dtype=torch.float32, device=dev)
+        _lib.check(lib.mdir_diffusion_batch_eps(_lib.ptr(index.db32[bslot]), nb, D, _lib.ptr(stats), _lib.ptr(eps), _lib.stream()),
+                   "mdir_diffusion_batch_eps")
+        rows = max(MERGE_TILE, SCREEN_PLANE_BYTES // (4 * nb) // MERGE_TILE * MERGE_TILE)
+        rows = min(rows, -(-n_target // MERGE_TILE) * MERGE_TILE)
+        plane = torch.empty((nb, rows), dtype=torch.float32, device=dev)
+        n_tiles = -(-n_target // MERGE_TILE)
+        cnt = torch.empty((n_tiles,), dtype=torch.int32, device=dev)
+        rep = torch.empty((n_tiles,), dtype=torch.int32, device=dev)
+
+        def run(r0, cap, tiles=None):
+            r1 = min(r0 + rows, n_target)
+            with self._phase("scan"):
+                _lib.check(lib.mdir_sim_scan_dense_bf16(_lib.ptr(index.db16[r0:r1]), r1 - r0, _lib.ptr(q16), nb, D, _lib.ptr(plane), rows,
+                                                        _lib.stream()), "mdir_sim_scan_dense_bf16")
+            n_run = -(-(r1 - r0) // MERGE_TILE) if tiles is None else int(tiles.numel())
+            seg = self._seg(2 * n_run * cap)
+            with self._phase("merge"):
+                _lib.check(lib.mdir_diffusion_merge(_lib.ptr(plane), rows, nb, r0, r1 - r0, _lib.ptr(tiles), n_run, _lib.ptr(live0),
+                                                    _lib.ptr(eps), _lib.ptr(bslot), _lib.ptr(index.db32), D, _lib.ptr(index.slot_id),
+                                                    _lib.ptr(self.knn_i), _lib.ptr(self.knn_s), self.k, _lib.ptr(seg), cap, _lib.ptr(cnt),
+                                                    _lib.ptr(rep), _lib.stream()), "mdir_diffusion_merge")
+
+        cap = MERGE_CAP
+        for r0 in range(0, n_target, rows):
+            run(r0, cap)
+        c, r = cnt.cpu().numpy(), rep.cpu().numpy()         # the call's synchronisation point
+        st = self.update_stats
+        st["screen_passed"] += int(c.sum())
+        over = np.flatnonzero(c > cap)
+        st["rescored"] += int(c.sum() - c[over].sum())
+        st["replaced"] += int(r.sum())
+        if over.size:
+            st["screen_reruns"] += int(over.size)
+            cap2 = int(c[over].max())
+            for r0 in sorted({int(t) * MERGE_TILE // rows * rows for t in over}):
+                t = over[(over * MERGE_TILE >= r0) & (over * MERGE_TILE < r0 + rows)]
+                run(r0, cap2, torch.from_numpy(t.astype(np.int32)).to(dev))
+            c2, r2 = cnt[torch.from_numpy(over).to(dev)].cpu().numpy(), rep[torch.from_numpy(over).to(dev)].cpu().numpy()
+            if (c2 > cap2).any():
+                raise _lib.MdirError("diffusion merge re-run overflowed its exact capacity (internal error)")
+            st["screen_passed"] += int(c2.sum())
+            st["rescored"] += int(c2.sum())
+            st["replaced"] += int(r2.sum())
+
+    def _seg(self, n):
+        """The reverse merge's candidate segments (uint64), grown on demand and kept."""
+        seg = getattr(self, "_seg_buf", None)
+        if seg is None or seg.numel() < n:
+            seg = self._seg_buf = torch.empty((n,), dtype=torch.int64, device=self.index.device)
+        return seg
+
+    def _insert(self, bslot, live0, n_target):
+        """Rows that became live (bslot): their own lists, then the reverse merge into everyone else's, then the graph."""
+        self._search_rows(bslot)
+        self._merge_batch(bslot, live0, n_target)
+        self._build_graph()
+
+    def add(self, vecs):
+        """index.add(vecs), and the graph follows; returns the new ids.  The new rows' lists come from the build's
+        search; every other live row's list takes in the new rows that beat its (k+1)-th entry (the reverse merge: a
+        certified bf16 screen of the new rows against the database, exact fp32 re-scores of the pairs that pass).  Cost:
+        one search of the new rows plus one dense bf16 scan of them against the used rows, then the graph kernels.
+        Errors (a full index, wrong shape) are raised by index.add before anything changes.  Runs on the current stream
+        and synchronises with the host: once for the merge's counters, besides the searches' own status checks."""
+        self._check_current()
+        index = self.index
+        s0, live0 = index._n_used, index.live.clone()
+        ids = index.add(vecs)
+        with torch.cuda.device(index.device):
+            if index._n_used > s0:
+                self._insert(torch.arange(s0, index._n_used, dtype=torch.int64, device=index.device), live0, s0)
+        self._finish()
+        return ids
+
+    def restore(self, ids):
+        """index.restore(ids), and the graph follows: the restored rows get lists from the build's search and enter the
+        other live rows' lists by the reverse merge of add().  Errors (an id never issued, or purged by compact) are
+        raised by index.restore before anything changes.  Synchronises with the host as add() does."""
+        self._check_current()
+        index = self.index
+        before, live0 = index._live_host.copy(), index.live.clone()
+        index.restore(ids)
+        with torch.cuda.device(index.device):
+            back = np.flatnonzero(index._live_host & ~before)
+            if back.size:
+                self._insert(torch.from_numpy(back).to(index.device), live0, index._n_used)
+        self._finish()
+
+    def remove(self, ids):
+        """index.remove(ids), and the graph follows: the removed rows' lists become padding and their graph rows empty;
+        the live rows whose lists held one of them (about k + 1 per removed row) are searched again with the build's
+        call.  The cost grows with that number: removing a large fraction of the rows approaches the cost of a rebuild.
+        Errors are raised by index.remove before anything changes.  Synchronises with the host once to find the rows to
+        search again, besides the searches' own status checks."""
+        self._check_current()
+        index = self.index
+        version = index._mutations
+        index.remove(ids)
+        if index._mutations != version:
+            lib = _lib.lib()
+            with torch.cuda.device(index.device):
+                n_used = index._n_used
+                flag = torch.empty((n_used,), dtype=torch.uint8, device=index.device)
+                with self._phase("stale"):
+                    _lib.check(lib.mdir_diffusion_stale_rows(_lib.ptr(self.knn_i), _lib.ptr(self.knn_s), n_used, self.k,
+                                                             _lib.ptr(index.slot_id), _lib.ptr(index.live), _lib.ptr(flag), _lib.stream()),
+                               "mdir_diffusion_stale_rows")
+                self._search_rows(torch.nonzero(flag).view(-1))
+                self._build_graph()
+        self._finish()
+
+    def compact(self):
+        """index.compact(), and the graph follows: the live slots' lists move to the front in the same stable order
+        (they hold ids, which compaction keeps, so no list changes) and the graph is rebuilt from them.  Returns the
+        number of rows purged.  Afterwards graph(), search() and its status words equal those of a new
+        Diffusion(index, k, gamma) bit for bit."""
+        self._check_current()
+        index = self.index
+        n_old = index._n_used
+        keep = np.flatnonzero(index._live_host[:n_old])
+        purged = index.compact()
+        if purged:
+            with torch.cuda.device(index.device):
+                keep_d = torch.from_numpy(keep).to(index.device)
+                n = keep.size
+                self.knn_i[:n] = self.knn_i[keep_d]
+                self.knn_s[:n] = self.knn_s[keep_d]
+                self.knn_i[n:n_old] = -1
+                self.knn_s[n:n_old] = float("-inf")
+                self.nbr[n:n_old] = -1
+                self.S[n:n_old] = 0.0
+                self.deg[n:n_old] = 0.0
+                self._build_graph()
+        self._finish()
+        return purged
 
     def search(self, q, k=100, trunc=1000, k_q=10, alpha=0.99, iters=20, rtol=1e-6):
         """q: (N_q, D) fp32 (host or device).  Returns (f (N_q, k) fp32, ids (N_q, k) int32) on the device: the shortlist
@@ -95,9 +308,7 @@ class Diffusion:
         (I - alpha S_LL) f = y with y_u = max(s_u, 0)^gamma on the first k_q rows of L; -inf / -1 padding past |L|."""
         check_search_params(k, trunc, k_q, alpha, iters, rtol)
         index = self.index
-        if index._mutations != self._version:
-            raise _lib.MdirError("the index was mutated (remove / restore / add / compact) after the diffusion graph was built: "
-                                 "build a new Diffusion")
+        self._check_current()
         k, trunc = int(k), int(trunc)
         dev = index.device
         with torch.cuda.device(dev):
@@ -113,7 +324,7 @@ class Diffusion:
             lib = _lib.lib()
             ws_bytes = lib.mdir_diffusion_solve_workspace_bytes(n_q, trunc, self.k)
             ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-            _lib.check(lib.mdir_diffusion_solve(_lib.ptr(ids), _lib.ptr(s), n_q, trunc, _lib.ptr(index.slot_id), self.nbr.shape[0],
+            _lib.check(lib.mdir_diffusion_solve(_lib.ptr(ids), _lib.ptr(s), n_q, trunc, _lib.ptr(index.slot_id), index._n_used,
                                                 _lib.ptr(self.nbr), _lib.ptr(self.S), self.k, int(k_q), self.gamma, float(alpha),
                                                 int(iters), float(rtol), k, _lib.ptr(ws), ws_bytes, _lib.ptr(f), _lib.ptr(out),
                                                 _lib.stream()), "mdir_diffusion_solve")
