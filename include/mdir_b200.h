@@ -449,6 +449,18 @@ int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int n_q, int tr
                          const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
                          int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, void* stream);
 
+/* Offline diffusion (mdir_b200.DiffusionTable; DESIGN 2.2e).  tab_ids / tab_f (>= n_used rows, width) = per slot the
+ *   top `width` (id, f) of that slot's row diffused as a query with k_q = 1 (mdir_diffusion_solve's output; -1 / -inf
+ *   padding).  mdir_diffusion_combine: per query q, L = L_ids / L_s (n_q, k_q), its certified fp32 top-k_q (-1 padding),
+ *   w_u = max(L_s[u], 0)^gamma in fp64; for every id j in the union of the table rows of L's slots, f_j = the sum over
+ *   u ascending of w_u * tab_f[slot(L_u)][e] (fp64, the product and the sum rounded separately; padding skipped).
+ *   f_out / ids_out (n_q, k_out) = the top k_out by ((float) f desc, id asc), -inf / -1 padding past the union.  Ids
+ *   outside the union are not candidates.  1 <= k_q <= 128, 1 <= width <= 1024, k_q * width <= 8192,
+ *   1 <= k_out <= 8192.  Bit-identical for a query alone or in any batch.                                            */
+int mdir_diffusion_combine(const int32_t* L_ids, const float* L_s, int n_q, int k_q, const uint32_t* slot_id, int64_t n_used,
+                           const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
+                           int32_t* ids_out, void* stream);
+
 /* Incremental update of the raw lists (Diffusion.add / restore / remove; DESIGN 2.2e).  A list entry's key is
  * mdir_make_key(score, id), smaller = better, all ones for padding; T_i = the key of entry k of slot i's list.
  * mdir_diffusion_batch_eps: eps[j] = the certified bf16 bound of row j of q32 (n_q, D) taken as a query (the formula of

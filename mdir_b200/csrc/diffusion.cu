@@ -11,6 +11,9 @@
 // Solve.  One CTA per query (a persistent grid over the queries); CG in fp64 on the fp32 graph weights.  Every step's arithmetic depends only on the query's
 // own shortlist and the graph, and every reduction runs in a fixed order (per-thread strided sums, an xor-shuffle tree
 // per warp, the warp partials summed in warp order), so a query's result is the same bits alone or in any batch.
+//
+// Combine (offline diffusion).  A table of every slot's own diffusion truncated to `width` entries, and per query the
+// weighted sum of the table rows of its top-k_q (diffusion_combine_kernel).
 #include <cuda_bf16.h>
 
 #include <cfloat>
@@ -477,6 +480,87 @@ __global__ void __launch_bounds__(256) diffusion_stale_kernel(int32_t* __restric
     if (lane == 0) flag[i] = stale ? 1 : 0;
 }
 
+// ---- offline diffusion (DiffusionTable.search) ------------------------------------------------------------------------
+// Table row of slot s: the top `width` (id, f) of that row's own diffusion (k_q = 1).  A query's f_j is the sum over the
+// k_q rows L_u of its top-k_q of w_u F[slot(L_u)][j], w_u = max(s_u, 0)^gamma, over the union of those table rows.
+constexpr int kCombMaxKq = 128;           // u takes 7 bits of a staged key
+constexpr int kCombMaxWidth = 1024;       // e takes 10 bits
+constexpr int kCombMaxEntries = 8192;     // k_q * width: 64-bit keys, fp32 sums and head flags, 104 KB of smem
+constexpr int kCombThreads = 512;
+constexpr int kCombCtas = 2 * kNumSMs;
+
+__host__ __device__ inline int comb_npow(int n) {
+    int p = 32;
+    while (p < n) p <<= 1;
+    return p;
+}
+__host__ __device__ inline size_t comb_smem_bytes(int n) { return ((size_t)comb_npow(n) * (8 + 4 + 1) + 15) & ~(size_t)15; }
+
+// One CTA per query (a persistent grid).  (1) L's ids -> slots, w_u in fp64; (2) key (id, u, e) per live table entry,
+// bitonic-sorted; (3) the first entry of each id's run sums its run in key order (ascending u) in fp64, as
+// f = f + w_u * F with separate roundings; (4) the run heads re-keyed make_key((float)f, id), sorted, top k_out emitted.
+// No atomics and fixed orders: a query's result is the same bits alone or in any batch.
+__global__ void __launch_bounds__(kCombThreads, 2) diffusion_combine_kernel(
+        const int32_t* __restrict__ L_ids, const float* __restrict__ L_s, int n_q, int k_q, const uint32_t* __restrict__ slot_id,
+        int64_t n_used, const int32_t* __restrict__ tab_ids, const float* __restrict__ tab_f, int width, float gamma, int k_out,
+        float* __restrict__ f_out, int32_t* __restrict__ ids_out) {
+    extern __shared__ __align__(16) uint8_t smem[];
+    __shared__ int64_t s_slot[kCombMaxKq];
+    __shared__ double s_w[kCombMaxKq];
+    const int n = k_q * width, npow = comb_npow(n);
+    uint64_t* keys = reinterpret_cast<uint64_t*>(smem);
+    float* fsum = reinterpret_cast<float*>(keys + npow);
+    uint8_t* head = reinterpret_cast<uint8_t*>(fsum + npow);
+    const int tid = threadIdx.x;
+    constexpr int kIdShift = 17;
+
+    for (int q = blockIdx.x; q < n_q; q += gridDim.x) {
+        for (int u = tid; u < k_q; u += kCombThreads) {
+            s_slot[u] = diff_slot_of(slot_id, n_used, L_ids[(int64_t)q * k_q + u]);
+            s_w[u] = pow((double)fmaxf(L_s[(int64_t)q * k_q + u], 0.f), (double)gamma);
+        }
+        __syncthreads();
+        for (int t = tid; t < npow; t += kCombThreads) {
+            uint64_t key = ~0ull;
+            if (t < n) {
+                const int u = t / width, e = t - u * width;
+                const int64_t s = s_slot[u];
+                const int32_t id = s >= 0 ? tab_ids[s * width + e] : -1;
+                if (id != -1) key = ((uint64_t)(uint32_t)id << kIdShift) | ((uint64_t)u << 10) | (uint64_t)e;
+            }
+            keys[t] = key;
+        }
+        __syncthreads();
+        bitonic_sort_smem(keys, npow);
+        for (int t = tid; t < npow; t += kCombThreads) {
+            const uint64_t kt = keys[t];
+            const uint64_t id = kt >> kIdShift;                    // padding: 2^47 - 1, no id
+            const bool h = kt != ~0ull && (t == 0 || (keys[t - 1] >> kIdShift) != id);
+            if (h) {
+                double f = 0.0;
+                for (int r = t; r < npow && (keys[r] >> kIdShift) == id; ++r) {
+                    const int u = (int)((keys[r] >> 10) & (kCombMaxKq - 1)), e = (int)(keys[r] & (kCombMaxWidth - 1));
+                    f = __dadd_rn(f, __dmul_rn(s_w[u], (double)tab_f[s_slot[u] * width + e]));
+                }
+                fsum[t] = (float)f;
+            }
+            head[t] = h;
+        }
+        __syncthreads();
+        for (int t = tid; t < npow; t += kCombThreads)
+            keys[t] = head[t] ? make_key(fsum[t], (uint32_t)(keys[t] >> kIdShift)) : ~0ull;
+        __syncthreads();
+        bitonic_sort_smem(keys, npow);
+        for (int j = tid; j < k_out; j += kCombThreads) {
+            const uint64_t kt = j < npow ? keys[j] : ~0ull;
+            const bool ok = kt != ~0ull;
+            f_out[(int64_t)q * k_out + j] = ok ? key_score(kt) : -INFINITY;
+            ids_out[(int64_t)q * k_out + j] = ok ? (int32_t)(uint32_t)kt : -1;
+        }
+        __syncthreads();                                                     // keys / s_slot are rewritten by the next query
+    }
+}
+
 }  // namespace mdir
 
 using namespace mdir;
@@ -558,6 +642,23 @@ extern "C" int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int 
     diffusion_solve_kernel<<<grid, kDiffThreads, kDiffSmem, (cudaStream_t)stream>>>(L_ids, L_s, n_q, trunc, slot_id, n_used, nbr, S, k, k_q,
                                                                                    gamma, alpha, iters, rtol, k_out, (uint8_t*)ws, f_out,
                                                                                    ids_out);
+    MDIR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int mdir_diffusion_combine(const int32_t* L_ids, const float* L_s, int n_q, int k_q, const uint32_t* slot_id, int64_t n_used,
+                                      const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
+                                      int32_t* ids_out, void* stream) {
+    MDIR_CHECK_ARG(L_ids && L_s && slot_id && tab_ids && tab_f && f_out && ids_out && n_q >= 0 && n_used >= 0);
+    MDIR_CHECK_ARG(k_q >= 1 && k_q <= kCombMaxKq && width >= 1 && width <= kCombMaxWidth && k_q * width <= kCombMaxEntries);
+    MDIR_CHECK_ARG(k_out >= 1 && k_out <= kCombMaxEntries && gamma > 0.f && gamma <= FLT_MAX);
+    if (n_q == 0) return 0;
+    static PerDeviceOnce once;
+    if (once.first() != 0)
+        MDIR_CUDA(cudaFuncSetAttribute(diffusion_combine_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)comb_smem_bytes(kCombMaxEntries)));
+    const int grid = n_q < kCombCtas ? n_q : kCombCtas;
+    diffusion_combine_kernel<<<grid, kCombThreads, comb_smem_bytes(k_q * width), (cudaStream_t)stream>>>(
+            L_ids, L_s, n_q, k_q, slot_id, n_used, tab_ids, tab_f, width, gamma, k_out, f_out, ids_out);
     MDIR_LAUNCH_CHECK();
     return 0;
 }

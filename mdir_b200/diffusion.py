@@ -4,7 +4,9 @@ NOT in the reference (parity unpinned, like qe.py): the semantics are restated i
 / diffusion_search.  The graph is built once per index from the certified fp32 top-(k+1) of every row and kept exact
 through add / remove / restore / compact made through the Diffusion (DESIGN 2.2e); a query's
 certified fp32 shortlist L is re-ranked by f, the truncated CG solution of (I - alpha S_LL) f = y, where y holds the
-query's top k_q scores raised to gamma.  The graph kernels and the per-query solve are mdir_b200/csrc/diffusion.cu."""
+query's top k_q scores raised to gamma.  The graph kernels and the per-query solve are mdir_b200/csrc/diffusion.cu.
+DiffusionTable is offline diffusion: every row's diffusion solved once, a query combines the rows of its top-k_q
+(tests/diffusion_offline_reference.py:offline_table / offline_search)."""
 import contextlib
 import math
 
@@ -23,6 +25,16 @@ MERGE_CAP = 1024     # candidate pairs one tile of the reverse merge holds; a ti
 # dense scan, 10,000 rows 26 Ki.  At R1M on a B200 (1,000 W) the 10,000-row scan in 38 chunks ran at ~1,020 TFLOP/s and
 # the 1,024-row scan in 4 chunks at ~1,100 (profiles/r12_diffusion_update_1gpu.log); other sizes were not measured.
 SCREEN_PLANE_BYTES = 1 << 30
+MAX_WIDTH = 1024     # entries per table row of DiffusionTable
+MAX_KQ = 128         # table rows one DiffusionTable query combines
+MAX_ENTRIES = 8192   # k_q * width (the combine sorts them in shared memory), and the largest k of DiffusionTable.search
+# DiffusionTable's build: rows per chunk (one top-trunc search + one mdir_diffusion_solve each) and queries per scan
+# pass.  At R1M (width 100, trunc 1000) on a B200 (1,000 W) the search passes took 14.4 s with 128-query passes, 18.1 s
+# with 256, 24.1 s with 512 and 31.8 s with 1,024 (WIDE_Q); the solves 0.71 s in chunks of 8,192 rows, 0.80 s in chunks
+# of 1,024 and 0.70 s in chunks of 32,768 (profiles/r13_diffusion_offline_1gpu.log).  Every choice gives the same table
+# bit for bit.
+OFFLINE_CHUNK = 8192
+OFFLINE_BLOCK_Q = 128
 
 
 def check_graph_params(k, gamma):
@@ -48,12 +60,31 @@ def check_search_params(k, trunc, k_q, alpha, iters, rtol):
         raise _lib.MdirError("diffusion needs rtol >= 0 (got %r)" % (rtol,))
 
 
+def check_offline_params(width, trunc, alpha, iters, rtol):
+    """MdirError unless 1 <= width <= min(trunc, 1024), trunc <= 2048 and the solve's parameters are valid."""
+    if not 1 <= int(width) <= MAX_WIDTH:
+        raise _lib.MdirError("offline diffusion needs 1 <= width <= %d (got %d)" % (MAX_WIDTH, int(width)))
+    check_search_params(width, trunc, 1, alpha, iters, rtol)
+
+
+def check_combine_params(k, k_q, width):
+    """MdirError unless 1 <= k_q <= 128, k_q * width <= 8192 and 1 <= k <= 8192."""
+    k, k_q = int(k), int(k_q)
+    if not 1 <= k_q <= MAX_KQ:
+        raise _lib.MdirError("offline diffusion needs 1 <= k_q <= %d (got %d)" % (MAX_KQ, k_q))
+    if k_q * int(width) > MAX_ENTRIES:
+        raise _lib.MdirError("offline diffusion needs k_q * width <= %d (got %d * %d)" % (MAX_ENTRIES, k_q, int(width)))
+    if not 1 <= k <= MAX_ENTRIES:
+        raise _lib.MdirError("offline diffusion needs 1 <= k <= %d (got %d)" % (MAX_ENTRIES, k))
+
+
 class Diffusion:
     """Diffusion search over a single-GPU Index.
 
         g = Diffusion(index, k=50, gamma=3.0)      # the graph: one wide search pass per 1,024 rows
         f, ids = g.search(q, k=100, trunc=1000, k_q=10, alpha=0.99, iters=20, rtol=1e-6)
         ids = g.add(vecs); g.remove(ids); g.restore(ids); g.compact()     # the index changes, the graph follows
+        tab = g.offline(width=100, trunc=1000)      # DiffusionTable: every row's diffusion, solved once
 
     The index needs the fp32 master copy and no removed rows among its used slots (call compact() first; a free
     capacity tail is fine).  add / remove / restore / compact through the Diffusion mutate the index and keep the graph
@@ -328,4 +359,107 @@ class Diffusion:
                                                 _lib.ptr(self.nbr), _lib.ptr(self.S), self.k, int(k_q), self.gamma, float(alpha),
                                                 int(iters), float(rtol), k, _lib.ptr(ws), ws_bytes, _lib.ptr(f), _lib.ptr(out),
                                                 _lib.stream()), "mdir_diffusion_solve")
+            return f, out
+
+    def offline(self, width=100, trunc=1000, alpha=0.99, iters=20, rtol=1e-6):
+        """The offline table (DiffusionTable): every used slot's row diffused as a query with k_q = 1, solved now and
+        truncated to its best `width` entries.  The graph must be current.  Cost: one certified fp32 top-trunc search
+        of every used row plus one solve per row (DESIGN 2.2e); memory 8 width bytes per slot of the index's capacity."""
+        return DiffusionTable(self, width, trunc, alpha, iters, rtol)
+
+
+class DiffusionTable:
+    """Offline diffusion (Yang, Hinami, Matsui, Ly, Satoh, AAAI 2019: diffusion decoupled into online and offline
+    processing): diffusion is linear in its right-hand side, so each database row's diffusion is solved once, and a
+    query's result is the weighted sum of the table rows of its top-k_q neighbours.  The query needs one top-k_q search
+    and one combine kernel, no shortlist of trunc rows and no solve.
+
+        tab = dif.offline(width=100, trunc=1000, alpha=0.99, iters=20, rtol=1e-6)
+        f, ids = tab.search(q, k=100, k_q=10)        # device tensors, like Diffusion.search
+        tab.status()                                  # status words of the k_q search
+        tab_ids, tab_f = tab.table()                  # (n_used, width) views on the device
+
+    Slot i's table row is Diffusion.search(db32[i:i+1], k=width, trunc, k_q=1, alpha, iters, rtol), ids (int32, -1
+    padding) and f (fp32, -inf padding) in the solve's order.  The right-hand side is seeded on the row's shortlist's first
+    entry: the row itself, or an exact duplicate with a lower id, which then wins the score tie, so both rows get the same
+    table row.  Rows are held at the index's capacity; slots past the used ones are padding.
+
+    The table is a snapshot: any mutation of the index after the build, through the Diffusion too (which keeps its graph
+    current, not the table), makes search() raise until offline() is run again."""
+
+    timed = False               # True: build_time gets the build's device time of the search passes and the solves (ms)
+
+    def __init__(self, diffusion, width=100, trunc=1000, alpha=0.99, iters=20, rtol=1e-6):
+        check_offline_params(width, trunc, alpha, iters, rtol)
+        index = diffusion.index
+        if isinstance(index, ShardedIndex) or not isinstance(index, Index):
+            raise _lib.MdirError("DiffusionTable needs a single-GPU Index (a ShardedIndex is not supported)")
+        diffusion._check_current()
+        self.index, self.gamma = index, diffusion.gamma
+        self.width, self.trunc, self.alpha, self.iters, self.rtol = int(width), int(trunc), float(alpha), int(iters), float(rtol)
+        self._version = index._mutations
+        self._n_used = index._n_used
+        self._status = None
+        self.build_time = {}
+        dev, lib = index.device, _lib.lib()
+        with torch.cuda.device(dev):
+            self.tab_ids = torch.full((index.n, self.width), -1, dtype=torch.int32, device=dev)
+            self.tab_f = torch.full((index.n, self.width), float("-inf"), dtype=torch.float32, device=dev)
+            chunk = int(OFFLINE_CHUNK)
+            ws_bytes = lib.mdir_diffusion_solve_workspace_bytes(min(chunk, max(self._n_used, 1)), self.trunc, diffusion.k)
+            ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+            events = []
+            for r0 in range(0, self._n_used, chunk):
+                r1 = min(r0 + chunk, self._n_used)
+                ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)] if self.timed else None
+                if ev:
+                    ev[0].record()
+                s, L = index.search(index.db32[r0:r1], self.trunc, precision="fp32", block_q=OFFLINE_BLOCK_Q)
+                if ev:
+                    ev[1].record()
+                _lib.check(lib.mdir_diffusion_solve(_lib.ptr(L), _lib.ptr(s), r1 - r0, self.trunc, _lib.ptr(index.slot_id), self._n_used,
+                                                    _lib.ptr(diffusion.nbr), _lib.ptr(diffusion.S), diffusion.k, 1, self.gamma, self.alpha,
+                                                    self.iters, self.rtol, self.width, _lib.ptr(ws), ws_bytes, _lib.ptr(self.tab_f[r0:r1]),
+                                                    _lib.ptr(self.tab_ids[r0:r1]), _lib.stream()), "mdir_diffusion_solve")
+                if ev:
+                    ev[2].record()
+                    events.append(ev)
+            if self.timed:
+                torch.cuda.current_stream().synchronize()
+                self.build_time = {"search": sum(a.elapsed_time(b) for a, b, _ in events),
+                                   "solve": sum(b.elapsed_time(c) for _, b, c in events)}
+
+    def table(self):
+        """(ids (n_used, width) int32, f (n_used, width) fp32) on the device, row r = slot r at build time."""
+        return self.tab_ids[:self._n_used], self.tab_f[:self._n_used]
+
+    def status(self):
+        """Per-query status words of the last search()'s k_q search (Index.status(): 0 = exact and certified)."""
+        return self._status
+
+    def search(self, q, k=100, k_q=10):
+        """q: (N_q, D) fp32 (host or device).  Returns (f (N_q, k) fp32, ids (N_q, k) int32) on the device.  L, s =
+        index.search(q, k_q, precision="fp32"); w_u = max(s_u, 0)^gamma; for every id j in the union of the table rows
+        of L's slots f_j = sum over u of w_u F[slot(L_u)][j] (fp64, ascending u); the top k by (fp32 f desc, id asc),
+        -inf / -1 padding past the union.  Rows outside the union are not candidates."""
+        check_combine_params(k, k_q, self.width)
+        index = self.index
+        if index._mutations != self._version:
+            raise _lib.MdirError("the index was mutated (remove / restore / add / compact) after the diffusion table was built: "
+                                 "run offline() again")
+        k, k_q = int(k), int(k_q)
+        dev = index.device
+        with torch.cuda.device(dev):
+            q32 = _as_dev_f32(q, dev)
+            n_q = q32.shape[0]
+            f = torch.empty((n_q, k), dtype=torch.float32, device=dev)
+            out = torch.empty((n_q, k), dtype=torch.int32, device=dev)
+            if n_q == 0:
+                self._status = torch.empty((0,), dtype=torch.int32, device=dev)
+                return f, out
+            s, L = index.search(q32, k_q, precision="fp32", check=True)
+            self._status = index.status()[:n_q].clone()
+            _lib.check(_lib.lib().mdir_diffusion_combine(_lib.ptr(L), _lib.ptr(s), n_q, k_q, _lib.ptr(index.slot_id), index._n_used,
+                                                         _lib.ptr(self.tab_ids), _lib.ptr(self.tab_f), self.width, self.gamma, k,
+                                                         _lib.ptr(f), _lib.ptr(out), _lib.stream()), "mdir_diffusion_combine")
             return f, out
