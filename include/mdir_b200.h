@@ -461,6 +461,23 @@ int mdir_diffusion_combine(const int32_t* L_ids, const float* L_s, int n_q, int 
                            const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
                            int32_t* ids_out, void* stream);
 
+/* Captured diffusion serving (mdir_b200.GraphedDiffusion / DiffusionPipeline; DESIGN 2.2f).  mdir_diffusion_solve_dev
+ *   and mdir_diffusion_combine_dev are mdir_diffusion_solve / mdir_diffusion_combine (same kernels, same checks, same
+ *   bits) with two optional device pointers, both read-only:
+ *   n_used_dev (1 int64): when non-NULL, the used-slot count of the slot -> id lookups is read from it on the device
+ *     (Index.n_scan, updated in stream order by add / compact), and the host's n_used is ignored, so a CUDA graph
+ *     keeps working after the index grows or shrinks.
+ *   status (n_q int32): when non-NULL, a query whose word is nonzero (its shortlist / top-k_q search was flagged)
+ *     does no work and gets -inf / -1 in all k_out columns.
+ *   The plain launchers are these with NULL, NULL.                                                                  */
+int mdir_diffusion_solve_dev(const int32_t* L_ids, const float* L_s, int n_q, int trunc, const uint32_t* slot_id, int64_t n_used,
+                             const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
+                             int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, const int64_t* n_used_dev,
+                             const int32_t* status, void* stream);
+int mdir_diffusion_combine_dev(const int32_t* L_ids, const float* L_s, int n_q, int k_q, const uint32_t* slot_id, int64_t n_used,
+                               const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
+                               int32_t* ids_out, const int64_t* n_used_dev, const int32_t* status, void* stream);
+
 /* Incremental update of the raw lists (Diffusion.add / restore / remove; DESIGN 2.2e).  A list entry's key is
  * mdir_make_key(score, id), smaller = better, all ones for padding; T_i = the key of entry k of slot i's list.
  * mdir_diffusion_batch_eps: eps[j] = the certified bf16 bound of row j of q32 (n_q, D) taken as a query (the formula of

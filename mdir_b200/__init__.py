@@ -6,8 +6,9 @@ hot path behind the reference's own plug-in surface (SURVEY.md section 8).
     clahe     clahe_u8, ChannelClahe / ImageClahe / ApplyClahe ...  (mdir transforms)
     search    rank(), Index, ShardedIndex, ranks_from_scores, topk_from_scores
     qe        alpha-QE / DBA (not in the reference; parity unpinned)
-    diffusion Diffusion: re-ranking on a mutual kNN graph of the database; DiffusionTable: its offline table (not in the
-              reference; parity unpinned)
+    diffusion Diffusion: re-ranking on a mutual kNN graph of the database; DiffusionTable: its offline table;
+              GraphedDiffusion / DiffusionPipeline: either one served from CUDA graphs (not in the reference; parity
+              unpinned)
     extract   batched extract_vectors (no per-image sync)            (cirtorch/networks/imageretrievalnet.py)
     evaluate  compute_map / compute_map_and_print on the device      (cirtorch/utils/evaluate.py)
     score     CirDatasetAp replacement + install()
@@ -20,7 +21,7 @@ from .wrappers import CirMultiscaleAggregation, CirtorchWhiten, RetrievalHead, w
 from .clahe import clahe_u8, image_clahe, ChannelClahe, ImageClahe, ApplyClahe, AddClaheFromRgb, CreateClahedImage  # noqa: F401
 from .search import (Index, ShardedIndex, GraphedSearch, SearchPipeline, GraphedRangeSearch, RangePipeline, rank,  # noqa: F401
                      ranks_from_scores, topk_from_scores)
-from .diffusion import Diffusion, DiffusionTable  # noqa: F401
+from .diffusion import Diffusion, DiffusionTable, GraphedDiffusion, DiffusionPipeline  # noqa: F401
 from .extract import extract_vectors, extract_from_tensors  # noqa: F401
 from .evaluate import compute_map, compute_map_and_print  # noqa: F401
 from .score import install  # noqa: F401

@@ -84,6 +84,8 @@ PROTOTYPES = {
     "mdir_diffusion_solve_workspace_bytes": (_sz, [_i, _i, _i]),
     "mdir_diffusion_solve": (_i, [_vp, _vp, _i, _i, _vp, _i64, _vp, _vp, _i, _i, _f, _d, _i, _d, _i, _vp, _sz, _vp, _vp, _vp]),
     "mdir_diffusion_combine": (_i, [_vp, _vp, _i, _i, _vp, _i64, _vp, _vp, _i, _f, _i, _vp, _vp, _vp]),
+    "mdir_diffusion_solve_dev": (_i, [_vp, _vp, _i, _i, _vp, _i64, _vp, _vp, _i, _i, _f, _d, _i, _d, _i, _vp, _sz, _vp, _vp, _vp, _vp, _vp]),
+    "mdir_diffusion_combine_dev": (_i, [_vp, _vp, _i, _i, _vp, _i64, _vp, _vp, _i, _f, _i, _vp, _vp, _vp, _vp, _vp]),
     "mdir_diffusion_batch_eps": (_i, [_vp, _i, _i, _vp, _vp, _vp]),
     "mdir_diffusion_merge": (_i, [_vp, _i64, _i, _i64, _i64, _vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp]),
     "mdir_diffusion_stale_rows": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),

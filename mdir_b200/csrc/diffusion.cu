@@ -132,7 +132,8 @@ __host__ __device__ inline size_t diff_ws_cta_bytes(int trunc, int k) {
 __global__ void __launch_bounds__(kDiffThreads) diffusion_solve_kernel(
         const int32_t* __restrict__ L_ids, const float* __restrict__ L_s, int n_q, int trunc, const uint32_t* __restrict__ slot_id,
         int64_t n_used, const int32_t* __restrict__ nbr, const float* __restrict__ S, int k, int k_q, float gamma, double alpha,
-        int iters, double rtol, int k_out, uint8_t* __restrict__ ws, float* __restrict__ f_out, int32_t* __restrict__ ids_out) {
+        int iters, double rtol, int k_out, uint8_t* __restrict__ ws, float* __restrict__ f_out, int32_t* __restrict__ ids_out,
+        const int64_t* __restrict__ n_used_dev, const int32_t* __restrict__ status) {
     extern __shared__ __align__(16) uint8_t smem[];
     uint64_t* keys = reinterpret_cast<uint64_t*>(smem);                       // kDiffMaxTrunc
     double* x = reinterpret_cast<double*>(keys + kDiffMaxTrunc);
@@ -142,12 +143,23 @@ __global__ void __launch_bounds__(kDiffThreads) diffusion_solve_kernel(
     uint16_t* cnt = reinterpret_cast<uint16_t*>(ap + kDiffMaxTrunc);
     __shared__ double red[kDiffWarps];
     __shared__ int s_n;
+    __shared__ int64_t s_used;
     // this CTA's local ELL of S_LL, column-major: entry c of row u at c * trunc + u (u16 local index, fp32 S)
     uint16_t* ell_idx = reinterpret_cast<uint16_t*>(ws + (size_t)blockIdx.x * diff_ws_cta_bytes(trunc, k));
     float* ell_val = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(ell_idx) + (((size_t)trunc * k * 2 + 255) & ~(size_t)255));
     const int tid = threadIdx.x;
+    if (tid == 0) s_used = n_used_dev ? *n_used_dev : n_used;
+    __syncthreads();
+    n_used = s_used;
 
     for (int q = blockIdx.x; q < n_q; q += gridDim.x) {
+        if (status && status[q] != 0) {                                      // a flagged shortlist: no rows
+            for (int j = tid; j < k_out; j += kDiffThreads) {
+                f_out[(int64_t)q * k_out + j] = -INFINITY;
+                ids_out[(int64_t)q * k_out + j] = -1;
+            }
+            continue;
+        }
         const int32_t* ids = L_ids + (int64_t)q * trunc;
         const float* sc = L_s + (int64_t)q * trunc;
         // (0) |L|: search pads its rows with id -1 after the live rows it found
@@ -503,18 +515,29 @@ __host__ __device__ inline size_t comb_smem_bytes(int n) { return ((size_t)comb_
 __global__ void __launch_bounds__(kCombThreads, 2) diffusion_combine_kernel(
         const int32_t* __restrict__ L_ids, const float* __restrict__ L_s, int n_q, int k_q, const uint32_t* __restrict__ slot_id,
         int64_t n_used, const int32_t* __restrict__ tab_ids, const float* __restrict__ tab_f, int width, float gamma, int k_out,
-        float* __restrict__ f_out, int32_t* __restrict__ ids_out) {
+        float* __restrict__ f_out, int32_t* __restrict__ ids_out, const int64_t* __restrict__ n_used_dev, const int32_t* __restrict__ status) {
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ int64_t s_slot[kCombMaxKq];
     __shared__ double s_w[kCombMaxKq];
+    __shared__ int64_t s_used;
     const int n = k_q * width, npow = comb_npow(n);
     uint64_t* keys = reinterpret_cast<uint64_t*>(smem);
     float* fsum = reinterpret_cast<float*>(keys + npow);
     uint8_t* head = reinterpret_cast<uint8_t*>(fsum + npow);
     const int tid = threadIdx.x;
     constexpr int kIdShift = 17;
+    if (tid == 0) s_used = n_used_dev ? *n_used_dev : n_used;
+    __syncthreads();
+    n_used = s_used;
 
     for (int q = blockIdx.x; q < n_q; q += gridDim.x) {
+        if (status && status[q] != 0) {                                      // a flagged top-k_q: no rows
+            for (int j = tid; j < k_out; j += kCombThreads) {
+                f_out[(int64_t)q * k_out + j] = -INFINITY;
+                ids_out[(int64_t)q * k_out + j] = -1;
+            }
+            continue;
+        }
         for (int u = tid; u < k_q; u += kCombThreads) {
             s_slot[u] = diff_slot_of(slot_id, n_used, L_ids[(int64_t)q * k_q + u]);
             s_w[u] = pow((double)fmaxf(L_s[(int64_t)q * k_q + u], 0.f), (double)gamma);
@@ -627,9 +650,10 @@ extern "C" size_t mdir_diffusion_solve_workspace_bytes(int n_q, int trunc, int k
     return (size_t)(n_q < kDiffCtas ? n_q : kDiffCtas) * diff_ws_cta_bytes(trunc, k);
 }
 
-extern "C" int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int n_q, int trunc, const uint32_t* slot_id, int64_t n_used,
-                                    const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
-                                    int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, void* stream) {
+extern "C" int mdir_diffusion_solve_dev(const int32_t* L_ids, const float* L_s, int n_q, int trunc, const uint32_t* slot_id, int64_t n_used,
+                                        const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
+                                        int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, const int64_t* n_used_dev,
+                                        const int32_t* status, void* stream) {
     MDIR_CHECK_ARG(L_ids && L_s && slot_id && nbr && S && f_out && ids_out && n_q >= 0 && n_used >= 0);
     MDIR_CHECK_ARG(trunc >= 1 && trunc <= kDiffMaxTrunc && k >= 1 && k <= kDiffMaxK);
     MDIR_CHECK_ARG(k_q >= 1 && k_q <= trunc && k_out >= 1 && k_out <= trunc);
@@ -641,14 +665,21 @@ extern "C" int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int 
     const int grid = n_q < kDiffCtas ? n_q : kDiffCtas;
     diffusion_solve_kernel<<<grid, kDiffThreads, kDiffSmem, (cudaStream_t)stream>>>(L_ids, L_s, n_q, trunc, slot_id, n_used, nbr, S, k, k_q,
                                                                                    gamma, alpha, iters, rtol, k_out, (uint8_t*)ws, f_out,
-                                                                                   ids_out);
+                                                                                   ids_out, n_used_dev, status);
     MDIR_LAUNCH_CHECK();
     return 0;
 }
 
-extern "C" int mdir_diffusion_combine(const int32_t* L_ids, const float* L_s, int n_q, int k_q, const uint32_t* slot_id, int64_t n_used,
-                                      const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
-                                      int32_t* ids_out, void* stream) {
+extern "C" int mdir_diffusion_solve(const int32_t* L_ids, const float* L_s, int n_q, int trunc, const uint32_t* slot_id, int64_t n_used,
+                                    const int32_t* nbr, const float* S, int k, int k_q, float gamma, double alpha, int iters, double rtol,
+                                    int k_out, void* ws, size_t ws_bytes, float* f_out, int32_t* ids_out, void* stream) {
+    return mdir_diffusion_solve_dev(L_ids, L_s, n_q, trunc, slot_id, n_used, nbr, S, k, k_q, gamma, alpha, iters, rtol, k_out, ws, ws_bytes,
+                                    f_out, ids_out, nullptr, nullptr, stream);
+}
+
+extern "C" int mdir_diffusion_combine_dev(const int32_t* L_ids, const float* L_s, int n_q, int k_q, const uint32_t* slot_id, int64_t n_used,
+                                          const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
+                                          int32_t* ids_out, const int64_t* n_used_dev, const int32_t* status, void* stream) {
     MDIR_CHECK_ARG(L_ids && L_s && slot_id && tab_ids && tab_f && f_out && ids_out && n_q >= 0 && n_used >= 0);
     MDIR_CHECK_ARG(k_q >= 1 && k_q <= kCombMaxKq && width >= 1 && width <= kCombMaxWidth && k_q * width <= kCombMaxEntries);
     MDIR_CHECK_ARG(k_out >= 1 && k_out <= kCombMaxEntries && gamma > 0.f && gamma <= FLT_MAX);
@@ -658,7 +689,14 @@ extern "C" int mdir_diffusion_combine(const int32_t* L_ids, const float* L_s, in
         MDIR_CUDA(cudaFuncSetAttribute(diffusion_combine_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)comb_smem_bytes(kCombMaxEntries)));
     const int grid = n_q < kCombCtas ? n_q : kCombCtas;
     diffusion_combine_kernel<<<grid, kCombThreads, comb_smem_bytes(k_q * width), (cudaStream_t)stream>>>(
-            L_ids, L_s, n_q, k_q, slot_id, n_used, tab_ids, tab_f, width, gamma, k_out, f_out, ids_out);
+            L_ids, L_s, n_q, k_q, slot_id, n_used, tab_ids, tab_f, width, gamma, k_out, f_out, ids_out, n_used_dev, status);
     MDIR_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int mdir_diffusion_combine(const int32_t* L_ids, const float* L_s, int n_q, int k_q, const uint32_t* slot_id, int64_t n_used,
+                                      const int32_t* tab_ids, const float* tab_f, int width, float gamma, int k_out, float* f_out,
+                                      int32_t* ids_out, void* stream) {
+    return mdir_diffusion_combine_dev(L_ids, L_s, n_q, k_q, slot_id, n_used, tab_ids, tab_f, width, gamma, k_out, f_out, ids_out, nullptr,
+                                      nullptr, stream);
 }

@@ -6,7 +6,8 @@ through add / remove / restore / compact made through the Diffusion (DESIGN 2.2e
 certified fp32 shortlist L is re-ranked by f, the truncated CG solution of (I - alpha S_LL) f = y, where y holds the
 query's top k_q scores raised to gamma.  The graph kernels and the per-query solve are mdir_b200/csrc/diffusion.cu.
 DiffusionTable is offline diffusion: every row's diffusion solved once, a query combines the rows of its top-k_q
-(tests/diffusion_offline_reference.py:offline_table / offline_search)."""
+(tests/diffusion_offline_reference.py:offline_table / offline_search).
+GraphedDiffusion and DiffusionPipeline serve either one from CUDA graphs (DESIGN 2.2f)."""
 import contextlib
 import math
 
@@ -15,7 +16,7 @@ import torch
 
 from . import _lib
 from .qe import DBA_BLOCK
-from .search import Index, ShardedIndex, WIDE_Q, _as_dev_f32
+from .search import Index, ShardedIndex, MAX_Q, STATUS_OVERFLOW, STATUS_UNCERTIFIED, WIDE_Q, _Pipeline, _as_dev_f32
 
 MAX_K = 255          # neighbours per database row
 MAX_TRUNC = 2048     # shortlist rows per query the solve kernel holds in shared memory
@@ -437,6 +438,11 @@ class DiffusionTable:
         """Per-query status words of the last search()'s k_q search (Index.status(): 0 = exact and certified)."""
         return self._status
 
+    def _check_current(self):
+        if self.index._mutations != self._version:
+            raise _lib.MdirError("the index was mutated (remove / restore / add / compact) after the diffusion table was built: "
+                                 "run offline() again")
+
     def search(self, q, k=100, k_q=10):
         """q: (N_q, D) fp32 (host or device).  Returns (f (N_q, k) fp32, ids (N_q, k) int32) on the device.  L, s =
         index.search(q, k_q, precision="fp32"); w_u = max(s_u, 0)^gamma; for every id j in the union of the table rows
@@ -444,9 +450,7 @@ class DiffusionTable:
         -inf / -1 padding past the union.  Rows outside the union are not candidates."""
         check_combine_params(k, k_q, self.width)
         index = self.index
-        if index._mutations != self._version:
-            raise _lib.MdirError("the index was mutated (remove / restore / add / compact) after the diffusion table was built: "
-                                 "run offline() again")
+        self._check_current()
         k, k_q = int(k), int(k_q)
         dev = index.device
         with torch.cuda.device(dev):
@@ -463,3 +467,237 @@ class DiffusionTable:
                                                          _lib.ptr(self.tab_ids), _lib.ptr(self.tab_f), self.width, self.gamma, k,
                                                          _lib.ptr(f), _lib.ptr(out), _lib.stream()), "mdir_diffusion_combine")
             return f, out
+
+
+def _serving_params(source, params):
+    """source.search's parameters for captured serving, defaults filled in: (trunc, k_q, alpha, iters, rtol) for a
+    Diffusion, (k_q,) for a DiffusionTable."""
+    if isinstance(source, Diffusion):
+        names = dict(trunc=1000, k_q=10, alpha=0.99, iters=20, rtol=1e-6)
+    elif isinstance(source, DiffusionTable):
+        names = dict(k_q=10)
+    else:
+        raise _lib.MdirError("diffusion serving needs a Diffusion or a DiffusionTable (got %s)" % type(source).__name__)
+    unknown = sorted(set(params) - set(names))
+    if unknown:
+        raise TypeError("%s.search() takes no parameter %s" % (type(source).__name__, ", ".join(unknown)))
+    return {**names, **params}
+
+
+class GraphedDiffusion:
+    """One diffusion step captured in a CUDA graph: static queries (n_q, D) fp32 in, static f (n_q, k) fp32, ids
+    (n_q, k) int32 and status (n_q,) int32 out.
+
+        gd = GraphedDiffusion(dif, n_q=70, k=100, trunc=1000, k_q=10)    # a Diffusion: Diffusion.search's parameters
+        gd = GraphedDiffusion(tab, n_q=70, k=100, k_q=10)                # a DiffusionTable: DiffusionTable.search's
+        f, ids = gd(q)                                                   # replay on the current stream
+
+    The graph runs the source's own shortlist search, index.search(q, trunc (table: k_q), precision="fp32",
+    check=False), copies its status words, then the solve (table: combine) kernel, which reads the used-slot count from
+    the index's device copy (Index.n_scan) and the status words from the graph.  A query whose word is nonzero (a
+    candidate segment overflowed, or the shortlist was not certified) gets no rows (-inf / -1) and keeps its word: the
+    graph has no widening, so whoever owns it redoes those queries with source.search (DiffusionPipeline does).  Every
+    other query is bit for bit source.search's row, alone or in any batch (DESIGN 2.2e).
+
+    add / remove / restore / compact made through the Diffusion need no re-capture: the graph reads the index's rows,
+    live bitmap, scan extent and slot -> id map and the Diffusion's graph arrays in place.  A replay raises, like
+    source.search, once the source is stale: a Diffusion whose index was mutated directly, or a table after any
+    mutation (a table's slot -> id lookups use its build-time count)."""
+
+    def __init__(self, source, n_q, k=100, **params):
+        p = _serving_params(source, params)
+        self.source, self.n_q, self.k, self.params = source, int(n_q), int(k), p
+        if not 1 <= self.n_q <= MAX_Q:
+            raise _lib.MdirError("GraphedDiffusion: n_q must be in [1, %d] (got %d)" % (MAX_Q, self.n_q))
+        online = isinstance(source, Diffusion)
+        if online:
+            check_search_params(self.k, p["trunc"], p["k_q"], p["alpha"], p["iters"], p["rtol"])
+        else:
+            check_combine_params(self.k, p["k_q"], source.width)
+        source._check_current()
+        self.index = index = source.index
+        dev, nq, k, lib = index.device, self.n_q, self.k, _lib.lib()
+        with torch.cuda.device(dev):
+            self.q = torch.zeros((nq, index.D), dtype=torch.float32, device=dev)
+            self.f = torch.empty((nq, k), dtype=torch.float32, device=dev)
+            self.ids = torch.empty((nq, k), dtype=torch.int32, device=dev)
+            self.status = torch.zeros((nq,), dtype=torch.int32, device=dev)
+            if online:
+                trunc = int(p["trunc"])
+                ws_bytes = lib.mdir_diffusion_solve_workspace_bytes(nq, trunc, source.k)
+                self._ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+
+            def step():
+                if online:
+                    s, L = index.search(self.q, trunc, precision="fp32", check=False)
+                    self.status.copy_(index.status()[:nq])
+                    _lib.check(lib.mdir_diffusion_solve_dev(_lib.ptr(L), _lib.ptr(s), nq, trunc, _lib.ptr(index.slot_id), index._n_used,
+                                                            _lib.ptr(source.nbr), _lib.ptr(source.S), source.k, int(p["k_q"]), source.gamma,
+                                                            float(p["alpha"]), int(p["iters"]), float(p["rtol"]), k, _lib.ptr(self._ws),
+                                                            ws_bytes, _lib.ptr(self.f), _lib.ptr(self.ids), _lib.ptr(index.n_scan),
+                                                            _lib.ptr(self.status), _lib.stream()), "mdir_diffusion_solve_dev")
+                else:
+                    s, L = index.search(self.q, int(p["k_q"]), precision="fp32", check=False)
+                    self.status.copy_(index.status()[:nq])
+                    _lib.check(lib.mdir_diffusion_combine_dev(_lib.ptr(L), _lib.ptr(s), nq, int(p["k_q"]), _lib.ptr(index.slot_id),
+                                                              source._n_used, _lib.ptr(source.tab_ids), _lib.ptr(source.tab_f), source.width,
+                                                              source.gamma, k, _lib.ptr(self.f), _lib.ptr(self.ids), None,
+                                                              _lib.ptr(self.status), _lib.stream()), "mdir_diffusion_combine_dev")
+                return s, L
+
+            prof, index.prof = getattr(index, "prof", None), None            # no timing events inside the graph
+            try:
+                side = torch.cuda.Stream(device=dev)
+                side.wait_stream(torch.cuda.current_stream(dev))
+                with torch.cuda.stream(side):                             # warm-up: stats, workspaces, kernel attributes
+                    step()
+                torch.cuda.current_stream(dev).wait_stream(side)
+                torch.cuda.synchronize(dev)
+                self.graph = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(self.graph):
+                    self._shortlist = step()      # held: the graph writes these buffers on every replay
+            finally:
+                index.prof = prof
+
+    def _check_current(self):
+        self.source._check_current()
+
+    def __call__(self, q=None):
+        """Replay on the current stream.  q: (n_q, D) fp32 (host, pinned for an asynchronous copy, or device) copied into
+        the static input; None keeps the previous queries.  Returns the static (f, ids); `status` holds the words.
+        MdirError, before anything is queued, when the source is stale."""
+        self._check_current()
+        if q is not None:
+            self.q.copy_(q, non_blocking=True)
+        self.graph.replay()
+        return self.f, self.ids
+
+
+class DiffusionPipeline(_Pipeline):
+    """Host-facing diffusion serving: query batches go up from pinned host buffers, GraphedDiffusion replays back to back
+    on one compute stream, and each ticket's (f, ids) and status words come back in pinned buffers, copies and replays
+    ordered by events only.
+
+        pipe = DiffusionPipeline(dif, n_q=70, k=100, trunc=1000, k_q=10)      # or (tab, n_q=70, k=100, k_q=10)
+        t0 = pipe.submit(q_0)
+        t1 = pipe.submit(q_1)
+        f, ids = pipe.result(t0)                   # numpy views, valid until `depth` more submits
+        pipe.add(vecs); pipe.remove(ids); pipe.restore(ids); pipe.compact()     # a Diffusion source only
+
+    result() is source.search's answer for the whole batch, bit for bit: the queries the graph flagged are redone, alone,
+    with source.search on the compute stream and written into the ticket's rows (both kernels are batch-invariant).
+    n_recovered counts tickets with such queries, recovered the queries by status bit (a query may count in both).
+
+    Mutations (a Diffusion source) go through the Diffusion's own methods on the compute stream, so its graph stays
+    current and no graph is re-captured.  They change the graph arrays and the slot -> id map in place, which a ticket
+    redone afterwards would read, so every pending ticket is settled first: waited for and its flagged queries redone
+    against the graph it was submitted under.  Tickets submitted before a mutation return the answer before it, later
+    ones the answer after it.  compact() refuses while tickets are pending, as in the other pipelines.  A table does
+    not follow updates: every mutation method raises."""
+
+    def __init__(self, source, n_q, k=100, depth=2, **params):
+        if int(depth) < 1:
+            raise _lib.MdirError("DiffusionPipeline: depth must be at least 1 (got %d)" % int(depth))
+        self.graphs = [GraphedDiffusion(source, n_q, k, **params) for _ in range(int(depth))]
+        self.source, self.params = source, self.graphs[0].params
+        # _Pipeline's remove / restore / add / compact call self.index's: the source's, which keep its graph current
+        self.index, self.local = source, source.index
+        self.n_q, self.k = int(n_q), int(k)
+        self.depth, self.overlap = int(depth), False
+        dev = self.local.device
+        with torch.cuda.device(dev):
+            self.compute, self.h2d, self.d2h = (torch.cuda.Stream(device=dev) for _ in range(3))
+            self.slots = [{
+                "q": torch.empty((self.n_q, self.local.D), dtype=torch.float32).pin_memory(),
+                "f": torch.empty((self.n_q, self.k), dtype=torch.float32).pin_memory(),
+                "ids": torch.empty((self.n_q, self.k), dtype=torch.int32).pin_memory(),
+                "status": torch.empty((self.n_q,), dtype=torch.int32).pin_memory(),
+                "up": torch.cuda.Event(), "done": torch.cuda.Event(), "down": torch.cuda.Event(),
+                "pending": False, "settled": False} for _ in range(self.depth)]
+            torch.cuda.synchronize(dev)
+        self.n_submitted = 0
+        self.n_recovered = 0            # tickets with at least one query redone eagerly
+        self.recovered = {"overflow": 0, "uncertified": 0}     # queries redone, by status bit
+
+    def submit(self, q):
+        """q: (n_q, D) fp32 (host or device), copied into the slot's pinned staging buffer here, so the caller may reuse
+        it at once.  Returns a ticket for result().  MdirError when the source is stale."""
+        t_new = self.n_submitted
+        slot, gd = self._free_slot(t_new), self.graphs[t_new % self.depth]
+        gd._check_current()
+        q = torch.as_tensor(q)
+        if tuple(q.shape) != tuple(gd.q.shape):
+            raise _lib.MdirError("DiffusionPipeline expects query batches of shape %s" % (tuple(gd.q.shape),))
+        slot["q"].copy_(q)
+        with torch.cuda.device(self.local.device):
+            with torch.cuda.stream(self.h2d):              # this slot's previous replay was collected by result()
+                gd.q.copy_(slot["q"], non_blocking=True)
+                slot["up"].record()
+            caller = torch.cuda.current_stream()
+            with torch.cuda.stream(self.compute):
+                self.compute.wait_event(slot["up"])
+                self.compute.wait_stream(caller)          # updates made on the Diffusion directly, on the caller's stream
+                gd.graph.replay()
+                slot["done"].record()
+            with torch.cuda.stream(self.d2h):
+                self.d2h.wait_event(slot["done"])
+                for name, src in (("f", gd.f), ("ids", gd.ids), ("status", gd.status)):
+                    slot[name].copy_(src, non_blocking=True)
+                slot["down"].record()
+        slot["pending"], slot["settled"] = True, False
+        self.n_submitted += 1
+        return t_new
+
+    def _settle(self, slot):
+        """Wait for a ticket and redo its flagged queries with source.search on the compute stream, into its rows."""
+        slot["down"].synchronize()
+        status = slot["status"].numpy()
+        flagged = np.flatnonzero(status)
+        if flagged.size:
+            self.n_recovered += 1
+            self.recovered["overflow"] += int(((status & STATUS_OVERFLOW) != 0).sum())
+            self.recovered["uncertified"] += int(((status & STATUS_UNCERTIFIED) != 0).sum())
+            rows = torch.from_numpy(flagged)
+            with torch.cuda.device(self.local.device), torch.cuda.stream(self.compute):
+                f, ids = self.source.search(slot["q"][rows], k=self.k, **self.params)
+                slot["f"][rows] = f.cpu()
+                slot["ids"][rows] = ids.cpu()
+        slot["settled"] = True
+
+    def result(self, ticket):
+        """Blocks until ticket's result is in host memory -> (f (n_q, k) fp32, ids (n_q, k) int32) numpy views of the
+        pinned buffers, valid until `depth` more submits."""
+        slot = self._pending_slot(ticket)
+        if not slot["settled"]:
+            self._settle(slot)
+        slot["pending"] = False
+        return slot["f"].numpy(), slot["ids"].numpy()
+
+    def _refuse_table(self):
+        if isinstance(self.source, DiffusionTable):
+            raise _lib.MdirError("DiffusionPipeline over a DiffusionTable: the table does not follow updates; mutate through the "
+                                 "Diffusion, run offline() again and build a new pipeline")
+
+    def compact(self):
+        """Diffusion.compact() on the compute stream; MdirError while a ticket is pending (see _Pipeline.compact)."""
+        self._refuse_table()
+        return super().compact()
+
+    def _mutate(self, fn):
+        """Settle every pending ticket, then run the source's mutation on the compute stream (after every replay queued
+        there).  A DiffusionTable raises."""
+        self._refuse_table()
+        for sl in self.slots:
+            if sl["pending"] and not sl["settled"]:
+                self._settle(sl)
+        with torch.cuda.device(self.local.device):
+            caller = torch.cuda.current_stream()
+            self.compute.wait_stream(caller)
+            with torch.cuda.stream(self.compute):
+                out = fn()
+            caller.wait_stream(self.compute)          # the caller's later work sees the updated index and graph
+            return out
+
+    def map(self, batches):
+        """Generator over an iterable of query batches, keeping `depth` tickets in flight."""
+        return self._map(batches, self.submit)
